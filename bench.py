@@ -2,6 +2,7 @@
 """Benchmark of the DANBO hot path on B200 (contract: see the task statement / DESIGN.md §Measurement).
 
     python bench.py --gpus 1 --steps 10 --warmup 3                 # this repo's CUDA path
+    python bench.py --gpus 1 --steps 10 --warmup 3 --dump-outputs DIR   # ... and write what the last timed step returned
     python bench.py --impl reference --steps 2 --warmup 1           # the unmodified reference (baseline/_ref) on host cores
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
@@ -118,6 +119,30 @@ def caster_kwargs(args, batch, device=None):
                 N_importance=args.N_importance, raw_noise_std=0., nanmean_chunk=args.chunk)
 
 
+DUMP_BYTES = 64 * 10 ** 6          # all files together, .npy headers included
+NPY_HEADER_BYTES = 1024            # an upper bound for the header np.save writes for these arrays
+
+
+def dump_outputs(ret, out_dir, budget=DUMP_BYTES, seed=0):
+    """Writes every array of a render call's returned dict as `out_dir/<name>.npy` (float64 stays float64, other
+    types become float32).  All arrays have one row per ray; when together they would exceed `budget` bytes, each keeps
+    the same rays: a fixed, seeded random sample in ray order, as many as fit.  Equal inputs thus give files that can be
+    compared one to one between two builds."""
+    arrays = {k: v.detach().cpu() for k, v in ret.items()}
+    arrays = {k: v if v.dtype == torch.float64 else v.float() for k, v in arrays.items()}
+    n = {v.shape[0] for v in arrays.values()}
+    assert len(n) == 1, {k: tuple(v.shape) for k, v in arrays.items()}
+    n = n.pop()
+    row_bytes = sum(v[:1].numel() * v.element_size() for v in arrays.values())
+    keep = min(n, max(budget - NPY_HEADER_BYTES * len(arrays), 0) // max(row_bytes, 1))
+    if keep < n:
+        rows = torch.randperm(n, generator=torch.Generator().manual_seed(seed))[:keep].sort().values
+        arrays = {k: v[rows] for k, v in arrays.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), v.numpy())
+
+
 def _mark(msg):
     if os.environ.get("DANBO_BENCH_VERBOSE"):
         sys.stderr.write(f"[bench rank {os.environ.get('RANK', '0')} t={time.perf_counter():.1f}] {msg}\n")
@@ -167,7 +192,7 @@ def run_ours(opt):
                 comm.wait_event(rendered[b])
                 gathered[b] = parallel.allgather_rows(pix, shard_sizes)
             pix.record_stream(comm)
-        return pix
+        return ret
 
     def drain():
         if world > 1:
@@ -203,7 +228,7 @@ def run_ours(opt):
     tail0, tail1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     for i in range(opt.steps):
         ev[i][0].record()
-        step_device(i=i)
+        ret = step_device(i=i)
         ev[i][1].record()
         flush.fill_(i)                                       # L2 flush between timed iterations (not timed)
     tail0.record()
@@ -212,6 +237,10 @@ def run_ours(opt):
     barrier()
     _mark("timed steps done")
     t_wall = time.perf_counter() - t_wall0
+    # every rank renders the same whole image, so rank 0's outputs are the complete result; dumped before any later call
+    # overwrites the graph's output buffers
+    if opt.dump_outputs and rank == 0:
+        dump_outputs(ret, opt.dump_outputs)
     dev_ms = sum(a.elapsed_time(b) for a, b in ev) + (tail0.elapsed_time(tail1) if world > 1 else 0.0)
     # the timed steps replay one CUDA graph; the same steps are run once more launch by launch with CUDA events around
     # the dominant kernel (and the launch counter on) for the roofline line
@@ -582,8 +611,8 @@ def workload_config(args, n_rays=None):
 def cpu_baseline(sample_rays=REF_SAMPLE_RAYS, repeats=1, threads=None):
     """The reference's CPU implementation of the path on the host cores, on a bounded sample of the same workload.
 
-    kind "reference": the UNMODIFIED reference (baseline/_ref, copied by scripts/vendor_ref.sh; /root/reference in the
-    authoring container) through its own `render` (core/trainer.py:96-162: ray assembly + `batchify_rays` in
+    kind "reference": the UNMODIFIED reference (baseline/_ref, copied by scripts/vendor_ref.sh, or $DANBO_REFERENCE)
+    through its own `render` (core/trainer.py:96-162: ray assembly + `batchify_rays` in
     `args.chunk` = 4096-ray chunks, as `render_path` calls it per image, run_nerf.py:92-96) and its own GraphCaster, with
     this repo's synthetic weights.  kind "port": the oracle restatement, only if the reference copy is absent."""
     sys.path.insert(0, os.path.join(ROOT, "oracle"))
@@ -609,6 +638,8 @@ def cpu_baseline(sample_rays=REF_SAMPLE_RAYS, repeats=1, threads=None):
             rh.reference_render_rays(render, kw_test, rargs, rays[:m, 0:3], rays[:m, 3:6], pose, cams[:m], H, W, 1.2 * H)
     else:
         kind = "port"
+        sys.stderr.write("bench.py: no copy of the original DANBO-pytorch ($DANBO_REFERENCE or baseline/_ref, see "
+                         "scripts/vendor_ref.sh): the CPU baseline runs the oracle port (kind \"port\")\n")
         import danbo_oracle as orc
         P = syn.synthetic_params(0)
         A = torch.from_numpy(sk.bone_align_transforms(syn.rest_pose())[0])
@@ -666,7 +697,14 @@ def main():
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the arrays the last timed step returned as DIR/<name>.npy (at most 64 MB in all; at N > 1 "
+                         "rank 0's: every rank renders the same whole image)")
     opt = ap.parse_args()
+    if opt.steps < 1:
+        ap.error("--steps must be at least 1")
+    if opt.dump_outputs and opt.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if opt.impl == "reference":
         run_reference(opt)
     else:

@@ -6,8 +6,8 @@ and bench.py's cpu_baseline / --impl reference legs may import it; the product p
 danbo-pytorch_b200/) never does and fails loudly when its CUDA library is missing.
 
 Pinning: the reference ships no tests or golden vectors (SURVEY §4), so the pins are outputs of the reference
-itself, produced in the authoring container by oracle/gen_golden.py (which imports /root/reference) and
-committed under tests/golden/.  tests/test_oracle_golden.py checks every function below against them.
+itself, produced by oracle/gen_golden.py (which imports the reference) and committed under tests/golden/.
+tests/test_oracle_golden.py checks every function below against them.
 
 Every function names the reference file:line it follows.  `P` is a flat dict of parameters keyed by the
 reference's own state_dict names (SURVEY appendix A), e.g. P["pts_linears.0.weight"].

@@ -1,11 +1,11 @@
-"""Generates tests/golden/*.npz by running the UNMODIFIED reference (authoring container only).
+"""Generates tests/golden/*.npz by running the UNMODIFIED reference (see oracle/ref_harness.py).
 
-    python oracle/gen_golden.py            # needs /root/reference; writes tests/golden/
+    python oracle/gen_golden.py            # needs the reference ($DANBO_REFERENCE or baseline/_ref); writes tests/golden/
 
 Every fixture holds the synthetic inputs (SURVEY §8d), the seed of the deterministic weights
 (danbo_b200.synthetic.synth_state_dict, numpy RandomState -> reproducible anywhere) and the reference's own
 tensors at each stage boundary of SURVEY §8(a), captured by wrapping the reference's functions in place.
-The reference is never copied; the GPU box only sees these vectors.
+The reference is never committed; the tests only need these vectors.
 """
 import os
 import sys
@@ -406,7 +406,7 @@ def run_grid_case(name, config, pose_seed, res, radius=0.9, weight_seed=0):
 
 
 def main():
-    assert rh.available(), "needs /root/reference (authoring container)"
+    assert rh.available(), "needs the reference ($DANBO_REFERENCE or baseline/_ref)"
     os.makedirs(OUT, exist_ok=True)
     torch.set_num_threads(8)
     only = sys.argv[1] if len(sys.argv) > 1 else None       # `python oracle/gen_golden.py anerf` regenerates that case only

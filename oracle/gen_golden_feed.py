@@ -1,7 +1,7 @@
-"""Generates tests/golden/feed_*.npz by running the UNMODIFIED reference data pipeline (authoring container only).
+"""Generates tests/golden/feed_*.npz by running the UNMODIFIED reference data pipeline (see oracle/ref_harness.py).
 TEST INFRASTRUCTURE.
 
-    python oracle/gen_golden_feed.py       # needs /root/reference; writes tests/golden/feed_plain.npz, feed_centers.npz
+    python oracle/gen_golden_feed.py       # needs the reference ($DANBO_REFERENCE or baseline/_ref); writes tests/golden/feed_plain.npz, feed_centers.npz
 
 Pins `danbo-pytorch_b200/feed.py` (SURVEY §8f rank 3): the reference's `BaseH5Dataset.__getitem__`
 (core/dataset.py:61-129) is run on a synthetic training set stored under the reference's HDF5 keys (read through the
@@ -56,7 +56,7 @@ def run_reference(arrays, image_idxs, rays_per_image, seed, mask_img=True, pertu
 
 def main():
     if not ref_harness.available():
-        raise SystemExit("needs /root/reference")
+        raise SystemExit("needs the reference ($DANBO_REFERENCE or baseline/_ref)")
     for name, centers in (("feed_plain", False), ("feed_centers", True)):
         arrays = feed.synthetic_arrays(centers=centers, **SPEC)
         out = run_reference(arrays, np.array([4, 0, 5, 2]), rays_per_image=12, seed=11)

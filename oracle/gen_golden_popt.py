@@ -1,7 +1,7 @@
-"""Generates tests/golden/popt.npz by running the UNMODIFIED reference pose layer (authoring container only).
+"""Generates tests/golden/popt.npz by running the UNMODIFIED reference pose layer (see oracle/ref_harness.py).
 TEST INFRASTRUCTURE.
 
-    python oracle/gen_golden_popt.py       # needs /root/reference
+    python oracle/gen_golden_popt.py       # needs the reference ($DANBO_REFERENCE or baseline/_ref)
 
 Pins `danbo-pytorch_b200/pose_opt.py` (SURVEY §8f rank 2): core/pose_opt.py's `PoseOptLayer` is built on synthetic
 poses (axis-angle and rot6d parameters, and the multi-view parameter split), its parameters are moved off their initial
@@ -81,7 +81,7 @@ def run_case(tag, out, use_rot6d=False, multiview=False):
 
 def main():
     if not ref_harness.available():
-        raise SystemExit("needs /root/reference")
+        raise SystemExit("needs the reference ($DANBO_REFERENCE or baseline/_ref)")
     out = {}
     rest, kps, bones = poses()
     out["rest_pose"], out["init_kps"], out["init_bones"], out["idxs"] = rest, kps, bones, IDXS

@@ -1,7 +1,7 @@
-"""Generates tests/golden/rays_box.npz by running the UNMODIFIED reference ray generation (authoring container only).
+"""Generates tests/golden/rays_box.npz by running the UNMODIFIED reference ray generation (see oracle/ref_harness.py).
 TEST INFRASTRUCTURE.
 
-    python oracle/gen_golden_rays.py       # needs /root/reference
+    python oracle/gen_golden_rays.py       # needs the reference ($DANBO_REFERENCE or baseline/_ref)
 
 Pins SURVEY §8f rank 1 (`render.rays_in_box`, `synthetic.cylinder_image_box`, `skeleton.bounding_cylinder`): the
 reference's `kp_to_valid_rays` (core/utils/ray_utils.py:84-138: `get_rays` :7-29, `get_kp_bounding_cylinder`
@@ -42,7 +42,7 @@ def run_reference(poses, c2ws, focal, given_cyls):
 
 def main():
     if not ref_harness.available():
-        raise SystemExit("needs /root/reference")
+        raise SystemExit("needs the reference ($DANBO_REFERENCE or baseline/_ref)")
     poses, c2ws, focal = inputs()
     out = {"H": H, "W": W, "n_views": N_VIEWS, "pose_seeds": np.array(POSE_SEEDS), "focal": focal}
     for tag, given in (("derived", False), ("given", True)):

@@ -1,6 +1,6 @@
-"""Runs the UNMODIFIED reference: /root/reference in the authoring container, else the git-ignored copy under
-baseline/_ref/ that scripts/vendor_ref.sh makes (it travels to the GPU box).  TEST / BASELINE INFRASTRUCTURE - nothing
-in the product imports this.
+"""Runs the UNMODIFIED reference, an original DANBO-pytorch checkout: the directory named by $DANBO_REFERENCE, else
+the git-ignored copy under baseline/_ref/ that scripts/vendor_ref.sh makes.  Without either, the tests that need it
+skip.  TEST / BASELINE INFRASTRUCTURE - nothing in the product imports this.
 
 Used by oracle/gen_golden.py to pin the oracle, by tests/test_oracle_vs_reference.py, by the drop-in tests
 (tests/test_gpu_dropin.py: the reference's own Trainer / render_path driving this repo's ray caster) and by bench.py's
@@ -17,8 +17,8 @@ import numpy as np
 import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-_CANDIDATES = [os.environ.get("DANBO_REFERENCE"), "/root/reference", os.path.join(os.path.dirname(_HERE), "baseline", "_ref")]
-REF = next((c for c in _CANDIDATES if c and os.path.isdir(os.path.join(c, "core"))), "/root/reference")
+_CANDIDATES = [os.environ.get("DANBO_REFERENCE"), os.path.join(os.path.dirname(_HERE), "baseline", "_ref")]
+REF = next((c for c in _CANDIDATES if c and os.path.isdir(os.path.join(c, "core"))), _CANDIDATES[-1])
 STUBS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "ref_stubs")
 
 

@@ -106,7 +106,7 @@ def test_ctypes_signatures_match_header_parameters():
 
 
 def test_reference_arm_prints_the_contract_line():
-    """`bench.py --impl reference` (the unmodified reference from baseline/_ref or /root/reference on the host cores; the
+    """`bench.py --impl reference` (the unmodified reference from baseline/_ref or $DANBO_REFERENCE on the host cores; the
     oracle port only where neither exists) prints one JSON line with the keys the driver reads."""
     import json
     import subprocess

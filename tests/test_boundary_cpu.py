@@ -4,6 +4,7 @@ the reference's trainer / run scripts touch on the caster, the checkpoint key sc
 import os
 import tempfile
 
+import numpy as np
 import pytest
 import torch
 
@@ -344,43 +345,41 @@ def test_create_raycaster_for_the_other_shipped_configs(tmp_path):
     assert db.create_raycaster(perf, _attrs(), device="cpu")[1]["ray_caster"].view_mode == "root_local"
 
 
-def test_dropin_hook_rebinds_create_raycaster_only():
+def test_dropin_hook_rebinds_create_raycaster_only(tmp_path):
     """`danbo_b200.install()` (dropin.py): the reference's `create_raycaster` name - in core.raycasters and in the modules
-    that copied it (run_nerf) - points at this repo's factory, nothing else changes, and `uninstall()` restores it.  Needs
-    the reference (`/root/reference` or the vendored baseline/_ref)."""
-    import ref_harness as rh                 # tests/conftest.py puts oracle/ on sys.path
-    if not rh.available():
-        pytest.skip("no reference copy")
-    import danbo_b200 as db
-    rc, run_nerf = rh._imports()
-    orig = rc.create_raycaster
-    names_before = {k: id(v) for k, v in vars(rc).items() if not k.startswith("__")}
-    db.install()
-    try:
-        assert getattr(rc.create_raycaster, "__danbo_b200__", False)
-        assert run_nerf.create_raycaster is rc.create_raycaster
-        changed = [k for k, v in vars(rc).items() if not k.startswith("__") and names_before.get(k) != id(v)]
-        assert changed == ["create_raycaster"], changed
-        # flags outside the supported subset raise through the hook as well (no fallback to the reference's caster)
-        args = rh.parse_args("h36m_zju/danbo_fast.txt", ["--agg_type", "relu"])
-        with pytest.raises(NotImplementedError):
-            rc.create_raycaster(args, {"rest_pose": None, "n_views": 8})
-    finally:
-        db.uninstall()
-    assert rc.create_raycaster is orig and run_nerf.create_raycaster is orig
+    that copied it (run_nerf) - points at this repo's factory, nothing else changes, and `uninstall()` restores it.  Runs
+    on the reference when a copy is given, else on a stand-in of its `core/` (tests/util.py `reference_core`)."""
+    import ref_harness as rh                 # tests/conftest.py puts oracle/ and tests/ on sys.path
+    from util import reference_modules
+    with reference_modules(tmp_path) as (rc, run_nerf):
+        args = (rh.parse_args("h36m_zju/danbo_fast.txt", ["--agg_type", "relu"]) if rh.available() else
+                db.make_args("danbo_fast", agg_type="relu"))
+        orig = rc.create_raycaster
+        names_before = {k: id(v) for k, v in vars(rc).items() if not k.startswith("__")}
+        db.install()
+        try:
+            assert getattr(rc.create_raycaster, "__danbo_b200__", False)
+            assert run_nerf.create_raycaster is rc.create_raycaster
+            changed = [k for k, v in vars(rc).items() if not k.startswith("__") and names_before.get(k) != id(v)]
+            assert changed == ["create_raycaster"], changed
+            # flags outside the supported subset raise through the hook as well (no fallback to the reference's caster)
+            with pytest.raises(NotImplementedError):
+                rc.create_raycaster(args, {"rest_pose": None, "n_views": 8})
+        finally:
+            db.uninstall()
+        assert rc.create_raycaster is orig and run_nerf.create_raycaster is orig
 
 
 def test_run_launcher_executes_a_reference_script_with_the_hook_installed(tmp_path):
     """`python -m danbo_b200.run <script> [args]`: the script runs as __main__ from the reference's root with
-    `create_raycaster` already rebound and its own argv.  A stand-in script is placed beside the reference's `core/`."""
+    `create_raycaster` already rebound and its own argv.  A stand-in script is placed beside the reference's `core/`
+    (or beside its stand-in, tests/util.py `reference_core`)."""
     import shutil
     import subprocess
     import sys
-    import ref_harness as rh
-    if not rh.available():
-        pytest.skip("no reference copy")
+    from util import reference_core
     root = tmp_path / "ref"
-    shutil.copytree(os.path.join(rh.REF, "core"), root / "core")
+    shutil.copytree(os.path.join(reference_core(tmp_path), "core"), root / "core")
     (root / "probe_script.py").write_text(
         "import sys, os\n"
         "from core.raycasters import create_raycaster\n"
@@ -430,3 +429,32 @@ def test_both_bench_arms_quote_the_same_config():
     assert a == b and a["rays_per_image"] == 261121 and a["samples_per_ray"] == 48 and a["chunk"] == 4096
     src = open(bench.__file__).read()
     assert src.count('"config": workload_config(args') == 2            # both JSON lines
+
+
+def test_bench_dump_outputs_writes_the_returned_arrays(tmp_path):
+    """`bench.py --dump-outputs DIR`: every returned array as DIR/<name>.npy in float32 (float64 kept); above the byte
+    budget every array keeps the same seeded sample of rays, in ray order, so that two runs write identical files."""
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    n = 1000
+    rid = torch.arange(n, dtype=torch.float32)
+    ret = {"rgb_map": rid[:, None].expand(n, 3).contiguous(), "acc_map": rid.to(torch.float64),
+           "T_i": rid[:, None].expand(n, 48).to(torch.bfloat16)}
+    bench.dump_outputs(ret, str(tmp_path / "all"))
+    full = {k: np.load(tmp_path / "all" / f"{k}.npy") for k in ret}
+    assert sorted(os.listdir(tmp_path / "all")) == ["T_i.npy", "acc_map.npy", "rgb_map.npy"]
+    assert full["acc_map"].dtype == np.float64 and full["rgb_map"].dtype == full["T_i"].dtype == np.float32
+    for k, v in ret.items():
+        np.testing.assert_array_equal(full[k], v.double().numpy())
+    budget = 100 * (3 * 4 + 8 + 48 * 4) + 3 * bench.NPY_HEADER_BYTES     # 100 rays' worth + the headers
+    for d in ("a", "b"):
+        bench.dump_outputs(ret, str(tmp_path / d), budget=budget)
+    part = {k: np.load(tmp_path / "a" / f"{k}.npy") for k in ret}
+    assert sum(os.path.getsize(tmp_path / "a" / f"{k}.npy") for k in ret) <= budget
+    rows = part["acc_map"].astype(np.int64)
+    assert len(rows) == 100 and np.all(np.diff(rows) > 0)
+    for k in ret:
+        np.testing.assert_array_equal(part[k], full[k][rows])
+        np.testing.assert_array_equal(part[k], np.load(tmp_path / "b" / f"{k}.npy"))

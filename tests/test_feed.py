@@ -13,7 +13,9 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "oracle"))
 import danbo_b200                                    # noqa: E402,F401
+import ref_harness                                   # noqa: E402
 from danbo_b200 import feed as fd                    # noqa: E402
 from danbo_b200 import synthetic as syn              # noqa: E402
 
@@ -184,11 +186,10 @@ def test_unsupported_flags_raise():
         fd.synthetic_feed(n_images=2, H=8, W=8, N_nms=1)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/core"), reason="authoring container only")
+@pytest.mark.skipif(not ref_harness.available(), reason="needs the original DANBO-pytorch (DANBO_REFERENCE or baseline/_ref)")
 def test_live_reference_other_draws():
     """The unmodified reference data pipeline, live, on draws that are not among the fixtures (focal per axis,
     identity camera rotation short-cut of dataset.py:393-394, no background arrays)."""
-    sys.path.insert(0, os.path.join(ROOT, "oracle"))
     import gen_golden_feed as gg
     arrays = fd.synthetic_arrays(n_images=5, H=18, W=14, seed=9, centers=True)
     arrays["focals"] = np.stack([arrays["focals"], arrays["focals"] * 1.1], -1)     # (N, 2): fx, fy

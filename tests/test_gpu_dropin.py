@@ -1,5 +1,5 @@
 """The reference's OWN callers on this repo's ray caster (run with -m gpu; needs the reference copy under baseline/_ref,
-made by scripts/vendor_ref.sh, or /root/reference).
+made by scripts/vendor_ref.sh, or $DANBO_REFERENCE).
 
 `danbo_b200.install()` rebinds `create_raycaster` (core/raycasters.py:17) - nothing else of the reference is touched - and
 then the unmodified `Trainer.train_batch` (core/trainer.py:257-300: render -> compute_loss -> backward -> Adam -> decay)
@@ -13,8 +13,8 @@ import torch
 import ref_harness as rh
 from danbo_b200 import synthetic as syn, skeleton as sk
 
-pytestmark = [pytest.mark.gpu, pytest.mark.timeout(600, method="thread"),
-              pytest.mark.skipif(not rh.available(), reason="no reference copy (run scripts/vendor_ref.sh)")]
+pytestmark = [pytest.mark.gpu, pytest.mark.timeout(600, method="thread")]
+needs_reference = pytest.mark.skipif(not rh.available(), reason="no reference copy (run scripts/vendor_ref.sh)")
 DEV = "cuda"
 N_POSES, RPP = 4, 96
 
@@ -72,18 +72,21 @@ def _ref_batch(device):
     return {k: v.contiguous().to(device) for k, v in rb.items()}, b
 
 
-def test_install_rebinds_create_raycaster_only():
+def test_install_rebinds_create_raycaster_only(tmp_path):
+    """On the reference when a copy is given, else on the stand-in of its `core/` (tests/util.py `reference_core`)."""
     import danbo_b200 as db
-    rc, run_nerf = rh._imports()
-    orig = rc.create_raycaster
-    db.install()
-    try:
-        assert getattr(rc.create_raycaster, "__danbo_b200__", False) and run_nerf.create_raycaster is rc.create_raycaster
-    finally:
-        db.uninstall()
-    assert rc.create_raycaster is orig and run_nerf.create_raycaster is orig
+    from util import reference_modules
+    with reference_modules(tmp_path) as (rc, run_nerf):
+        orig = rc.create_raycaster
+        db.install()
+        try:
+            assert getattr(rc.create_raycaster, "__danbo_b200__", False) and run_nerf.create_raycaster is rc.create_raycaster
+        finally:
+            db.uninstall()
+        assert rc.create_raycaster is orig and run_nerf.create_raycaster is orig
 
 
+@needs_reference
 @pytest.mark.parametrize("perturb", [0.0, 1.0])
 def test_reference_trainer_train_batch_on_this_caster(perturb):
     import danbo_b200 as db
@@ -147,6 +150,7 @@ def test_reference_trainer_train_batch_on_this_caster(perturb):
 
 
 
+@needs_reference
 def test_reference_render_path_on_this_caster():
     """BASELINE config #1 shape: danbo_base, one 64x64 image, through the reference's render_path on both casters."""
     import danbo_b200 as db

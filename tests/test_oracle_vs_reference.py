@@ -1,6 +1,6 @@
 """Live comparison of the CPU oracle with the UNMODIFIED reference on inputs that are NOT among the committed fixtures
-(other poses, ray subsets and weight seeds).  Needs /root/reference, so it runs in the authoring container only and is
-skipped on the GPU box (nothing under tests/ reads the reference there)."""
+(other poses, ray subsets and weight seeds).  Needs an original DANBO-pytorch checkout ($DANBO_REFERENCE or the copy
+under baseline/_ref/, see oracle/ref_harness.py) and skips without one."""
 import os
 import sys
 
@@ -11,7 +11,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
 import ref_harness as rh  # noqa: E402
 
-pytestmark = pytest.mark.skipif(not rh.available(), reason="/root/reference is not present (GPU box)")
+pytestmark = pytest.mark.skipif(not rh.available(), reason="needs the original DANBO-pytorch (DANBO_REFERENCE or baseline/_ref)")
 
 
 def _render_both(config, extra, pose_seed, weight_seed, n_rays, agg_type="sigmoid", lindisp=False):

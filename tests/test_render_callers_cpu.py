@@ -12,7 +12,9 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "oracle"))
 import danbo_b200                                    # noqa: E402,F401
+import ref_harness                                   # noqa: E402
 from danbo_b200 import render, skeleton as sk, synthetic as syn  # noqa: E402
 
 FX = np.load(os.path.join(ROOT, "tests", "golden", "rays_box.npz"))
@@ -58,7 +60,7 @@ def test_rays_in_box_match_reference(tag):
     assert len(n_rays) > 1                                              # ... differently from view to view
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/core"), reason="authoring container only")
+@pytest.mark.skipif(not ref_harness.available(), reason="needs the original DANBO-pytorch (DANBO_REFERENCE or baseline/_ref)")
 def test_live_reference_other_cameras():
     sys.path.insert(0, os.path.join(ROOT, "oracle"))
     import gen_golden_rays as gg
@@ -113,10 +115,8 @@ def test_render_chunks_like_batchify_rays():
     assert ra["rgb_map"].shape == (10, 3) and ra["T_i"].shape == (10, 5, 4)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/core"), reason="authoring container only")
+@pytest.mark.skipif(not ref_harness.available(), reason="needs the original DANBO-pytorch (DANBO_REFERENCE or baseline/_ref)")
 def test_render_hands_the_caster_what_the_reference_does():
-    sys.path.insert(0, os.path.join(ROOT, "oracle"))
-    import ref_harness
     ref_harness._imports()
     import core.trainer as tr
     rays, kw = _render_inputs()

@@ -1,4 +1,5 @@
 """Shared helpers for the parity tests: fixture loading and parameter rebuilding."""
+import contextlib
 import os
 
 import numpy as np
@@ -226,3 +227,44 @@ def field_mlp_bf16_ste(x, view, P):
     g = torch.relu(feat @ bf(Wv[:, :256]).t() + view @ Wv[:, 256:].t() + P["views_linears.0.bias"])
     rgb = g @ P["rgb_linear.weight"].t() + P["rgb_linear.bias"]
     return torch.cat([rgb, sigma], -1)
+
+
+def reference_core(tmp_path):
+    """-> a directory holding the reference's `core/` and `run_nerf.py`: the reference itself when a copy is given
+    ($DANBO_REFERENCE or the vendored baseline/_ref), else a stand-in with just the seam the drop-in hook works on - a
+    `core.raycasters` that defines `create_raycaster` and a `run_nerf` that copies the name (run_nerf.py:20)."""
+    import ref_harness as rh
+    if rh.available():
+        return rh.REF
+    root = tmp_path / "stand_in"
+    (root / "core").mkdir(parents=True)
+    (root / "core" / "__init__.py").write_text("")
+    (root / "core" / "raycasters.py").write_text(
+        "import os\n\nRAY_CHUNK = 4096\n\n\ndef create_raycaster(args, data_attrs, device=None):\n"
+        "    raise AssertionError('the stand-in factory must not be called')\n")
+    (root / "run_nerf.py").write_text("from core.raycasters import create_raycaster\n")
+    return str(root)
+
+
+@contextlib.contextmanager
+def reference_modules(tmp_path):
+    """-> (core.raycasters, run_nerf) of the reference copy when one is given, else of the `reference_core` stand-in.
+    The stand-in's modules and path entry are gone again on exit, and modules of those names that were loaded
+    before are put back."""
+    import importlib
+    import sys
+    import ref_harness as rh
+    if rh.available():
+        yield rh._imports()
+        return
+    root = reference_core(tmp_path)
+    names = ("core", "core.raycasters", "run_nerf")
+    saved = {n: sys.modules.pop(n) for n in names if n in sys.modules}
+    sys.path.insert(0, root)
+    try:
+        yield importlib.import_module("core.raycasters"), importlib.import_module("run_nerf")
+    finally:
+        sys.path.remove(root)
+        for n in names:
+            sys.modules.pop(n, None)
+        sys.modules.update(saved)
