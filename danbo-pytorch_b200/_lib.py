@@ -37,6 +37,7 @@ _SIGNATURES = {
     "danbo_anerf_save_bytes": [c_i, c_p],
     "danbo_anerf_mlp_save": [c_p, c_p, c_p, c_p, c_p, c_p, c_i, c_i, c_p, c_i, c_i, c_p, c_p],
     "danbo_anerf_untile": [c_p, ctypes.c_longlong, c_i, c_i, c_p, c_p],
+    "danbo_anerf_embed_bwd": [c_p, c_i, c_i, c_i, c_p, c_p, c_i, c_i, c_p, c_p, c_f, c_p, c_p, c_p, c_p],
     "danbo_pack_mlp_weights": [c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p],
     "danbo_mlp_forward": [c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_i, c_p, c_i, c_i, c_i, c_p],
     "danbo_mlp_forward_trace": [c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_i, c_p, c_i, c_i, c_i, c_p, c_p],

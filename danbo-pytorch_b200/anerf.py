@@ -5,7 +5,8 @@ plus the cutoff embedders' `cutoff_dist` / `tau` entries, cutoff_embedder.py:128
 `AnerfCaster` mirrors raycasters.py:205-546 for this network type: cylinder near/far only (:419-420), every sample
 goes through the field, single_net fine pass on the S_f new samples (F9).  Train mode (single_net configs): the forward
 keeps every layer's activation tile image (`danbo_anerf_mlp_save`) and `_AnerfBlock.backward` turns d (rgb, acc) into the
-MLP / frame-code gradients with the compositing backward kernels and `kernels.anerf_mlp_backward`.
+MLP / frame-code gradients with the compositing backward kernels and `kernels.anerf_mlp_backward`; when the poses require
+a gradient (--opt_pose) it also returns d loss / d skts through `kernels.anerf_embed_bwd`.
 """
 import torch
 import torch.nn as nn
@@ -214,7 +215,8 @@ class AnerfCaster(RayCaster):
         if save:
             keep.update(dict(rays=rays, cam_idx=cam_idx, codes=codes, code_bias=code_bias, S_c=S_c, S_f=S_f, inv_B=inv_B,
                              z0=z0, raw0=raw0, ones0=ones0, noise0=noise0, xd0=xd, xv0=xv, sv0=sv0, raw1=raw1, ones1=ones1,
-                             noise1=noise1, xd1=xd1, xv1=xv1, sv1=sv1, z_all=c0["z_all"], order=c0["order"]))
+                             noise1=noise1, xd1=xd1, xv1=xv1, sv1=sv1, z_all=c0["z_all"], order=c0["order"],
+                             z1=z1, ray_enc=enc, p_skts=p_skts, skip=skip, align=align, tau=tau))
         ret = {"rgb_map": c1["rgb_map"], "disp_map": c1["disp_map"], "acc_map": c1["acc_map"], "alpha": c1["alpha"],
                "T_i": c1["weights"], "rgb0": c0["rgb_map"], "disp0": c0["disp_map"], "acc0": c0["acc_map"],
                "alpha0": c0["alpha"]}
@@ -288,13 +290,15 @@ ANERF_DIFF_KEYS = ("rgb_map", "acc_map", "rgb0", "acc0")
 class _AnerfBlock(torch.autograd.Function):
     """Autograd root of A-NeRF training: forward = the render kernels with saved activations; backward = compositing
     backward kernels (composite.cu) + kernels.anerf_mlp_backward.  Differentiable outputs are what the trainer's losses
-    read (core/trainer.py:396-422): rgb_map, acc_map, rgb0, acc0."""
+    read (core/trainer.py:396-422): rgb_map, acc_map, rgb0, acc0.  The per-pose world-to-bone matrices are an input:
+    when they require a gradient (the pose layer under --opt_pose, core/trainer.py:314-341) each pass also forms the MLP's
+    input gradient and `danbo_anerf_embed_bwd` turns it into d loss / d skts."""
 
     @staticmethod
-    def forward(ctx, caster, cfg, *params):
+    def forward(ctx, caster, cfg, pose_skts, *params):
         keep = {}
         with torch.no_grad():
-            ret = caster._render_block_anerf(cfg["rays"], 0, cfg["skip"], cfg["pose_skts"], cfg["pose_cyls"], cfg["cam_idx"],
+            ret = caster._render_block_anerf(cfg["rays"], 0, cfg["skip"], pose_skts, cfg["pose_cyls"], cfg["cam_idx"],
                                              cfg["codes"], cfg["align"], cfg["packed"], cfg["tau"], cfg["S_c"], cfg["S_f"],
                                              cfg["B"], cfg["nanmean_chunk"], cfg["stages"], lindisp=cfg["lindisp"],
                                              rand=cfg["rand"], raw_noise_std=cfg["raw_noise_std"], keep=keep)
@@ -318,19 +322,27 @@ class _AnerfBlock(torch.autograd.Function):
                               None, None)
         K.composite_bwd(rays, S_c, k["raw0"], k["ones0"], k["z0"], k["noise0"], k["inv_B"], cg(g["rgb0"], n, 3),
                         cg(g["acc0"], n), d_raw0)
-        for d_raw, S, xd, xv, sv in ((d_raw0, S_c, k["xd0"], k["xv0"], k["sv0"]), (d_raw1, S_f, k["xd1"], k["xv1"], k["sv1"])):
-            K.anerf_mlp_backward(P, G, d_raw, n * S, S, xd, xv, sv, k["code_bias"], k["cam_idx"], k["codes"])
+        want_pose = ctx.needs_input_grad[2]
+        d_skts = zeros(*k["p_skts"].shape) if want_pose else None         # p0 == 0: a training block holds every pose
+        for d_raw, S, z, xd, xv, sv in ((d_raw0, S_c, k["z0"], k["xd0"], k["xv0"], k["sv0"]),
+                                        (d_raw1, S_f, k["z1"], k["xd1"], k["xv1"], k["sv1"])):
+            dx = K.anerf_mlp_backward(P, G, d_raw, n * S, S, xd, xv, sv, k["code_bias"], k["cam_idx"], k["codes"],
+                                      want_dx=want_pose)
+            if want_pose:
+                K.anerf_embed_bwd(rays, S, z, k["p_skts"], k["skip"], k["align"], k["ray_enc"], k["tau"], dx[0], dx[1],
+                                  d_skts)
+                del dx
         ctx.keep = None
-        return (None, None) + tuple(G[name] for name in ANERF_PARAM_NAMES)
+        return (None, None, d_skts) + tuple(G[name] for name in ANERF_PARAM_NAMES)
 
 
 def _anerf_block_with_grad(caster, rays, skip, pose_skts, pose_cyls, cam_idx, codes, align, packed, tau, S_c, S_f, B,
                            nanmean_chunk, lindisp, rand, raw_noise_std, stages):
     named = dict(caster.network.named_parameters())
-    cfg = dict(rays=rays, skip=skip, pose_skts=pose_skts, pose_cyls=pose_cyls, cam_idx=cam_idx, codes=codes, align=align,
+    cfg = dict(rays=rays, skip=skip, pose_cyls=pose_cyls, cam_idx=cam_idx, codes=codes, align=align,
                packed=packed, tau=tau, S_c=S_c, S_f=S_f, B=B, nanmean_chunk=nanmean_chunk, lindisp=lindisp, rand=rand,
                raw_noise_std=raw_noise_std, stages=stages)
-    outs = _AnerfBlock.apply(caster, cfg, *[named[n] for n in ANERF_PARAM_NAMES])
+    outs = _AnerfBlock.apply(caster, cfg, pose_skts, *[named[n] for n in ANERF_PARAM_NAMES])
     return dict(zip(ANERF_OUT_KEYS, outs))
 
 

@@ -805,10 +805,13 @@ class _RowCount:
         self.capacity = int(rows)
 
 
-def anerf_mlp_backward(P, G, d_raw, rows, S, xd, xv, save, code_bias, cam_idx, codes_with_mean):
+def anerf_mlp_backward(P, G, d_raw, rows, S, xd, xv, save, code_bias, cam_idx, codes_with_mean, want_dx=False):
     """Backward of the A-NeRF MLP (core/networks/nerf.py:164-209 under autograd, trainer.py:573) over the `rows` dense
-    rows of one pass: parameter gradients are ADDED to G (reference names).  No input gradient is needed: the encodings
-    have no trainable parameter (opt_cutoff = False) and the poses are not optimised on this path.
+    rows of one pass: parameter gradients are ADDED to G (reference names).  The encodings have no trainable parameter
+    (opt_cutoff = False), so the input gradient is only formed when the poses are optimised (want_dx): then
+    -> (d xd (rows,432), d xv (rows,648)) fp32, d xd = delta0 . W0 + delta5 . W5[:, :432] (layer 0 and the skip input of
+    layer 5), d xv = delta9 . Wv[:, 448:1096], three more danbo_gemm_dgrad launches.  Otherwise None, and the launch
+    sequence is the one without them.
 
     d_raw (>= rows,4) [d rgb, d sigma]; xd / xv: the pass's operand tile images; save: what danbo_anerf_mlp_save kept;
     code_bias (n_rays,224) from danbo_anerf_ray_encode.  Built from the generic fp32 GEMM kernels of backward_mlp.cu
@@ -834,6 +837,11 @@ def anerf_mlp_backward(P, G, d_raw, rows, S, xd, xv, save, code_bias, cam_idx, c
     # rgb head
     d9 = f32(rows, VW)
     _dgrad(_Ptr(d_raw.view(-1), 0, ld=4), f32c(P["rgb_linear.weight"]), VW, d9, VW, rc, VW, 3, mask=z9.to(torch.bfloat16))
+    dXd = dXv = None
+    if want_dx:
+        dXv = f32(rows, XV)
+        with _Timed("anerf_mlp_dx"):
+            _dgrad(d9, _Ptr(Wv.view(-1), W), W + XV + 128, dXv, XV, rc, XV, VW)
     _wgrad(_Ptr(d_raw.view(-1), 0, ld=4), g, G["rgb_linear.weight"], VW, rc, 3, VW)
     _colsum(_Ptr(d_raw.view(-1), 0, ld=4), G["rgb_linear.bias"], rc, 3)
     # view layer: weights of the feature / direction / frame-code column blocks, bias, frame codes
@@ -867,9 +875,41 @@ def anerf_mlp_backward(P, G, d_raw, rows, S, xd, xv, save, code_bias, cam_idx, c
             _wgrad(cur, xd_r, dW, XD + W, rc, W, XD)
             _wgrad(cur, a_in, _Ptr(dW.view(-1), XD), XD + W, rc, W, W)
             _dgrad(cur, _Ptr(Wl.view(-1), XD), XD + W, nxt, W, rc, W, W, mask=a_in)
+            if want_dx:
+                dXd = f32(rows, XD)
+                with _Timed("anerf_mlp_dx"):
+                    _dgrad(cur, Wl, XD + W, dXd, XD, rc, XD, W)
         else:
             _wgrad(cur, a_in, G[f"pts_linears.{L}.weight"], W, rc, W, W)
             _dgrad(cur, Wl, W, nxt, W, rc, W, W, mask=a_in)
         cur, nxt = nxt, cur
     _colsum(cur, G["pts_linears.0.bias"], rc, W)
     _wgrad(cur, xd_r, G["pts_linears.0.weight"], XD, rc, W, XD)
+    if want_dx:
+        with _Timed("anerf_mlp_dx"):
+            _dgrad(cur, f32c(P["pts_linears.0.weight"]), XD, dXd, XD, rc, XD, W, accumulate=True)
+        return dXd, dXv
+    return None
+
+
+def anerf_embed_bwd(rays, S, z, pose_skts, rays_per_pose, align, ray_enc, tau, d_xd, d_xv, d_skts):
+    """d skts (n_poses,24,4,4) += d loss / d skts of one pass's encodings (danbo_anerf_embed_bwd), given the MLP's input
+    gradient d_xd (n*S,432), d_xv (n*S,648) and the pass's forward inputs (z (n,S), ray_enc from anerf_ray_encode)."""
+    _need_cuda(rays, z, pose_skts, align, ray_enc, d_xd, d_xv, d_skts)
+    n = rays.shape[0]
+    f32 = torch.float32
+    assert rays.dtype == f32 and rays.dim() == 2 and rays.shape[1] >= 6 and rays.stride(1) == 1
+    assert z.dtype == f32 and z.shape == (n, S) and z.is_contiguous()
+    assert ray_enc.dtype == f32 and ray_enc.shape[0] >= n and ray_enc.shape[1] == 648 and ray_enc.is_contiguous()
+    assert pose_skts.dtype == f32 and pose_skts.shape[1:] == (24, 4, 4) and pose_skts.is_contiguous()
+    assert align.dtype == f32 and align.shape == (24, 4, 4) and align.is_contiguous()
+    assert d_xd.dtype == f32 and d_xv.dtype == f32
+    assert d_xd.shape == (n * S, 432) and d_xv.shape == (n * S, 648) and d_xd.is_contiguous() and d_xv.is_contiguous()
+    assert d_skts.shape == pose_skts.shape and d_skts.dtype == torch.float32 and d_skts.is_contiguous()
+    with _Timed("anerf_embed_bwd"):
+        _lib.check(_lib.load().danbo_anerf_embed_bwd(_p(rays), rays.stride(0), n, int(S), _p(z), _p(pose_skts),
+                                                     int(rays_per_pose), pose_skts.shape[0], _p(align), _p(ray_enc),
+                                                     float(tau), _p(d_xd), _p(d_xv), _p(d_skts), _stream()),
+                   "danbo_anerf_embed_bwd")
+    _count(1)
+    return d_skts

@@ -307,6 +307,16 @@ int danbo_anerf_mlp_save(const void* xd, const void* xv, const void* wstream, co
  * row-major bf16 out (n_rows, n_chunks * 64): how the A-NeRF backward reads xd / xv / saved activations. */
 int danbo_anerf_untile(const void* img, long long tile_stride, int n_rows, int n_chunks, void* out, void* stream);
 
+/* Backward of danbo_anerf_embed and of the direction part of danbo_anerf_ray_encode to the poses (pose refinement,
+ * --opt_pose): autograd of core/encoders.py:288-303,305-317,442-444,639-651,774-795 and core/cutoff_embedder.py:151-214
+ * (encode_pts / encode_views, core/networks/nerf.py:222-279) with respect to skts.  Rows are dense (row = ray * S + s);
+ * z, pose_skts, align, ray_enc and tau are what the forward calls of the pass read.  d_xd (n_rays*S,432) and d_xv
+ * (n_rays*S,648) fp32, row-major: d loss / d the density and view inputs.  d_skts (n_poses,24,4,4) fp32 is added to
+ * (zero it first); rows 0-2 only, the homogeneous row gets nothing.  Near/far and the sample depths are constants. */
+int danbo_anerf_embed_bwd(const float* rays, int ray_stride, int n_rays, int S, const float* z, const float* pose_skts,
+                          int rays_per_pose, int n_poses, const float* align, const float* ray_enc, float tau,
+                          const float* d_xd, const float* d_xv, float* d_skts, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
