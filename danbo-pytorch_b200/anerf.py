@@ -197,7 +197,7 @@ class AnerfCaster(RayCaster):
         inv_B = 1.0 / B
         noise0 = (rand["noise0"] * (raw_noise_std * B)).contiguous() if ("noise0" in rand and raw_noise_std > 0) else None
         c0 = K.composite_resample(rays, S_c, S_f, raw0, ones0, z0, noise=noise0, inv_B=inv_B, u_rand=rand.get("u"),
-                                  want_inds=stages is not None, smooth=self.single_net)
+                                  want_inds=stages is not None, smooth=self.single_net, want_weights=stages is not None)
         z1 = c0["z_samples"]
         if not self.single_net:
             return self._fine_network_pass(rays, p_skts, skip, cam_idx, align, S_c, S_f, B, c0, near, far, z0, raw0, stages)

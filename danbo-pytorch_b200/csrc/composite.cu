@@ -2,10 +2,9 @@
 // Reference: core/networks/nerf.py:281-347 (raw2outputs), core/utils/ray_utils.py:159-203,257-291
 // (sample_pdf / isample_from_lineseg), core/raycasters.py:484-514,745-761 (_merge_encodings / merge_samples).
 //
-// One warp per ray; every lane owns a contiguous run of samples, products and prefix sums are done as
-// lane-local sequential work plus one warp scan.  cumprod / cumsum accumulate in fp64 like ATen's CPU kernels
-// (acc_type<float>) and round each output to fp32.  HBM bound: 16 B raw + 4 B z in, 8 B (weight, alpha) out
-// per sample, 20 B per ray.
+// Forward: a group of kL lanes per ray, 32 / kL rays per warp; backward: one warp per ray.  cumprod / cumsum
+// accumulate in fp64 like ATen's CPU kernels (acc_type<float>) and round each output to fp32.  16 B raw + 4 B z in,
+// 8 B (weight, alpha) out per sample: too few bytes to bind the forward kernels to HBM, they are bound by instruction issue.
 #include "common.cuh"
 #include <math.h>
 
@@ -39,194 +38,286 @@ __device__ __forceinline__ double warp_excl_sum(double v, int lane) {
     return lane == 0 ? 0.0 : ex;
 }
 
-// Composites one ray whose S samples are described by fetch(i) -> raw (rgb, sigma).  sm.z must hold z[0..S).
-// Writes weights / alpha rows and the per-ray maps; leaves the weights in sm.w.
-// kE = samples per lane = ceil(S / 32), a template parameter so that the per-lane loops have no dead iterations (the
-// generic 5-element loops spent 4 of 5 iterations on predicated-off work at S = 32).
-template <int kE, class Fetch>
-__device__ __forceinline__ void composite_ray(RaySmem& sm, int S, int lane, float norm_d, float inv_B,
-                                              const float* __restrict__ noise_row, Fetch fetch,
-                                              float* __restrict__ w_row, float* __restrict__ alpha_row,
-                                              float* __restrict__ rgb_out, float* __restrict__ disp_out,
-                                              float* __restrict__ acc_out) {
-    constexpr int epl = kE;
-    float al[kE], cr[kE], cg[kE], cb[kE];
-    double lp = 1.0;
+// ---- forward kernels: a group of kL lanes composites one ray, a warp holds 32 / kL rays.  The per-ray work that does
+// not grow with S (setup, scans, reductions, the map stores, the merge bookkeeping) is then shared by the rays of a warp
+// instead of being repeated by all 32 lanes for every ray.
+//
+// Sample layout.  The fp32 sums behind the maps (rgb, disp, acc) are defined on a 32-lane layout: virtual lane v holds
+// the kEo = ceil(S / 32) samples v*kEo .. v*kEo + kEo - 1, sums them in order, and the 32 partial sums meet in an xor
+// butterfly (16, 8, 4, 2, 1).  Lane g of a group holds the virtual lanes g, g + kL, g + 2 kL, ..., so the butterfly levels
+// >= kL are lane-local and the rest are shuffles of width kL: the maps come out bit-identical for every kL.
+// The fp64 transmittance product is scanned per round of kL virtual lanes; that association differs from a 32-lane scan
+// and can move a weight by one fp32 ulp only when the fp64 product lies within 2^-29 (relative) of an fp32 rounding tie.
+// The pdf and cdf sums are fp64 sums of fp32 terms no smaller than 1e-5 / total and are exact in any order.
+//
+// Every lane of a warp stays to the end: a group past the last ray computes on the last ray and stores nothing, so the
+// full-warp shuffles of its neighbours stay defined.  Shuffles use width kL, votes and __syncwarp the group's mask.
+
+template <int kL>
+__device__ __forceinline__ unsigned group_mask(int lane) {
+    return kL == 32 ? 0xffffffffu : ((1u << kL) - 1u) << (lane & ~(kL - 1));
+}
+template <int kL>
+__device__ __forceinline__ double group_incl_prod(double v, int g) {
 #pragma unroll
-    for (int e = 0; e < kE; ++e) {
-        const int i = lane * epl + e;
-        al[e] = 0.f; cr[e] = cg[e] = cb[e] = 0.f;
-        if (i < S) {
-            const float4 raw = fetch(i);
-            float d = (i + 1 < S) ? __fsub_rn(sm.z[i + 1], sm.z[i]) : 1e10f;
-            d = __fmul_rn(d, norm_d);
-            cr[e] = (1.f / (1.f + expf(-raw.x))) * 1.002f - 0.001f;
-            cg[e] = (1.f / (1.f + expf(-raw.y))) * 1.002f - 0.001f;
-            cb[e] = (1.f / (1.f + expf(-raw.z))) * 1.002f - 0.001f;
-            float sg = __fmul_rn(raw.w, inv_B);
-            if (noise_row) sg = __fadd_rn(sg, noise_row[i]);
-            sg = fmaxf(sg, 0.f);
-            al[e] = __fsub_rn(1.f, expf(-__fmul_rn(sg, d)));
-            lp *= (double)__fadd_rn(__fsub_rn(1.f, al[e]), 1e-10f);
+    for (int o = 1; o < kL; o <<= 1) { const double u = __shfl_up_sync(0xffffffffu, v, o, kL); if (g >= o) v *= u; }
+    return v;
+}
+template <int kL>
+__device__ __forceinline__ double group_incl_sum(double v, int g) {
+#pragma unroll
+    for (int o = 1; o < kL; o <<= 1) { const double u = __shfl_up_sync(0xffffffffu, v, o, kL); if (g >= o) v += u; }
+    return v;
+}
+template <int kL, class T>
+__device__ __forceinline__ T group_sum(T v) {
+#pragma unroll
+    for (int o = kL / 2; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o, kL);
+    return v;
+}
+
+// Composites one ray of S samples (z[0..S), fetch(i) -> raw (rgb, sigma)) on the kL lanes of its group; kEo = ceil(S / 32).
+// Writes the weights / alpha rows and the maps when `store`; leaves the weights in w_sm when it is given.
+template <int kL, int kEo, class Fetch>
+__device__ __forceinline__ void composite_group(const float* z, int S, int g, unsigned gmask, bool store, float norm_d,
+                                                float inv_B, const float* __restrict__ noise_row, Fetch fetch, float* w_sm,
+                                                float* __restrict__ w_row, float* __restrict__ alpha_row,
+                                                float* __restrict__ rgb_out, float* __restrict__ disp_out,
+                                                float* __restrict__ acc_out) {
+    constexpr int R = 32 / kL;                          // virtual lanes per lane
+    float al[R][kEo], cr[R][kEo], cg[R][kEo], cb[R][kEo];
+    double lp[R];
+#pragma unroll
+    for (int j = 0; j < R; ++j) {
+        lp[j] = 1.0;
+#pragma unroll
+        for (int e = 0; e < kEo; ++e) {
+            const int i = (j * kL + g) * kEo + e;
+            al[j][e] = 0.f; cr[j][e] = cg[j][e] = cb[j][e] = 0.f;
+            if (i < S) {
+                const float4 raw = fetch(i);
+                float d = (i + 1 < S) ? __fsub_rn(z[i + 1], z[i]) : 1e10f;
+                d = __fmul_rn(d, norm_d);
+                cr[j][e] = (1.f / (1.f + expf(-raw.x))) * 1.002f - 0.001f;
+                cg[j][e] = (1.f / (1.f + expf(-raw.y))) * 1.002f - 0.001f;
+                cb[j][e] = (1.f / (1.f + expf(-raw.z))) * 1.002f - 0.001f;
+                float sg = __fmul_rn(raw.w, inv_B);
+                if (noise_row) sg = __fadd_rn(sg, noise_row[i]);
+                sg = fmaxf(sg, 0.f);
+                al[j][e] = __fsub_rn(1.f, expf(-__fmul_rn(sg, d)));
+                lp[j] *= (double)__fadd_rn(__fsub_rn(1.f, al[j][e]), 1e-10f);
+            }
         }
     }
-    double T = warp_excl_prod(lp, lane);
-    float sr = 0.f, sg_ = 0.f, sb = 0.f, sd = 0.f, sw = 0.f;
+    // exclusive product before each virtual lane: a group scan per round, times the product of the rounds before it
+    double T[R];
+    double carry = 1.0;
 #pragma unroll
-    for (int e = 0; e < kE; ++e) {
-        const int i = lane * epl + e;
-        if (i < S) {
-            const float w = __fmul_rn(al[e], (float)T);
-            T *= (double)__fadd_rn(__fsub_rn(1.f, al[e]), 1e-10f);
-            sm.w[i] = w;
-            if (w_row) w_row[i] = w;
-            if (alpha_row) alpha_row[i] = al[e];
-            sr = fmaf(w, cr[e], sr); sg_ = fmaf(w, cg[e], sg_); sb = fmaf(w, cb[e], sb);
-            sd = fmaf(w, sm.z[i], sd); sw += w;
+    for (int j = 0; j < R; ++j) {
+        const double inc = group_incl_prod<kL>(lp[j], g);
+        const double ex = __shfl_up_sync(0xffffffffu, inc, 1, kL);
+        T[j] = carry * (g == 0 ? 1.0 : ex);
+        if (j + 1 < R) carry *= __shfl_sync(0xffffffffu, inc, kL - 1, kL);
+    }
+    float pr[R], pg[R], pb[R], pd[R], pw[R];
+#pragma unroll
+    for (int j = 0; j < R; ++j) {
+        double t = T[j];
+        pr[j] = pg[j] = pb[j] = pd[j] = pw[j] = 0.f;
+#pragma unroll
+        for (int e = 0; e < kEo; ++e) {
+            const int i = (j * kL + g) * kEo + e;
+            if (i < S) {
+                const float w = __fmul_rn(al[j][e], (float)t);
+                t *= (double)__fadd_rn(__fsub_rn(1.f, al[j][e]), 1e-10f);
+                if (w_sm) w_sm[i] = w;
+                if (store) {
+                    if (w_row) w_row[i] = w;
+                    alpha_row[i] = al[j][e];
+                }
+                pr[j] = fmaf(w, cr[j][e], pr[j]); pg[j] = fmaf(w, cg[j][e], pg[j]); pb[j] = fmaf(w, cb[j][e], pb[j]);
+                pd[j] = fmaf(w, z[i], pd[j]); pw[j] += w;
+            }
         }
     }
-    sr = warp_sum(sr); sg_ = warp_sum(sg_); sb = warp_sum(sb); sd = warp_sum(sd); sw = warp_sum(sw);
-    if (lane == 0) {
-        rgb_out[0] = sr; rgb_out[1] = sg_; rgb_out[2] = sb;
+    // butterfly levels 16 .. kL: virtual lanes j*kL + g and (j + m)*kL + g sit in the same lane
+#pragma unroll
+    for (int m = R / 2; m > 0; m >>= 1)
+#pragma unroll
+        for (int j = 0; j < m; ++j) {
+            pr[j] += pr[j + m]; pg[j] += pg[j + m]; pb[j] += pb[j + m]; pd[j] += pd[j + m]; pw[j] += pw[j + m];
+        }
+    const float sr = group_sum<kL>(pr[0]), sg = group_sum<kL>(pg[0]), sb = group_sum<kL>(pb[0]);
+    const float sd = group_sum<kL>(pd[0]), sw = group_sum<kL>(pw[0]);
+    if (store && g == 0) {
+        rgb_out[0] = sr; rgb_out[1] = sg; rgb_out[2] = sb;
         float disp = 1.f / fmaxf(1e-10f, sd / (sw + 1e-10f));
         if (fabsf(sw) <= 1e-8f) disp = 0.f;                         // torch.isclose(sum w, 0) -> disparity 0
         *disp_out = disp;
         *acc_out = fminf(sw, 1.f);
     }
-    __syncwarp();
+    __syncwarp(gmask);
 }
 
-// Coarse pass: composite + inverse-CDF importance sampling + merge order.
-template <int kE>
+// Coarse pass: composite + inverse-CDF importance sampling + merge order.  Dynamic shared memory: per ray, z[S], w[S],
+// cdf[S], and for S_f > 0 the fine samples zs[S_f] with their stable sort (values, indices) when they are out of order.
+template <int kL, int kEo>
 __global__ void __launch_bounds__(32 * kWarpsPerBlock)
 composite_resample_kernel(const float* __restrict__ rays, int ray_stride, int n_rays, int S, int S_f,
                           const float* __restrict__ raw /* (n_rays*S + n_rays, 4); tail = per-ray empty sample */,
                           const uint32_t* __restrict__ mask, const float* __restrict__ z,
                           const float* __restrict__ noise, float inv_B, const float* __restrict__ u_vals /* (S_f) or null */,
                           const float* __restrict__ u_rand /* (n_rays,S_f) or null */,
-                          float* __restrict__ weights, float* __restrict__ alpha, float* __restrict__ rgb0,
+                          float* __restrict__ weights /* or null */, float* __restrict__ alpha, float* __restrict__ rgb0,
                           float* __restrict__ disp0, float* __restrict__ acc0, float* __restrict__ z_samples,
                           float* __restrict__ z_all, int* __restrict__ order_out, int* __restrict__ inds_out,
                           int smooth /* 1: single_net weights (is_only, ray_utils.py:272-279); 0: the interior weights */) {
-    __shared__ RaySmem smem[kWarpsPerBlock];
-    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-    const int n = blockIdx.x * kWarpsPerBlock + wib;
-    if (n >= n_rays) return;
-    RaySmem& sm = smem[wib];
+    extern __shared__ float dsm[];
+    constexpr int kE = (32 / kL) * kEo;                 // samples per lane
+    const int lane = threadIdx.x & 31, g = lane & (kL - 1), slot = threadIdx.x / kL;
+    const unsigned gmask = group_mask<kL>(lane);
+    const int n_slot = blockIdx.x * (blockDim.x / kL) + slot;
+    const bool valid = n_slot < n_rays;
+    const int n = valid ? n_slot : n_rays - 1;
+    float* sz = dsm + (size_t)slot * (3 * S + 3 * S_f);
+    float* sw = sz + S;
+    float* scdf = sw + S;
+    float* szs = scdf + S;
+    float* sfz = szs + S_f;
+    int* sfi = reinterpret_cast<int*>(sfz + S_f);
     const float* r = rays + (size_t)n * ray_stride;
     const float norm_d = __fsqrt_rn(__fadd_rn(__fadd_rn(__fmul_rn(r[3], r[3]), __fmul_rn(r[4], r[4])), __fmul_rn(r[5], r[5])));
-    for (int i = lane; i < S; i += 32) sm.z[i] = z[(size_t)n * S + i];
-    __syncwarp();
+    for (int i = g; i < S; i += kL) sz[i] = z[(size_t)n * S + i];
+    __syncwarp(gmask);
     const float4* raw4 = reinterpret_cast<const float4*>(raw);
     const float4 empty = raw4[(size_t)n_rays * S + n];
+    // the raw row is read only for an active sample: DANBO's coarse masks are sparse, and an inactive row would cost 16 B
     auto fetch = [&](int i) { return mask[(size_t)n * S + i] ? raw4[(size_t)n * S + i] : empty; };
-    composite_ray<kE>(sm, S, lane, norm_d, inv_B, noise ? noise + (size_t)n * S : nullptr, fetch,
-                      weights + (size_t)n * S, alpha + (size_t)n * S, rgb0 + (size_t)n * 3, disp0 + n, acc0 + n);
+    composite_group<kL, kEo>(sz, S, g, gmask, valid, norm_d, inv_B, noise ? noise + (size_t)n * S : nullptr, fetch,
+                             S_f > 0 ? sw : nullptr, weights ? weights + (size_t)n * S : nullptr, alpha + (size_t)n * S,
+                             rgb0 + (size_t)n * 3, disp0 + n, acc0 + n);
     if (S_f <= 0) return;
-    // ---- R1: pdf over the S-2 interior bins, cdf with a leading zero (ray_utils.py:161-164,272-279)
+    // ---- R1: pdf over the S-2 interior bins, cdf with a leading zero (ray_utils.py:161-164,272-279); lane g holds the
+    // contiguous bins g*K .. g*K + K - 1
     const int nb = S - 2;
-    const int epl = (nb + 31) / 32;                     // <= kE
+    const int K = (nb + kL - 1) / kL;                   // <= kE
     float dw[kE];
     double lsum = 0.0;
 #pragma unroll
     for (int e = 0; e < kE; ++e) {
-        const int k = lane * epl + e;
+        const int k = g * K + e;
         dw[e] = 0.f;
-        if (e < epl && k < nb) {
+        if (e < K && k < nb) {
             if (smooth) {
-                const float a = fmaxf(sm.w[k], sm.w[k + 1]), b = fmaxf(sm.w[k + 1], sm.w[k + 2]);
+                const float a = fmaxf(sw[k], sw[k + 1]), b = fmaxf(sw[k + 1], sw[k + 2]);
                 dw[e] = __fadd_rn(__fadd_rn(__fmul_rn(0.5f, __fadd_rn(a, b)), 0.01f), 1e-5f);
             } else {
-                dw[e] = __fadd_rn(sm.w[k + 1], 1e-5f);                     // weights[..., 1:-1] + 1e-5 (sample_pdf)
+                dw[e] = __fadd_rn(sw[k + 1], 1e-5f);                        // weights[..., 1:-1] + 1e-5 (sample_pdf)
             }
             lsum += (double)dw[e];
         }
     }
-    double tot = lsum;
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) tot += __shfl_xor_sync(0xffffffffu, tot, o);
-    const float total = (float)tot;
+    const float total = (float)group_sum<kL>(lsum);
     double lpdf = 0.0;
 #pragma unroll
     for (int e = 0; e < kE; ++e) {
-        const int k = lane * epl + e;
-        if (e < epl && k < nb) { dw[e] = __fdiv_rn(dw[e], total); lpdf += (double)dw[e]; }
+        const int k = g * K + e;
+        if (e < K && k < nb) { dw[e] = __fdiv_rn(dw[e], total); lpdf += (double)dw[e]; }
     }
-    double run = warp_excl_sum(lpdf, lane);
-    if (lane == 0) sm.cdf[0] = 0.f;
+    const double inc = group_incl_sum<kL>(lpdf, g);
+    const double ex = __shfl_up_sync(0xffffffffu, inc, 1, kL);
+    double run = g == 0 ? 0.0 : ex;
+    if (g == 0) scdf[0] = 0.f;
 #pragma unroll
     for (int e = 0; e < kE; ++e) {
-        const int k = lane * epl + e;
-        if (e < epl && k < nb) { run += (double)dw[e]; sm.cdf[k + 1] = (float)run; }
+        const int k = g * K + e;
+        if (e < K && k < nb) { run += (double)dw[e]; scdf[k + 1] = (float)run; }
     }
-    __syncwarp();
+    __syncwarp(gmask);
     const int n_cdf = S - 1;
-    for (int j = lane; j < S_f; j += 32) {
+    for (int j = g; j < S_f; j += kL) {
         const float u = u_rand ? u_rand[(size_t)n * S_f + j] : u_vals[j];
         // searchsorted(cdf, u, right=True) = #{k : cdf[k] <= u}; the cdf is non-decreasing (a running sum of
         // non-negative terms), so the count is the first index with cdf > u: binary search
         int lo = 0, hi = n_cdf;
-        while (lo < hi) { const int mid = (lo + hi) >> 1; if (sm.cdf[mid] <= u) lo = mid + 1; else hi = mid; }
+        while (lo < hi) { const int mid = (lo + hi) >> 1; if (scdf[mid] <= u) lo = mid + 1; else hi = mid; }
         const int ind = lo;
         const int below = ind - 1 > 0 ? ind - 1 : 0;
         const int above = ind < n_cdf - 1 ? ind : n_cdf - 1;
-        const float cb = sm.cdf[below], ca = sm.cdf[above];
-        const float bb = __fmul_rn(.5f, __fadd_rn(sm.z[below + 1], sm.z[below]));
-        const float ba = __fmul_rn(.5f, __fadd_rn(sm.z[above + 1], sm.z[above]));
+        const float cb = scdf[below], ca = scdf[above];
+        const float bb = __fmul_rn(.5f, __fadd_rn(sz[below + 1], sz[below]));
+        const float ba = __fmul_rn(.5f, __fadd_rn(sz[above + 1], sz[above]));
         float den = __fsub_rn(ca, cb);
         if (den < 1e-5f) den = 1.f;
         const float t = __fdiv_rn(__fsub_rn(u, cb), den);
         const float zsv = __fadd_rn(bb, __fmul_rn(t, __fsub_rn(ba, bb)));
-        sm.zs[j] = zsv;
-        z_samples[(size_t)n * S_f + j] = zsv;
-        if (inds_out) inds_out[(size_t)n * S_f + j] = ind;
+        szs[j] = zsv;
+        if (valid) {
+            z_samples[(size_t)n * S_f + j] = zsv;
+            if (inds_out) inds_out[(size_t)n * S_f + j] = ind;
+        }
     }
-    __syncwarp();
-    // ---- sorted merge of [z ; z_samples] (stable: ties keep concatenation order)
+    __syncwarp(gmask);
+    // ---- stable merge of [z ; z_samples] (ties keep concatenation order).  The rank of element i is
+    //   #{k : cat[k] < cat[i] or (cat[k] == cat[i] and k < i)}.
+    // With z non-decreasing (every sampler's output) and the fine samples stably sorted by (value, index) into fz / fi,
+    //   coarse i: i + #{fine < z_i}        fine at sorted position p: #{z <= fz[p]} + p
+    // by one binary search each.  Eval draws sorted u, so the fine samples are already in order; train mode draws a
+    // random u per ray, and its fine samples are sorted by counting, O(S_f) per sample.  Both checks vote per ray.
     const int St = S + S_f;
-    for (int i = lane; i < St; i += 32) sm.cat[i] = i < S ? sm.z[i] : sm.zs[i - S];
-    __syncwarp();
-    // rank of element i in the stable sort = #{k : cat[k] < cat[i] or (cat[k] == cat[i] and k < i)}.  When both halves are
-    // already non-decreasing (always for z; for z_samples whenever u is sorted, i.e. eval) this is
-    //   coarse i: i + #{z_samples < z_i}        fine j: S + j' ... = #{z <= zs_j} + j
-    // by two binary searches; otherwise (train mode, random u) the general count.  Checked per ray, so exact either way.
-    bool sorted = true;
-    for (int i = lane; i < St; i += 32)
-        if (i + 1 < St && i + 1 != S) sorted = sorted && !(sm.cat[i + 1] < sm.cat[i]);
-    sorted = __all_sync(0xffffffffu, sorted);
-    if (sorted) {
-        for (int i = lane; i < St; i += 32) {
-            const float v = sm.cat[i];
-            int rank;
-            if (i < S) {
-                int lo = 0, hi = S_f;                               // first fine index with zs >= v
-                while (lo < hi) { const int mid = (lo + hi) >> 1; if (sm.zs[mid] < v) lo = mid + 1; else hi = mid; }
-                rank = i + lo;
-            } else {
-                int lo = 0, hi = S;                                 // first coarse index with z > v
-                while (lo < hi) { const int mid = (lo + hi) >> 1; if (sm.z[mid] <= v) lo = mid + 1; else hi = mid; }
-                rank = lo + (i - S);
-            }
-            sm.order[rank] = i;
-        }
-    } else {
-        for (int i = lane; i < St; i += 32) {
-            const float v = sm.cat[i];
+    int* out_o = order_out + (size_t)n * St;
+    float* out_z = z_all + (size_t)n * St;
+    bool z_ok = true, zs_ok = true;
+    for (int i = g; i + 1 < S; i += kL) z_ok = z_ok && !(sz[i + 1] < sz[i]);
+    for (int j = g; j + 1 < S_f; j += kL) zs_ok = zs_ok && !(szs[j + 1] < szs[j]);
+    const unsigned z_bad = __ballot_sync(gmask, !z_ok) & gmask, zs_bad = __ballot_sync(gmask, !zs_ok) & gmask;
+    if (z_bad) {                                        // coarse z out of order (no sampler produces it): the plain count
+        for (int i = g; i < St; i += kL) {
+            const float v = i < S ? sz[i] : szs[i - S];
             int rank = 0;
-            for (int k = 0; k < St; ++k) { const float c = sm.cat[k]; rank += (c < v || (c == v && k < i)) ? 1 : 0; }
-            sm.order[rank] = i;
+            for (int k = 0; k < St; ++k) { const float c = k < S ? sz[k] : szs[k - S]; rank += (c < v || (c == v && k < i)) ? 1 : 0; }
+            if (valid) { out_o[rank] = i; out_z[rank] = v; }
         }
+        return;
     }
-    __syncwarp();
-    for (int i = lane; i < St; i += 32) {
-        const int src = sm.order[i];
-        order_out[(size_t)n * St + i] = src;
-        z_all[(size_t)n * St + i] = sm.cat[src];
+    const float* fz = szs;
+    const int* fi = nullptr;
+    if (zs_bad) {
+        for (int j = g; j < S_f; j += kL) {
+            const float v = szs[j];
+            int p = 0;
+            for (int k = 0; k < S_f; ++k) { const float c = szs[k]; p += (c < v || (c == v && k < j)) ? 1 : 0; }
+            sfz[p] = v;
+            sfi[p] = j;
+        }
+        __syncwarp(gmask);
+        fz = sfz;
+        fi = sfi;
+    }
+    for (int i = g; i < St; i += kL) {
+        float v;
+        int rank, src;
+        if (i < S) {
+            v = sz[i];
+            int lo = 0, hi = S_f;                               // first fine sample >= v
+            while (lo < hi) { const int mid = (lo + hi) >> 1; if (fz[mid] < v) lo = mid + 1; else hi = mid; }
+            rank = i + lo;
+            src = i;
+        } else {
+            const int p = i - S;
+            v = fz[p];
+            int lo = 0, hi = S;                                 // first coarse sample > v
+            while (lo < hi) { const int mid = (lo + hi) >> 1; if (sz[mid] <= v) lo = mid + 1; else hi = mid; }
+            rank = lo + p;
+            src = S + (fi ? fi[p] : p);
+        }
+        if (valid) { out_o[rank] = src; out_z[rank] = v; }
     }
 }
 
-// Fine pass: gather coarse / fine raw by merge order, composite the S_t samples.
-template <int kE>
+// Fine pass: gather coarse / fine raw by merge order, composite the S_t samples.  No shared memory: z and the merge order
+// are read from their rows in global memory.
+template <int kL, int kEo>
 __global__ void __launch_bounds__(32 * kWarpsPerBlock)
 merge_composite_kernel(const float* __restrict__ rays, int ray_stride, int n_rays, int S_c, int S_f,
                        const float* __restrict__ raw0 /* (n_rays*S_c + n_rays, 4) */, const uint32_t* __restrict__ mask0,
@@ -236,33 +327,35 @@ merge_composite_kernel(const float* __restrict__ rays, int ray_stride, int n_ray
                        float* __restrict__ disp, float* __restrict__ acc, float* __restrict__ raw_merged /* (n,St,4) or null */,
                        const float* __restrict__ confd0, const float* __restrict__ confd1,
                        float* __restrict__ confd_merged /* (n,St,24) or null */, float* __restrict__ invalid_merged /* or null */) {
-    __shared__ RaySmem smem[kWarpsPerBlock];
-    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-    const int n = blockIdx.x * kWarpsPerBlock + wib;
-    if (n >= n_rays) return;
-    RaySmem& sm = smem[wib];
+    const int lane = threadIdx.x & 31, g = lane & (kL - 1), slot = threadIdx.x / kL;
+    const unsigned gmask = group_mask<kL>(lane);
+    const int n_slot = blockIdx.x * (blockDim.x / kL) + slot;
+    const bool valid = n_slot < n_rays;
+    const int n = valid ? n_slot : n_rays - 1;
     const int St = S_c + S_f;
     const float* r = rays + (size_t)n * ray_stride;
     const float norm_d = __fsqrt_rn(__fadd_rn(__fadd_rn(__fmul_rn(r[3], r[3]), __fmul_rn(r[4], r[4])), __fmul_rn(r[5], r[5])));
-    for (int i = lane; i < St; i += 32) { sm.z[i] = z_all[(size_t)n * St + i]; sm.order[i] = order[(size_t)n * St + i]; }
-    __syncwarp();
+    const int* ord = order + (size_t)n * St;
     const float4* r0 = reinterpret_cast<const float4*>(raw0);
     const float4* r1 = reinterpret_cast<const float4*>(raw1);
     const float4 empty = r0[(size_t)n_rays * S_c + n];
     auto fetch = [&](int i) {
-        const int src = sm.order[i];
-        float4 v;
-        if (src < S_c) v = mask0[(size_t)n * S_c + src] ? r0[(size_t)n * S_c + src] : empty;
-        else           v = mask1[(size_t)n * S_f + src - S_c] ? r1[(size_t)n * S_f + src - S_c] : empty;
-        if (raw_merged) reinterpret_cast<float4*>(raw_merged)[(size_t)n * St + i] = v;
+        const int src = ord[i];
+        const bool coarse = src < S_c;
+        const size_t sidx = coarse ? (size_t)n * S_c + src : (size_t)n * S_f + src - S_c;
+        const uint32_t m = (coarse ? mask0 : mask1)[sidx];  // mask and raw loads issue together; an inactive row is dropped
+        const float4 raw = (coarse ? r0 : r1)[sidx];
+        const float4 v = m ? raw : empty;
+        if (raw_merged && valid) reinterpret_cast<float4*>(raw_merged)[(size_t)n * St + i] = v;
         return v;
     };
-    composite_ray<kE>(sm, St, lane, norm_d, inv_B, noise ? noise + (size_t)n * St : nullptr, fetch,
-                      weights + (size_t)n * St, alpha + (size_t)n * St, rgb + (size_t)n * 3, disp + n, acc + n);
-    if (confd_merged || invalid_merged) {                          // training outputs (raycasters.py:710-716)
-        for (int e = lane; e < St * DANBO_J; e += 32) {
+    composite_group<kL, kEo>(z_all + (size_t)n * St, St, g, gmask, valid, norm_d, inv_B,
+                             noise ? noise + (size_t)n * St : nullptr, fetch, nullptr, weights + (size_t)n * St,
+                             alpha + (size_t)n * St, rgb + (size_t)n * 3, disp + n, acc + n);
+    if ((confd_merged || invalid_merged) && valid) {       // training outputs (raycasters.py:710-716)
+        for (int e = g; e < St * DANBO_J; e += kL) {
             const int i = e / DANBO_J, j = e - i * DANBO_J;
-            const int src = sm.order[i];
+            const int src = ord[i];
             const bool coarse = src < S_c;
             const size_t sidx = coarse ? (size_t)n * S_c + src : (size_t)n * S_f + src - S_c;
             const uint32_t m = coarse ? mask0[sidx] : mask1[sidx];
@@ -277,19 +370,26 @@ merge_composite_kernel(const float* __restrict__ rays, int ray_stride, int n_ray
 
 using namespace danbo;
 
+// Lanes per ray of each launcher, indexed by kEo - 1 = ceil(S / 32) - 1.  Each entry is the fastest of 8, 16 and 32 lanes
+// on the B200 for that kernel and sample count (scripts/composite_lanes_bench.py, DESIGN §4).
+constexpr int kCrLanes[5] = {8, 16, 16, 32, 32};
+constexpr int kMcLanes[5] = {8, 16, 32, 32, 32};
+
 extern "C" int danbo_composite_resample(const float* rays, int ray_stride, int n_rays, int S, int S_f, const float* raw,
                                         const unsigned int* mask, const float* z, const float* noise, float inv_B,
                                         const float* u_vals, const float* u_rand, float* weights, float* alpha,
                                         float* rgb0, float* disp0, float* acc0, float* z_samples, float* z_all,
                                         int* order, int* inds, int smooth_weights, void* stream) {
     if (n_rays <= 0) return 0;
-    if (S < 3 || S > kMaxS || S + S_f > kMaxS) return -1;
+    if (S < 3 || S > kMaxS || S_f < 0 || S + S_f > kMaxS) return -1;
     if (S_f > 0 && !u_vals && !u_rand) return -2;
-    const int G = (n_rays + kWarpsPerBlock - 1) / kWarpsPerBlock;
-#define DANBO_CR_LAUNCH(E) composite_resample_kernel<E><<<G, 32 * kWarpsPerBlock, 0, (cudaStream_t)stream>>>( \
+    const size_t smem_per_ray = (size_t)(3 * S + 3 * S_f) * sizeof(float);
+#define DANBO_CR_LAUNCH(E) composite_resample_kernel<kCrLanes[E - 1], E>                                              \
+        <<<(n_rays + 32 * kWarpsPerBlock / kCrLanes[E - 1] - 1) / (32 * kWarpsPerBlock / kCrLanes[E - 1]),               \
+           32 * kWarpsPerBlock, 32 * kWarpsPerBlock / kCrLanes[E - 1] * smem_per_ray, (cudaStream_t)stream>>>(           \
         rays, ray_stride, n_rays, S, S_f, raw, mask, z, noise, inv_B, u_vals, u_rand, weights, alpha, rgb0, disp0, acc0, \
         z_samples, z_all, order, inds, smooth_weights)
-    switch ((S + 31) / 32) {                                 // samples per lane: the kernel is specialised on it
+    switch ((S + 31) / 32) {                                 // samples per virtual lane: the kernel is specialised on it
         case 1: DANBO_CR_LAUNCH(1); break;
         case 2: DANBO_CR_LAUNCH(2); break;
         case 3: DANBO_CR_LAUNCH(3); break;
@@ -309,9 +409,10 @@ extern "C" int danbo_merge_composite(const float* rays, int ray_stride, int n_ra
                                      float* invalid_merged, void* stream) {
     if (n_rays <= 0) return 0;
     if (S_c + S_f > kMaxS) return -1;
-    const int G = (n_rays + kWarpsPerBlock - 1) / kWarpsPerBlock;
-#define DANBO_MC_LAUNCH(E) merge_composite_kernel<E><<<G, 32 * kWarpsPerBlock, 0, (cudaStream_t)stream>>>( \
-        rays, ray_stride, n_rays, S_c, S_f, raw0, mask0, raw1, mask1, z_all, order, noise, inv_B, weights, alpha, rgb, \
+#define DANBO_MC_LAUNCH(E) merge_composite_kernel<kMcLanes[E - 1], E>                                                 \
+        <<<(n_rays + 32 * kWarpsPerBlock / kMcLanes[E - 1] - 1) / (32 * kWarpsPerBlock / kMcLanes[E - 1]),               \
+           32 * kWarpsPerBlock, 0, (cudaStream_t)stream>>>(                                                              \
+        rays, ray_stride, n_rays, S_c, S_f, raw0, mask0, raw1, mask1, z_all, order, noise, inv_B, weights, alpha, rgb,  \
         disp, acc, raw_merged, confd0, confd1, confd_merged, invalid_merged)
     switch ((S_c + S_f + 31) / 32) {
         case 1: DANBO_MC_LAUNCH(1); break;

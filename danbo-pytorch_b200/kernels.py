@@ -336,15 +336,18 @@ def mlp_forward(xtiles, packed, rbias, active, row_ray, out, density_only=False,
     return out
 
 
-def composite_resample(rays, S, S_f, raw, mask, z, noise=None, inv_B=1.0, u_rand=None, want_inds=False, smooth=True):
+def composite_resample(rays, S, S_f, raw, mask, z, noise=None, inv_B=1.0, u_rand=None, want_inds=False, smooth=True,
+                       want_weights=True):
     """C1 + R1 on the coarse samples.  raw (n*S+n,4).  -> dict.  smooth: single_net importance weights (is_only);
-    S_f = 0: compositing only."""
+    S_f = 0: compositing only.  want_weights=False: no "weights" entry, and the (n, S) weight row is not written."""
     _need_cuda(rays, raw, mask, z, noise, u_rand)
     lib = _lib.load()
     n = rays.shape[0]
     dev = rays.device
     f = lambda *s: torch.empty(*s, device=dev, dtype=torch.float32)
-    out = {"weights": f(n, S), "alpha": f(n, S), "rgb_map": f(n, 3), "disp_map": f(n), "acc_map": f(n)}
+    out = {"alpha": f(n, S), "rgb_map": f(n, 3), "disp_map": f(n), "acc_map": f(n)}
+    if want_weights:
+        out["weights"] = f(n, S)
     u_vals = None
     if S_f > 0:
         out["z_samples"], out["z_all"] = f(n, S_f), f(n, S + S_f)
@@ -355,7 +358,7 @@ def composite_resample(rays, S, S_f, raw, mask, z, noise=None, inv_B=1.0, u_rand
             u_vals = _linspace01(S_f, dev.index if dev.index is not None else torch.cuda.current_device())
     with _Timed("composite_resample"):
         _lib.check(lib.danbo_composite_resample(_p(rays), rays.stride(0), n, S, S_f, _p(raw), _p(mask), _p(z), _p(noise),
-                                                float(inv_B), _p(u_vals), _p(u_rand), _p(out["weights"]), _p(out["alpha"]),
+                                                float(inv_B), _p(u_vals), _p(u_rand), _p(out.get("weights")), _p(out["alpha"]),
                                                 _p(out["rgb_map"]), _p(out["disp_map"]), _p(out["acc_map"]),
                                                 _p(out.get("z_samples")), _p(out.get("z_all")), _p(out.get("order")),
                                                 _p(out.get("inds")), int(bool(smooth)), _stream()), "danbo_composite_resample")

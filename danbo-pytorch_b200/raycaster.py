@@ -357,7 +357,7 @@ class RayCaster(nn.Module):
             K.mlp_forward(f0.xtiles, packed, rbias, act0, f0.row_ray, raw0)
         noise0 = (rand["noise0"] * (raw_noise_std * B)).contiguous() if ("noise0" in rand and raw_noise_std > 0) else None
         c0 = K.composite_resample(rays, S_c, S_f, raw0, mask0, z0, noise=noise0, inv_B=inv_B, u_rand=rand.get("u"),
-                                  want_inds=stages is not None)
+                                  want_inds=stages is not None, want_weights=stages is not None)
         if "z_fine" in rand:
             # test hook: evaluate the fine pass at given importance samples (z_fine, z_all, order as the reference
             # produced them) instead of this pass's own - cuts the coarse -> fine coupling for stage-wise parity checks

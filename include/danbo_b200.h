@@ -137,7 +137,7 @@ int danbo_mlp_set_cta_pair(int enable);
  * read the ray's empty entry.  noise (n,S) already scaled, or NULL.  u_vals = linspace(0,1,S_f) (eval) or u_rand
  * (n,S_f) (train).  order (n,S+S_f) int32 = sorted_idxs.  smooth_weights 1: the single_net importance weights
  * (is_only: 0.5 (max(w_k-1, w_k) + max(w_k, w_k+1)) + 0.01); 0: the interior weights themselves (separate fine network,
- * raycasters.py:348).  S_f = 0 composites only. */
+ * raycasters.py:348).  S_f = 0 composites only.  weights may be NULL: the (n,S) weight row is then not written. */
 int danbo_composite_resample(const float* rays, int ray_stride, int n_rays, int S, int S_f, const float* raw,
                              const unsigned int* mask, const float* z, const float* noise, float inv_B,
                              const float* u_vals, const float* u_rand, float* weights, float* alpha, float* rgb0,
