@@ -3,10 +3,11 @@
 `AnerfField` owns the parameters under the reference's names (core/networks/nerf.py:73-105 with W = 448, view_W = 224,
 plus the cutoff embedders' `cutoff_dist` / `tau` entries, cutoff_embedder.py:128-133) so reference checkpoints load.
 `AnerfCaster` mirrors raycasters.py:205-546 for this network type: cylinder near/far only (:419-420), every sample
-goes through the field, single_net fine pass on the S_f new samples (F9).  Train mode (single_net configs): the forward
-keeps every layer's activation tile image (`danbo_anerf_mlp_save`) and `_AnerfBlock.backward` turns d (rgb, acc) into the
-MLP / frame-code gradients with the compositing backward kernels and `kernels.anerf_mlp_backward`; when the poses require
-a gradient (--opt_pose) it also returns d loss / d skts through `kernels.anerf_embed_bwd`.
+goes through the field, single_net fine pass on the S_f new samples (F9), or a separate fine network on all S_c + S_f
+merged samples (anerf_h).  Train mode: the forward keeps every layer's activation tile image (`danbo_anerf_mlp_save`)
+and `_AnerfBlock.backward` turns d (rgb, acc) into the MLP / frame-code gradients of each network with the compositing
+backward kernels and `kernels.anerf_mlp_backward`; when the poses require a gradient (--opt_pose) it also returns
+d loss / d skts through `kernels.anerf_embed_bwd`.
 """
 import torch
 import torch.nn as nn
@@ -138,10 +139,11 @@ class AnerfCaster(RayCaster):
                     "u": torch.rand(N, N_importance, device=dev), "noise1": torch.randn(N, S_t, device=dev)}
         rand = {k: v.to(dev).contiguous() for k, v in rand.items()}
         if self.training and torch.is_grad_enabled():
+            # rows the networks evaluate per ray: a separate fine network runs on all S_c + S_f merged samples
+            rows = N_samples + (N_samples + N_importance if not self.single_net else N_importance)
+            max_train = max(MAX_RAYS_PER_LAUNCH * 24 // rows // 4096, 1) * 4096
             if not self.single_net:
-                raise NotImplementedError("training with a separate fine network (single_net=False, anerf_h.txt) is not "
-                                          "implemented: the backward pass covers the single_net configs")
-            max_train = max(MAX_RAYS_PER_LAUNCH * 24 // (N_samples + N_importance) // 4096, 1) * 4096
+                self._packed_mlp(self.network_fine)         # the unconditional train-mode pack, as for the coarse network
             if N > max_train:
                 raise NotImplementedError(f"A-NeRF training batches above {max_train} rays are not implemented")
             return _anerf_block_with_grad(self, rays, skip, pose_skts, pose_cyls, cam_idx, codes, align, packed, tau,
@@ -199,8 +201,13 @@ class AnerfCaster(RayCaster):
         c0 = K.composite_resample(rays, S_c, S_f, raw0, ones0, z0, noise=noise0, inv_B=inv_B, u_rand=rand.get("u"),
                                   want_inds=stages is not None, smooth=self.single_net, want_weights=stages is not None)
         z1 = c0["z_samples"]
+        if save:
+            keep.update(dict(rays=rays, cam_idx=cam_idx, codes=codes, code_bias=code_bias, S_c=S_c, S_f=S_f, inv_B=inv_B,
+                             z0=z0, raw0=raw0, ones0=ones0, noise0=noise0, xd0=xd, xv0=xv, sv0=sv0, ray_enc=enc,
+                             p_skts=p_skts, skip=skip, align=align, tau=tau))
         if not self.single_net:
-            return self._fine_network_pass(rays, p_skts, skip, cam_idx, align, S_c, S_f, B, c0, near, far, z0, raw0, stages)
+            return self._fine_network_pass(rays, p_skts, skip, cam_idx, align, S_c, S_f, B, c0, near, far, z0, raw0, stages,
+                                           rand=rand, raw_noise_std=raw_noise_std, keep=keep)
         if save:                                             # the coarse pass's operand images are read again by the backward
             xd1, xv1 = K.anerf_embed(rays, S_f, z1, p_skts, skip, align, enc, tau)
         else:
@@ -213,10 +220,8 @@ class AnerfCaster(RayCaster):
         c1 = K.merge_composite(rays, S_c, S_f, raw0, ones0, raw1, ones1, c0["z_all"], c0["order"], noise=noise1,
                                inv_B=inv_B, want_raw=stages is not None)
         if save:
-            keep.update(dict(rays=rays, cam_idx=cam_idx, codes=codes, code_bias=code_bias, S_c=S_c, S_f=S_f, inv_B=inv_B,
-                             z0=z0, raw0=raw0, ones0=ones0, noise0=noise0, xd0=xd, xv0=xv, sv0=sv0, raw1=raw1, ones1=ones1,
-                             noise1=noise1, xd1=xd1, xv1=xv1, sv1=sv1, z_all=c0["z_all"], order=c0["order"],
-                             z1=z1, ray_enc=enc, p_skts=p_skts, skip=skip, align=align, tau=tau))
+            keep.update(dict(raw1=raw1, ones1=ones1, noise1=noise1, xd1=xd1, xv1=xv1, sv1=sv1, z_all=c0["z_all"],
+                             order=c0["order"], z1=z1))
         ret = {"rgb_map": c1["rgb_map"], "disp_map": c1["disp_map"], "acc_map": c1["acc_map"], "alpha": c1["alpha"],
                "T_i": c1["weights"], "rgb0": c0["rgb_map"], "disp0": c0["disp_map"], "acc0": c0["acc_map"],
                "alpha0": c0["alpha"]}
@@ -226,19 +231,30 @@ class AnerfCaster(RayCaster):
                            "raw": c1.get("raw"), "ray_enc": enc, "code_bias": code_bias})
         return ret
 
-    def _fine_network_pass(self, rays, p_skts, skip, cam_idx, align, S_c, S_f, B, c0, near, far, z0, raw0, stages):
-        """single_net=False (raycasters.py:350-376): the fine network on all S_c + S_f merged samples, then raw2outputs."""
+    def _fine_network_pass(self, rays, p_skts, skip, cam_idx, align, S_c, S_f, B, c0, near, far, z0, raw0, stages,
+                           rand=None, raw_noise_std=0., keep=None):
+        """single_net=False (raycasters.py:350-376): the fine network on all S_c + S_f merged samples, then raw2outputs
+        (with the train-mode density noise `noise1`, as raw2outputs adds it whenever raw_noise_std > 0).  keep: as in
+        _render_block_anerf."""
+        rand = rand or {}
         n, dev = rays.shape[0], rays.device
         fine = self.network_fine
         S_t = S_c + S_f
         packed_f = self._packed_mlp(fine)
-        enc_f, code_bias_f = K.anerf_ray_encode(rays, p_skts, skip, cam_idx, self._codes_of(fine), packed_f)
+        codes_f, tau_f = self._codes_of(fine), self._tau(fine)
+        enc_f, code_bias_f = K.anerf_ray_encode(rays, p_skts, skip, cam_idx, codes_f, packed_f)
         z_all = c0["z_all"]
-        xd, xv = K.anerf_embed(rays, S_t, z_all, p_skts, skip, align, enc_f, self._tau(fine))
+        xd, xv = K.anerf_embed(rays, S_t, z_all, p_skts, skip, align, enc_f, tau_f)
         raw = torch.empty(n * S_t + n, 4, device=dev, dtype=torch.float32)       # tail rows: unused empty entries
-        K.anerf_mlp(xd, xv, packed_f, code_bias_f, n * S_t, S_t, raw)
+        sv = K.anerf_save_buffer(n * S_t, dev) if keep is not None else None
+        K.anerf_mlp(xd, xv, packed_f, code_bias_f, n * S_t, S_t, raw, save=sv)
         ones = torch.ones(n, S_t, device=dev, dtype=torch.int32)
-        c1 = K.composite_resample(rays, S_t, 0, raw, ones, z_all, inv_B=1.0 / B)
+        inv_B = 1.0 / B
+        noise1 = (rand["noise1"] * (raw_noise_std * B)).contiguous() if ("noise1" in rand and raw_noise_std > 0) else None
+        c1 = K.composite_resample(rays, S_t, 0, raw, ones, z_all, noise=noise1, inv_B=inv_B)
+        if keep is not None:
+            keep.update(dict(raw_f=raw, ones_f=ones, z_all=z_all, noise1=noise1, xd_f=xd, xv_f=xv, sv_f=sv,
+                             code_bias_f=code_bias_f, codes_f=codes_f, ray_enc_f=enc_f, tau_f=tau_f))
         ret = {"rgb_map": c1["rgb_map"], "disp_map": c1["disp_map"], "acc_map": c1["acc_map"], "alpha": c1["alpha"],
                "T_i": c1["weights"], "rgb0": c0["rgb_map"], "disp0": c0["disp_map"], "acc0": c0["acc_map"],
                "alpha0": c0["alpha"]}
@@ -292,7 +308,8 @@ class _AnerfBlock(torch.autograd.Function):
     backward kernels (composite.cu) + kernels.anerf_mlp_backward.  Differentiable outputs are what the trainer's losses
     read (core/trainer.py:396-422): rgb_map, acc_map, rgb0, acc0.  The per-pose world-to-bone matrices are an input:
     when they require a gradient (the pose layer under --opt_pose, core/trainer.py:314-341) each pass also forms the MLP's
-    input gradient and `danbo_anerf_embed_bwd` turns it into d loss / d skts."""
+    input gradient and `danbo_anerf_embed_bwd` turns it into d loss / d skts.  `params`: the 25 tensors of the network in
+    ANERF_PARAM_NAMES order, then those of a separate fine network (single_net=False)."""
 
     @staticmethod
     def forward(ctx, caster, cfg, pose_skts, *params):
@@ -316,33 +333,54 @@ class _AnerfBlock(torch.autograd.Function):
         cg = lambda t, *s: zeros(*s) if t is None else t.contiguous().float()
         P = dict(zip(ANERF_PARAM_NAMES, ctx.params))
         G = {name: torch.zeros_like(p, dtype=torch.float32) for name, p in P.items()}
-        d_raw0, d_raw1 = zeros(n * S_c + n, 4), zeros(n * S_f, 4)
-        K.merge_composite_bwd(rays, S_c, S_f, k["raw0"], k["ones0"], k["raw1"], k["ones1"], k["z_all"], k["order"],
-                              k["noise1"], k["inv_B"], cg(g["rgb_map"], n, 3), cg(g["acc_map"], n), None, d_raw0, d_raw1,
-                              None, None)
+        separate = "raw_f" in k
+        if separate:
+            # the fine network's composite over all S_t merged samples; the importance samples are detached
+            # (ray_utils.py:287), so the fine outputs reach only the fine network and the coarse outputs only the coarse
+            S_t = S_c + S_f
+            P_f = dict(zip(ANERF_PARAM_NAMES, ctx.params[len(ANERF_PARAM_NAMES):]))
+            G_f = {name: torch.zeros_like(p, dtype=torch.float32) for name, p in P_f.items()}
+            d_raw_f, d_raw0 = zeros(n * S_t + n, 4), zeros(n * S_c + n, 4)
+            K.composite_bwd(rays, S_t, k["raw_f"], k["ones_f"], k["z_all"], k["noise1"], k["inv_B"], cg(g["rgb_map"], n, 3),
+                            cg(g["acc_map"], n), d_raw_f)
+        else:
+            d_raw0, d_raw1 = zeros(n * S_c + n, 4), zeros(n * S_f, 4)
+            K.merge_composite_bwd(rays, S_c, S_f, k["raw0"], k["ones0"], k["raw1"], k["ones1"], k["z_all"], k["order"],
+                                  k["noise1"], k["inv_B"], cg(g["rgb_map"], n, 3), cg(g["acc_map"], n), None, d_raw0,
+                                  d_raw1, None, None)
         K.composite_bwd(rays, S_c, k["raw0"], k["ones0"], k["z0"], k["noise0"], k["inv_B"], cg(g["rgb0"], n, 3),
                         cg(g["acc0"], n), d_raw0)
         want_pose = ctx.needs_input_grad[2]
         d_skts = zeros(*k["p_skts"].shape) if want_pose else None         # p0 == 0: a training block holds every pose
-        for d_raw, S, z, xd, xv, sv in ((d_raw0, S_c, k["z0"], k["xd0"], k["xv0"], k["sv0"]),
-                                        (d_raw1, S_f, k["z1"], k["xd1"], k["xv1"], k["sv1"])):
-            dx = K.anerf_mlp_backward(P, G, d_raw, n * S, S, xd, xv, sv, k["code_bias"], k["cam_idx"], k["codes"],
-                                      want_dx=want_pose)
+        coarse = (P, G, d_raw0, S_c, k["z0"], k["xd0"], k["xv0"], k["sv0"], k["code_bias"], k["codes"], k["ray_enc"],
+                  k["tau"])
+        if separate:
+            fine = (P_f, G_f, d_raw_f, S_t, k["z_all"], k["xd_f"], k["xv_f"], k["sv_f"], k["code_bias_f"], k["codes_f"],
+                    k["ray_enc_f"], k["tau_f"])
+        else:
+            fine = (P, G, d_raw1, S_f, k["z1"], k["xd1"], k["xv1"], k["sv1"], k["code_bias"], k["codes"], k["ray_enc"],
+                    k["tau"])
+        for Pn, Gn, d_raw, S, z, xd, xv, sv, code_bias, codes, enc, tau in (coarse, fine):
+            dx = K.anerf_mlp_backward(Pn, Gn, d_raw, n * S, S, xd, xv, sv, code_bias, k["cam_idx"], codes, want_dx=want_pose)
             if want_pose:
-                K.anerf_embed_bwd(rays, S, z, k["p_skts"], k["skip"], k["align"], k["ray_enc"], k["tau"], dx[0], dx[1],
-                                  d_skts)
+                K.anerf_embed_bwd(rays, S, z, k["p_skts"], k["skip"], k["align"], enc, tau, dx[0], dx[1], d_skts)
                 del dx
         ctx.keep = None
-        return (None, None, d_skts) + tuple(G[name] for name in ANERF_PARAM_NAMES)
+        grads = tuple(G[name] for name in ANERF_PARAM_NAMES)
+        if separate:
+            grads += tuple(G_f[name] for name in ANERF_PARAM_NAMES)
+        return (None, None, d_skts) + grads
 
 
 def _anerf_block_with_grad(caster, rays, skip, pose_skts, pose_cyls, cam_idx, codes, align, packed, tau, S_c, S_f, B,
                            nanmean_chunk, lindisp, rand, raw_noise_std, stages):
-    named = dict(caster.network.named_parameters())
+    params = [dict(caster.network.named_parameters())[n] for n in ANERF_PARAM_NAMES]
+    if not caster.single_net:
+        params += [dict(caster.network_fine.named_parameters())[n] for n in ANERF_PARAM_NAMES]
     cfg = dict(rays=rays, skip=skip, pose_cyls=pose_cyls, cam_idx=cam_idx, codes=codes, align=align,
                packed=packed, tau=tau, S_c=S_c, S_f=S_f, B=B, nanmean_chunk=nanmean_chunk, lindisp=lindisp, rand=rand,
                raw_noise_std=raw_noise_std, stages=stages)
-    outs = _AnerfBlock.apply(caster, cfg, pose_skts, *[named[n] for n in ANERF_PARAM_NAMES])
+    outs = _AnerfBlock.apply(caster, cfg, pose_skts, *params)
     return dict(zip(ANERF_OUT_KEYS, outs))
 
 

@@ -216,7 +216,15 @@ class TrainStep:
             self.popt["popt_anchors"] = {k: (v.to(dev) if torch.is_tensor(v) else v)
                                          for k, v in self.popt["popt_anchors"].items()}
         self.fused_loss = fused_loss           # False: the trainer's losses as PyTorch ops + autograd (compute_loss)
-        params = [p for p in caster.network.parameters() if p.requires_grad]
+        # create_raycaster's grad_vars order (raycasters.py:188): the network, then a separate fine network.  The bucket,
+        # the optimizer state and so the checkpoints index the reference's Adam over grad_vars.
+        nets = [caster.network]
+        fine = getattr(caster, "network_fine", caster.network)
+        if fine is not caster.network:
+            if graph:
+                raise NotImplementedError("graph capture of a training step with a separate fine network is not implemented")
+            nets.append(fine)
+        params = [p for net in nets for p in net.parameters() if p.requires_grad]
         self.bucket = parallel.GradBucket(params)
         caster.grads_in_place = True            # backward kernels add into the bucket's views (see autograd._RenderBlock)
         caster.network.grads_in_place = True    # ... and so does the graph net's backward (autograd._GraphNet)
