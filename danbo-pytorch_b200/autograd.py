@@ -7,7 +7,8 @@ trainer's losses read (core/trainer.py:396-422,507-536); disp / alpha / T_i / pa
 the reference where they are used only under comparisons.  The per-pose graph net is its own node (`_GraphNet`, or the
 PyTorch ops when the pose itself needs a gradient): its output `vol` is an input of this Function and receives d vol.
 The per-pose world-to-bone matrices are an input too: when they require a gradient (the pose layer under --opt_pose,
-core/trainer.py:314-341) `danbo_field_agg_bwd` also accumulates d loss / d skts.
+core/trainer.py:314-341) `danbo_field_agg_bwd` also accumulates d loss / d skts, and with root-local view directions
+(perfcap configs) `danbo_view_root_bwd` adds the view branch's part.
 """
 import torch
 
@@ -129,15 +130,22 @@ class _RenderBlock(torch.autograd.Function):
                                 agg_grads, d_skts=d_skts)
         if side2 is not None:
             cur.wait_stream(side2)
+        # root-local view directions (perfcap configs) depend on the root rotation: with a pose leaf, d ray_bias also
+        # flows to d skts (adds into the same tensor as field_agg_bwd's atomics)
+        view_root = d_skts is not None and getattr(ctx.caster, "view_mode", "world") == "root_local"
         if side is not None:
             # d_ray_bias is complete once the second pass's head backward has run: the side stream already waits for it
             with torch.cuda.stream(side):
                 K.ray_bias_bwd(k["rays_v"], k["cam_idx"], k["codes"], P["views_linears.0.weight"], d_ray_bias,
                                G["views_linears.0.weight"], G["views_linears.0.bias"], G["framecodes.codes.weight"])
+                if view_root:
+                    K.view_root_bwd(rays, k["p_skts"], k["skip"], P["views_linears.0.weight"], d_ray_bias, d_skts)
             cur.wait_stream(side)
         else:
             K.ray_bias_bwd(k["rays_v"], k["cam_idx"], k["codes"], P["views_linears.0.weight"], d_ray_bias,
                            G["views_linears.0.weight"], G["views_linears.0.bias"], G["framecodes.codes.weight"])
+            if view_root:
+                K.view_root_bwd(rays, k["p_skts"], k["skip"], P["views_linears.0.weight"], d_ray_bias, d_skts)
         ctx.keep = None
         del alive, wss
         if in_place:
@@ -156,9 +164,6 @@ def render_block_with_grad(caster, rays, skip, pose_skts, pose_cyls, vol, cam_id
         named["views_linears.0.weight"] = torch.nn.functional.pad(named["views_linears.0.weight"], (0, 128))
         named["framecodes.codes.weight"] = torch.zeros(1, 128, device=rays.device)
     params = [named[n] for n in PARAM_NAMES]
-    if pose_skts.requires_grad and getattr(caster, "view_mode", "world") != "world":
-        raise NotImplementedError("pose gradients with root-local view directions (perfcap configs): the view branch's "
-                                  "dependence on the root rotation is not differentiated")
     cfg = dict(rays=rays, skip=skip, pose_cyls=pose_cyls, cam_idx=cam_idx, codes=codes, consts=consts,
                packed=packed, S_c=S_c, S_f=S_f, B=B, raw_noise_std=raw_noise_std, perturb=perturb,
                nanmean_chunk=nanmean_chunk, rand=rand, stages=stages, lindisp=lindisp)

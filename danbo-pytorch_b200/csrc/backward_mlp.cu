@@ -7,6 +7,7 @@
 //   gemm_wgrad      : dW[M x N] += A[rows x M]^T . B[rows x N], split over rows, fp32 atomics
 //   colsum          : bias gradients
 //   ray_bias_bwd    : grads of views_linears.0[:, 256:], its bias and the frame codes
+//   view_root_bwd   : d skts of the root rotation through root-local view directions (perfcap configs, --opt_pose)
 // All row counts are device scalars (the active counters), so nothing synchronises with the host.
 // Training batches hold ~4e4 active rows, so these are launch/latency bound; the tensor-core (tcgen05) versions are the
 // next step once the training step is correct end to end (DESIGN.md §Backward).
@@ -307,6 +308,118 @@ ray_bias_bwd_kernel(const float* __restrict__ rays, int ray_stride, int n_rays, 
         if (i < nc) atomicAdd(d_w_view + (size_t)o * 411 + 256 + c0 + i, acc[i]);
 }
 
+// V1 backward to the root rotation (perfcap configs: ray_tr_type=root_local + view_type=relray, pose refinement).  There
+// the view branch encodes dn = normalize(m), m = R0 d_ray, R0 = skts[pose, 0, :3, :3] (RootLocalEncoder
+// encoders.py:570-578, VecNormEncoder :774-795), and PE(dn) = [dn, sin(2^f dn), cos(2^f dn)]_{f<4} meets columns 256..282
+// of W_v.  Per ray:
+//   g = W_v[:, 256:283]^T d_ray_bias,   d dn_a = g_a + sum_f 2^f (g_sin,f,a cos(2^f dn_a) - g_cos,f,a sin(2^f dn_a)),
+//   d m = (d dn - (dn . d dn) dn) / |m|,   d skts[pose, 0, 0:3, 0:3] += d m (x) d_ray.
+// Work layout: 32 rays per block of 4 warps.  The block stages its 32 d_ray_bias rows (float4 loads, a row is 512
+// contiguous bytes) and the 128 x 27 weight slice in shared memory.  Then lane = ray and warp w forms the columns
+// 7w..7w+6 of g: the d_ray_bias reads are conflict-free (row stride 129) and the weight reads are broadcasts.  Warp
+// a < 3 forms d dn_a (four sincos per lane), and warp 0 finishes the per-ray chain.  When all rays of the block share a
+// pose (rays are image-major, so almost always) it sums the 9 entries over the block and issues one set of atomics;
+// otherwise every ray issues its own.  Three barriers order the phases: staging -> o-loop, gs stores -> the cross-warp gs
+// reads (and the reuse of db), d dn -> warp 0.  57 registers, no spills, 36.6 KB of shared memory (-Xptxas -v).
+constexpr int VR_RAYS = 32, VR_COLS = 27, VR_GRP = 7;
+
+__global__ void __launch_bounds__(128)
+view_root_bwd_kernel(const float* __restrict__ rays, int ray_stride, int n_rays, const float* __restrict__ pose_skts,
+                     int rays_per_pose, int n_poses, const float* __restrict__ w_view /* (128,411) */,
+                     const float* __restrict__ d_ray_bias /* (n,128) */, float* __restrict__ d_skts) {
+    __shared__ float db[VR_RAYS][129];
+    __shared__ __align__(16) float ws[4][128][8];          // [warp][o][column 7w + s], slot 7 zero
+    __shared__ float gs[VR_RAYS][VR_COLS + 2];              // row stride 29: conflict-free for lane = ray
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int base = blockIdx.x * VR_RAYS;
+    const int nr = min(VR_RAYS, n_rays - base);
+    for (int i = tid; i < VR_RAYS * 32; i += 128) {
+        const int r = i >> 5, q = i & 31;
+        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (r < nr) v = __ldg(reinterpret_cast<const float4*>(d_ray_bias + (size_t)(base + r) * 128) + q);
+        db[r][4 * q + 0] = v.x; db[r][4 * q + 1] = v.y; db[r][4 * q + 2] = v.z; db[r][4 * q + 3] = v.w;
+    }
+    for (int i = tid; i < 4 * 128 * 8; i += 128) {
+        const int w = i >> 10, o = (i >> 3) & 127, s = i & 7, c = w * VR_GRP + s;
+        ws[w][o][s] = (s < VR_GRP && c < VR_COLS) ? __ldg(w_view + (size_t)o * 411 + 256 + c) : 0.f;
+    }
+    __syncthreads();
+    float acc[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+#pragma unroll 4
+    for (int o = 0; o < 128; ++o) {
+        const float d = db[lane][o];
+        const float4 a = *reinterpret_cast<const float4*>(&ws[warp][o][0]);
+        const float4 b = *reinterpret_cast<const float4*>(&ws[warp][o][4]);
+        acc[0] = fmaf(a.x, d, acc[0]); acc[1] = fmaf(a.y, d, acc[1]); acc[2] = fmaf(a.z, d, acc[2]);
+        acc[3] = fmaf(a.w, d, acc[3]); acc[4] = fmaf(b.x, d, acc[4]); acc[5] = fmaf(b.y, d, acc[5]);
+        acc[6] = fmaf(b.z, d, acc[6]);
+    }
+#pragma unroll
+    for (int s = 0; s < VR_GRP; ++s)
+        if (warp * VR_GRP + s < VR_COLS) gs[lane][warp * VR_GRP + s] = acc[s];
+    // every warp reads columns the other warps wrote, and warps 0-2 overwrite db, which every warp's o-loop reads
+    __syncthreads();
+    const bool live = lane < nr;
+    const int n = base + lane;
+    const int pose = live ? min(n / rays_per_pose, n_poses - 1) : 0;
+    float dx = 0.f, dy = 0.f, dz = 0.f, nrm = 1.f, dn[3] = {0.f, 0.f, 0.f};
+    if (live) {
+        const float* r = rays + (size_t)n * ray_stride + 3;
+        dx = r[0]; dy = r[1]; dz = r[2];
+        const float* R = pose_skts + (size_t)pose * DANBO_J * 16;          // joint 0
+        const float m[3] = {fmaf(__ldg(R + 2), dz, fmaf(__ldg(R + 1), dy, __ldg(R + 0) * dx)),
+                            fmaf(__ldg(R + 6), dz, fmaf(__ldg(R + 5), dy, __ldg(R + 4) * dx)),
+                            fmaf(__ldg(R + 10), dz, fmaf(__ldg(R + 9), dy, __ldg(R + 8) * dx))};
+        nrm = fmaxf(sqrtf(m[0] * m[0] + m[1] * m[1] + m[2] * m[2]), 1e-12f);
+        dn[0] = m[0] / nrm; dn[1] = m[1] / nrm; dn[2] = m[2] / nrm;
+    }
+    // d dn_a of ray `lane` by warp a < 3 (4 sincos per lane instead of 12 on one warp)
+    if (warp < 3 && live) {
+        const int a = warp;
+        const float da = warp == 0 ? dn[0] : (warp == 1 ? dn[1] : dn[2]);
+        float g = gs[lane][a];
+#pragma unroll
+        for (int f = 0; f < 4; ++f) {
+            const float fr = (float)(1 << f);
+            float sn, cs;
+            sincosf(da * fr, &sn, &cs);                                  // ray_bias_kernel's sin / cos arguments
+            g = fmaf(fr * cs, gs[lane][3 + 6 * f + a], g);
+            g = fmaf(-fr * sn, gs[lane][6 + 6 * f + a], g);
+        }
+        db[lane][a] = g;                                                 // the d_ray_bias tile is consumed
+    }
+    __syncthreads();
+    if (warp != 0) return;
+    float out[9];
+#pragma unroll
+    for (int i = 0; i < 9; ++i) out[i] = 0.f;
+    if (live) {
+        const float ddn[3] = {db[lane][0], db[lane][1], db[lane][2]};
+        const float p = dn[0] * ddn[0] + dn[1] * ddn[1] + dn[2] * ddn[2];
+#pragma unroll
+        for (int i = 0; i < 3; ++i) {
+            const float dm = (ddn[i] - p * dn[i]) / nrm;
+            out[3 * i + 0] = dm * dx; out[3 * i + 1] = dm * dy; out[3 * i + 2] = dm * dz;
+        }
+    }
+    const int pose_first = min(base / rays_per_pose, n_poses - 1);
+    const int pose_last = min((base + nr - 1) / rays_per_pose, n_poses - 1);
+    if (pose_first == pose_last) {
+        float* dst = d_skts + (size_t)pose_first * DANBO_J * 16;
+#pragma unroll
+        for (int i = 0; i < 9; ++i) {
+            float v = out[i];
+#pragma unroll
+            for (int off = 16; off > 0; off >>= 1) v += __shfl_xor_sync(0xffffffffu, v, off);
+            if (lane == 0) atomicAdd(dst + (i / 3) * 4 + i % 3, v);
+        }
+    } else if (live) {
+        float* dst = d_skts + (size_t)pose * DANBO_J * 16;
+#pragma unroll
+        for (int i = 0; i < 9; ++i) atomicAdd(dst + (i / 3) * 4 + i % 3, out[i]);
+    }
+}
+
 }  // namespace bwd
 }  // namespace danbo
 
@@ -375,6 +488,19 @@ extern "C" int danbo_ray_bias_bwd(const float* rays, int ray_stride, int n_rays,
     if (rb_blocks > 1184) rb_blocks = 1184;
     bwd::ray_bias_bwd_kernel<<<rb_blocks, 256, 0, (cudaStream_t)stream>>>(
         rays, ray_stride, n_rays, cam_idx, codes, n_codes, w_view, d_ray_bias, d_w_view, d_b_view, d_codes);
+    DANBO_CHECK_LAUNCH();
+    return 0;
+}
+
+extern "C" int danbo_view_root_bwd(const float* rays, int ray_stride, int n_rays, const float* pose_skts,
+                                   int rays_per_pose, int n_poses, const float* w_view, const float* d_ray_bias,
+                                   float* d_skts, void* stream) {
+    if (n_rays <= 0) return 0;
+    if (!rays || !pose_skts || !w_view || !d_ray_bias || !d_skts || ray_stride < 6 || rays_per_pose <= 0 || n_poses <= 0)
+        return -1;
+    if (reinterpret_cast<uintptr_t>(d_ray_bias) & 15) return -1;       // rows are read as float4
+    bwd::view_root_bwd_kernel<<<(n_rays + bwd::VR_RAYS - 1) / bwd::VR_RAYS, 128, 0, (cudaStream_t)stream>>>(
+        rays, ray_stride, n_rays, pose_skts, rays_per_pose, n_poses, w_view, d_ray_bias, d_skts);
     DANBO_CHECK_LAUNCH();
     return 0;
 }

@@ -586,6 +586,38 @@ def ray_bias_bwd(rays, cam_idx, codes_with_mean, w_view, d_ray_bias, d_w_view, d
     _count(1)
 
 
+def view_root_bwd(rays, pose_skts, rays_per_pose, w_view, d_ray_bias, d_skts):
+    """d skts (n_poses,24,4,4) += d loss / d skts through root-local view directions (perfcap configs under --opt_pose,
+    danbo_view_root_bwd): rows 0-2, columns 0-2 of joint 0 only.  rays (n,>=6) with unit column stride, w_view the
+    (128,411) view weight, d_ray_bias (n,128) the gradient of danbo_ray_bias's output."""
+    tensors = dict(rays=rays, pose_skts=pose_skts, w_view=w_view, d_ray_bias=d_ray_bias, d_skts=d_skts)
+    _need_cuda(*tensors.values())
+    for name, t in tensors.items():
+        if t.dtype != torch.float32:
+            raise ValueError(f"view_root_bwd: {name} must be fp32, got {t.dtype}")
+        if t.device != rays.device:
+            raise ValueError(f"view_root_bwd: {name} is on {t.device}, rays on {rays.device}")
+    n = rays.shape[0]
+    if rays.dim() != 2 or rays.shape[1] < 6 or rays.stride(1) != 1:
+        raise ValueError("view_root_bwd: rays must be (n, >=6) with contiguous rows")
+    if pose_skts.dim() != 4 or tuple(pose_skts.shape[1:]) != (J, 4, 4) or not pose_skts.is_contiguous():
+        raise ValueError("view_root_bwd: pose_skts must be a contiguous (n_poses,24,4,4) tensor")
+    if tuple(w_view.shape) != (128, 411) or not w_view.is_contiguous():
+        raise ValueError("view_root_bwd: w_view must be a contiguous (128,411) tensor")
+    if tuple(d_ray_bias.shape) != (n, 128) or not d_ray_bias.is_contiguous() or d_ray_bias.data_ptr() % 16:
+        raise ValueError("view_root_bwd: d_ray_bias must be a contiguous, 16-byte aligned (n,128) tensor")
+    if d_skts.shape != pose_skts.shape or not d_skts.is_contiguous():
+        raise ValueError("view_root_bwd: d_skts must be a contiguous tensor of pose_skts' shape")
+    if int(rays_per_pose) <= 0:
+        raise ValueError("view_root_bwd: rays_per_pose must be positive")
+    with _Timed("view_root_bwd"):
+        _lib.check(_lib.load().danbo_view_root_bwd(_p(rays), rays.stride(0), n, _p(pose_skts), int(rays_per_pose),
+                                                   pose_skts.shape[0], _p(w_view), _p(d_ray_bias), _p(d_skts),
+                                                   _stream()), "danbo_view_root_bwd")
+    _count(1)
+    return d_skts
+
+
 def field_agg_bwd(rays, S, z, mask, active, pose_skts, pose_vol, rays_per_pose, consts, fo, dX, g_logit_ext, grads,
                   d_skts=None):
     """grads: list of the 9 fp32 parameter / volume accumulators in the order of danbo_field_agg_bwd (see danbo_b200.h);

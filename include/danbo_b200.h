@@ -210,6 +210,15 @@ int danbo_ray_bias_bwd(const float* rays, int ray_stride, int n_rays, const int*
                        const float* w_view, const float* d_ray_bias, float* d_w_view, float* d_b_view, float* d_codes,
                        void* stream);
 
+/* V1 backward to the root rotation under root-local view directions (perfcap configs: ray_tr_type=root_local,
+ * view_type=relray; pose refinement, --opt_pose): autograd of RootLocalEncoder (core/encoders.py:570-578) and
+ * VecNormEncoder (:774-795), i.e. of dn = normalize(skts[pose, 0, :3, :3] . rays_d) and its 4-octave encoding, which
+ * danbo_ray_bias multiplies by W_v[:, 256:283], with respect to skts.  Ray n belongs to pose min(n / rays_per_pose,
+ * n_poses - 1).  w_view (128,411) fp32 and d_ray_bias (n_rays,128) fp32 row-major (16-byte aligned).  d_skts
+ * (n_poses,24,4,4) fp32 is added to (zero it first); only rows 0-2, columns 0-2 of joint 0 receive anything. */
+int danbo_view_root_bwd(const float* rays, int ray_stride, int n_rays, const float* pose_skts, int rays_per_pose,
+                        int n_poses, const float* w_view, const float* d_ray_bias, float* d_skts, void* stream);
+
 /* G1/G2 + A1-A3 + PE backward (danbo.py:261-302, gnn_backbone.py:787-828, misc.py:331-351): d X (rows,208) and the
  * extra logit gradient -> grads[10] = { w0, adj_w, b0, w1, b1, w2, b2 of prob_linears, d vol (n_poses,24,240),
  * d axis_scale (24,3), d skts (n_poses,24,4,4) or NULL } (fp32, accumulated).  d skts is the gradient with respect to
