@@ -26,6 +26,10 @@ _SIGNATURES = {
     "danbo_mlp_set_cta_pair": [c_i],
     "danbo_graph_net_fwd": [c_p, c_i, c_p, c_p, c_p, c_p],
     "danbo_graph_net_bwd": [c_i, c_p, c_p, c_p, c_p, c_p, c_p],
+    "danbo_graph_net_bwd_pose": [c_p, c_i, c_p, c_p, c_p, c_p, c_p],
+    "danbo_pose_fwd": [c_p, c_p, c_p, c_p, c_p, c_i, c_p, c_p, c_i, c_i, c_p, c_p, c_f, c_f, c_f, c_p, c_p, c_p, c_p, c_p],
+    "danbo_pose_bwd": [c_p, c_p, c_p, c_p, c_p, c_i, c_p, c_p, c_i, c_i, c_p, c_p, c_p, c_p, c_p, c_f, c_f, c_p, c_p, c_p,
+                       c_p],
     "danbo_train_loss": [c_p, c_p, c_p, c_p, c_p, c_p, c_f, c_i, c_i, c_i, c_f, c_f, c_p, c_p, c_p, c_p, c_i, c_f, c_p, c_p, c_f,
                          c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p],
     "danbo_adam_step": [c_p, c_p, c_p, c_p, ctypes.c_longlong, c_p, c_f, c_f, c_f, c_p, c_i, c_p],

@@ -173,15 +173,16 @@ def render_block_with_grad(caster, rays, skip, pose_skts, pose_cyls, vol, cam_id
 
 class _GraphNet(torch.autograd.Function):
     """GN1 + GN2 (pose -> bone feature lines) as four launches each way; gradients go to the ten graph-net parameters
-    (the pose itself is not optimised on this path: opt_pose is off in every shipped config)."""
+    and, when the pose requires one (the pose layer's kernel path, `pose_layer`), one more launch gives d pose_bones."""
 
     @staticmethod
     def forward(ctx, net, pose_bones, *params):
         named = {n: p for n, p in zip(K.GN_GRADS, params)}
         gn = net.graph_net
         named["layers.0.adj"], named["layers.1.adj"] = gn.layers[0].adj, gn.layers[1].adj
+        pose_bones = pose_bones.detach().float().contiguous()
         vol, saved = K.graph_net_fwd(pose_bones, [named[n].detach() for n in K.GN_PARAMS])
-        ctx.saved_bufs, ctx.net, ctx.params = saved, net, params
+        ctx.saved_bufs, ctx.net, ctx.params, ctx.pose_bones = saved, net, params, pose_bones
         return vol
 
     @staticmethod
@@ -192,17 +193,73 @@ class _GraphNet(torch.autograd.Function):
             p.grad is not None and p.grad.dtype == torch.float32 and p.grad.is_contiguous() and p.grad.shape == p.shape
             for p in params)
         grads = [p.grad if in_place else torch.zeros_like(p, dtype=torch.float32) for p in params]
-        K.graph_net_bwd(ctx.saved_bufs, d_vol, grads)
-        ctx.saved_bufs = None
+        work = K.graph_net_bwd(ctx.saved_bufs, d_vol, grads)
+        # a pose that needs a gradient (the pose layer's kernel path): d pose_bones through layer 0's inputs
+        d_pose = K.graph_net_bwd_pose(ctx.saved_bufs, work, ctx.pose_bones) if ctx.needs_input_grad[1] else None
+        ctx.saved_bufs = ctx.pose_bones = None
         if in_place:
-            return (None, None) + (None,) * len(params)
-        return (None, None) + tuple(grads)
+            return (None, d_pose) + (None,) * len(params)
+        return (None, d_pose) + tuple(grads)
 
 
 def graph_net_volumes(net, pose_bones):
     named = dict(net.graph_net.named_parameters())
     params = [named[n] for n in K.GN_GRADS]
-    if torch.is_grad_enabled() and any(p.requires_grad for p in params):
+    if torch.is_grad_enabled() and (pose_bones.requires_grad or any(p.requires_grad for p in params)):
         return _GraphNet.apply(net, pose_bones, *params)
     named["layers.0.adj"], named["layers.1.adj"] = net.graph_net.layers[0].adj, net.graph_net.layers[1].adj
     return K.graph_net_fwd(pose_bones, [named[n].detach() for n in K.GN_PARAMS])[0]
+
+
+class _PoseLayer(torch.autograd.Function):
+    """The pose layer's forward (`pose_opt.PoseOptLayer.calculate_kinematic` for the batch's unique poses) and the
+    trainer's pose regulariser (`pose_opt.kp_loss` without the temporal term) as one launch (danbo_pose_fwd); the
+    backward of both as one launch (danbo_pose_bwd) that adds into the layer's parameter gradients."""
+
+    @staticmethod
+    def forward(ctx, spec, idx, *params):
+        layer = dict(spec["buffers"], **{n: p.detach() for n, p in zip(spec["names"], params)})
+        kps, bones, skts, stats = K.pose_fwd(layer, idx, spec["skip"], spec["G"], anchors=spec["anchors"],
+                                             tol=spec["tol"], coef=spec["coef"], ext_scale=spec["ext_scale"])
+        ctx.spec, ctx.layer, ctx.idx, ctx.params = spec, layer, idx, params
+        mpjpc = stats[1]
+        ctx.mark_non_differentiable(mpjpc)
+        return kps, bones, skts, stats[0], mpjpc
+
+    @staticmethod
+    def backward(ctx, d_kps, d_bones, d_skts, d_reg, _d_mpjpc):
+        spec, params = ctx.spec, ctx.params
+        # with a pose optimizer over one flat, pre-zeroed gradient bucket (training.FlatAdam) the kernel adds straight
+        # into the parameters' .grad views, as the render block does for the network
+        in_place = spec["grads_in_place"] and all(
+            p.grad is not None and p.grad.dtype == torch.float32 and p.grad.is_contiguous() and p.grad.shape == p.shape
+            for p in params)
+        grads = {n: (p.grad if in_place else torch.zeros_like(p, dtype=torch.float32)) for n, p in zip(spec["names"], params)}
+        c = lambda t: None if t is None else t.float().contiguous()
+        if d_skts is None:
+            d_skts = torch.zeros(spec["G"], K.J, 4, 4, device=ctx.idx.device)
+        K.pose_bwd(ctx.layer, ctx.idx, spec["skip"], spec["G"], c(d_skts), grads, d_bones=c(d_bones), d_kps=c(d_kps),
+                   anchor_bones=spec["anchors"]["bones"] if d_reg is not None else None,
+                   d_reg=None if d_reg is None else c(d_reg).reshape(()), tol=spec["tol"], coef=spec["coef"])
+        ctx.layer = ctx.params = None
+        if in_place:
+            return (None, None) + (None,) * len(params)
+        return (None, None) + tuple(grads[n] for n in spec["names"])
+
+
+def pose_layer(layer, idx, skip, G, anchors, rest_idx=None, tol=0., coef=0., ext_scale=0.001, grads_in_place=False):
+    """Poses idx[0], idx[skip], ... (G of them, idx int64 on the layer's device) of a `pose_opt.PoseOptLayer`
+    (axis-angle; the multi-view split too) through the kernels.  anchors: {'kps', 'bones'} fp32 (F,24,3) on the layer's
+    device; rest_idx: the layer's `rest_pose_idxs` as an int64 device tensor when it holds several rest poses.
+    -> kps (G,24,3), bones (G,24,3), skts (G,24,4,4), kp_loss (differentiable scalar), MPJPC (scalar)."""
+    names = [n for n, _ in layer.named_parameters()]
+    buffers = {"rest_pose": layer.rest_pose.float().contiguous()}
+    if layer.kp_map is not None:
+        buffers["kp_map"] = layer.kp_map
+    if layer.rest_pose.shape[0] > 1:
+        if rest_idx is None:
+            raise ValueError("pose_layer: a layer with several rest poses needs rest_idx")
+        buffers["rest_idx"] = rest_idx
+    spec = dict(names=names, buffers=buffers, skip=int(skip), G=int(G), anchors=anchors, tol=float(tol),
+                coef=float(coef), ext_scale=float(ext_scale), grads_in_place=bool(grads_in_place))
+    return _PoseLayer.apply(spec, idx, *[p for _, p in layer.named_parameters()])

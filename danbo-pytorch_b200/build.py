@@ -9,7 +9,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libdanbo_b200.so")
-SOURCES = ["version.cu", "field.cu", "field_mma.cu", "composite.cu", "mlp_tcgen05.cu", "backward_mlp.cu", "backward_field.cu", "mlp_bwd_tcgen05.cu", "anerf.cu", "anerf_bwd.cu", "loss.cu", "graphnet.cu"]
+SOURCES = ["version.cu", "field.cu", "field_mma.cu", "composite.cu", "mlp_tcgen05.cu", "backward_mlp.cu", "backward_field.cu", "mlp_bwd_tcgen05.cu", "anerf.cu", "anerf_bwd.cu", "loss.cu", "graphnet.cu", "pose.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr", "--expt-extended-lambda"]
 

@@ -15,6 +15,7 @@
 // backward blocks own a 16-row slice of the node's weight matrix, for both its gradient (one owner thread per entry:
 // plain += unless there are several pose groups) and the transposed product.  4 launches forward, 4 backward, fp32.
 #include "common.cuh"
+#include "rotation.cuh"
 #include <math.h>
 
 namespace danbo {
@@ -44,7 +45,9 @@ struct Grads {                     // accumulated into (+=)
 
 // Graph inputs of (pose g, joint j): rot6d of the axis-angle (quaternion route, skeleton_utils.py:411-418) and its
 // 5-octave encoding [x, sin 2^0 x, cos 2^0 x, sin 2^1 x, ...] in blocks of 6, zeroed for the root (mask_root).
-// One thread per (pose, rot6d component i): it writes the 11 entries that derive from component i.
+// One thread per (pose, rot6d component i): it writes the 11 entries that derive from component i.  It computes only
+// the entry it needs rather than calling axisang_to_rot (rotation.cuh), which compiles one sum differently (an FADD
+// becomes an FFMA) and would change the graph net's outputs in the last bit.
 __device__ __forceinline__ void graph_inputs(const float* __restrict__ aa, int j, int i, float* row, float* keep) {
     const float ax = aa[0], ay = aa[1], az = aa[2];
     const float ang = sqrtf(ax * ax + ay * ay + az * az), half = 0.5f * ang;
@@ -285,6 +288,62 @@ bwd_kernel(int G, Params P, Saved S, const float* __restrict__ d_in, Grads Gr, f
     }
 }
 
+// ---- d pose: layer 0's d pre-activation -> d axis-angle --------------------------------------------------------
+// d lin0 = A0^T d pre0 (the transposed mix), d w_in = mask_root (W0[j] d lin0), then back through the 5-octave PE with
+// the sin / cos values the forward kept in saved[0] (d sin(2^f x) / dx = 2^f cos(2^f x)), rot6d = (R00 R01 R10 R11
+// R20 R21) and the quaternion route.  Block = (node, pose), 128 threads: thread = column of d lin0, then warp = rows of
+// W0[j]; the root's row is zero (mask_root).
+__global__ void __launch_bounds__(kW)
+bwd_pose_kernel(const float* __restrict__ bones, Params P, Saved S, const float* __restrict__ d_pre0,
+                float* __restrict__ d_bones) {
+    __shared__ float dl[kW];
+    __shared__ float dw[kIn];
+    const int node = blockIdx.x, g = blockIdx.y, tid = threadIdx.x, lane = tid & 31;
+    const size_t at = (size_t)g * DANBO_J + node;
+    if (node == 0) {
+        if (tid < 3) d_bones[at * 3 + tid] = 0.f;
+        return;
+    }
+    float acc = 0.f;
+    for (int o = 0; o < DANBO_J; ++o) {
+        const int e = o * DANBO_J + node;
+        const float m = __ldg(P.adj0 + e);
+        if (m == 0.f) continue;
+        acc = fmaf(__ldg(P.adjw0 + e) * m, d_pre0[((size_t)g * DANBO_J + o) * kW + tid], acc);
+    }
+    dl[tid] = acc;
+    __syncthreads();
+    for (int i = tid >> 5; i < kIn; i += kW / 32) {
+        const float* w = P.w0 + ((size_t)node * kIn + i) * kW;
+        float s = 0.f;
+#pragma unroll
+        for (int c = lane; c < kW; c += 32) s = fmaf(__ldg(w + c), dl[c], s);
+        s = warp_sum(s);
+        if (lane == 0) dw[i] = s;
+    }
+    __syncthreads();
+    if (tid >= 32) return;
+    float dx = 0.f;
+    if (lane < 6) {
+        const float* keep = S.w_in + at * kIn;
+        dx = dw[lane];
+#pragma unroll
+        for (int f = 0; f < 5; ++f)
+            dx += (float)(1 << f) * (keep[12 + 12 * f + lane] * dw[6 + 12 * f + lane]
+                                     - keep[6 + 12 * f + lane] * dw[12 + 12 * f + lane]);
+    }
+    float gR[9] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+    gR[0] = __shfl_sync(0xffffffffu, dx, 0); gR[1] = __shfl_sync(0xffffffffu, dx, 1);
+    gR[3] = __shfl_sync(0xffffffffu, dx, 2); gR[4] = __shfl_sync(0xffffffffu, dx, 3);
+    gR[6] = __shfl_sync(0xffffffffu, dx, 4); gR[7] = __shfl_sync(0xffffffffu, dx, 5);
+    if (lane == 0) {
+        const float a[3] = {bones[at * 3], bones[at * 3 + 1], bones[at * 3 + 2]};
+        float da[3];
+        axisang_to_rot_bwd(a, gR, da);
+        d_bones[at * 3] = da[0]; d_bones[at * 3 + 1] = da[1]; d_bones[at * 3 + 2] = da[2];
+    }
+}
+
 }  // namespace gn
 }  // namespace danbo
 
@@ -338,6 +397,19 @@ extern "C" int danbo_graph_net_bwd(int n_poses, const float* const* params, floa
     gn::bwd_kernel<1><<<g128, gn::kThreads, 0, st>>>(n_poses, P, S, d_pre1, Gr, d_pre0);
     DANBO_CHECK_LAUNCH();
     gn::bwd_kernel<0><<<g66, gn::kThreads, 0, st>>>(n_poses, P, S, d_pre0, Gr, nullptr);
+    DANBO_CHECK_LAUNCH();
+    return 0;
+}
+
+extern "C" int danbo_graph_net_bwd_pose(const float* pose_bones, int n_poses, const float* const* params,
+                                        float* const* saved, const float* work, float* d_pose_bones, void* stream) {
+    if (n_poses <= 0) return 0;
+    if (!pose_bones || !params || !saved || !work || !d_pose_bones) return -1;
+    const gn::Params P = gn_params(params);
+    const gn::Saved S = gn_saved(saved);
+    const float* d_pre0 = work + (size_t)n_poses * DANBO_J * gn::kW;     // where danbo_graph_net_bwd leaves it
+    gn::bwd_pose_kernel<<<dim3(DANBO_J, n_poses), gn::kW, 0, (cudaStream_t)stream>>>(pose_bones, P, S, d_pre0,
+                                                                                      d_pose_bones);
     DANBO_CHECK_LAUNCH();
     return 0;
 }

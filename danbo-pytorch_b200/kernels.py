@@ -678,6 +678,120 @@ def graph_net_bwd(saved, d_vol, grads):
     ga = (ctypes.c_void_p * 10)(*[g.data_ptr() for g in grads])
     _lib.check(lib.danbo_graph_net_bwd(G, pa, sa, _p(d_vol), ga, _p(work), _stream()), "danbo_graph_net_bwd")
     _count(4)
+    return work
+
+
+def graph_net_bwd_pose(saved, work, pose_bones):
+    """d loss / d pose_bones (G,24,3) of the graph net (danbo_graph_net_bwd_pose), after graph_net_bwd returned `work`
+    for the same `saved`; pose_bones is what graph_net_fwd read.  The root's row is zero (mask_root)."""
+    tensors, bufs = saved
+    _need_cuda(pose_bones, work)
+    G = bufs[0].shape[0]
+    if pose_bones.dtype != torch.float32 or tuple(pose_bones.shape) != (G, J, 3) or not pose_bones.is_contiguous():
+        raise ValueError(f"graph_net_bwd_pose: pose_bones must be a contiguous fp32 ({G},24,3) tensor")
+    if work.dtype != torch.float32 or work.numel() != 2 * G * J * 128 or not work.is_contiguous():
+        raise ValueError("graph_net_bwd_pose: work must be graph_net_bwd's workspace of the same poses")
+    if pose_bones.device != work.device or bufs[0].device != work.device:
+        raise ValueError("graph_net_bwd_pose: pose_bones, work and saved must be on one device")
+    d_bones = torch.empty(G, J, 3, device=work.device)
+    pa = (ctypes.c_void_p * 12)(*[t.data_ptr() for t in tensors])
+    sa = (ctypes.c_void_p * 6)(*[t.data_ptr() for t in bufs])
+    with _Timed("graph_net_bwd_pose"):
+        _lib.check(_lib.load().danbo_graph_net_bwd_pose(_p(pose_bones), G, pa, sa, _p(work), _p(d_bones), _stream()),
+                   "danbo_graph_net_bwd_pose")
+    _count(1)
+    return d_bones
+
+
+def _pose_layer_args(fn, layer, idx, idx_stride, n_poses):
+    """Checks the pose layer's tensors for pose_fwd / pose_bwd -> the leading arguments of danbo_pose_fwd/_bwd."""
+    pelvis, bones, rest = layer["pelvis"], layer["bones"], layer["rest_pose"]
+    root_bones, kp_map, rest_idx = layer.get("root_bones"), layer.get("kp_map"), layer.get("rest_idx")
+    _need_cuda(pelvis, bones, rest, idx, root_bones, kp_map, rest_idx)
+    dev = pelvis.device
+    for name, t, dt in (("pelvis", pelvis, torch.float32), ("bones", bones, torch.float32), ("rest_pose", rest, torch.float32),
+                        ("root_bones", root_bones, torch.float32), ("kp_map", kp_map, torch.int64),
+                        ("rest_idx", rest_idx, torch.int64), ("idx", idx, torch.int64)):
+        if t is None:
+            continue
+        if t.dtype != dt or not t.is_contiguous() or t.device != dev:
+            raise ValueError(f"{fn}: {name} must be a contiguous {dt} tensor on {dev}")
+    F_ = pelvis.shape[0]
+    if tuple(pelvis.shape) != (F_, 3):
+        raise ValueError(f"{fn}: pelvis must be (F,3)")
+    if (root_bones is None) != (kp_map is None):
+        raise ValueError(f"{fn}: root_bones and kp_map go together (the multi-view split)")
+    if root_bones is None:
+        if tuple(bones.shape) != (F_, J, 3):
+            raise ValueError(f"{fn}: bones must be (F,24,3) axis-angle")
+    elif tuple(root_bones.shape) != (F_, 3) or bones.dim() != 3 or tuple(bones.shape[1:]) != (J - 1, 3) \
+            or tuple(kp_map.shape) != (F_,):
+        raise ValueError(f"{fn}: the multi-view split needs root_bones (F,3), bones (U,23,3) and kp_map (F)")
+    if rest.dim() != 3 or tuple(rest.shape[1:]) != (J, 3):
+        raise ValueError(f"{fn}: rest_pose must be (R,24,3)")
+    if rest.shape[0] > 1 and (rest_idx is None or tuple(rest_idx.shape) != (F_,)):
+        raise ValueError(f"{fn}: several rest poses need a per-frame row table rest_idx (F)")
+    if idx.dim() != 1 or int(idx_stride) <= 0 or (int(n_poses) - 1) * int(idx_stride) >= max(idx.shape[0], 1):
+        raise ValueError(f"{fn}: idx must be 1-D and hold n_poses entries at stride idx_stride")
+    return [_p(pelvis), _p(bones), _p(root_bones), _p(kp_map), _p(rest), rest.shape[0],
+            _p(rest_idx if rest.shape[0] > 1 else None), _p(idx), int(idx_stride), int(n_poses)]
+
+
+def pose_fwd(layer, idx, idx_stride, n_poses, anchors=None, tol=0., coef=0., ext_scale=0.001):
+    """The pose layer's forward for poses idx[0], idx[stride], ... (danbo_pose_fwd).  layer: dict of the parameter and
+    buffer tensors (pelvis, bones[, root_bones, kp_map], rest_pose[, rest_idx]); anchors: {'kps', 'bones'} (F,24,3)
+    for the regulariser and MPJPC, or None.  -> kps (G,24,3), bones (G,24,3), skts (G,24,4,4), stats (2,) or None."""
+    args = _pose_layer_args("pose_fwd", layer, idx, idx_stride, n_poses)
+    dev, F_ = layer["pelvis"].device, layer["pelvis"].shape[0]
+    ak = ab = stats = None
+    if anchors is not None:
+        ak, ab = anchors["kps"], anchors["bones"]
+        for name, t in (("kps", ak), ("bones", ab)):
+            _need_cuda(t)
+            if t.dtype != torch.float32 or not t.is_contiguous() or t.device != dev or tuple(t.shape) != (F_, J, 3):
+                raise ValueError(f"pose_fwd: anchor {name} must be a contiguous fp32 ({F_},24,3) tensor on {dev}")
+        if not float(ext_scale) > 0:
+            raise ValueError("pose_fwd: ext_scale must be positive")
+        stats = torch.empty(2, device=dev)
+    G = int(n_poses)
+    kps, bones, skts = torch.empty(G, J, 3, device=dev), torch.empty(G, J, 3, device=dev), torch.empty(G, J, 4, 4, device=dev)
+    with _Timed("pose_fwd"):
+        _lib.check(_lib.load().danbo_pose_fwd(*args, _p(ak), _p(ab), float(tol), float(coef), float(ext_scale), _p(kps),
+                                              _p(bones), _p(skts), _p(stats), _stream()), "danbo_pose_fwd")
+    _count(1)
+    return kps, bones, skts, stats
+
+
+def pose_bwd(layer, idx, idx_stride, n_poses, d_skts, grads, d_bones=None, d_kps=None, anchor_bones=None, d_reg=None,
+             tol=0., coef=0.):
+    """Backward of pose_fwd (danbo_pose_bwd): ADDS d loss / d parameters into grads {'pelvis', 'bones'[,
+    'root_bones']} (fp32, the parameters' shapes).  d_reg: device scalar d loss / d kp_loss, or None (no regulariser)."""
+    args = _pose_layer_args("pose_bwd", layer, idx, idx_stride, n_poses)
+    dev, G = layer["pelvis"].device, int(n_poses)
+    for name, t, shape in (("d_skts", d_skts, (G, J, 4, 4)), ("d_bones", d_bones, (G, J, 3)), ("d_kps", d_kps, (G, J, 3)),
+                           ("d_reg", d_reg, ()), ("anchor_bones", anchor_bones, (layer["pelvis"].shape[0], J, 3))):
+        if t is None:
+            continue
+        _need_cuda(t)
+        if t.dtype != torch.float32 or not t.is_contiguous() or t.device != dev or tuple(t.shape) != shape:
+            raise ValueError(f"pose_bwd: {name} must be a contiguous fp32 {shape} tensor on {dev}")
+    if d_skts is None:
+        raise ValueError("pose_bwd: d_skts is required")
+    if d_reg is not None and anchor_bones is None:
+        raise ValueError("pose_bwd: the regulariser's gradient needs anchor_bones")
+    names = ("pelvis", "bones") + (("root_bones",) if layer.get("root_bones") is not None else ())
+    if set(grads) != set(names):
+        raise ValueError(f"pose_bwd: grads must hold exactly {names}")
+    for nm in names:
+        g = grads[nm]
+        _need_cuda(g)
+        if g.dtype != torch.float32 or not g.is_contiguous() or g.device != dev or g.shape != layer[nm].shape:
+            raise ValueError(f"pose_bwd: grads[{nm!r}] must be a contiguous fp32 tensor of the parameter's shape")
+    with _Timed("pose_bwd"):
+        _lib.check(_lib.load().danbo_pose_bwd(*args, _p(d_skts), _p(d_bones), _p(d_kps), _p(anchor_bones), _p(d_reg),
+                                              float(tol), float(coef), _p(grads["pelvis"]), _p(grads["bones"]),
+                                              _p(grads.get("root_bones")), _stream()), "danbo_pose_bwd")
+    _count(1)
 
 
 LOSS_KINDS = {"L1": 0, "MSE": 1}

@@ -225,12 +225,15 @@ class DanboField(nn.Module):
 
     # ---- GN1 + GN2 (PyTorch, per unique pose) ---------------------------------------------------------------
     fused_graph_net = True        # GN1 + GN2 as danbo_graph_net_fwd/_bwd (CUDA tensors); False: the PyTorch ops below
+    # set by training.TrainStep around the forward pass of its pose-kernel path (a captured --opt_pose iteration): the
+    # pose's gradient then comes from the graph-net kernels (danbo_graph_net_bwd_pose) too
+    pose_kernels = False
 
     def bone_volumes(self, pose_bones):
         """pose_bones (G,24,3) axis-angle -> (G,24,240) feature lines (encoders.py:460-473,859-877; danbo.py:190-194)."""
-        # a pose that itself needs a gradient (pose layer under --opt_pose) takes the PyTorch ops below: the graph-net
-        # kernels' backward stops at the parameters
-        pose_grad = torch.is_grad_enabled() and pose_bones.requires_grad
+        # a pose that itself needs a gradient (pose layer under --opt_pose) takes the PyTorch ops below unless the pose
+        # kernels serve the step: eager training with a pose layer keeps them as its reference path
+        pose_grad = torch.is_grad_enabled() and pose_bones.requires_grad and not self.pose_kernels
         six = pose_bones.shape[-1] == 6          # a rot6d pose layer hands its parameters over as they are (encoders.py:873-877)
         if self.fused_graph_net and pose_bones.is_cuda and not pose_grad and not six:
             from .autograd import graph_net_volumes

@@ -256,8 +256,12 @@ class PoseOptLayer(nn.Module):
 
 
 # ---- construction / checkpoints ---------------------------------------------------------------------------------
-def create_popt(args, data_attrs, ckpt=None, device=None):
-    """pose_opt.py:14-83 -> (pose_optimizer, {'popt_anchors', 'popt_layer', 'skel_type'})."""
+def create_popt(args, data_attrs, ckpt=None, device=None, flat=False):
+    """pose_opt.py:14-83 -> (pose_optimizer, {'popt_anchors', 'popt_layer', 'skel_type'}).
+
+    flat=True: the optimizer is a `training.FlatAdam` over a `parallel.GradBucket` of the layer's parameters (CUDA
+    only) instead of `torch.optim.Adam`: one launch per step, and what `training.TrainStep(graph=True)` needs to capture
+    an --opt_pose iteration.  Its state_dict is in torch.optim.Adam's format, so checkpoints load either way."""
     skel_type = data_attrs.get("skel_type", sk.SMPLSkeleton)
     J = len(skel_type.joint_names)
     rest_pose = torch.as_tensor(np.asarray(data_attrs["rest_pose"])).reshape(-1, J, 3).float()
@@ -268,8 +272,12 @@ def create_popt(args, data_attrs, ckpt=None, device=None):
                          kp_map=data_attrs.get("kp_map"), kp_uidxs=data_attrs.get("kp_uidxs"),
                          rest_pose_idxs=data_attrs.get("rest_pose_idxs"), use_cache=False,
                          use_rot6d=bool(getattr(args, "opt_rot6d", False))).to(device)
-    optimizer = torch.optim.Adam(params=list(layer.parameters()), lr=getattr(args, "opt_pose_lrate", 5e-4),
-                                 betas=(0.9, 0.999))
+    params, lr = list(layer.parameters()), getattr(args, "opt_pose_lrate", 5e-4)
+    if flat:
+        from . import parallel, training
+        optimizer = training.FlatAdam(params, parallel.GradBucket(params), lr=lr, betas=(0.9, 0.999))
+    else:
+        optimizer = torch.optim.Adam(params=params, lr=lr, betas=(0.9, 0.999))
     anchor_kps, anchor_bones, anchor_beta = init_kps, init_bones, beta
     init = getattr(args, "init_poseopt", None)
     if (ckpt is not None or init is not None) and not getattr(args, "no_poseopt_reload", False):

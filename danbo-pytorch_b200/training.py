@@ -159,6 +159,10 @@ class FlatAdam(torch.optim.Optimizer):
         self.param_groups[0]["lr"] = float(lr)
         self.lr_dev.fill_(float(lr))
 
+    def zero_grad(self, set_to_none=True):
+        """Zeroes the gradient bucket in place: the parameters' .grad must stay views of it (set_to_none is ignored)."""
+        self.bucket.zero()
+
     def state_dict(self):
         """torch.optim.Adam's format (one host read of the step counter)."""
         return adam_state_to_dict(self.bucket.params, self.exp_avg, self.exp_avg_sq, float(self.step_dev.item()),
@@ -187,6 +191,39 @@ class FlatAdam(torch.optim.Optimizer):
                 torch.autograd.graph.increment_version(p)
 
 
+def pose_batch_poses(batch):
+    """(G, skip) of an --opt_pose batch: the poses are kp_idx[::skip], one per image of an image-major batch of
+    N_uniques equal runs (what the data feed builds).  A batch that does not divide so is refused: finding its poses
+    would need torch.unique, a host synchronisation, which a captured step cannot hold."""
+    n, G = int(batch["kp_idx"].shape[0]), int(batch["N_uniques"])
+    if G <= 0 or n % G:
+        raise NotImplementedError(f"a captured --opt_pose step needs N_uniques ({G}) to divide the batch ({n} rays): "
+                                  "other batches need torch.unique, a host synchronisation")
+    return G, n // G
+
+
+def _refuse_pose_graph(args, caster, world_size, pose_optimizer, layer):
+    """What a captured iteration with a pose layer does not cover: raise, naming the reason, before any device work."""
+    why = None
+    if getattr(caster.network, "graph_net", None) is None:
+        why = "the A-NeRF field (the pose kernels serve the DANBO field's graph net and bone transforms)"
+    elif getattr(caster, "network_fine", caster.network) is not caster.network:
+        why = "a separate fine network"
+    elif world_size > 1:
+        why = "world_size > 1 (the pose gradients' all-reduce is not part of the captured step)"
+    elif layer.use_rot6d or getattr(args, "opt_rot6d", False):
+        why = "opt_rot6d (the pose kernels take axis-angle parameters)"
+    elif getattr(args, "use_temp_loss", False):
+        why = "use_temp_loss (the temporal pose term is not part of the pose kernels)"
+    elif layer.use_cache or getattr(args, "opt_pose_cache", False):
+        why = "opt_pose_cache (the cache is refreshed on the host after every pose step)"
+    elif not isinstance(pose_optimizer, FlatAdam):
+        why = ("a pose optimizer that is not a training.FlatAdam (pass pose_opt.create_popt(..., flat=True)): a captured "
+               "backward writes into fixed gradient storage, which zero_grad(set_to_none=True) would detach")
+    if why is not None:
+        raise NotImplementedError(f"graph capture of a training step with a pose layer is not implemented for {why}")
+
+
 class TrainStep:
     """forward -> losses -> backward -> (all-reduce of one flat fp32 gradient bucket) -> Adam."""
 
@@ -207,14 +244,24 @@ class TrainStep:
         self.last_stats = {}
         self.n_steps = 0                        # optimizer steps taken (the `step` of Adam's state; restored by resume())
         self.lrate = float(args.lrate)
+        # a captured iteration runs the pose layer, its regulariser and their backward as kernels (autograd.pose_layer);
+        # eager steps keep the PyTorch ops of pose_opt
+        self._pose_kernels = self.popt is not None and graph
         if self.popt is not None:
+            layer = self.popt["popt_layer"]
             if graph:
-                raise NotImplementedError("graph capture of a training step with a pose layer is not implemented")
+                _refuse_pose_graph(args, caster, world_size, pose_optimizer, layer)
             dev = next(caster.network.parameters()).device
-            self.popt["popt_layer"].to(dev)
+            layer.to(dev)
             # anchors on the layer's device once: indexing them by the batch's kp_idx then needs no host round trip
             self.popt["popt_anchors"] = {k: (v.to(dev) if torch.is_tensor(v) else v)
                                          for k, v in self.popt["popt_anchors"].items()}
+            if self._pose_kernels:
+                a = self.popt["popt_anchors"]
+                self._pose_anchors = {k: a[k].float().contiguous() for k in ("kps", "bones")}
+                self._rest_idx = None
+                if layer.rest_pose.shape[0] > 1:
+                    self._rest_idx = torch.as_tensor(layer.rest_pose_idxs, device=dev).long()
         self.fused_loss = fused_loss           # False: the trainer's losses as PyTorch ops + autograd (compute_loss)
         # create_raycaster's grad_vars order (raycasters.py:188): the network, then a separate fine network.  The bucket,
         # the optimizer state and so the checkpoints index the reference's Adam over grad_vars.
@@ -248,15 +295,28 @@ class TrainStep:
 
             def run(**b):
                 loss, preds = self._step(b) if self._graph_whole else self._fwd_bwd(b)
-                return {"loss": loss, "rgb_map": preds["rgb_map"], "acc_map": preds["acc_map"]}
-            # building the graph must not train: parameters, moments and the step counter are restored after capture
+                out = {"loss": loss, "rgb_map": preds["rgb_map"], "acc_map": preds["acc_map"]}
+                if self.popt is not None:
+                    out["MPJPC"] = self.last_stats["MPJPC"]
+                return out
+            # building the graph must not train: parameters, moments and the step counters (the network's and the
+            # pose layer's) are restored after capture
             state = [optimizer.flat, optimizer.exp_avg, optimizer.exp_avg_sq, optimizer.step_dev] if flat else []
+            if self.popt is not None:
+                po = pose_optimizer
+                state += [po.flat, po.exp_avg, po.exp_avg_sq, po.step_dev]
             self._graphed = GraphedFn(run, params[0].device, warmup=3, state=state if self._graph_whole else [],
                                       capture_error_mode="thread_local" if world_size > 1 else "global")
 
     def __call__(self, batch):
         if self._graphed is not None:
+            if self.popt is not None:
+                pose_batch_poses(batch)          # refused before any device work
+                # the poses come from the layer: the feed's tables would only be copied into static buffers
+                batch = {k: v for k, v in batch.items() if k not in ("kp_batch", "skts", "bones")}
             out = self._graphed(**batch)
+            if self.popt is not None:
+                self.last_stats = {"MPJPC": out["MPJPC"]}
             if not self._graph_whole:
                 if self.world > 1:
                     self.bucket.allreduce(average=True)
@@ -340,7 +400,20 @@ class TrainStep:
         self.caster.train()
         self.bucket.zero()
         extra = None
-        if self.popt is not None:
+        if self._pose_kernels:
+            from .autograd import pose_layer
+            G, skip = pose_batch_poses(batch)
+            n = G * skip
+            self.pose_optimizer.zero_grad()
+            kps, bones, skts, extra, mpjpc = pose_layer(
+                self.popt["popt_layer"], batch["kp_idx"].long(), skip, G, self._pose_anchors, rest_idx=self._rest_idx,
+                tol=getattr(a, "opt_pose_tol", 0.), coef=getattr(a, "opt_pose_coef", 0.),
+                ext_scale=getattr(a, "ext_scale", 0.001), grads_in_place=True)
+            # per-ray rows as stride-0 expands, as PoseOptLayer.calculate_kinematic returns them
+            ex = lambda t: t[:, None].expand(G, skip, *t.shape[1:]).reshape(n, *t.shape[1:])
+            batch = dict(batch, kp_batch=ex(kps), skts=ex(skts), bones=ex(bones))
+            self.last_stats = {"MPJPC": mpjpc}
+        elif self.popt is not None:
             from . import pose_opt
             layer = self.popt["popt_layer"]
             if self.pose_optimizer is not None:
@@ -352,9 +425,14 @@ class TrainStep:
                                                        {"kp_batch": kps, "bones": bones, "rots": rots}, popt_layer=layer,
                                                        temp_val=batch.get("temp_val"))
             extra = sum(losses.values())
-        preds = self.caster(batch["ray_batch"], N_samples=a.N_samples, kp_batch=batch["kp_batch"], skts=batch["skts"],
-                            cyls=batch["cyls"], bones=batch["bones"], cams=batch["cams"], N_uniques=batch["N_uniques"],
-                            perturb=a.perturb, N_importance=a.N_importance, raw_noise_std=a.raw_noise_std)
+        net = self.caster.network
+        net.pose_kernels = self._pose_kernels        # the graph net's kernels then also return d pose
+        try:
+            preds = self.caster(batch["ray_batch"], N_samples=a.N_samples, kp_batch=batch["kp_batch"], skts=batch["skts"],
+                                cyls=batch["cyls"], bones=batch["bones"], cams=batch["cams"], N_uniques=batch["N_uniques"],
+                                perturb=a.perturb, N_importance=a.N_importance, raw_noise_std=a.raw_noise_std)
+        finally:
+            net.pose_kernels = False
         # every rank holds 1/world of the batch: mean-reduced data terms are averaged by the all-reduce; the parameter-only
         # volume penalty is identical on every rank, so averaging leaves it unchanged
         if self.fused_loss and fused_loss_supported(a, preds):

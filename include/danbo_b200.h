@@ -247,6 +247,36 @@ int danbo_graph_net_fwd(const float* pose_bones, int n_poses, const float* const
 int danbo_graph_net_bwd(int n_poses, const float* const* params, float* const* saved, const float* d_vol,
                         float* const* grads, float* work, void* stream);
 
+/* d pose from the graph net (encode_graph_inputs core/encoders.py:460-473, AxisAngtoRot6DEncoder :859-877, Embedder
+ * core/cutoff_embedder.py:62-73, mask_root gnn_backbone.py:669-670): after danbo_graph_net_bwd, with the same params,
+ * saved and work, d_pose_bones (n_poses,24,3) = d loss / d pose_bones through the layer-0 input (written; the root's row
+ * is zero).  pose_bones is the axis-angle the forward call read. */
+int danbo_graph_net_bwd_pose(const float* pose_bones, int n_poses, const float* const* params, float* const* saved,
+                             const float* work, float* d_pose_bones, void* stream);
+
+/* Pose layer (PoseOptLayer.calculate_kinematic core/pose_opt.py:210-224,264-339; axis_angle_to_matrix
+ * core/utils/skeleton_utils.py:411-418) for n_poses poses, pose g being frame idx[g * idx_stride] (int64).  Parameters:
+ * pelvis (F,3) and bones (F,24,3) axis-angle, or with the multi-view split root_bones (F,3), bones (U,23,3) and kp_map
+ * (F, int64; both NULL otherwise).  rest_pose (n_rest,24,3); with n_rest > 1 frame f uses row rest_idx[f] (int64).
+ * Writes kps (n_poses,24,3), the gathered axis-angle bones_out (n_poses,24,3) and skts (n_poses,24,4,4) = the rigid
+ * inverse of the local-to-world matrices.  stats (or NULL) = { kp_loss, MPJPC } (Trainer._compute_kp_loss
+ * core/trainer.py:446-505 without the temporal term: coef * mean over poses and joints 1..23 of
+ * sum_c max((anchor_bones - bones)^2 - tol, 0), and the mean |anchor_kps - kps| / ext_scale), anchors (F,24,3). */
+int danbo_pose_fwd(const float* pelvis, const float* bones, const float* root_bones, const long long* kp_map,
+                   const float* rest_pose, int n_rest, const long long* rest_idx, const long long* idx, int idx_stride,
+                   int n_poses, const float* anchor_kps, const float* anchor_bones, float tol, float coef,
+                   float ext_scale, float* kps, float* bones_out, float* skts, float* stats, void* stream);
+
+/* Backward of danbo_pose_fwd (same layer arguments): d_skts (n_poses,24,4,4; the homogeneous row is ignored), d_bones
+ * (n_poses,24,3) or NULL, d_kps (n_poses,24,3) or NULL, and, when d_reg (a device scalar, d loss / d kp_loss) is not
+ * NULL, the regulariser's gradient with anchor_bones, tol and coef.  ADDS (atomics) into g_pelvis (F,3) and g_bones
+ * (F,24,3), or g_root_bones (F,3) and g_bones (U,23,3) with the multi-view split. */
+int danbo_pose_bwd(const float* pelvis, const float* bones, const float* root_bones, const long long* kp_map,
+                   const float* rest_pose, int n_rest, const long long* rest_idx, const long long* idx, int idx_stride,
+                   int n_poses, const float* d_skts, const float* d_bones, const float* d_kps,
+                   const float* anchor_bones, const float* d_reg, float tol, float coef, float* g_pelvis,
+                   float* g_bones, float* g_root_bones, void* stream);
+
 /* L*: the trainer's losses on the outputs of the path, value and gradients in one launch (core/trainer.py:396-422
  * _compute_nerf_loss with loss_fn L1 (loss_kind 0) or MSE (1) on rgb + (1 - acc) bg for the fine and, if rgb0 != NULL,
  * the coarse maps; :507-536 _compute_soft_softmax_loss when confd != NULL; :538-553 _compute_volume_scale_loss when
