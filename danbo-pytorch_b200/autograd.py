@@ -9,6 +9,12 @@ PyTorch ops when the pose itself needs a gradient): its output `vol` is an input
 The per-pose world-to-bone matrices are an input too: when they require a gradient (the pose layer under --opt_pose,
 core/trainer.py:314-341) `danbo_field_agg_bwd` also accumulates d loss / d skts, and with root-local view directions
 (perfcap configs) `danbo_view_root_bwd` adds the view branch's part.
+
+When no network parameter needs a gradient and the poses do (training.PoseFitStep fits poses to a frozen field), both
+nodes take the pose-only path: the same data-gradient chain through compositing, MLP, field and graph net, with the
+kernel variants that form no weight gradient (no K = rows GEMMs, transposes, bias sums, aggregation-net or graph-net
+weight atomics, no ray-bias backward) and a transposed weight pack that is keyed on the weights instead of redone per
+call (RayCaster._packed_dgrad).
 """
 import torch
 
@@ -24,6 +30,22 @@ OTHER_NAMES = ["framecodes.codes.weight", "graph_net.axis_scale"]
 PARAM_NAMES = MLP_NAMES + AGG_NAMES + OTHER_NAMES
 OUT_KEYS = ["rgb_map", "disp_map", "acc_map", "alpha", "T_i", "rgb0", "disp0", "acc0", "alpha0", "confd", "part_invalid"]
 DIFF_KEYS = ("rgb_map", "acc_map", "rgb0", "acc0", "confd")
+N_TRAINED = len(MLP_NAMES) + len(AGG_NAMES)      # parameters every training configuration trains (OTHER_NAMES may not)
+
+
+def weight_grads(flags, core=None):
+    """Whether a backward node trains the network's weights, from the requires-grad flags of its parameter inputs.
+    True when each of the first `core` flags (default: all) is set - the others may be constants, as axis_scale without
+    opt_scale or the zero code table of a field without frame codes; False when no flag is set (the pose-only path).
+    Anything in between is refused: a backward that trains some of the field's weights is not implemented."""
+    flags = [bool(f) for f in flags]
+    core = len(flags) if core is None else int(core)
+    if all(flags[:core]):
+        return True
+    if not any(flags):
+        return False
+    raise NotImplementedError("a backward in which only some of the field's parameters need a gradient is not implemented: "
+                              "train all of them (training.TrainStep) or none (training.PoseFitStep)")
 
 
 class _RenderBlock(torch.autograd.Function):
@@ -56,6 +78,8 @@ class _RenderBlock(torch.autograd.Function):
         g_rgb0, g_acc0 = cg(g["rgb0"], n, 3), cg(g["acc0"], n)
         g_confd = None if g["confd"] is None else g["confd"].contiguous().float()
         P = dict(zip(PARAM_NAMES, ctx.params))
+        if not weight_grads(ctx.needs_input_grad[4:], N_TRAINED):
+            return _RenderBlock._pose_only(ctx, P, g_rgb, g_acc, g_rgb0, g_acc0, g_confd)
         # Every backward kernel ACCUMULATES into its gradient buffers.  When the trainer keeps all gradients in one flat,
         # pre-zeroed bucket (parallel.GradBucket, opted in through caster.grads_in_place) the kernels add straight into
         # the parameters' .grad views and this node returns no parameter gradients: that removes one zero-fill and one
@@ -152,6 +176,60 @@ class _RenderBlock(torch.autograd.Function):
             return (None, None, d_vol, d_skts) + (None,) * len(PARAM_NAMES)
         return (None, None, d_vol, d_skts) + tuple(G[name] for name in PARAM_NAMES)
 
+    @staticmethod
+    def _pose_only(ctx, P, g_rgb, g_acc, g_rgb0, g_acc0, g_confd):
+        """Backward to d vol and d skts only.  Compositing as in training; per pass the dX-only MLP chain (head backward
+        only where d ray_bias is read: root-local view directions) and the field backward without the aggregation-net
+        and axis-scale accumulators; no ray-bias backward; danbo_view_root_bwd on root-local view directions."""
+        if K.BACKWARD_IMPL != "tc":
+            raise NotImplementedError("the pose-only backward runs on the tensor-core MLP kernels (BACKWARD_IMPL='tc')")
+        k = ctx.keep
+        rays, dev = k["rays"], k["rays"].device
+        n, S_c, S_f = rays.shape[0], k["S_c"], k["S_f"]
+        zeros = lambda *s: torch.zeros(*s, device=dev, dtype=torch.float32)
+        d_raw0, d_raw1 = zeros(n * S_c + n, 4), zeros(n * S_f, 4)
+        gl0 = gl1 = None
+        if g_confd is not None:
+            gl0 = torch.empty(n * S_c, K.J, device=dev, dtype=torch.float32)
+            gl1 = torch.empty(n * S_f, K.J, device=dev, dtype=torch.float32)
+        K.merge_composite_bwd(rays, S_c, S_f, k["raw0"], k["mask0"], k["raw1"], k["mask1"], k["z_all"], k["order"],
+                              k["noise1"], k["inv_B"], g_rgb, g_acc, g_confd, d_raw0, d_raw1, gl0, gl1)
+        K.composite_bwd(rays, S_c, k["raw0"], k["mask0"], k["z0"], k["noise0"], k["inv_B"], g_rgb0, g_acc0, d_raw0)
+        d_vol = zeros(*ctx.vol_shape)
+        grads = [None] * 7 + [d_vol[k["p0"]:], None]
+        d_skts = zeros(*k["p_skts"].shape) if ctx.needs_input_grad[3] else None
+        view_root = d_skts is not None and getattr(ctx.caster, "view_mode", "world") == "root_local"
+        d_ray_bias = zeros(n, 128) if view_root else None
+        packed_t = ctx.caster._packed_dgrad()
+        cur = torch.cuda.current_stream(dev)
+        side2 = None
+        if K.BACKWARD_STREAMS > 1:
+            # as in training: the coarse pass's field backward overlaps the fine pass's MLP backward
+            side2 = getattr(ctx.caster, "_bwd_side_stream2", None)
+            if side2 is None or side2.device != dev:
+                side2 = ctx.caster._bwd_side_stream2 = torch.cuda.Stream(device=dev)
+        alive = []
+        for ip, (d_raw, S, z, mask, act, fo, sv, gl) in enumerate((
+                (d_raw0, S_c, k["z0"], k["mask0"], k["act0"], k["f0"], k["sv0"], gl0),
+                (d_raw1, S_f, k["z1"], k["mask1"], k["act1"], k["f1"], k["sv1"], gl1))):
+            dX = K.mlp_backward_pose(P, d_raw, act, fo, sv, packed_t, d_ray_bias)
+            alive.append(dX)
+            if side2 is not None and ip == 0:
+                side2.wait_stream(cur)
+                with torch.cuda.stream(side2):
+                    K.field_agg_bwd(rays, S, z, mask, act, k["p_skts"], k["p_vol"], k["skip"], k["consts"], fo, dX, gl,
+                                    grads, d_skts=d_skts)
+            else:
+                K.field_agg_bwd(rays, S, z, mask, act, k["p_skts"], k["p_vol"], k["skip"], k["consts"], fo, dX, gl,
+                                grads, d_skts=d_skts)
+        if side2 is not None:
+            cur.wait_stream(side2)
+        if view_root:
+            K.view_root_bwd(rays, k["p_skts"], k["skip"], P["views_linears.0.weight"], d_ray_bias, d_skts)
+        ctx.keep = None
+        del alive
+        return (None, None, d_vol if ctx.needs_input_grad[2] else None, d_skts) + (None,) * len(PARAM_NAMES)
+
 
 def render_block_with_grad(caster, rays, skip, pose_skts, pose_cyls, vol, cam_idx, codes, consts, packed, S_c, S_f, B,
                            raw_noise_std, perturb, nanmean_chunk, rand, stages, lindisp=False):
@@ -164,6 +242,7 @@ def render_block_with_grad(caster, rays, skip, pose_skts, pose_cyls, vol, cam_id
         named["views_linears.0.weight"] = torch.nn.functional.pad(named["views_linears.0.weight"], (0, 128))
         named["framecodes.codes.weight"] = torch.zeros(1, 128, device=rays.device)
     params = [named[n] for n in PARAM_NAMES]
+    weight_grads([p.requires_grad for p in params], N_TRAINED)          # a mixed set is refused before any launch
     cfg = dict(rays=rays, skip=skip, pose_cyls=pose_cyls, cam_idx=cam_idx, codes=codes, consts=consts,
                packed=packed, S_c=S_c, S_f=S_f, B=B, raw_noise_std=raw_noise_std, perturb=perturb,
                nanmean_chunk=nanmean_chunk, rand=rand, stages=stages, lindisp=lindisp)
@@ -188,6 +267,12 @@ class _GraphNet(torch.autograd.Function):
     @staticmethod
     def backward(ctx, d_vol):
         params = ctx.params
+        if not weight_grads(ctx.needs_input_grad[2:]):
+            # pose-only (training.PoseFitStep): the transposed products only, then d pose as below
+            work = K.graph_net_bwd(ctx.saved_bufs, d_vol, None)
+            d_pose = K.graph_net_bwd_pose(ctx.saved_bufs, work, ctx.pose_bones)
+            ctx.saved_bufs = ctx.pose_bones = None
+            return (None, d_pose) + (None,) * len(params)
         # same contract as _RenderBlock: with a pre-zeroed flat gradient bucket the kernels add straight into .grad
         in_place = bool(getattr(ctx.net, "grads_in_place", False)) and all(
             p.grad is not None and p.grad.dtype == torch.float32 and p.grad.is_contiguous() and p.grad.shape == p.shape
@@ -206,6 +291,7 @@ def graph_net_volumes(net, pose_bones):
     named = dict(net.graph_net.named_parameters())
     params = [named[n] for n in K.GN_GRADS]
     if torch.is_grad_enabled() and (pose_bones.requires_grad or any(p.requires_grad for p in params)):
+        weight_grads([p.requires_grad for p in params])                  # a mixed set is refused before any launch
         return _GraphNet.apply(net, pose_bones, *params)
     named["layers.0.adj"], named["layers.1.adj"] = net.graph_net.layers[0].adj, net.graph_net.layers[1].adj
     return K.graph_net_fwd(pose_bones, [named[n].detach() for n in K.GN_PARAMS])[0]

@@ -112,8 +112,10 @@ __device__ __forceinline__ float tile_colsum(const float* T, int lane) {
 }
 
 // kSoftmax: agg_mode 1 (dense pair lists, blend weight of the pair from the row's masked softmax); the sigmoid
-// instantiation carries none of that code.
-template <bool kSoftmax>
+// instantiation carries none of that code.  kWeightGrads = false (pose-only backward, the field is frozen): the
+// aggregation net's weight / bias tile sums and atomics and the axis-scale gradient are compiled out; the backward
+// through the three layers to each pair's d x, and from there to d vol and d skts, stays.
+template <bool kSoftmax, bool kWeightGrads>
 __global__ void __launch_bounds__(128)
 pair_logits_bwd_kernel(const float* __restrict__ rays, int ray_stride, int S, const float* __restrict__ z,
                        const int* __restrict__ active_ids, const float* __restrict__ pose_skts,
@@ -192,45 +194,51 @@ pair_logits_bwd_kernel(const float* __restrict__ rays, int ray_stride, int S, co
         if (!live) da = 0.f;
 #pragma unroll
         for (int o = 0; o < DANBO_AGG_W; ++o) {
-            const float o2 = fmaxf(d1[o], 0.f);
-            T1[lane * kTileLd + o] = da * o2;                           // -> dW2
+            if (kWeightGrads) T1[lane * kTileLd + o] = da * fmaxf(d1[o], 0.f);          // -> dW2
             d1[o] = d1[o] > 0.f ? da * __ldg(fc.agg_w2 + j * DANBO_AGG_W + o) : 0.f;   // delta1
-            T2[lane * kTileLd + o] = d1[o];
+            if (kWeightGrads) T2[lane * kTileLd + o] = d1[o];
         }
-        __syncwarp();
-        atomicAdd(G.w2 + j * DANBO_AGG_W + lane, tile_colsum(T1, lane));
-        atomicAdd(G.b1 + j * DANBO_AGG_W + lane, tile_colsum(T2, lane));
-        { const float s = warp_sum(da); if (lane == 0) atomicAdd(G.b2 + j, s); }
-        __syncwarp();
-        // ---- layer 1 backward: dW1[j][i][o] += o1[i] delta1[o];  d o1[i] = sum_o delta1[o] W1[j][i][o]
+        if (kWeightGrads) {
+            __syncwarp();
+            atomicAdd(G.w2 + j * DANBO_AGG_W + lane, tile_colsum(T1, lane));
+            atomicAdd(G.b1 + j * DANBO_AGG_W + lane, tile_colsum(T2, lane));
+            { const float s = warp_sum(da); if (lane == 0) atomicAdd(G.b2 + j, s); }
+            __syncwarp();
+            // ---- layer 1 backward: dW1[j][i][o] += o1[i] delta1[o];  d o1[i] = sum_o delta1[o] W1[j][i][o]
 #pragma unroll
-        for (int o = 0; o < DANBO_AGG_W; ++o) T1[lane * kTileLd + o] = mix[o];      // o1 of every pair
-        __syncwarp();
-        {
-            float acc[DANBO_AGG_W];                      // lane = weight row i
+            for (int o = 0; o < DANBO_AGG_W; ++o) T1[lane * kTileLd + o] = mix[o];      // o1 of every pair
+            __syncwarp();
+            {
+                float acc[DANBO_AGG_W];                      // lane = weight row i
 #pragma unroll
-            for (int o = 0; o < DANBO_AGG_W; ++o) acc[o] = 0.f;
-            for (int p = 0; p < 32; ++p) {
-                const float a = T1[p * kTileLd + lane];
+                for (int o = 0; o < DANBO_AGG_W; ++o) acc[o] = 0.f;
+                for (int p = 0; p < 32; ++p) {
+                    const float a = T1[p * kTileLd + lane];
 #pragma unroll
-                for (int o = 0; o < DANBO_AGG_W; ++o) acc[o] = fmaf(a, T2[p * kTileLd + o], acc[o]);
+                    for (int o = 0; o < DANBO_AGG_W; ++o) acc[o] = fmaf(a, T2[p * kTileLd + o], acc[o]);
+                }
+#pragma unroll
+                for (int o = 0; o < DANBO_AGG_W; ++o) atomicAdd(G.w1 + ((size_t)j * DANBO_AGG_W + lane) * DANBO_AGG_W + o, acc[o]);
             }
-#pragma unroll
-            for (int o = 0; o < DANBO_AGG_W; ++o) atomicAdd(G.w1 + ((size_t)j * DANBO_AGG_W + lane) * DANBO_AGG_W + o, acc[o]);
+            __syncwarp();
         }
-        __syncwarp();
         float d0[DANBO_AGG_W];                           // delta0 = d o1 * [o1 > 0]
 #pragma unroll
         for (int i = 0; i < DANBO_AGG_W; ++i) {
             float s = 0.f;
+            // a plain load in the pose-only variant: with no atomics in between, ptxas would otherwise keep all 1 024 W1
+            // values of the forward recompute's __ldg loads live for this loop (255 registers, 2.6 KB of spills)
 #pragma unroll
-            for (int o = 0; o < DANBO_AGG_W; ++o) s = fmaf(d1[o], __ldg(w1 + i * DANBO_AGG_W + o), s);
+            for (int o = 0; o < DANBO_AGG_W; ++o)
+                s = fmaf(d1[o], kWeightGrads ? __ldg(w1 + i * DANBO_AGG_W + o) : w1[i * DANBO_AGG_W + o], s);
             d0[i] = mix[i] > 0.f ? s : 0.f;
-            T2[lane * kTileLd + i] = d0[i];
+            if (kWeightGrads) T2[lane * kTileLd + i] = d0[i];
         }
-        __syncwarp();
-        atomicAdd(G.b0 + lane, tile_colsum(T2, lane));
-        __syncwarp();
+        if (kWeightGrads) {
+            __syncwarp();
+            atomicAdd(G.b0 + lane, tile_colsum(T2, lane));
+            __syncwarp();
+        }
         // ---- layer 0 + adjacency mix + feature gather, per tree neighbour
         for (uint32_t nb = kNbrMask[j]; nb;) {
             const int k = __ffs(nb) - 1; nb &= nb - 1;
@@ -250,26 +258,28 @@ pair_logits_bwd_kernel(const float* __restrict__ rays, int ray_stride, int S, co
                 dadj = fmaf(h[i], s, dadj);
                 dh[i] = adj * s;
             }
-            { const float s = warp_sum(live ? dadj : 0.f); if (lane == 0) atomicAdd(G.adjw + j * DANBO_J + k, s * adjm); }
-            // dW0[k][i][o] += h[i] * adj * delta0[o]: tiles T1 = h (15 cols), T2 = adj * delta0
+            if (kWeightGrads) {
+                { const float s = warp_sum(live ? dadj : 0.f); if (lane == 0) atomicAdd(G.adjw + j * DANBO_J + k, s * adjm); }
+                // dW0[k][i][o] += h[i] * adj * delta0[o]: tiles T1 = h (15 cols), T2 = adj * delta0
 #pragma unroll
-            for (int i = 0; i < DANBO_FEAT; ++i) T1[lane * kTileLd + i] = live ? h[i] : 0.f;
+                for (int i = 0; i < DANBO_FEAT; ++i) T1[lane * kTileLd + i] = live ? h[i] : 0.f;
 #pragma unroll
-            for (int o = 0; o < DANBO_AGG_W; ++o) T2[lane * kTileLd + o] = adj * d0[o];
-            __syncwarp();
-            {
-                float acc[DANBO_FEAT];                   // lane = output unit o
+                for (int o = 0; o < DANBO_AGG_W; ++o) T2[lane * kTileLd + o] = adj * d0[o];
+                __syncwarp();
+                {
+                    float acc[DANBO_FEAT];                   // lane = output unit o
 #pragma unroll
-                for (int i = 0; i < DANBO_FEAT; ++i) acc[i] = 0.f;
-                for (int p = 0; p < 32; ++p) {
-                    const float t = T2[p * kTileLd + lane];
+                    for (int i = 0; i < DANBO_FEAT; ++i) acc[i] = 0.f;
+                    for (int p = 0; p < 32; ++p) {
+                        const float t = T2[p * kTileLd + lane];
 #pragma unroll
-                    for (int i = 0; i < DANBO_FEAT; ++i) acc[i] = fmaf(T1[p * kTileLd + i], t, acc[i]);
+                        for (int i = 0; i < DANBO_FEAT; ++i) acc[i] = fmaf(T1[p * kTileLd + i], t, acc[i]);
+                    }
+#pragma unroll
+                    for (int i = 0; i < DANBO_FEAT; ++i) atomicAdd(G.w0 + ((size_t)k * DANBO_FEAT + i) * DANBO_AGG_W + lane, acc[i]);
                 }
-#pragma unroll
-                for (int i = 0; i < DANBO_FEAT; ++i) atomicAdd(G.w0 + ((size_t)k * DANBO_FEAT + i) * DANBO_AGG_W + lane, acc[i]);
+                __syncwarp();
             }
-            __syncwarp();
             if (k == j && live) {                        // direct path: hbar = sum_j p_j h_j
 #pragma unroll
                 for (int i = 0; i < DANBO_FEAT; ++i) dh[i] = fmaf(pj, d_hbar[(size_t)row * 16 + i], dh[i]);
@@ -300,9 +310,11 @@ pair_logits_bwd_kernel(const float* __restrict__ rays, int ray_stride, int S, co
                 }
                 dxa *= 0.5f * (float)DANBO_RES;                      // d iy / d x
                 const float sc = __ldg(fc.axis_scale + k * 3 + a);
-                // x = t / |s|  ->  d x / d s = -x / |s| * sign(s) = -x / s
-                const float ds = warp_sum(live ? -dxa * x[a] / sc : 0.f);
-                if (lane == 0) atomicAdd(G.axis_scale + k * 3 + a, ds);
+                if (kWeightGrads) {
+                    // x = t / |s|  ->  d x / d s = -x / |s| * sign(s) = -x / s
+                    const float ds = warp_sum(live ? -dxa * x[a] / sc : 0.f);
+                    if (lane == 0) atomicAdd(G.axis_scale + k * 3 + a, ds);
+                }
                 dt[a] = live ? dxa / fabsf(sc) : 0.f;
             }
             if (G.skts != nullptr) {
@@ -353,7 +365,8 @@ static FieldConsts make_consts_b(const float* const* p) {
 
 // grads[10] = { d_w0 (24,15,32), d_adj_w (24,24), d_b0 (32), d_w1 (24,32,32), d_b1 (24,32), d_w2 (24,32), d_b2 (24),
 //               d_vol (n_poses,24,240), d_axis_scale (24,3), d_skts (n_poses,24,4,4) or NULL }: fp32 accumulators, added
-//               to (zero them first).  d_skts = NULL (poses are constants) skips that gradient.
+//               to (zero them first).  d_skts = NULL (poses are constants) skips that gradient.  grads[0..6] and
+//               grads[8] all NULL (all or none) select the pose-only variant: no aggregation-net or axis-scale gradient.
 // work / pair_capacity: the SAME workspace the forward danbo_field_agg call filled (pair lists are reused).
 extern "C" int danbo_field_agg_bwd(const float* rays, int ray_stride, int n_rays, int S, const float* z,
                                    const unsigned int* mask, const int* active_ids, const int* active_count,
@@ -364,6 +377,11 @@ extern "C" int danbo_field_agg_bwd(const float* rays, int ray_stride, int n_rays
                                    void* stream) {
     if (capacity <= 0) return 0;
     if (agg_mode < 0 || agg_mode > 1) return -1;
+    if (grads == nullptr || grads[7] == nullptr) return -1;
+    int n_weight = grads[8] != nullptr;
+    for (int i = 0; i < 7; ++i) n_weight += grads[i] != nullptr;
+    if (n_weight != 0 && n_weight != 8) return -1;
+    const bool wg = n_weight == 8;
     cudaStream_t st = (cudaStream_t)stream;
     const FieldConsts fc = make_consts_b(consts);
     int rblocks = (capacity + 127) / 128;
@@ -376,14 +394,10 @@ extern "C" int danbo_field_agg_bwd(const float* rays, int ray_stride, int n_rays
     PairWork pw{const_cast<int*>(work)};
     int pblocks = (pair_capacity / 32 + 3) / 4;
     if (pblocks > num_sms * 4) pblocks = num_sms * 4;
-    if (agg_mode == 1)
-        pair_logits_bwd_kernel<true><<<pblocks, 128, 0, st>>>(rays, ray_stride, S, z, active_ids, pose_skts, pose_vol,
-                                                               rays_per_pose, n_poses, fc, pw, pair_capacity, logits,
-                                                               d_logit, d_hbar, G, mask);
-    else
-        pair_logits_bwd_kernel<false><<<pblocks, 128, 0, st>>>(rays, ray_stride, S, z, active_ids, pose_skts, pose_vol,
-                                                                rays_per_pose, n_poses, fc, pw, pair_capacity, logits,
-                                                                d_logit, d_hbar, G, mask);
+    auto kern = agg_mode == 1 ? (wg ? pair_logits_bwd_kernel<true, true> : pair_logits_bwd_kernel<true, false>)
+                              : (wg ? pair_logits_bwd_kernel<false, true> : pair_logits_bwd_kernel<false, false>);
+    kern<<<pblocks, 128, 0, st>>>(rays, ray_stride, S, z, active_ids, pose_skts, pose_vol, rays_per_pose, n_poses, fc, pw,
+                                  pair_capacity, logits, d_logit, d_hbar, G, mask);
     DANBO_CHECK_LAUNCH();
     return 0;
 }

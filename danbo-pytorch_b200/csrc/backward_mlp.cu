@@ -159,6 +159,9 @@ colsum_kernel(const float* __restrict__ A, int lda, float* __restrict__ db, cons
 // Heads.  One warp per row.
 //   d_raw (per sample id, 4) -> delta9 (rows,128) = (d_rgb . W_rgb) * [g > 0];  d_a7 (rows,256) = d_sigma * w_alpha
 //   grads: rgb_linear (3,128)+(3), alpha_linear (256)+(1); d ray_bias[ray] += delta9
+// kHeadGrads / kRayBias = false compile those reductions / that output out (pose-only backward: the heads are frozen,
+// and d ray_bias is needed only where the view directions depend on the pose).
+template <bool kHeadGrads, bool kRayBias>
 __global__ void __launch_bounds__(256)
 head_bwd_kernel(const float* __restrict__ d_raw, const int* __restrict__ row_sample, const int* __restrict__ row_ray,
                 const int* __restrict__ rows_ptr, const __nv_bfloat16* __restrict__ g_save /* (rows,128) */,
@@ -169,11 +172,13 @@ head_bwd_kernel(const float* __restrict__ d_raw, const int* __restrict__ row_sam
     const int R = *rows_ptr;
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
     __shared__ float s_wrgb[3][128], s_walpha[256], s_brgb[3], s_balpha;
-    for (int i = threadIdx.x; i < 384; i += 256) s_wrgb[i / 128][i % 128] = 0.f;
-    for (int i = threadIdx.x; i < 256; i += 256) s_walpha[i] = 0.f;
-    if (threadIdx.x < 3) s_brgb[threadIdx.x] = 0.f;
-    if (threadIdx.x == 0) s_balpha = 0.f;
-    __syncthreads();
+    if (kHeadGrads) {
+        for (int i = threadIdx.x; i < 384; i += 256) s_wrgb[i / 128][i % 128] = 0.f;
+        for (int i = threadIdx.x; i < 256; i += 256) s_walpha[i] = 0.f;
+        if (threadIdx.x < 3) s_brgb[threadIdx.x] = 0.f;
+        if (threadIdx.x == 0) s_balpha = 0.f;
+        __syncthreads();
+    }
     for (int r = blockIdx.x * 8 + wib; r < R; r += gridDim.x * 8) {
         const float4 g = reinterpret_cast<const float4*>(d_raw)[row_sample[r]];
         const int ray = row_ray[r];
@@ -183,17 +188,18 @@ head_bwd_kernel(const float* __restrict__ d_raw, const int* __restrict__ row_sam
             const float gv = __bfloat162float(g_save[(size_t)r * 128 + c]);
             const float d = gv > 0.f ? (g.x * w_rgb[c] + g.y * w_rgb[128 + c] + g.z * w_rgb[256 + c]) : 0.f;
             if (delta9) delta9[(size_t)r * 128 + c] = d;
-            atomicAdd(d_ray_bias + (size_t)ray * 128 + c, d);
-            atomicAdd(&s_wrgb[0][c], g.x * gv); atomicAdd(&s_wrgb[1][c], g.y * gv); atomicAdd(&s_wrgb[2][c], g.z * gv);
+            if (kRayBias) atomicAdd(d_ray_bias + (size_t)ray * 128 + c, d);
+            if (kHeadGrads) { atomicAdd(&s_wrgb[0][c], g.x * gv); atomicAdd(&s_wrgb[1][c], g.y * gv); atomicAdd(&s_wrgb[2][c], g.z * gv); }
         }
 #pragma unroll
         for (int q = 0; q < 8; ++q) {
             const int c = lane + 32 * q;
             if (d_a7) d_a7[(size_t)r * 256 + c] = g.w * w_alpha[c];
-            atomicAdd(&s_walpha[c], g.w * __bfloat162float(a7_save[(size_t)r * 256 + c]));
+            if (kHeadGrads) atomicAdd(&s_walpha[c], g.w * __bfloat162float(a7_save[(size_t)r * 256 + c]));
         }
-        if (lane == 0) { atomicAdd(&s_brgb[0], g.x); atomicAdd(&s_brgb[1], g.y); atomicAdd(&s_brgb[2], g.z); atomicAdd(&s_balpha, g.w); }
+        if (kHeadGrads && lane == 0) { atomicAdd(&s_brgb[0], g.x); atomicAdd(&s_brgb[1], g.y); atomicAdd(&s_brgb[2], g.z); atomicAdd(&s_balpha, g.w); }
     }
+    if (!kHeadGrads) return;
     __syncthreads();
     for (int i = threadIdx.x; i < 384; i += 256) atomicAdd(d_w_rgb + i, s_wrgb[i / 128][i % 128]);
     for (int i = threadIdx.x; i < 256; i += 256) atomicAdd(d_w_alpha + i, s_walpha[i]);
@@ -470,9 +476,15 @@ extern "C" int danbo_mlp_head_bwd(const float* d_raw, const int* row_sample, con
                                   const float* w_alpha, float* delta9, float* d_a7, float* d_w_rgb, float* d_b_rgb,
                                   float* d_w_alpha, float* d_b_alpha, float* d_ray_bias, int num_sms, void* stream) {
     if (max_rows <= 0) return 0;
+    const int n_head = (d_w_rgb != nullptr) + (d_b_rgb != nullptr) + (d_w_alpha != nullptr) + (d_b_alpha != nullptr);
+    if (n_head != 0 && n_head != 4) return -1;
+    const bool head = n_head == 4, rb = d_ray_bias != nullptr;
+    if (!head && !rb && delta9 == nullptr && d_a7 == nullptr) return 0;      // nothing asked for: no launch
     int blocks = (max_rows + 7) / 8;
     if (blocks > num_sms * 4) blocks = num_sms * 4;
-    bwd::head_bwd_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(
+    auto kern = head ? (rb ? bwd::head_bwd_kernel<true, true> : bwd::head_bwd_kernel<true, false>)
+                     : (rb ? bwd::head_bwd_kernel<false, true> : bwd::head_bwd_kernel<false, false>);
+    kern<<<blocks, 256, 0, (cudaStream_t)stream>>>(
         d_raw, row_sample, row_ray, rows_dev, (const __nv_bfloat16*)g_save, (const __nv_bfloat16*)a7_save, w_rgb, w_alpha,
         delta9, d_a7, d_w_rgb, d_b_rgb, d_w_alpha, d_b_alpha, d_ray_bias);
     DANBO_CHECK_LAUNCH();

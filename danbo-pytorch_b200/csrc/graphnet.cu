@@ -173,8 +173,10 @@ fwd_kernel(const float* __restrict__ bones, int G, Params P, Saved S, float* __r
 // ---- backward ---------------------------------------------------------------------------------------------------
 // MODE 3: d out -> dW3, db3, d pre2.   MODE 2: d pre2 -> dW2, db2, d pre1, db1.   MODE 1: d pre1 -> (un-mix) d lin1 ->
 // dA1, dW1, d pre0, db0.   MODE 0: d pre0 -> d lin0 -> dA0, dW0.   Block = (node, 16-row slice of its weight matrix,
-// pose group).
-template <int MODE>
+// pose group).  kGrads = false (pose-only backward, the graph net is frozen): the transposed products only, i.e. MODE
+// 3..1 leave d pre2, d pre1 and d pre0 (what bwd_pose_kernel reads) and no weight, bias or adjacency gradient; MODE 0
+// then has nothing to do and is not launched.
+template <int MODE, bool kGrads>
 __global__ void __launch_bounds__(kThreads)
 bwd_kernel(int G, Params P, Saved S, const float* __restrict__ d_in, Grads Gr, float* __restrict__ d_next) {
     constexpr int n_in = MODE == 0 ? kIn : kW;              // rows of the weight matrix
@@ -202,7 +204,7 @@ bwd_kernel(int G, Params P, Saved S, const float* __restrict__ d_in, Grads Gr, f
         const int c = tid & (kW - 1), half = tid >> 7;
 #pragma unroll
         for (int u = 0; u < kG / 2; ++u) d_s[(half * (kG / 2) + u) * pd + c] = dl[u];
-        if (first) {
+        if (kGrads && first) {
             // d A[j][node] = sum_{g,c} d pre[g][j][c] lin[g][node][c];  d adj_w = d A * adj
             const float* lin = MODE == 1 ? S.lin1 : S.lin0;
             float* d_adjw = MODE == 1 ? Gr.adjw1 : Gr.adjw0;
@@ -252,7 +254,7 @@ bwd_kernel(int G, Params P, Saved S, const float* __restrict__ d_in, Grads Gr, f
     // ---- dW[i][c] += sum_g act[g][i] d[g][c] for the slice's rows: one owner thread per entry
     float* dW = MODE == 3 ? Gr.w3 + (size_t)node * kW * kOut : MODE == 2 ? Gr.w2 + (size_t)node * kW * kW
               : MODE == 1 ? Gr.w1 + (size_t)node * kW * kW : Gr.w0 + (size_t)node * kIn * kW;
-    for (int e = tid; e < nr * n_out; e += kThreads) {
+    for (int e = tid; kGrads && e < nr * n_out; e += kThreads) {
         const int il = e / n_out, c = e - il * n_out;
         float s = 0.f;
 #pragma unroll
@@ -261,7 +263,7 @@ bwd_kernel(int G, Params P, Saved S, const float* __restrict__ d_in, Grads Gr, f
         if (excl) *dst += s; else atomicAdd(dst, s);
     }
     // ---- per-joint bias of layers 2 and 3
-    if (MODE >= 2 && first) {
+    if (kGrads && MODE >= 2 && first) {
         float* db = MODE == 3 ? Gr.b3 + node * kOut : Gr.b2 + node * kW;
         for (int c = tid; c < n_out; c += kThreads) {
             float s = 0.f;
@@ -279,7 +281,7 @@ bwd_kernel(int G, Params P, Saved S, const float* __restrict__ d_in, Grads Gr, f
         float v = a_s[g * kSlice + il] > 0.f ? (MODE == 1 ? s + s : s) : 0.f;      // n1 = relu(2 pre0)
         if (g >= ng || il >= nr) v = 0.f;
         if (g < ng && il < nr) d_next[((size_t)(g0 + g) * DANBO_J + node) * kW + i0 + il] = v;
-        if (MODE <= 2) {                                     // shared biases b1 / b0: summed over poses and nodes
+        if (kGrads && MODE <= 2) {                           // shared biases b1 / b0: summed over poses and nodes
             float sb = v;
 #pragma unroll
             for (int o = kG / 2; o > 0; o >>= 1) sb += __shfl_xor_sync(0xffffffffu, sb, o);
@@ -377,26 +379,38 @@ extern "C" int danbo_graph_net_fwd(const float* pose_bones, int n_poses, const f
     return 0;
 }
 
+// grads = NULL: the pose-only variant (three launches, no weight gradients); work then still holds d pre0 for
+// danbo_graph_net_bwd_pose.
 extern "C" int danbo_graph_net_bwd(int n_poses, const float* const* params, float* const* saved, const float* d_vol,
                                    float* const* grads, float* work /* 2 * n_poses*24*128 floats */, void* stream) {
     if (n_poses <= 0) return 0;
-    if (!params || !saved || !d_vol || !grads || !work) return -1;
+    if (!params || !saved || !d_vol || !work) return -1;
     cudaStream_t st = (cudaStream_t)stream;
     const gn::Params P = gn_params(params);
     const gn::Saved S = gn_saved(saved);
-    const gn::Grads Gr{grads[0], grads[1], grads[2], grads[3], grads[4], grads[5], grads[6], grads[7], grads[8], grads[9]};
     float* d_pre1 = work;
     float* d_pre0 = work + (size_t)n_poses * DANBO_J * gn::kW;
     const int groups = (n_poses + gn::kG - 1) / gn::kG;
     const dim3 g128(DANBO_J, gn::kW / gn::kSlice, groups), g66(DANBO_J, (gn::kIn + gn::kSlice - 1) / gn::kSlice, groups);
+    if (grads == nullptr) {
+        const gn::Grads none{};
+        gn::bwd_kernel<3, false><<<g128, gn::kThreads, 0, st>>>(n_poses, P, S, d_vol, none, d_pre0);
+        DANBO_CHECK_LAUNCH();
+        gn::bwd_kernel<2, false><<<g128, gn::kThreads, 0, st>>>(n_poses, P, S, d_pre0, none, d_pre1);
+        DANBO_CHECK_LAUNCH();
+        gn::bwd_kernel<1, false><<<g128, gn::kThreads, 0, st>>>(n_poses, P, S, d_pre1, none, d_pre0);
+        DANBO_CHECK_LAUNCH();
+        return 0;
+    }
+    const gn::Grads Gr{grads[0], grads[1], grads[2], grads[3], grads[4], grads[5], grads[6], grads[7], grads[8], grads[9]};
     // d_pre2 lives in d_pre0's buffer: it is consumed (by <2>) before <1> writes d_pre0
-    gn::bwd_kernel<3><<<g128, gn::kThreads, 0, st>>>(n_poses, P, S, d_vol, Gr, d_pre0);
+    gn::bwd_kernel<3, true><<<g128, gn::kThreads, 0, st>>>(n_poses, P, S, d_vol, Gr, d_pre0);
     DANBO_CHECK_LAUNCH();
-    gn::bwd_kernel<2><<<g128, gn::kThreads, 0, st>>>(n_poses, P, S, d_pre0, Gr, d_pre1);
+    gn::bwd_kernel<2, true><<<g128, gn::kThreads, 0, st>>>(n_poses, P, S, d_pre0, Gr, d_pre1);
     DANBO_CHECK_LAUNCH();
-    gn::bwd_kernel<1><<<g128, gn::kThreads, 0, st>>>(n_poses, P, S, d_pre1, Gr, d_pre0);
+    gn::bwd_kernel<1, true><<<g128, gn::kThreads, 0, st>>>(n_poses, P, S, d_pre1, Gr, d_pre0);
     DANBO_CHECK_LAUNCH();
-    gn::bwd_kernel<0><<<g66, gn::kThreads, 0, st>>>(n_poses, P, S, d_pre0, Gr, nullptr);
+    gn::bwd_kernel<0, true><<<g66, gn::kThreads, 0, st>>>(n_poses, P, S, d_pre0, Gr, nullptr);
     DANBO_CHECK_LAUNCH();
     return 0;
 }

@@ -113,7 +113,8 @@ __device__ __forceinline__ void epi_dx(const EpiArgs& E) {
 }
 
 // delta stages: accumulator (+ sigma-head term) gated by the saved activation -> bf16 delta in TMEM (next A operand) + HBM
-template <bool kAlpha, bool kMask>
+// (kSave: the pose-only variant keeps the delta in TMEM only, no HBM plane and no transposed image)
+template <bool kAlpha, bool kMask, bool kSave>
 __device__ __forceinline__ void epi_delta(const EpiArgs& E) {
     uint4 m[8];
     if (kMask) {
@@ -149,15 +150,18 @@ __device__ __forceinline__ void epi_delta(const EpiArgs& E) {
             }
         }
         tmem_st16(E.act_out + 16 * gq, *reinterpret_cast<const uint32_t(*)[16]>(&pk[gq * 16]));
-        if (E.delta_out != nullptr) {
+        if (kSave && E.delta_out != nullptr) {
 #pragma unroll
             for (int i = 0; i < 4; ++i)
                 E.delta_out[gq * 4 + i] = make_uint4(pk[gq * 16 + 4 * i], pk[gq * 16 + 4 * i + 1], pk[gq * 16 + 4 * i + 2], pk[gq * 16 + 4 * i + 3]);
         }
     }
-    if (E.delta_t != nullptr) store_transposed(E.stage, E.lane, pk, E.delta_t, E.block64, E.rowgroup0, E.col0);
+    if (kSave && E.delta_t != nullptr) store_transposed(E.stage, E.lane, pk, E.delta_t, E.block64, E.rowgroup0, E.col0);
 }
 
+// kSaveDeltas = false: the pose-only variant (no weight gradients follow), whose epilogue writes dX only; delta_save and
+// delta_t are not touched.
+template <bool kSaveDeltas>
 __global__ void __launch_bounds__(kThreads, 1)
 dgrad_kernel(const uint8_t* __restrict__ wstream,            // [84][16 KB] transposed-weight tiles (pack_dgrad)
              const float* __restrict__ w_rgb, const float* __restrict__ w_alpha,
@@ -279,12 +283,12 @@ dgrad_kernel(const uint8_t* __restrict__ wstream,            // [84][16 KB] tran
                 const uint32_t a0 = tmem + lane_addr + kActCol + 32u * ch;          // buffer 0, packed columns
                 tmem_st16(a0, *reinterpret_cast<const uint32_t(*)[16]>(&pk[0]));
                 tmem_st16(a0 + 16, *reinterpret_cast<const uint32_t(*)[16]>(&pk[16]));
-                if (grow < cap) {
+                if (kSaveDeltas && grow < cap) {
                     uint4* dst = reinterpret_cast<uint4*>(delta_save + (size_t)grow * 256 + ch * 64);
 #pragma unroll
                     for (int i = 0; i < 8; ++i) dst[i] = make_uint4(pk[4 * i], pk[4 * i + 1], pk[4 * i + 2], pk[4 * i + 3]);
                 }
-                if (delta_t != nullptr && blk64 < n_blk64)
+                if (kSaveDeltas && delta_t != nullptr && blk64 < n_blk64)
                     store_transposed(stage_addr, lane, pk, delta_t, blk64, (q & 1) * 4, ch * 64);
                 tmem_wait_st();
                 tc_fence_before();
@@ -310,9 +314,9 @@ dgrad_kernel(const uint8_t* __restrict__ wstream,            // [84][16 KB] tran
                     E.dx = dX + (size_t)(valid ? grow : 0) * 208;
                     if (s == 4) epi_dx<false>(E);
                     else if (s == 10) epi_dx<true>(E);
-                    else if (s == 0) epi_delta<false, false>(E);
-                    else if (s == 1) epi_delta<true, true>(E);
-                    else epi_delta<false, true>(E);
+                    else if (s == 0) epi_delta<false, false, kSaveDeltas>(E);
+                    else if (s == 1) epi_delta<true, true, kSaveDeltas>(E);
+                    else epi_delta<false, true, kSaveDeltas>(E);
                     tmem_wait_st();
                     tc_fence_before();
                     __syncwarp();
@@ -557,27 +561,42 @@ extern "C" int danbo_pack_mlp_dgrad(const float* const* w_pts, const float* w_fe
     return 0;
 }
 
-// Fused data-gradient chain.  delta_save planes: 0 = delta of views_linears.0 (128 wide), 1 = d feature, 2..9 = deltas
-// of pts_linears.7..0.  dX (cap,208) fp32 is fully written for valid rows.
-extern "C" int danbo_mlp_dgrad(const void* wstream_t, const float* w_rgb, const float* w_alpha, const float* d_raw,
-                               const int* row_sample, const int* rows_dev, int max_rows, const void* act_save,
-                               const void* g_save, int cap, void* delta_save, void* delta_t, float* dX, int num_sms,
-                               void* stream) {
-    if (max_rows <= 0) return 0;
+template <bool kSaveDeltas>
+static int launch_dgrad(const void* wstream_t, const float* w_rgb, const float* w_alpha, const float* d_raw,
+                        const int* row_sample, const int* rows_dev, int max_rows, const void* act_save,
+                        const void* g_save, int cap, void* delta_save, void* delta_t, float* dX, int num_sms,
+                        void* stream) {
     const int smem = (int)sizeof(mlpb::Smem) + 1024;
     static bool attr = false;
     if (!attr) {
-        cudaError_t e = cudaFuncSetAttribute(mlpb::dgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+        cudaError_t e = cudaFuncSetAttribute(mlpb::dgrad_kernel<kSaveDeltas>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
         if (e != cudaSuccess) return (int)e;
         attr = true;
     }
     int tiles = (max_rows + DANBO_TILE_M - 1) / DANBO_TILE_M;
     int grid = num_sms < tiles ? num_sms : tiles;
-    mlpb::dgrad_kernel<<<grid, mlpb::kThreads, smem, (cudaStream_t)stream>>>(
+    mlpb::dgrad_kernel<kSaveDeltas><<<grid, mlpb::kThreads, smem, (cudaStream_t)stream>>>(
         (const uint8_t*)wstream_t, w_rgb, w_alpha, d_raw, row_sample, rows_dev, (const __nv_bfloat16*)act_save,
         (const __nv_bfloat16*)g_save, cap, (__nv_bfloat16*)delta_save, (uint8_t*)delta_t, dX);
     DANBO_CHECK_LAUNCH();
     return 0;
+}
+
+// Fused data-gradient chain.  delta_save planes: 0 = delta of views_linears.0 (128 wide), 1 = d feature, 2..9 = deltas
+// of pts_linears.7..0.  dX (cap,208) fp32 is fully written for valid rows.  delta_save = NULL (then delta_t must be
+// NULL too) selects the variant that writes dX only: no weight gradient will read the planes (pose-only backward).
+extern "C" int danbo_mlp_dgrad(const void* wstream_t, const float* w_rgb, const float* w_alpha, const float* d_raw,
+                               const int* row_sample, const int* rows_dev, int max_rows, const void* act_save,
+                               const void* g_save, int cap, void* delta_save, void* delta_t, float* dX, int num_sms,
+                               void* stream) {
+    if (max_rows <= 0) return 0;
+    if (delta_save == nullptr) {
+        if (delta_t != nullptr) return -1;
+        return launch_dgrad<false>(wstream_t, w_rgb, w_alpha, d_raw, row_sample, rows_dev, max_rows, act_save, g_save,
+                                   cap, nullptr, nullptr, dX, num_sms, stream);
+    }
+    return launch_dgrad<true>(wstream_t, w_rgb, w_alpha, d_raw, row_sample, rows_dev, max_rows, act_save, g_save, cap,
+                              delta_save, delta_t, dX, num_sms, stream);
 }
 
 // Weight + bias gradients from the saved deltas / activations.

@@ -578,6 +578,54 @@ def mlp_backward_tc(P, G, d_raw, active, fo, save, d_ray_bias, ws, repack=True, 
     return dX
 
 
+class PackedDgrad:
+    """The transposed bf16 weight tiles danbo_mlp_dgrad reads, kept across calls: a backward that trains no weight
+    (the pose-only path) repacks them only when the weights changed (`RayCaster._packed_dgrad`), not per iteration."""
+
+    def __init__(self, device):
+        sizes = [ctypes.c_longlong() for _ in range(5)]
+        ns = ctypes.c_int()
+        _lib.load().danbo_mlp_bwd_workspace(1, *[ctypes.byref(x) for x in sizes], ctypes.byref(ns))
+        self.wstream = torch.empty(sizes[0].value, device=device, dtype=torch.uint8)
+
+    def pack(self, P):
+        """P: the reference's parameter names -> fp32 CUDA tensors (pts_linears.i.weight, feature_linear.weight,
+        views_linears.0.weight)."""
+        ws = [f32c(P[f"pts_linears.{i}.weight"]) for i in range(8)]
+        wf, wv = f32c(P["feature_linear.weight"]), f32c(P["views_linears.0.weight"])
+        _need_cuda(*ws, wf, wv)
+        wa = (ctypes.c_void_p * 8)(*[t.data_ptr() for t in ws])
+        _lib.check(_lib.load().danbo_pack_mlp_dgrad(wa, _p(wf), _p(wv), _p(self.wstream), _stream()),
+                   "danbo_pack_mlp_dgrad")
+        self._keep = (ws, wf, wv)              # sources alive until the stream has consumed them
+        _count(1)
+        return self
+
+
+def mlp_backward_pose(P, d_raw, active, fo, save, packed_t, d_ray_bias=None):
+    """Backward of the fused MLP when no weight needs a gradient (pose-only path) -> dX (cap,208) fp32.  The head
+    backward runs only for d_ray_bias ((n,128) fp32, added to; None: not formed, and then no head launch at all); the
+    data-gradient chain is the dX-only variant of danbo_mlp_dgrad (no delta planes).  packed_t: a PackedDgrad of the
+    current weights.  No transposes, no K = rows GEMMs, no bias sums."""
+    lib = _lib.load()
+    dev = d_raw.device
+    cap = active.capacity
+    assert save.cap == cap
+    idx = dev.index if dev.index is not None else torch.cuda.current_device()
+    if d_ray_bias is not None:
+        _lib.check(lib.danbo_mlp_head_bwd(_p(d_raw), _p(active.ids), _p(fo.row_ray), _p(active.count), cap, _p(save.g),
+                                          _p(save.act[7]), _p(P["rgb_linear.weight"]), _p(P["alpha_linear.weight"]),
+                                          None, None, None, None, None, None, _p(d_ray_bias), num_sms(idx), _stream()),
+                   "danbo_mlp_head_bwd")
+        _count(1)
+    dX = torch.empty(cap, 208, device=dev, dtype=torch.float32)
+    _lib.check(lib.danbo_mlp_dgrad(_p(packed_t.wstream), _p(P["rgb_linear.weight"]), _p(P["alpha_linear.weight"]),
+                                   _p(d_raw), _p(active.ids), _p(active.count), cap, _p(save.act), _p(save.g), cap, None,
+                                   None, _p(dX), num_sms(idx), _stream()), "danbo_mlp_dgrad")
+    _count(1)
+    return dX
+
+
 def ray_bias_bwd(rays, cam_idx, codes_with_mean, w_view, d_ray_bias, d_w_view, d_b_view, d_codes):
     lib = _lib.load()
     _lib.check(lib.danbo_ray_bias_bwd(_p(rays), rays.stride(0), rays.shape[0], _p(cam_idx), _p(codes_with_mean),
@@ -621,7 +669,9 @@ def view_root_bwd(rays, pose_skts, rays_per_pose, w_view, d_ray_bias, d_skts):
 def field_agg_bwd(rays, S, z, mask, active, pose_skts, pose_vol, rays_per_pose, consts, fo, dX, g_logit_ext, grads,
                   d_skts=None):
     """grads: list of the 9 fp32 parameter / volume accumulators in the order of danbo_field_agg_bwd (see danbo_b200.h);
-    d_skts: (n_poses,24,4,4) fp32 accumulator of the gradient w.r.t. the world-to-bone matrices, or None."""
+    entries 0-6 and 8 (aggregation net, axis_scale) all None select the pose-only kernel variant, entry 7 (d vol) is
+    always required.  d_skts: (n_poses,24,4,4) fp32 accumulator of the gradient w.r.t. the world-to-bone matrices, or
+    None."""
     lib = _lib.load()
     dev = rays.device
     n = rays.shape[0]
@@ -629,11 +679,15 @@ def field_agg_bwd(rays, S, z, mask, active, pose_skts, pose_vol, rays_per_pose, 
     d_logit = torch.empty(n * S, J, device=dev, dtype=torch.float32)
     if len(grads) != 9:
         raise ValueError("field_agg_bwd takes 9 accumulators (+ d_skts)")
+    n_weight = sum(g is not None for i, g in enumerate(grads) if i != 7)
+    if grads[7] is None or n_weight not in (0, 8):
+        raise ValueError("field_agg_bwd: d vol (grads[7]) is required; the other 8 accumulators are all given or all None")
     if d_skts is not None:
         _need_cuda(d_skts)
         if d_skts.dtype != torch.float32 or not d_skts.is_contiguous() or tuple(d_skts.shape) != (pose_skts.shape[0], J, 4, 4):
             raise ValueError("d_skts must be a contiguous fp32 (n_poses,24,4,4) tensor")
-    ga = (ctypes.c_void_p * 10)(*([g.data_ptr() for g in grads] + [None if d_skts is None else d_skts.data_ptr()]))
+    ga = (ctypes.c_void_p * 10)(*([None if g is None else g.data_ptr() for g in grads] +
+                                  [None if d_skts is None else d_skts.data_ptr()]))
     idx = dev.index if dev.index is not None else torch.cuda.current_device()
     _lib.check(lib.danbo_field_agg_bwd(_p(rays), rays.stride(0), n, S, _p(z), _p(mask), _p(active.ids), _p(active.count),
                                        active.capacity, _p(pose_skts), _p(pose_vol), int(rays_per_pose),
@@ -667,7 +721,8 @@ def graph_net_fwd(pose_bones, tensors):
 
 
 def graph_net_bwd(saved, d_vol, grads):
-    """grads: the 10 fp32 accumulators in GN_GRADS order (added to)."""
+    """grads: the 10 fp32 accumulators in GN_GRADS order (added to), or None: the pose-only variant (three launches,
+    no weight gradient), whose `work` graph_net_bwd_pose reads all the same."""
     lib = _lib.load()
     tensors, bufs = saved
     d_vol = f32c(d_vol)
@@ -675,9 +730,9 @@ def graph_net_bwd(saved, d_vol, grads):
     work = torch.empty(2 * G * J * 128, device=dev)
     pa = (ctypes.c_void_p * 12)(*[t.data_ptr() for t in tensors])
     sa = (ctypes.c_void_p * 6)(*[t.data_ptr() for t in bufs])
-    ga = (ctypes.c_void_p * 10)(*[g.data_ptr() for g in grads])
+    ga = None if grads is None else (ctypes.c_void_p * 10)(*[g.data_ptr() for g in grads])
     _lib.check(lib.danbo_graph_net_bwd(G, pa, sa, _p(d_vol), ga, _p(work), _stream()), "danbo_graph_net_bwd")
-    _count(4)
+    _count(3 if grads is None else 4)
     return work
 
 

@@ -56,6 +56,9 @@ class RayCaster(nn.Module):
         self.child_idxs = child
         self._packed = None
         self._packed_key = None
+        self._pack_gen = 0                        # bumped by every weight pack: the transposed pack follows it
+        self._packed_t = None
+        self._packed_t_gen = -1
         self._align_dev = None
         self._graphed = None
         self.block_streams = BLOCK_STREAMS
@@ -157,8 +160,10 @@ class RayCaster(nn.Module):
         # previous replay's Adam wrote.  Eval calls rely on the key: it changes with every torch in-place op
         # (`_version`), `load_state_dict`, `TrainStep` (which invalidates it after every iteration) and `FlatAdam.step`
         # (which bumps the parameters' versions); `render_graphed` checks it EAGERLY before each replay and repacks into
-        # the same static buffers, so an eval graph holds no pack launch and still never sees stale weights.
-        force = self.training and torch.is_grad_enabled()
+        # the same static buffers, so an eval graph holds no pack launch and still never sees stale weights.  A train-mode
+        # forward in which no MLP weight needs a gradient (training.PoseFitStep: the field is frozen) is keyed the same
+        # way; PoseFitStep checks the key eagerly before each replay of its graph.
+        force = self.training and torch.is_grad_enabled() and any(P[n].requires_grad for n in names)
         # a forced (training) pack skips the empty-sample constants, which only calls without a backward pass read
         if force or key != self._packed_key or not self._packed.has_empty:
             tensors = {n: P[n] for n in names}
@@ -168,7 +173,26 @@ class RayCaster(nn.Module):
                 tensors["views_linears.0.weight"] = F.pad(P["views_linears.0.weight"].detach(), (0, 128))
             self._packed.pack(tensors, want_empty=not force)
             self._packed_key = key
+            self._pack_gen += 1
         return self._packed
+
+    def _packed_dgrad(self):
+        """The transposed weight tiles of the MLP's data-gradient chain for a backward that trains no weight (the
+        pose-only path): repacked only when `_packed_mlp` last repacked, so it follows the same key.  (A training
+        backward packs them into its own workspace every iteration, autograd._RenderBlock.)"""
+        packed = self._packed_mlp()
+        if self._packed_t is None or self._packed_t.wstream.device != self._device():
+            self._packed_t = K.PackedDgrad(self._device())
+            self._packed_t_gen = -1
+        if self._packed_t_gen != self._pack_gen:
+            P = dict(self.network.named_parameters())
+            tensors = {n: P[n] for n in ["feature_linear.weight", "views_linears.0.weight"] +
+                       [f"pts_linears.{i}.weight" for i in range(8)]}
+            if not getattr(self.network, "opt_framecode", True):     # the kernels' 411-column view layout, as above
+                tensors["views_linears.0.weight"] = F.pad(P["views_linears.0.weight"].detach(), (0, 128))
+            self._packed_t.pack(tensors)
+            self._packed_t_gen = self._pack_gen
+        return self._packed_t
 
     def _codes_with_mean(self):
         if not getattr(self.network, "opt_framecode", True):

@@ -124,7 +124,8 @@ def save_checkpoint(path, global_step, caster, optimizer, popt_kwargs=None, pose
         popt_sd = popt_kwargs["popt_layer"].state_dict()
         poptim_sd = pose_optimizer.state_dict() if pose_optimizer is not None else None
         anchors = popt_kwargs.get("popt_anchors")
-    torch.save({"global_step": global_step, "optimizer_state_dict": optimizer.state_dict(),
+    torch.save({"global_step": global_step,
+                "optimizer_state_dict": optimizer.state_dict() if optimizer is not None else None,
                 "poseopt_layer_state_dict": popt_sd, "pose_optimizer_state_dict": poptim_sd, "poseopt_anchors": anchors,
                 **caster.state_dict()}, path)
 
@@ -202,8 +203,10 @@ def pose_batch_poses(batch):
     return G, n // G
 
 
-def _refuse_pose_graph(args, caster, world_size, pose_optimizer, layer):
-    """What a captured iteration with a pose layer does not cover: raise, naming the reason, before any device work."""
+def _refuse_pose_graph(args, caster, world_size, pose_optimizer, layer,
+                       what="graph capture of a training step with a pose layer"):
+    """What a captured iteration with a pose layer (and PoseFitStep, which runs the same kernels) does not cover: raise,
+    naming the reason, before any device work."""
     why = None
     if getattr(caster.network, "graph_net", None) is None:
         why = "the A-NeRF field (the pose kernels serve the DANBO field's graph net and bone transforms)"
@@ -221,7 +224,7 @@ def _refuse_pose_graph(args, caster, world_size, pose_optimizer, layer):
         why = ("a pose optimizer that is not a training.FlatAdam (pass pose_opt.create_popt(..., flat=True)): a captured "
                "backward writes into fixed gradient storage, which zero_grad(set_to_none=True) would detach")
     if why is not None:
-        raise NotImplementedError(f"graph capture of a training step with a pose layer is not implemented for {why}")
+        raise NotImplementedError(f"{what} is not implemented for {why}")
 
 
 class TrainStep:
@@ -443,3 +446,138 @@ class TrainStep:
             loss = loss + extra
         loss.backward()
         return loss.detach(), preds
+
+
+class PoseFitStep:
+    """Fits the SMPL poses of frames to their images with the field frozen: forward -> losses -> pose-only backward ->
+    pose backward -> the pose optimizer's Adam.  Call shape of TrainStep: `loss, preds = step(batch)`,
+    `step.last_stats["MPJPC"]`, `step.save(path, global_step)`, `step.resume(ckpt)`.
+
+    Only the pose layer's parameters change, through `pose_optimizer` (a FlatAdam, `pose_opt.create_popt(..., flat=True)`).
+    The network's parameters, their .grad, `caster.state_dict()` and any network optimizer are left as they are: the
+    network's parameters are passed to the render with requires_grad off for the duration of a call, so its backward
+    nodes take the pose-only path (autograd.weight_grads) and form no weight gradient.  No learning-rate decay and no
+    `update_embed_fns` schedule is applied to the network.
+
+    Loss: the trainer's image terms as TrainStep computes them (rgb_loss, rgb_loss0, soft_softmax_loss) plus the pose
+    regulariser (kp_loss, danbo_pose_fwd).  vol_scale_loss depends on the network's axis_scale only, has no pose
+    gradient and is left out.  Frames the field was not trained on have no frame code: give them cams < 0 in the batch
+    and they are rendered with the mean code (danbo_ray_bias's last code row).
+
+    graph=True captures the whole iteration as one CUDA graph (graphs.GraphedFn); capture applies no pose step (the pose
+    arena, its moments and its step counter are restored).  The MLP weight packs are keyed on the weights and checked
+    before each replay, outside the graph, so a `caster.load_state_dict` between steps is seen.  graph=False runs the
+    same kernels eagerly.  Refused (NotImplementedError, before any device work): the A-NeRF field, a separate fine
+    network, world_size > 1, opt_rot6d, use_temp_loss, opt_pose_cache, a pose optimizer that is not a FlatAdam, and a
+    batch whose N_uniques does not divide it."""
+
+    def __init__(self, caster, args, popt_kwargs, pose_optimizer, graph=False, world_size=1):
+        if not popt_kwargs or popt_kwargs.get("popt_layer") is None:
+            raise ValueError("PoseFitStep needs the pose layer of pose_opt.create_popt (popt_kwargs['popt_layer'])")
+        layer = popt_kwargs["popt_layer"]
+        _refuse_pose_graph(args, caster, world_size, pose_optimizer, layer, what="pose fitting (PoseFitStep)")
+        self.caster, self.args, self.popt, self.pose_optimizer = caster, args, popt_kwargs, pose_optimizer
+        self.last_stats = {}
+        dev = next(caster.network.parameters()).device
+        layer.to(dev)
+        self.popt["popt_anchors"] = {k: (v.to(dev) if torch.is_tensor(v) else v)
+                                     for k, v in self.popt["popt_anchors"].items()}
+        a = self.popt["popt_anchors"]
+        self._pose_anchors = {k: a[k].float().contiguous() for k in ("kps", "bones")}
+        self._rest_idx = None
+        if layer.rest_pose.shape[0] > 1:
+            self._rest_idx = torch.as_tensor(layer.rest_pose_idxs, device=dev).long()
+        self._graphed = None
+        if graph:
+            from .graphs import GraphedFn
+
+            def run(_param_ptrs=None, **b):
+                loss, preds = self._step(b)
+                return {"loss": loss, "rgb_map": preds["rgb_map"], "acc_map": preds["acc_map"],
+                        "MPJPC": self.last_stats["MPJPC"]}
+            po = pose_optimizer
+            self._graphed = GraphedFn(run, dev, warmup=3, state=[po.flat, po.exp_avg, po.exp_avg_sq, po.step_dev])
+
+    def _frozen(self):
+        """Context: the network's parameters with requires_grad off (restored on exit)."""
+        import contextlib
+        nets = [self.caster.network]
+
+        @contextlib.contextmanager
+        def ctx():
+            saved = [(p, p.requires_grad) for net in nets for p in net.parameters()]
+            try:
+                for p, _ in saved:
+                    p.requires_grad_(False)
+                yield
+            finally:
+                for p, r in saved:
+                    p.requires_grad_(r)
+        return ctx()
+
+    def __call__(self, batch):
+        pose_batch_poses(batch)                  # refused before any device work
+        if self._graphed is None:
+            return self._step(batch)
+        # the poses come from the layer: the feed's tables would only be copied into static buffers
+        batch = {k: v for k, v in batch.items() if k not in ("kp_batch", "skts", "bones")}
+        self.caster.train()
+        with self._frozen():
+            # eager, outside the graph: repack the MLP weights (both packs, into the buffers the graph reads) iff they
+            # changed since the last pack
+            self.caster._packed_dgrad()
+        # the graph reads the parameters through the raw pointers they had at capture: re-pointed storage recaptures
+        ptrs = hash(tuple(p.data_ptr() for p in self.caster.network.parameters()))
+        out = self._graphed(_param_ptrs=ptrs, **batch)
+        self.last_stats = {"MPJPC": out["MPJPC"]}
+        return out["loss"], out
+
+    def _step(self, batch):
+        from .autograd import pose_layer
+        a = self.args
+        caster, net = self.caster, self.caster.network
+        caster.train()
+        G, skip = pose_batch_poses(batch)
+        n = G * skip
+        self.pose_optimizer.zero_grad()
+        kps, bones, skts, reg, mpjpc = pose_layer(
+            self.popt["popt_layer"], batch["kp_idx"].long(), skip, G, self._pose_anchors, rest_idx=self._rest_idx,
+            tol=getattr(a, "opt_pose_tol", 0.), coef=getattr(a, "opt_pose_coef", 0.),
+            ext_scale=getattr(a, "ext_scale", 0.001), grads_in_place=True)
+        ex = lambda t: t[:, None].expand(G, skip, *t.shape[1:]).reshape(n, *t.shape[1:])
+        batch = dict(batch, kp_batch=ex(kps), skts=ex(skts), bones=ex(bones))
+        self.last_stats = {"MPJPC": mpjpc}
+        net.pose_kernels = True                  # the graph net's kernels return d pose
+        try:
+            with self._frozen():
+                preds = caster(batch["ray_batch"], N_samples=a.N_samples, kp_batch=batch["kp_batch"],
+                               skts=batch["skts"], cyls=batch["cyls"], bones=batch["bones"], cams=batch["cams"],
+                               N_uniques=batch["N_uniques"], perturb=a.perturb, N_importance=a.N_importance,
+                               raw_noise_std=a.raw_noise_std)
+                if fused_loss_supported(a, preds):
+                    # axis_scale needs no gradient here, so the fused loss forms no volume-scale term
+                    loss, _ = fused_loss_backward(a, preds, batch, net, extra_loss=reg)
+                else:
+                    _, terms = compute_loss(a, preds, batch, net)
+                    terms.pop("vol_scale_loss", None)
+                    total = sum(terms.values()) + reg
+                    total.backward()
+                    loss = total.detach()
+        finally:
+            net.pose_kernels = False
+        self.pose_optimizer.step()
+        return loss, preds
+
+    def save(self, path, global_step):
+        """Checkpoint in the reference's format with the (unchanged) network, the pose layer and the pose optimizer;
+        there is no network optimizer state (optimizer_state_dict is None)."""
+        save_checkpoint(path, global_step, self.caster, None, self.popt, self.pose_optimizer)
+
+    def resume(self, ckpt):
+        """The pose layer and pose optimizer state of a loaded checkpoint dict (nothing of the network).
+        -> global_step."""
+        if ckpt.get("poseopt_layer_state_dict") is not None:
+            self.popt["popt_layer"].load_state_dict(ckpt["poseopt_layer_state_dict"])
+            if ckpt.get("pose_optimizer_state_dict") is not None:
+                self.pose_optimizer.load_state_dict(ckpt["pose_optimizer_state_dict"])
+        return int(ckpt.get("global_step", 0))

@@ -173,7 +173,9 @@ int danbo_merge_composite_bwd(const float* rays, int ray_stride, int n_rays, int
                               float* d_logit1, void* stream);
 
 /* M1 backward building blocks (fp32).  rows_dev = device scalar row count.
- * head_bwd : d raw -> delta of views_linears.0 (rows,128), d a7 (rows,256) and the rgb/alpha head + ray-bias grads
+ * head_bwd : d raw -> delta of views_linears.0 (rows,128), d a7 (rows,256) and the rgb/alpha head + ray-bias grads;
+ *            delta9, d_a7 and d_ray_bias may each be NULL (not formed); the four head gradients are all given or all
+ *            NULL (not formed: pose-only backward); nothing asked for launches nothing
  * gemm_dgrad: D[rows x N] = A[rows x K] . B[K x N] (+ D) (* [mask > 0]);  gemm_wgrad: dW[M x N] += A^T . B;
  * colsum: db[N] += sum_rows A. */
 int danbo_mlp_head_bwd(const float* d_raw, const int* row_sample, const int* row_ray, const int* rows_dev, int max_rows,
@@ -191,7 +193,8 @@ int danbo_colsum(const float* A, int lda, float* db, const int* rows_dev, int ma
  * bf16 weight tiles (once per iteration); danbo_mlp_dgrad: fused data-gradient chain (deltas of every layer saved as
  * bf16 planes [10][cap][256]: 0 = views_linears.0, 1 = d feature, 2..9 = pts_linears.7..0; dX (cap,208) fp32; with
  * delta_t != NULL the planes are also written row-transposed (the deltaT workspace: operand images of the K = rows GEMMs),
- * and danbo_mlp_wgrad is told so with delta_t_ready = 1 and skips that transpose pass);
+ * and danbo_mlp_wgrad is told so with delta_t_ready = 1 and skips that transpose pass; delta_save = NULL, with delta_t
+ * NULL too, selects the variant that writes dX only, for a backward that forms no weight gradient);
  * danbo_mlp_wgrad: dW = delta^T . act (K = rows) for dw[10] = { views_linears.0.weight, feature_linear.weight,
  * pts_linears.7, .6, .5, .4, .3, .2, .1, .0 } and db[9] = { feature_linear.bias, pts_linears.7..0 bias }, accumulated. */
 int danbo_mlp_bwd_workspace(int cap, long long* wstream_bytes, long long* delta_bytes, long long* deltaT_bytes,
@@ -223,8 +226,9 @@ int danbo_view_root_bwd(const float* rays, int ray_stride, int n_rays, const flo
  * extra logit gradient -> grads[10] = { w0, adj_w, b0, w1, b1, w2, b2 of prob_linears, d vol (n_poses,24,240),
  * d axis_scale (24,3), d skts (n_poses,24,4,4) or NULL } (fp32, accumulated).  d skts is the gradient with respect to
  * the world-to-bone matrices (what the pose layer, core/pose_opt.py:264-339, receives under --opt_pose; rows 0-2 only,
- * the homogeneous row gets none); NULL when the poses are constants.  work = the workspace the forward danbo_field_agg
- * filled; agg_mode as in that call. */
+ * the homogeneous row gets none); NULL when the poses are constants.  grads[0..6] and grads[8] all NULL (all or none)
+ * select the pose-only variant: no aggregation-net or axis-scale gradient, d vol and d skts as before.  work = the
+ * workspace the forward danbo_field_agg filled; agg_mode as in that call. */
 int danbo_field_agg_bwd(const float* rays, int ray_stride, int n_rays, int S, const float* z, const unsigned int* mask,
                         const int* active_ids, const int* active_count, int capacity, const float* pose_skts,
                         const float* pose_vol, int rays_per_pose, int n_poses, const float* const* consts,
@@ -243,7 +247,8 @@ int danbo_graph_net_fwd(const float* pose_bones, int n_poses, const float* const
                         float* vol_out, void* stream);
 
 /* grads[10] = d { 0.lin.weight, 0.adj_w, 0.bias, 1.lin.weight, 1.adj_w, 1.bias, 2.weight, 2.bias, 3.weight, 3.bias } (fp32,
- * added to); d_vol (n_poses,24,240); work = 2 * n_poses*24*128 floats. */
+ * added to); d_vol (n_poses,24,240); work = 2 * n_poses*24*128 floats.  grads = NULL: the pose-only variant (3 launches,
+ * the transposed products only), which leaves in work what danbo_graph_net_bwd_pose reads. */
 int danbo_graph_net_bwd(int n_poses, const float* const* params, float* const* saved, const float* d_vol,
                         float* const* grads, float* work, void* stream);
 
