@@ -55,6 +55,7 @@ _SIGNATURES = {
     "danbo_ray_bias_bwd": [c_p, c_i, c_i, c_p, c_p, c_i, c_p, c_p, c_p, c_p, c_p, c_p],
     "danbo_view_root_bwd": [c_p, c_i, c_i, c_p, c_i, c_i, c_p, c_p, c_p, c_p],
     "danbo_field_agg_bwd": [c_p, c_i, c_i, c_i, c_p, c_p, c_p, c_p, c_i, c_p, c_p, c_i, c_i, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_i, c_p, c_i, c_i, c_p],
+    "danbo_field_agg_bwd_pts": [c_p, c_i, c_i, c_i, c_p, c_p, c_p, c_p, c_i, c_p, c_p, c_i, c_i, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_i, c_p, c_p, c_p, c_i, c_i, c_p],
     "danbo_mlp_bwd_workspace": [c_i, c_p, c_p, c_p, c_p, c_p, c_p],
     "danbo_pack_mlp_dgrad": [c_p, c_p, c_p, c_p, c_p],
     "danbo_mlp_dgrad": [c_p, c_p, c_p, c_p, c_p, c_p, c_i, c_p, c_p, c_i, c_p, c_p, c_p, c_i, c_p],

@@ -115,13 +115,19 @@ __device__ __forceinline__ float tile_colsum(const float* T, int lane) {
 // instantiation carries none of that code.  kWeightGrads = false (pose-only backward, the field is frozen): the
 // aggregation net's weight / bias tile sums and atomics and the axis-scale gradient are compiled out; the backward
 // through the three layers to each pair's d x, and from there to d vol and d skts, stays.
-template <bool kSoftmax, bool kWeightGrads>
-__global__ void __launch_bounds__(128)
-pair_logits_bwd_kernel(const float* __restrict__ rays, int ray_stride, int S, const float* __restrict__ z,
-                       const int* __restrict__ active_ids, const float* __restrict__ pose_skts,
-                       const float* __restrict__ pose_vol, int rays_per_pose, int n_poses, FieldConsts fc, PairWork pw,
-                       int pair_capacity, const float* __restrict__ logits, const float* __restrict__ d_logit,
-                       const float* __restrict__ d_hbar, AggGrads G, const uint32_t* __restrict__ mask) {
+// kPointGrad (requires !kWeightGrads; the point-gradient backward, danbo_field_agg_bwd_pts): every pair also adds
+// sum_k R_k^T A_k^T d t_k over the tree neighbours k of its bone to d_pts[id] (3 per-lane atomics: a warp's 32 pairs
+// belong to different rows), d vol / d skts are skipped when their accumulator is NULL, and d t includes the
+// derivative of the feature window exp(-2 sum x^6) - the true gradient of the field, where training detaches it.
+template <bool kSoftmax, bool kWeightGrads, bool kPointGrad>
+__device__ __forceinline__ void
+pair_logits_bwd_body(const float* __restrict__ rays, int ray_stride, int S, const float* __restrict__ z,
+                     const int* __restrict__ active_ids, const float* __restrict__ pose_skts,
+                     const float* __restrict__ pose_vol, int rays_per_pose, int n_poses, const FieldConsts& fc,
+                     const PairWork& pw, int pair_capacity, const float* __restrict__ logits,
+                     const float* __restrict__ d_logit, const float* __restrict__ d_hbar, const AggGrads& G,
+                     const uint32_t* __restrict__ mask, float* __restrict__ d_pts) {
+    static_assert(!(kPointGrad && kWeightGrads), "the point-gradient variant forms no weight gradient");
     __shared__ float tiles[4][2][32 * kTileLd];
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
     float* T1 = tiles[wib][0];
@@ -240,6 +246,7 @@ pair_logits_bwd_kernel(const float* __restrict__ rays, int ray_stride, int S, co
             __syncwarp();
         }
         // ---- layer 0 + adjacency mix + feature gather, per tree neighbour
+        float gp[3] = {0.f, 0.f, 0.f};                   // kPointGrad: d / d p, summed over the neighbours
         for (uint32_t nb = kNbrMask[j]; nb;) {
             const int k = __ffs(nb) - 1; nb &= nb - 1;
             float x[3], h[DANBO_FEAT];
@@ -287,9 +294,11 @@ pair_logits_bwd_kernel(const float* __restrict__ rays, int ray_stride, int S, co
             // ---- feature gather backward (window detached): taps -> d vol, interpolation weight -> d x -> d axis_scale
             const float a2 = x[0] * x[0], b2 = x[1] * x[1], c2 = x[2] * x[2];
             const float win = expf(-2.f * (a2 * a2 * a2 + b2 * b2 * b2 + c2 * c2 * c2));
-            float* dvol = G.vol + ((size_t)pose * DANBO_J + k) * DANBO_VOL;
+            const bool dvol_on = !kPointGrad || G.vol != nullptr;
+            float* dvol = dvol_on ? G.vol + ((size_t)pose * DANBO_J + k) * DANBO_VOL : nullptr;
             const float* volk = vol + k * DANBO_VOL;
             float dt[3];                                             // d loss / d t, t = A_k (R_k p + t_k) + a_k = x |s|
+            float sw = 0.f;                                          // kPointGrad: sum_c dh[c] * un-windowed h[c]
 #pragma unroll
             for (int a = 0; a < 3; ++a) {
                 const float iy = ((x[a] + 1.f) * (float)DANBO_RES - 1.f) * 0.5f;
@@ -304,9 +313,10 @@ pair_logits_bwd_kernel(const float* __restrict__ rays, int ray_stride, int S, co
                     const int base = f * (DANBO_RES * 3) + a;
                     const float v0 = ok0 ? __ldg(volk + base + i0 * 3) : 0.f;
                     const float v1 = ok1 ? __ldg(volk + base + i1 * 3) : 0.f;
-                    if (live && ok0) atomicAdd(dvol + base + i0 * 3, g * wt0);
-                    if (live && ok1) atomicAdd(dvol + base + i1 * 3, g * wt1);
+                    if (live && ok0 && dvol_on) atomicAdd(dvol + base + i0 * 3, g * wt0);
+                    if (live && ok1 && dvol_on) atomicAdd(dvol + base + i1 * 3, g * wt1);
                     dxa = fmaf(g, v1 - v0, dxa);
+                    if (kPointGrad) sw = fmaf(dh[f * 3 + a], v0 * wt0 + v1 * wt1, sw);
                 }
                 dxa *= 0.5f * (float)DANBO_RES;                      // d iy / d x
                 const float sc = __ldg(fc.axis_scale + k * 3 + a);
@@ -317,7 +327,17 @@ pair_logits_bwd_kernel(const float* __restrict__ rays, int ray_stride, int S, co
                 }
                 dt[a] = live ? dxa / fabsf(sc) : 0.f;
             }
-            if (G.skts != nullptr) {
+            if (kPointGrad) {
+                // the window's own derivative: d win / d x_a = -12 x_a^5 win, times the un-windowed taps of all 15
+                // channels (d h[c] / d x_a = h[c] / win * d win / d x_a)
+                const float cw = -12.f * win * sw;
+#pragma unroll
+                for (int a = 0; a < 3; ++a) {
+                    const float x2 = x[a] * x[a];
+                    if (live) dt[a] += cw * x2 * x2 * x[a] / fabsf(__ldg(fc.axis_scale + k * 3 + a));
+                }
+            }
+            if (kPointGrad || G.skts != nullptr) {
                 // ---- d x -> d skts[pose][k] (encoders.py:288-303, :442-444): t = A l + a, l = R p + t_k, so
                 // d l = A^T d t and d [R | t_k] = d l (x) [p, 1].  A warp's pairs usually share their pose (rays are
                 // image-major): one warp reduction and 12 atomics; mixed warps fall back to per-lane atomics.
@@ -326,8 +346,14 @@ pair_logits_bwd_kernel(const float* __restrict__ rays, int ray_stride, int S, co
 #pragma unroll
                 for (int i = 0; i < 3; ++i)
                     dl[i] = fmaf(__ldg(A + 8 + i), dt[2], fmaf(__ldg(A + 4 + i), dt[1], __ldg(A + i) * dt[0]));
+                if (kPointGrad) {                                    // d p = R^T d l
+                    const float* R = skt + k * 16;
+#pragma unroll
+                    for (int c = 0; c < 3; ++c)
+                        gp[c] = fmaf(__ldg(R + 8 + c), dl[2], fmaf(__ldg(R + 4 + c), dl[1], fmaf(__ldg(R + c), dl[0], gp[c])));
+                }
                 const uint32_t lm = __ballot_sync(0xffffffffu, live);
-                if (lm != 0u) {
+                if ((!kPointGrad || G.skts != nullptr) && lm != 0u) {
                     const int pose_ref = __shfl_sync(0xffffffffu, pose, __ffs(lm) - 1);
                     const float pw4[4] = {px, py, pz, 1.f};
                     if (__all_sync(0xffffffffu, !live || pose == pose_ref)) {
@@ -349,7 +375,36 @@ pair_logits_bwd_kernel(const float* __restrict__ rays, int ray_stride, int S, co
                 }
             }
         }
+        if (kPointGrad && live) {
+#pragma unroll
+            for (int c = 0; c < 3; ++c) atomicAdd(d_pts + (size_t)id * 3 + c, gp[c]);
+        }
     }
+}
+
+template <bool kSoftmax, bool kWeightGrads>
+__global__ void __launch_bounds__(128)
+pair_logits_bwd_kernel(const float* __restrict__ rays, int ray_stride, int S, const float* __restrict__ z,
+                       const int* __restrict__ active_ids, const float* __restrict__ pose_skts,
+                       const float* __restrict__ pose_vol, int rays_per_pose, int n_poses, FieldConsts fc, PairWork pw,
+                       int pair_capacity, const float* __restrict__ logits, const float* __restrict__ d_logit,
+                       const float* __restrict__ d_hbar, AggGrads G, const uint32_t* __restrict__ mask) {
+    pair_logits_bwd_body<kSoftmax, kWeightGrads, false>(rays, ray_stride, S, z, active_ids, pose_skts, pose_vol,
+                                                        rays_per_pose, n_poses, fc, pw, pair_capacity, logits, d_logit,
+                                                        d_hbar, G, mask, nullptr);
+}
+
+// d_pts (n_rays*S, 3): d / d sample position, added to; G.vol / G.skts may be NULL, the other accumulators are unused
+template <bool kSoftmax>
+__global__ void __launch_bounds__(128)
+pair_logits_bwd_pts_kernel(const float* __restrict__ rays, int ray_stride, int S, const float* __restrict__ z,
+                           const int* __restrict__ active_ids, const float* __restrict__ pose_skts,
+                           const float* __restrict__ pose_vol, int rays_per_pose, int n_poses, FieldConsts fc,
+                           PairWork pw, int pair_capacity, const float* __restrict__ logits,
+                           const float* __restrict__ d_logit, const float* __restrict__ d_hbar, AggGrads G,
+                           const uint32_t* __restrict__ mask, float* __restrict__ d_pts) {
+    pair_logits_bwd_body<kSoftmax, false, true>(rays, ray_stride, S, z, active_ids, pose_skts, pose_vol, rays_per_pose,
+                                                n_poses, fc, pw, pair_capacity, logits, d_logit, d_hbar, G, mask, d_pts);
 }
 
 }  // namespace danbo
@@ -398,6 +453,38 @@ extern "C" int danbo_field_agg_bwd(const float* rays, int ray_stride, int n_rays
                               : (wg ? pair_logits_bwd_kernel<false, true> : pair_logits_bwd_kernel<false, false>);
     kern<<<pblocks, 128, 0, st>>>(rays, ray_stride, S, z, active_ids, pose_skts, pose_vol, rays_per_pose, n_poses, fc, pw,
                                   pair_capacity, logits, d_logit, d_hbar, G, mask);
+    DANBO_CHECK_LAUNCH();
+    return 0;
+}
+
+// The point-gradient backward: field_rows_bwd as above, then the kPointGrad pair kernel.  d_pts (n_rays*S, 3) receives
+// d / d p of every sample (added to); d_vol (n_poses,24,240) and d_skts (n_poses,24,4,4) are optional (NULL: skipped).
+// The feature window is NOT detached here (see pair_logits_bwd_body), so d_skts is the true derivative, not training's.
+extern "C" int danbo_field_agg_bwd_pts(const float* rays, int ray_stride, int n_rays, int S, const float* z,
+                                       const unsigned int* mask, const int* active_ids, const int* active_count,
+                                       int capacity, const float* pose_skts, const float* pose_vol, int rays_per_pose,
+                                       int n_poses, const float* const* consts, const float* logits, const float* hbar,
+                                       const float* dX, const float* g_logit_ext, float* d_hbar, float* d_logit,
+                                       const int* work, int pair_capacity, float* d_pts, float* d_vol, float* d_skts,
+                                       int num_sms, int agg_mode, void* stream) {
+    if (capacity <= 0) return 0;
+    if (agg_mode < 0 || agg_mode > 1) return -1;
+    if (d_pts == nullptr) return -1;
+    cudaStream_t st = (cudaStream_t)stream;
+    const FieldConsts fc = make_consts_b(consts);
+    int rblocks = (capacity + 127) / 128;
+    if (rblocks > num_sms * 16) rblocks = num_sms * 16;
+    field_rows_bwd_kernel<<<rblocks, 128, 0, st>>>(rays, ray_stride, n_rays, S, z, mask, active_ids, active_count,
+                                                    capacity, pose_skts, pose_vol, rays_per_pose, n_poses, fc, logits,
+                                                    hbar, dX, g_logit_ext, d_hbar, d_logit, agg_mode);
+    DANBO_CHECK_LAUNCH();
+    AggGrads G{nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, d_vol, nullptr, d_skts};
+    PairWork pw{const_cast<int*>(work)};
+    int pblocks = (pair_capacity / 32 + 3) / 4;
+    if (pblocks > num_sms * 4) pblocks = num_sms * 4;
+    auto kern = agg_mode == 1 ? pair_logits_bwd_pts_kernel<true> : pair_logits_bwd_pts_kernel<false>;
+    kern<<<pblocks, 128, 0, st>>>(rays, ray_stride, S, z, active_ids, pose_skts, pose_vol, rays_per_pose, n_poses, fc, pw,
+                                  pair_capacity, logits, d_logit, d_hbar, G, mask, d_pts);
     DANBO_CHECK_LAUNCH();
     return 0;
 }

@@ -697,7 +697,42 @@ def field_agg_bwd(rays, S, z, mask, active, pose_skts, pose_vol, rays_per_pose, 
     _count(2)
 
 
-GN_PARAMS = ["layers.0.lin.weight", "layers.0.adj_w", "layers.0.adj", "layers.0.bias", "layers.1.lin.weight",
+def field_agg_bwd_pts(rays, S, z, mask, active, pose_skts, pose_vol, rays_per_pose, consts, fo, dX, d_pts, d_vol=None,
+                      d_skts=None):
+    """d / d (sample position) of the field's output through the same chain as field_agg_bwd (danbo_field_agg_bwd_pts):
+    d_pts (n*S,3) fp32, added to, is required; d_vol (pose_vol's shape) and d_skts (n_poses,24,4,4) are optional
+    accumulators (None: not formed).  The feature window's derivative is included (training detaches it), so these are
+    the field's true derivatives.  fo: the forward field_agg of the same call, with want_hbar."""
+    lib = _lib.load()
+    dev = rays.device
+    n = rays.shape[0]
+    if fo.hbar is None:
+        raise ValueError("field_agg_bwd_pts: the forward field_agg must keep hbar (want_hbar=True)")
+    for name, t, shape in (("d_pts", d_pts, (n * S, 3)), ("d_vol", d_vol, tuple(pose_vol.shape)),
+                           ("d_skts", d_skts, (pose_skts.shape[0], J, 4, 4))):
+        if t is None:
+            if name == "d_pts":
+                raise ValueError("field_agg_bwd_pts: d_pts is required")
+            continue
+        _need_cuda(t)
+        if t.dtype != torch.float32 or not t.is_contiguous() or tuple(t.shape) != shape or t.device != dev:
+            raise ValueError(f"field_agg_bwd_pts: {name} must be a contiguous fp32 {shape} tensor on {dev}")
+    if tuple(dX.shape) != (active.capacity, 208) or dX.dtype != torch.float32 or not dX.is_contiguous():
+        raise ValueError("field_agg_bwd_pts: dX must be the contiguous fp32 (capacity,208) output of the MLP backward")
+    d_hbar = torch.empty(active.capacity, 16, device=dev, dtype=torch.float32)
+    d_logit = torch.empty(n * S, J, device=dev, dtype=torch.float32)
+    idx = dev.index if dev.index is not None else torch.cuda.current_device()
+    _lib.check(lib.danbo_field_agg_bwd_pts(_p(rays), rays.stride(0), n, S, _p(z), _p(mask), _p(active.ids),
+                                           _p(active.count), active.capacity, _p(pose_skts), _p(pose_vol),
+                                           int(rays_per_pose), pose_skts.shape[0], consts.array, _p(fo.logits),
+                                           _p(fo.hbar), _p(dX), None, _p(d_hbar), _p(d_logit), _p(fo.work), fo.pair_cap,
+                                           _p(d_pts), _p(d_vol), _p(d_skts), num_sms(idx), fo.agg_mode, _stream()),
+               "danbo_field_agg_bwd_pts")
+    _count(2)
+    return d_pts
+
+
+GN_PARAMS =["layers.0.lin.weight", "layers.0.adj_w", "layers.0.adj", "layers.0.bias", "layers.1.lin.weight",
              "layers.1.adj_w", "layers.1.adj", "layers.1.bias", "layers.2.weight", "layers.2.bias", "layers.3.weight",
              "layers.3.bias"]                                    # order of danbo_graph_net_fwd's params[12]
 GN_GRADS = [n for n in GN_PARAMS if not n.endswith(".adj")]     # order of danbo_graph_net_bwd's grads[10]

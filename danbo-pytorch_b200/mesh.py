@@ -151,12 +151,21 @@ def mesh_volume(vertices, triangles):
 
 
 # ---- writers (trimesh.export / imageio.imwrite of run_render.py:1280,1343-1346) -----------------------------------
-def write_ply(path, vertices, triangles):
-    """Binary little-endian PLY with float32 vertices and int32 triangle indices."""
+def write_ply(path, vertices, triangles, normals=None):
+    """Binary little-endian PLY with float32 vertices and int32 triangle indices; with `normals` (V,3) each vertex also
+    carries float32 nx ny nz (viewers then shade the mesh smoothly).  Without normals the bytes are those of a plain
+    vertex + face file."""
     v = np.ascontiguousarray(torch.as_tensor(vertices).detach().cpu().numpy(), dtype="<f4")
     f = np.ascontiguousarray(torch.as_tensor(triangles).detach().cpu().numpy(), dtype="<i4")
+    props = "property float x\nproperty float y\nproperty float z\n"
+    if normals is not None:
+        nrm = np.ascontiguousarray(torch.as_tensor(normals).detach().cpu().numpy(), dtype="<f4")
+        if nrm.shape != v.shape:
+            raise ValueError(f"write_ply: normals {nrm.shape} must match vertices {v.shape}")
+        v = np.ascontiguousarray(np.concatenate([v.reshape(-1, 3), nrm.reshape(-1, 3)], 1))
+        props += "property float nx\nproperty float ny\nproperty float nz\n"
     head = ("ply\nformat binary_little_endian 1.0\n"
-            f"element vertex {len(v)}\nproperty float x\nproperty float y\nproperty float z\n"
+            f"element vertex {len(v)}\n{props}"
             f"element face {len(f)}\nproperty list uchar int vertex_indices\nend_header\n").encode("ascii")
     rec = np.empty(len(f), dtype=[("n", "u1"), ("idx", "<i4", (3,))])
     rec["n"], rec["idx"] = 3, f
@@ -166,17 +175,24 @@ def write_ply(path, vertices, triangles):
         fh.write(rec.tobytes())
 
 
-def read_ply(path):
-    """Inverse of write_ply (for tests and round trips)."""
+def read_ply(path, with_normals=False):
+    """Inverse of write_ply (for tests and round trips) -> (vertices, triangles), or (vertices, triangles, normals) with
+    `with_normals` (a file without nx ny nz raises)."""
     with open(path, "rb") as fh:
         data = fh.read()
     end = data.index(b"end_header\n") + len(b"end_header\n")
     head = data[:end].decode("ascii").split("\n")
     nv = int([l for l in head if l.startswith("element vertex")][0].split()[-1])
     nf = int([l for l in head if l.startswith("element face")][0].split()[-1])
-    v = np.frombuffer(data, dtype="<f4", count=nv * 3, offset=end).reshape(nv, 3)
-    rec = np.frombuffer(data, dtype=[("n", "u1"), ("idx", "<i4", (3,))], count=nf, offset=end + nv * 12)
-    return v.copy(), rec["idx"].copy()
+    has_n = "property float nx" in head
+    if with_normals and not has_n:
+        raise ValueError(f"{path} has no vertex normals")
+    width = 6 if has_n else 3
+    vn = np.frombuffer(data, dtype="<f4", count=nv * width, offset=end).reshape(nv, width)
+    rec = np.frombuffer(data, dtype=[("n", "u1"), ("idx", "<i4", (3,))], count=nf, offset=end + nv * 4 * width)
+    if with_normals:
+        return vn[:, :3].copy(), rec["idx"].copy(), vn[:, 3:].copy()
+    return vn[:, :3].copy(), rec["idx"].copy()
 
 
 def write_png(path, img):
@@ -230,11 +246,22 @@ def save_renders(basedir, rgbs, accs, fps=14):
 
 
 @torch.no_grad()
-def render_mesh(ray_caster, kps, skts, bones, radius=1.80, res=255, threshold=10., out_dir=None, preproc_kwargs=None):
+def render_mesh(ray_caster, kps, skts, bones, radius=1.80, res=255, threshold=10., out_dir=None, preproc_kwargs=None,
+                normals=False):
     """run_render.py:1266-1281: per pose, the (res+1)^3 raw-density lattice (`fwd_type='mesh'`), relu, marching cubes at
     `threshold`, vertices scaled to `v / res - 0.5`; written as `meshes/{i:03d}.ply` when out_dir is given.
-    -> list of (vertices, triangles)."""
+    -> list of (vertices, triangles).
+
+    normals=True: -> list of (vertices, triangles, normals), the same vertices and triangles, with the unit outward
+    normal -grad sigma / |grad sigma| of the field at every vertex (0 where the gradient is 0), from
+    `render_pts_gradient` at the vertex's world position root + 2 radius v (the lattice is in xyz index order around
+    the root joint, `render_mesh_density`); the PLY files carry them as nx ny nz."""
     import os
+    caster = getattr(ray_caster, "module", ray_caster)          # the training handle wraps the caster
+    if normals:
+        if not hasattr(caster, "render_pts_gradient"):
+            raise NotImplementedError("render_mesh(normals=True) needs a caster with render_pts_gradient")
+        caster._refuse_normals("render_mesh(normals=True)")
     out = []
     if out_dir is not None:
         os.makedirs(os.path.join(out_dir, "meshes"), exist_ok=True)
@@ -243,7 +270,12 @@ def render_mesh(ray_caster, kps, skts, bones, radius=1.80, res=255, threshold=10
                          render_kwargs=preproc_kwargs, fwd_type="mesh")
         v, t = marching_cubes(torch.relu(raw.reshape(res + 1, res + 1, res + 1)), threshold)
         v = v / res - 0.5
+        n = None
+        if normals:
+            root = torch.as_tensor(kps[i:i + 1]).reshape(1, -1, 3)[0, 0].to(v.device).float()
+            _, g = caster.render_pts_gradient(root + 2. * radius * v, kps[i:i + 1], skts[i:i + 1], bones[i:i + 1])
+            n = caster._unit_normals(g).to(v.device)
         if out_dir is not None:
-            write_ply(os.path.join(out_dir, "meshes", f"{i:03d}.ply"), v, t)
-        out.append((v, t))
+            write_ply(os.path.join(out_dir, "meshes", f"{i:03d}.ply"), v, t, normals=n)
+        out.append((v, t) if n is None else (v, t, n))
     return out

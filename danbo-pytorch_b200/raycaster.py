@@ -24,12 +24,17 @@ MAX_RAYS_PER_LAUNCH = 262144          # multiple of every sane `chunk`; bounds t
 # sequences are issued on separate streams, so that the issue-/LSU-bound kernels of one block can fill the SM time the
 # tensor-bound MLP kernel of the other leaves (and the gaps between dependent launches).  1 = one stream, as measured.
 BLOCK_STREAMS = int(os.environ.get("DANBO_BLOCK_STREAMS", "1"))
+# Rows (samples) per launch sequence of the surface-normal paths (render_pts_gradient, render_rays(want_normals=True)):
+# they keep the bf16 MLP activations and the encoded rows for a backward pass, about 7 KB per row, so 2^18 rows hold
+# about 1.8 GB.
+NORMAL_BLOCK_ROWS = 1 << 18
 
 
 class RayCaster(nn.Module):
     """GraphCaster of the reference (raycasters.py:642-716) on B200 kernels."""
 
     _supports_fine_network = False        # a separate fine network (single_net=False): the A-NeRF caster only
+    _supports_normals = True              # density gradients / normals (render_pts_gradient, want_normals): DANBO only
 
     def __init__(self, network, network_fine=None, single_net=True, rest_poses=None, align_bones="align",
                  skel_type=None, use_volume_near_far=False, view_mode="world", **kwargs):
@@ -88,6 +93,9 @@ class RayCaster(nn.Module):
         from .graphs import GraphedFn
         if self.training:
             raise RuntimeError("render_graphed is for eval mode")
+        if ignored.get("want_normals"):
+            raise NotImplementedError("want_normals is not implemented for render_graphed (normals are not captured): "
+                                      "use the plain call")
         if ignored.get("ray_noise_std", 0.) > 0 or ignored.get("pytest"):
             raise NotImplementedError("ray_noise_std > 0 and pytest are not implemented")
         B = float((preproc_kwargs or {}).get("density_scale", 1.0))
@@ -227,12 +235,19 @@ class RayCaster(nn.Module):
                     subject_idxs=None, retraw=False, lindisp=False, perturb=0., N_importance=0, network_fine=None,
                     raw_noise_std=0., ray_noise_std=0., verbose=False, ext_scale=0.001, pytest=False, N_uniques=1,
                     render_confd=False, render_entropy=False, preproc_kwargs=None, netchunk=1024 * 64,
-                    nerf_type="danbo", use_viewdirs=True, nanmean_chunk=None, _rand=None, _stages=None):
+                    nerf_type="danbo", use_viewdirs=True, nanmean_chunk=None, want_normals=False, _rand=None,
+                    _stages=None):
         """Same arguments and returned dict as raycasters.py:245-377,516-546,710-716.
 
         Extra (optional) keywords: `nanmean_chunk` keeps the reference's per-chunk near/far fill (F8) when more than
-        one reference chunk is passed in a single call; `_rand`/`_stages` are test hooks (inject the four random
-        tensors / collect stage tensors)."""
+        one reference chunk is passed in a single call; `want_normals` adds `normal_map` (n,3), the composite of the
+        samples' unit normals (`_render_normals`; eval mode without gradients only); `_rand`/`_stages` are test hooks
+        (inject the four random tensors / collect stage tensors)."""
+        if want_normals:
+            self._refuse_normals("render_rays(want_normals=True)")
+            if self.training or torch.is_grad_enabled():
+                raise NotImplementedError("want_normals is for eval mode without gradients (caster.eval(), torch.no_grad()): "
+                                          "normals in training are not implemented")
         # render_confd / render_entropy / verbose / retraw are accepted and ignored, as in the reference's render_rays
         # (raycasters.py:245-377 never reads them)
         if ray_noise_std > 0 or pytest:
@@ -249,6 +264,9 @@ class RayCaster(nn.Module):
             raise NotImplementedError("density_type other than 'relu' is not implemented")
         B = float(pk.get("density_scale", 1.0))
         rays, pose_skts, pose_bones, pose_cyls, cam_idx, skip = self._prepare(ray_batch, skts, cyls, bones, cams, N_uniques)
+        if want_normals:
+            return self._render_normals(rays, pose_skts, pose_bones, pose_cyls, cam_idx, skip, N_samples, N_importance, B,
+                                        nanmean_chunk, bool(lindisp), _stages)
         return self._render_prepared(rays, pose_skts, pose_bones, pose_cyls, cam_idx, skip=skip, N_samples=N_samples,
                                      N_importance=N_importance, B=B, raw_noise_std=raw_noise_std, perturb=perturb,
                                      nanmean_chunk=nanmean_chunk, lindisp=bool(lindisp), _rand=_rand, _stages=_stages)
@@ -341,9 +359,11 @@ class RayCaster(nn.Module):
         return block, n_streams
 
     def _render_block(self, rays, ray0, skip, pose_skts, pose_cyls, vol, cam_idx, codes, consts, packed, S_c, S_f, B,
-                      raw_noise_std, perturb, training, nanmean_chunk, rand, stages, keep=None, lindisp=False):
+                      raw_noise_std, perturb, training, nanmean_chunk, rand, stages, keep=None, lindisp=False,
+                      nearfar=None):
         """One launch sequence over <= MAX_RAYS_PER_LAUNCH rays.  `keep` (dict) receives every intermediate the
-        backward pass needs (train mode with gradients)."""
+        backward pass needs (train mode with gradients, and the normal map).  `nearfar`: the block's (near, far), when
+        the caller computed them over a larger range of rays (the normal map's blocks)."""
         n = rays.shape[0]
         # poses of this block: ray (ray0 + i) -> pose (ray0 + i) // skip
         if pose_skts.shape[0] == 1:
@@ -353,8 +373,11 @@ class RayCaster(nn.Module):
             p0 = ray0 // skip
         p_skts, p_cyls, p_vol = pose_skts[p0:], pose_cyls[p0:], vol[p0:]
         seg = 0 if not nanmean_chunk else int(nanmean_chunk)
-        near, far = K.nearfar(rays, p_cyls, p_skts, skip, consts.align, consts.axis_scale, seg_len=seg,
-                              use_box=self.use_volume_near_far, bound=1.3)
+        if nearfar is None:
+            near, far = K.nearfar(rays, p_cyls, p_skts, skip, consts.align, consts.axis_scale, seg_len=seg,
+                                  use_box=self.use_volume_near_far, bound=1.3)
+        else:
+            near, far = nearfar
         rays_v = self._view_rays(rays, p_skts, skip)
         rbias = K.ray_bias(rays_v, cam_idx, codes, packed)
         inv_B = 1.0 / B
@@ -419,6 +442,123 @@ class RayCaster(nn.Module):
                            "raw": c1.get("raw"), "n_active0": act0.count, "n_active1": act1.count,
                            "ray_bias": rbias})
         return ret
+
+    # ------------------------------------------------------------------------------------------------ normals
+    def _refuse_normals(self, what):
+        if not self._supports_normals:
+            raise NotImplementedError(f"{what}: density gradients are implemented for the DANBO field only (the A-NeRF "
+                                      "field's density depends on the point through its cut-off encodings as well)")
+
+    def _pass_gradient(self, rays, S, z, mask, act, fo, sv, p_skts, p_vol, skip, consts, packed_t):
+        """d raw sigma / d p of every sample of one saved pass, from one backward pass seeded with d raw = (0,0,0,1) on
+        every row (rows are independent, so each sample gets its own gradient) -> (n*S, 3).  A sample no bone sees has
+        no active row and gets exactly 0."""
+        dev = rays.device
+        n = rays.shape[0]
+        d_raw = torch.zeros(n * S + n, 4, device=dev)           # covers the appended empty entries (ids >= n*S) too
+        d_raw[:, 3] = 1.
+        P = dict(self.network.named_parameters())
+        dX = K.mlp_backward_pose({k: P[k].detach() for k in ("rgb_linear.weight", "alpha_linear.weight")}, d_raw, act,
+                                 fo, sv, packed_t)
+        d_pts = torch.zeros(n * S, 3, device=dev)
+        K.field_agg_bwd_pts(rays, S, z, mask, act, p_skts, p_vol, skip, consts, fo, dX, d_pts)
+        return d_pts
+
+    @staticmethod
+    def _unit_normals(grad):
+        """-grad / |grad| (the outward normal of a density level set); exactly 0 where the gradient is 0."""
+        nrm = grad.norm(dim=-1, keepdim=True)
+        return torch.where(nrm > 0, -grad / torch.where(nrm > 0, nrm, torch.ones_like(nrm)), torch.zeros_like(grad))
+
+    @torch.no_grad()
+    def render_pts_gradient(self, pts, kps, skts, bones, netchunk=NORMAL_BLOCK_ROWS):
+        """Raw sigma and its gradient with respect to the point, in world coordinates, at points (P,1,3) or (P,3) for
+        ONE pose -> (sigma (P,1), grad (P,3)).  sigma is what render_pts_density returns.  The gradient is the field's
+        true derivative (the feature window is differentiated, where training detaches it); a point no bone sees gets
+        exactly 0.  Points go in chunks of `netchunk` (the saved activations take about 7 KB per point).  No autograd:
+        the network's parameters and their .grad are untouched."""
+        self._refuse_normals("render_pts_gradient")
+        if kps.shape[0] != 1 or skts.shape[0] != 1 or bones.shape[0] != 1:
+            raise NotImplementedError("render_pts_gradient takes one pose (kps, skts, bones with a leading 1)")
+        dev = self._device()
+        P = pts.shape[0]
+        p_all = pts.reshape(P, 3).to(dev).float()
+        consts, packed, packed_t = self._consts(), self._packed_mlp(), self._packed_dgrad()
+        p_skts = skts.to(dev).float().contiguous()
+        vol = self.network.bone_volumes(bones.to(dev).float()).float().contiguous()
+        agg_mode = self.network.agg_mode
+        sigma = torch.empty(P, device=dev)
+        grad = torch.empty(P, 3, device=dev)
+        chunk = max(int(netchunk), 1)
+        for c0 in range(0, P, chunk):
+            c1 = min(P, c0 + chunk)
+            m = c1 - c0
+            rays = torch.zeros(m, 8, device=dev)                    # "rays" with o = point, d = 0, z = 0
+            rays[:, :3] = p_all[c0:c1]
+            z = torch.zeros(m, 1, device=dev)
+            # append_empty=2: one extra entry (id 2m-1) carries sigma of a point that no bone sees, as in render_pts_density
+            _, mask, act = K.sample_mask(rays, 1, p_skts, m, consts, z_in=z, append_empty=2, capacity=m + 1)
+            fo = K.field_agg(rays, 1, z, mask, act, p_skts, vol, m, consts, want_hbar=True, want_xrows=True,
+                             agg_mode=agg_mode)
+            if not torch.cuda.is_current_stream_capturing() and fo.overflowed():
+                fo = K.field_agg(rays, 1, z, mask, act, p_skts, vol, m, consts, want_hbar=True, want_xrows=True,
+                                 agg_mode=agg_mode, pairs_per_row=K.J)
+            raw = torch.empty(2 * m, 4, device=dev)
+            sv = K.ActSave(act.capacity, dev)
+            # the colour head reads a view bias; sigma does not, and its backward seed has no colour component
+            K.mlp_forward_save(fo.xtiles, packed, torch.zeros(m, 128, device=dev), act, fo.row_ray, raw, sv)
+            grad[c0:c1] = self._pass_gradient(rays, 1, z, mask, act, fo, sv, p_skts, vol, m, consts, packed_t)
+            sigma[c0:c1] = torch.where(mask.reshape(-1) != 0, raw[:m, 3], raw[2 * m - 1, 3])
+        return (sigma.reshape(P, 1, 1) if pts.dim() == 3 else sigma.reshape(P, 1)), grad
+
+    def _render_normals(self, rays, pose_skts, pose_bones, pose_cyls, cam_idx, skip, S_c, S_f, B, nanmean_chunk,
+                        lindisp, stages):
+        """render_rays(want_normals=True): the eval render (no perturbation, no noise) with its intermediates kept, the
+        seeded backward of render_pts_gradient on both passes, and normal_map = sum_m w_m n_m over the merged samples
+        with the fine composite's weights (world frame, not renormalised).  The plain call's blocks (and their near /
+        far fill segments) are kept; each is cut into ray blocks of at most NORMAL_BLOCK_ROWS samples of a single
+        pose."""
+        dev = self._device()
+        N = rays.shape[0]
+        net = self.network
+        consts, packed, packed_t = self._consts(), self._packed_mlp(), self._packed_dgrad()
+        vol = net.bone_volumes(pose_bones).float().contiguous()
+        codes = self._codes_with_mean()
+        G = pose_skts.shape[0]
+        block, _ = self._plan_blocks(N, G, skip, nanmean_chunk, 1)
+        seg = 0 if not nanmean_chunk else int(nanmean_chunk)
+        sub_rays = max(1, NORMAL_BLOCK_ROWS // (S_c + S_f + 1))
+        outs = []
+        for s0 in range(0, N, block):
+            s1 = min(N, s0 + block)
+            p0 = 0 if G == 1 else s0 // skip
+            near, far = K.nearfar(rays[s0:s1], pose_cyls[p0:], pose_skts[p0:], skip, consts.align, consts.axis_scale,
+                                  seg_len=seg, use_box=self.use_volume_near_far, bound=1.3)
+            # sub-blocks of one pose each: ray i of the call belongs to pose min(i // skip, G - 1)
+            a = s0
+            while a < s1:
+                g = min(a // skip, G - 1)
+                pose_end = s1 if g == G - 1 else min(s1, (g + 1) * skip)
+                b = min(pose_end, a + sub_rays)
+                keep = {}
+                ret = self._render_block(rays[a:b], 0, b - a, pose_skts[g:g + 1], pose_cyls[g:g + 1], vol[g:g + 1],
+                                         cam_idx[a:b], codes, consts, packed, S_c, S_f, B, 0., 0., False, nanmean_chunk,
+                                         {}, stages, keep=keep, lindisp=lindisp,
+                                         nearfar=(near[a - s0:b - s0], far[a - s0:b - s0]))
+                k = keep
+                n = b - a
+                g0 = self._pass_gradient(k["rays"], S_c, k["z0"], k["mask0"], k["act0"], k["f0"], k["sv0"], k["p_skts"],
+                                         k["p_vol"], k["skip"], consts, packed_t)
+                g1 = self._pass_gradient(k["rays"], S_f, k["z1"], k["mask1"], k["act1"], k["f1"], k["sv1"], k["p_skts"],
+                                         k["p_vol"], k["skip"], consts, packed_t)
+                nrm = self._unit_normals(torch.cat([g0.reshape(n, S_c, 3), g1.reshape(n, S_f, 3)], 1))
+                nrm = torch.gather(nrm, 1, k["order"].long()[..., None].expand(-1, -1, 3))      # merge order (z_all)
+                ret["normal_map"] = (ret["T_i"][..., None] * nrm).sum(1)
+                outs.append(ret)
+                a = b
+        if len(outs) == 1:
+            return outs[0]
+        return {k: torch.cat([o[k] for o in outs], 0) for k in outs[0]}
 
     # ------------------------------------------------------------------------------------------------ density grid
     @torch.no_grad()

@@ -69,15 +69,27 @@ def rays_in_box(H, W, focal, c2w, cyl, device, c2w_dev=None):
 
 @torch.no_grad()
 def render_images(caster, args, c2ws, poses, H, W, focal=None, cam_idx=0, white_bkgd=True, near=syn.NEAR, far=syn.FAR,
-                  graphed=False, distributed=False):
+                  graphed=False, distributed=False, normals=False):
     """Render one image per (camera, pose) pair.  poses: list of dicts from synthetic.make_pose (kps, skts, bones, cyl);
     image k uses c2ws[k] and poses[k % len(poses)], like render_path.  With distributed=True images are dealt round
-    robin to the ranks and the finished images all-gathered: every rank returns all images (n, H, W, 3) float32."""
+    robin to the ranks and the finished images all-gathered: every rank returns all images (n, H, W, 3) float32.
+    normals=True (single process, not graphed): -> (images, normal_images), the second (n, H, W, 3) float32 world-frame
+    normal maps (`render_rays(want_normals=True)`), 0 on the background."""
+    if normals:
+        if graphed:
+            raise NotImplementedError("render_images(normals=True) with graphed=True: normals are not captured")
+        if distributed:
+            raise NotImplementedError("render_images(normals=True) with distributed=True is not implemented")
+        if hasattr(caster, "_refuse_normals"):
+            caster._refuse_normals("render_images(normals=True)")
+        if caster.training:
+            raise NotImplementedError("render_images(normals=True) is for eval mode (caster.eval())")
     dev = next(caster.parameters()).device
     focal = 1.2 * H if focal is None else focal
     rank, world = parallel.world() if distributed else (0, 1)
     mine = list(range(rank, len(c2ws), world))
     out = torch.ones(len(mine), H * W, 3, device=dev) if white_bkgd else torch.zeros(len(mine), H * W, 3, device=dev)
+    nmaps = torch.zeros(len(mine), H * W, 3, device=dev) if normals else None
     call = caster.render_graphed if graphed else caster
     # every pose table and camera of this rank's images goes to the device ONCE (5 copies), not per image: a pageable
     # host-to-device copy is synchronous, and one per tensor per image kept the GPU idle for half of each image
@@ -97,10 +109,15 @@ def render_images(caster, args, c2ws, poses, H, W, focal=None, cam_idx=0, white_
                    skts=tab["skts"][ps:ps + 1].expand(n, -1, -1, -1), cyls=tab["cyl"][ps:ps + 1].expand(n, -1),
                    bones=tab["bones"][ps:ps + 1].expand(n, -1, -1),
                    cams=torch.full((n, 1), cam_idx, dtype=torch.long, device=dev), N_uniques=1, perturb=False,
-                   N_importance=args.N_importance, raw_noise_std=0., nanmean_chunk=args.chunk)
+                   N_importance=args.N_importance, raw_noise_std=0., nanmean_chunk=args.chunk,
+                   **({"want_normals": True} if normals else {}))
         bg = 1.0 if white_bkgd else 0.0
         out[slot, idx] = ret["rgb_map"] + (1. - ret["acc_map"])[:, None] * bg         # run_nerf.py:103-133
+        if normals:
+            nmaps[slot, idx] = ret["normal_map"]
     out = out.reshape(len(mine), H, W, 3)
+    if normals:
+        return out, nmaps.reshape(len(mine), H, W, 3)
     if world == 1:
         return out
     counts = [len(range(r, len(c2ws), world)) for r in range(world)]

@@ -236,6 +236,19 @@ int danbo_field_agg_bwd(const float* rays, int ray_stride, int n_rays, int S, co
                         float* d_logit, const int* work, int pair_capacity, float* const* grads, int num_sms,
                         int agg_mode, void* stream);
 
+/* The gradient of the field with respect to the sample positions p = o + z d (surface normals: seed d raw with
+ * (0,0,0,1) on every row and the rows' own gradients come out of one pass).  Arguments as danbo_field_agg_bwd, with
+ * three accumulators (fp32, added to) in place of grads: d_pts (n_rays*S, 3), required; d_vol (n_poses,24,240) and
+ * d_skts (n_poses,24,4,4), each optional (NULL: not formed).  No aggregation-net or axis-scale gradient.  Unlike
+ * danbo_field_agg_bwd, the derivative of the feature window exp(-2 sum x^6) is included (the true gradient; training
+ * detaches the window), in d_pts and d_skts alike.  2 launches. */
+int danbo_field_agg_bwd_pts(const float* rays, int ray_stride, int n_rays, int S, const float* z, const unsigned int* mask,
+                            const int* active_ids, const int* active_count, int capacity, const float* pose_skts,
+                            const float* pose_vol, int rays_per_pose, int n_poses, const float* const* consts,
+                            const float* logits, const float* hbar, const float* dX, const float* g_logit_ext,
+                            float* d_hbar, float* d_logit, const int* work, int pair_capacity, float* d_pts,
+                            float* d_vol, float* d_skts, int num_sms, int agg_mode, void* stream);
+
 /* GN1 + GN2: the per-pose skeleton graph net, pose_bones (n_poses,24,3) axis-angle -> vol_out (n_poses,24,240) bone
  * feature lines (encode_graph_inputs core/encoders.py:460-473,859-877; BodyGNN.forward on FactorizeGNN
  * core/networks/gnn_backbone.py:683-704,225-274; ParallelLinear core/networks/misc.py:174-183; incl. the doubled layer-0
