@@ -30,6 +30,7 @@ _SIGNATURES = {
     "danbo_pose_fwd": [c_p, c_p, c_p, c_p, c_p, c_i, c_p, c_p, c_i, c_i, c_p, c_p, c_f, c_f, c_f, c_p, c_p, c_p, c_p, c_p],
     "danbo_pose_bwd": [c_p, c_p, c_p, c_p, c_p, c_i, c_p, c_p, c_i, c_i, c_p, c_p, c_p, c_p, c_p, c_f, c_f, c_p, c_p, c_p,
                        c_p],
+    "danbo_pose_kp2d": [c_p, c_p, c_p, c_i, c_f, c_f, c_p, c_p, c_p],
     "danbo_train_loss": [c_p, c_p, c_p, c_p, c_p, c_p, c_f, c_i, c_i, c_i, c_f, c_f, c_p, c_p, c_p, c_p, c_i, c_f, c_p, c_p, c_f,
                          c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p],
     "danbo_adam_step": [c_p, c_p, c_p, c_p, ctypes.c_longlong, c_p, c_f, c_f, c_f, c_p, c_i, c_p],

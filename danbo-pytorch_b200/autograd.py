@@ -349,3 +349,27 @@ def pose_layer(layer, idx, skip, G, anchors, rest_idx=None, tol=0., coef=0., ext
     spec = dict(names=names, buffers=buffers, skip=int(skip), G=int(G), anchors=anchors, tol=float(tol),
                 coef=float(coef), ext_scale=float(ext_scale), grads_in_place=bool(grads_in_place))
     return _PoseLayer.apply(spec, idx, *[p for _, p in layer.named_parameters()])
+
+
+class _PoseKp2d(torch.autograd.Function):
+    """The 2D keypoint reprojection term (`pose_opt.kp2d_loss`) as one launch (danbo_pose_kp2d), which writes d loss /
+    d kps with the loss; the backward scales it.  Under the pose layer, that gradient reaches danbo_pose_bwd as its
+    d_kps (`_PoseLayer.backward`)."""
+
+    @staticmethod
+    def forward(ctx, kps, kp2d, proj, sigma, coef):
+        loss, px, d_kps = K.pose_kp2d(kps.detach().contiguous(), kp2d, proj, sigma, coef)
+        ctx.save_for_backward(d_kps)
+        ctx.mark_non_differentiable(px)
+        return loss, px
+
+    @staticmethod
+    def backward(ctx, d_loss, _d_px):
+        (d_kps,) = ctx.saved_tensors
+        return d_loss * d_kps, None, None, None, None
+
+
+def pose_kp2d(kps, kp2d, proj, sigma, coef):
+    """kps (G,24,3) fp32 (the pose layer's output), kp2d (G,24,3) detections (u, v, confidence), proj (G,3,4), both
+    contiguous fp32 on kps' device.  -> (loss, kp2d_px): the differentiable scalar term and the mean pixel error."""
+    return _PoseKp2d.apply(kps, kp2d, proj, float(sigma), float(coef))

@@ -50,6 +50,11 @@ PRESETS = {
 }
 
 
+# flags of this package that the reference does not have: the 2D keypoint reprojection term of pose fitting and
+# --opt_pose training (training.kp2d_batch); kp2d_coef = 0 leaves it off
+PACKAGE_DEFAULTS = dict(kp2d_sigma=100.0, kp2d_coef=0.0)
+
+
 def _coerce(v):
     if v in ("True", "False"):
         return v == "True"
@@ -76,7 +81,7 @@ def read_config_file(path):
 
 
 def make_args(preset=None, config_file=None, **overrides):
-    d = dict(DEFAULTS)
+    d = dict(DEFAULTS, **PACKAGE_DEFAULTS)
     if config_file is not None:
         d.update(read_config_file(config_file))
     if preset is not None:

@@ -241,6 +241,55 @@ __global__ void bwd_kernel(Layer L, const float* __restrict__ d_skts, const floa
     }
 }
 
+// 2D keypoint reprojection term: joint j of pose g projects through P_g (3x4) to (u, v) = (P0 X, P1 X) / P2 X with
+// X = [kps_j, 1]; the residual against the detection (u^, v^, c) is penalised per coordinate with Geman-McClure,
+// rho(r) = s^2 r^2 / (s^2 + r^2), weighted by c.  loss = coef / (G * 24) * sum c (rho(r_u) + rho(r_v)); d kps is
+// written in the same pass (d rho / d r = 2 s^4 r / (s^2 + r^2)^2, d u / d X = (P0 - u P2) / w).  A joint at or behind
+// the camera (w <= 1e-6) adds nothing to the loss, the pixel error or the gradient.  Same layout as fwd_kernel: one
+// block, warp w takes poses w, w + warps, ..., lane = joint; the loss and the pixel error are reduced in the block.
+__global__ void kp2d_kernel(const float* __restrict__ kps, const float* __restrict__ kp2d, const float* __restrict__ proj,
+                            int n_poses, float sigma, float coef, float* __restrict__ d_kps, float* __restrict__ stats) {
+    __shared__ float red[3][kMaxWarps];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+    const float s2 = sigma * sigma, scale = coef / (float)(n_poses * DANBO_J);
+    float loss = 0.f, px = 0.f, seen = 0.f;
+    for (int g = warp; g < n_poses; g += nw) {
+        if (lane >= DANBO_J) continue;
+        const size_t at = (size_t)g * DANBO_J + lane;
+        const float* P = proj + (size_t)g * 12;
+        const float X[3] = {kps[at * 3], kps[at * 3 + 1], kps[at * 3 + 2]};
+        float h[3];
+#pragma unroll
+        for (int r = 0; r < 3; ++r) h[r] = P[r * 4] * X[0] + P[r * 4 + 1] * X[1] + P[r * 4 + 2] * X[2] + P[r * 4 + 3];
+        const float c = kp2d[at * 3 + 2];
+        float d[3] = {0.f, 0.f, 0.f};
+        if (h[2] > 1e-6f) {
+            const float u = h[0] / h[2], v = h[1] / h[2];
+            const float ru = u - kp2d[at * 3], rv = v - kp2d[at * 3 + 1];
+            const float qu = s2 + ru * ru, qv = s2 + rv * rv;
+            loss += c * (s2 * ru * ru / qu + s2 * rv * rv / qv);
+            if (c > 0.f) { px += sqrtf(ru * ru + rv * rv); seen += 1.f; }
+            const float gu = scale * c * 2.f * s2 * s2 * ru / (qu * qu) / h[2];
+            const float gv = scale * c * 2.f * s2 * s2 * rv / (qv * qv) / h[2];
+#pragma unroll
+            for (int k = 0; k < 3; ++k) d[k] = gu * (P[k] - u * P[8 + k]) + gv * (P[4 + k] - v * P[8 + k]);
+        }
+#pragma unroll
+        for (int k = 0; k < 3; ++k) d_kps[at * 3 + k] = d[k];
+    }
+    loss = warp_sum(loss);
+    px = warp_sum(px);
+    seen = warp_sum(seen);
+    if (lane == 0) { red[0][warp] = loss; red[1][warp] = px; red[2][warp] = seen; }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        float a = 0.f, b = 0.f, n = 0.f;
+        for (int w = 0; w < nw; ++w) { a += red[0][w]; b += red[1][w]; n += red[2][w]; }
+        stats[0] = a * scale;
+        stats[1] = n > 0.f ? b / n : 0.f;
+    }
+}
+
 static int threads_for(int n_poses) { return 32 * (n_poses < kMaxWarps ? n_poses : kMaxWarps); }
 
 static bool layer_ok(const Layer& L) {
@@ -282,6 +331,16 @@ extern "C" int danbo_pose_bwd(const float* pelvis, const float* bones, const flo
     if (d_reg && !anchor_bones) return -1;
     pose::bwd_kernel<<<1, pose::threads_for(n_poses), 0, (cudaStream_t)stream>>>(
         L, d_skts, d_bones, d_kps, anchor_bones, d_reg, tol, coef, g_pelvis, g_bones, g_root_bones);
+    DANBO_CHECK_LAUNCH();
+    return 0;
+}
+
+extern "C" int danbo_pose_kp2d(const float* kps, const float* kp2d, const float* proj, int n_poses, float sigma,
+                               float coef, float* d_kps, float* stats, void* stream) {
+    if (n_poses <= 0) return 0;
+    if (!kps || !kp2d || !proj || !d_kps || !stats || !(sigma > 0.f)) return -1;
+    pose::kp2d_kernel<<<1, pose::threads_for(n_poses), 0, (cudaStream_t)stream>>>(kps, kp2d, proj, n_poses, sigma, coef,
+                                                                                  d_kps, stats);
     DANBO_CHECK_LAUNCH();
     return 0;
 }

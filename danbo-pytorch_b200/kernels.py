@@ -884,6 +884,26 @@ def pose_bwd(layer, idx, idx_stride, n_poses, d_skts, grads, d_bones=None, d_kps
     _count(1)
 
 
+def pose_kp2d(kps, kp2d, proj, sigma, coef):
+    """The 2D keypoint reprojection term (danbo_pose_kp2d) of kps (G,24,3) against detections kp2d (G,24,3) = (u, v,
+    confidence) through projection matrices proj (G,3,4), all contiguous fp32 on one device.
+    -> loss (scalar), kp2d_px (scalar, mean pixel error over the joints with confidence > 0), d loss / d kps (G,24,3)."""
+    _need_cuda(kps, kp2d, proj)
+    dev, G = kps.device, kps.shape[0]
+    for name, t, shape in (("kps", kps, (G, J, 3)), ("kp2d", kp2d, (G, J, 3)), ("proj", proj, (G, 3, 4))):
+        if t.dtype != torch.float32 or not t.is_contiguous() or t.device != dev or tuple(t.shape) != shape:
+            raise ValueError(f"pose_kp2d: {name} must be a contiguous fp32 {shape} tensor on {dev}")
+    if not float(sigma) > 0:
+        raise ValueError("pose_kp2d: sigma must be positive")
+    d_kps = torch.empty(G, J, 3, device=dev)
+    stats = torch.empty(2, device=dev)
+    with _Timed("pose_kp2d"):
+        _lib.check(_lib.load().danbo_pose_kp2d(_p(kps), _p(kp2d), _p(proj), int(G), float(sigma), float(coef),
+                                               _p(d_kps), _p(stats), _stream()), "danbo_pose_kp2d")
+    _count(1)
+    return stats[0], stats[1], d_kps
+
+
 LOSS_KINDS = {"L1": 0, "MSE": 1}
 
 

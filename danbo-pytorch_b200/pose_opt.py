@@ -374,3 +374,25 @@ def kp_loss(args, anchors, kp_idx, kp_opts, popt_layer=None, temp_val=None):
         losses["temp_loss"] = ((ang + vel) * temp_val[..., None].to(dev)).mean() * float(args.temp_coef)
     pjpc = (pick(anchors["kps"]) - kp_opts["kp_batch"].detach()).pow(2.).sum(-1).pow(0.5)
     return losses, {"MPJPC": pjpc.mean() / float(getattr(args, "ext_scale", 0.001))}
+
+
+# ---- 2D keypoint reprojection term (the torch statement of danbo_pose_kp2d, csrc/pose.cu) ---------------------------
+def kp2d_loss(kps, kp2d, proj, sigma, coef):
+    """kps (G,24,3) world-frame joints, kp2d (G,24,3) detections (pixel u, pixel v, confidence c >= 0) in SMPL joint
+    order, proj (G,3,4) projection matrices.  -> (loss, kp2d_px): coef / (G*24) * sum c (rho(r_u) + rho(r_v)) with the
+    Geman-McClure rho(r) = sigma^2 r^2 / (sigma^2 + r^2) on the pixel residuals, and the mean |r| over the joints with
+    c > 0 (detached).  Joints at or behind the camera (w = P2 [kps, 1] <= 1e-6) contribute nothing, gradient included."""
+    G, J = kps.shape[:2]
+    X = torch.cat([kps, torch.ones_like(kps[..., :1])], -1)
+    h = (proj[:, None] @ X[..., None])[..., 0]                                 # (G,J,3)
+    front = h[..., 2] > 1e-6
+    w = torch.where(front, h[..., 2], torch.ones_like(h[..., 2]))
+    r = h[..., :2] / w[..., None] - kp2d[..., :2]
+    r = torch.where(front[..., None], r, torch.zeros_like(r))
+    s2 = float(sigma) ** 2
+    rho = (s2 * r * r / (s2 + r * r)).sum(-1)
+    c = kp2d[..., 2]
+    loss = (c * rho).sum() * (float(coef) / (G * J))
+    seen = (front & (c > 0)).to(r.dtype)
+    px = (r.detach().norm(dim=-1) * seen).sum() / seen.sum().clamp(min=1)
+    return loss, px

@@ -67,6 +67,18 @@ def rays_in_box(H, W, focal, c2w, cyl, device, c2w_dev=None):
     return rays_o, rays_d, idx
 
 
+def projection_matrix(c2w, H, W, focal):
+    """The 3x4 projection P of the pinhole cameras of `rays_in_box` and `synthetic` (looking down -z; pixel (i, j) on
+    the direction ((i - W/2)/f, -(j - H/2)/f, -1) in the camera frame): a world point X projects to pixel
+    (P0 [X,1], P1 [X,1]) / P2 [X,1].  P = [[f, 0, -W/2], [0, -f, -H/2], [0, 0, -1]] [R^T | -R^T t] with c2w = [R | t].
+    c2w: (4,4) or (3,4), or a batch (..., 3|4, 4), numpy or torch.  -> float64 numpy (..., 3, 4)."""
+    c2w = np.asarray(c2w.detach().cpu() if torch.is_tensor(c2w) else c2w, dtype=np.float64)[..., :3, :4]
+    R, t = c2w[..., :3, :3], c2w[..., :3, 3:]
+    Rt = np.swapaxes(R, -1, -2)
+    K = np.array([[focal, 0., -W * 0.5], [0., -focal, -H * 0.5], [0., 0., -1.]], dtype=np.float64)
+    return K @ np.concatenate([Rt, -Rt @ t], -1)
+
+
 @torch.no_grad()
 def render_images(caster, args, c2ws, poses, H, W, focal=None, cam_idx=0, white_bkgd=True, near=syn.NEAR, far=syn.FAR,
                   graphed=False, distributed=False, normals=False):

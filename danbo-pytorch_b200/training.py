@@ -203,6 +203,47 @@ def pose_batch_poses(batch):
     return G, n // G
 
 
+KP2D_KEYS = ("kp2d", "kp2d_proj")
+
+
+def kp2d_batch(args, batch, pose_layer=True):
+    """The 2D keypoint term's inputs of a batch: (kp2d (G,24,3) detections (u, v, confidence), kp2d_proj (G,3,4)),
+    G = N_uniques, when the batch carries both and args.kp2d_coef > 0; None when the term is off.  A batch with one of
+    the two keys, with other shapes, or with the term on and no pose layer raises ValueError (host-side checks only:
+    nothing has run on the device yet)."""
+    has = [k in batch for k in KP2D_KEYS]
+    if not any(has):
+        return None
+    if not all(has):
+        raise ValueError(f"the 2D keypoint term needs both batch['kp2d'] and batch['kp2d_proj'] (got only "
+                         f"{KP2D_KEYS[has.index(True)]!r})")
+    G = int(batch["N_uniques"])
+    kp2d, proj = batch["kp2d"], batch["kp2d_proj"]
+    if tuple(kp2d.shape) != (G, 24, 3) or tuple(proj.shape) != (G, 3, 4):
+        raise ValueError(f"batch['kp2d'] must be (N_uniques, 24, 3) = ({G}, 24, 3) and batch['kp2d_proj'] ({G}, 3, 4); "
+                         f"got {tuple(kp2d.shape)} and {tuple(proj.shape)}")
+    if G <= 0 or int(batch["kp_idx"].shape[0]) % G:
+        raise ValueError(f"the 2D keypoint term needs an image-major batch of N_uniques ({G}) equal runs")
+    if not float(getattr(args, "kp2d_coef", 0.)) > 0:
+        return None
+    if not pose_layer:
+        raise ValueError("the 2D keypoint term (kp2d_coef > 0) needs a pose layer (popt_kwargs of pose_opt.create_popt)")
+    if not float(getattr(args, "kp2d_sigma", 100.)) > 0:
+        raise ValueError("kp2d_sigma must be positive")
+    return kp2d, proj
+
+
+def _kp2d_term(args, kps, kp2d, kernels):
+    """(loss, kp2d_px) of the 2D keypoint term on the pose layer's (G,24,3) kps: the kernel (autograd.pose_kp2d) or the
+    PyTorch ops (pose_opt.kp2d_loss)."""
+    from . import autograd, pose_opt
+    det, proj = (t.to(device=kps.device, dtype=torch.float32).contiguous() for t in kp2d)
+    sigma, coef = float(getattr(args, "kp2d_sigma", 100.)), float(args.kp2d_coef)
+    if kernels:
+        return autograd.pose_kp2d(kps, det, proj, sigma, coef)
+    return pose_opt.kp2d_loss(kps, det, proj, sigma, coef)
+
+
 def _refuse_pose_graph(args, caster, world_size, pose_optimizer, layer,
                        what="graph capture of a training step with a pose layer"):
     """What a captured iteration with a pose layer (and PoseFitStep, which runs the same kernels) does not cover: raise,
@@ -234,7 +275,9 @@ class TrainStep:
                  pose_optimizer=None):
         """`popt_kwargs` / `pose_optimizer`: what `pose_opt.create_popt` returns (--opt_pose, core/trainer.py:314-341):
         the batch's poses then come from the pose layer (indexed by `batch['kp_idx']`), the pose regulariser
-        (`pose_opt.kp_loss`) joins the loss and the pose optimiser steps with the network's."""
+        (`pose_opt.kp_loss`) joins the loss and the pose optimiser steps with the network's.  A batch with `kp2d` and
+        `kp2d_proj` adds the 2D keypoint term when args.kp2d_coef > 0 (`kp2d_batch`): danbo_pose_kp2d in a captured
+        step, `pose_opt.kp2d_loss` in an eager one; `last_stats["kp2d_px"]` is its mean pixel error."""
         self.caster, self.args, self.world = caster, args, world_size
         # flags the reference trainer honours and this step does not implement: raise, never ignore (no shipped config
         # sets any of them)
@@ -300,7 +343,7 @@ class TrainStep:
                 loss, preds = self._step(b) if self._graph_whole else self._fwd_bwd(b)
                 out = {"loss": loss, "rgb_map": preds["rgb_map"], "acc_map": preds["acc_map"]}
                 if self.popt is not None:
-                    out["MPJPC"] = self.last_stats["MPJPC"]
+                    out.update(self.last_stats)
                 return out
             # building the graph must not train: parameters, moments and the step counters (the network's and the
             # pose layer's) are restored after capture
@@ -312,6 +355,9 @@ class TrainStep:
                                       capture_error_mode="thread_local" if world_size > 1 else "global")
 
     def __call__(self, batch):
+        kp2d = kp2d_batch(self.args, batch, self.popt is not None)     # refused before any device work
+        if kp2d is None and any(k in batch for k in KP2D_KEYS):
+            batch = {k: v for k, v in batch.items() if k not in KP2D_KEYS}     # the term is off: nothing of it runs
         if self._graphed is not None:
             if self.popt is not None:
                 pose_batch_poses(batch)          # refused before any device work
@@ -319,7 +365,7 @@ class TrainStep:
                 batch = {k: v for k, v in batch.items() if k not in ("kp_batch", "skts", "bones")}
             out = self._graphed(**batch)
             if self.popt is not None:
-                self.last_stats = {"MPJPC": out["MPJPC"]}
+                self.last_stats = {k: out[k] for k in ("MPJPC", "kp2d_px") if k in out}
             if not self._graph_whole:
                 if self.world > 1:
                     self.bucket.allreduce(average=True)
@@ -403,6 +449,7 @@ class TrainStep:
         self.caster.train()
         self.bucket.zero()
         extra = None
+        kp2d = kp2d_batch(a, batch, self.popt is not None)
         if self._pose_kernels:
             from .autograd import pose_layer
             G, skip = pose_batch_poses(batch)
@@ -416,6 +463,9 @@ class TrainStep:
             ex = lambda t: t[:, None].expand(G, skip, *t.shape[1:]).reshape(n, *t.shape[1:])
             batch = dict(batch, kp_batch=ex(kps), skts=ex(skts), bones=ex(bones))
             self.last_stats = {"MPJPC": mpjpc}
+            if kp2d is not None:
+                l2d, self.last_stats["kp2d_px"] = _kp2d_term(a, kps, kp2d, kernels=True)
+                extra = extra + l2d
         elif self.popt is not None:
             from . import pose_opt
             layer = self.popt["popt_layer"]
@@ -428,6 +478,10 @@ class TrainStep:
                                                        {"kp_batch": kps, "bones": bones, "rots": rots}, popt_layer=layer,
                                                        temp_val=batch.get("temp_val"))
             extra = sum(losses.values())
+            if kp2d is not None:
+                skip = int(batch["kp_idx"].shape[0]) // int(batch["N_uniques"])      # one row per pose of the batch
+                l2d, self.last_stats["kp2d_px"] = _kp2d_term(a, kps[::skip], kp2d, kernels=False)
+                extra = extra + l2d
         net = self.caster.network
         net.pose_kernels = self._pose_kernels        # the graph net's kernels then also return d pose
         try:
@@ -460,9 +514,11 @@ class PoseFitStep:
     `update_embed_fns` schedule is applied to the network.
 
     Loss: the trainer's image terms as TrainStep computes them (rgb_loss, rgb_loss0, soft_softmax_loss) plus the pose
-    regulariser (kp_loss, danbo_pose_fwd).  vol_scale_loss depends on the network's axis_scale only, has no pose
-    gradient and is left out.  Frames the field was not trained on have no frame code: give them cams < 0 in the batch
-    and they are rendered with the mean code (danbo_ray_bias's last code row).
+    regulariser (kp_loss, danbo_pose_fwd), and the 2D keypoint reprojection term when the batch carries `kp2d` and
+    `kp2d_proj` and args.kp2d_coef > 0 (`kp2d_batch`; danbo_pose_kp2d; `last_stats["kp2d_px"]`).  vol_scale_loss
+    depends on the network's axis_scale only, has no pose gradient and is left out.  Frames the field was not trained
+    on have no frame code: give them cams < 0 in the batch and they are rendered with the mean code (danbo_ray_bias's
+    last code row).
 
     graph=True captures the whole iteration as one CUDA graph (graphs.GraphedFn); capture applies no pose step (the pose
     arena, its moments and its step counter are restored).  The MLP weight packs are keyed on the weights and checked
@@ -493,8 +549,7 @@ class PoseFitStep:
 
             def run(_param_ptrs=None, **b):
                 loss, preds = self._step(b)
-                return {"loss": loss, "rgb_map": preds["rgb_map"], "acc_map": preds["acc_map"],
-                        "MPJPC": self.last_stats["MPJPC"]}
+                return dict(self.last_stats, loss=loss, rgb_map=preds["rgb_map"], acc_map=preds["acc_map"])
             po = pose_optimizer
             self._graphed = GraphedFn(run, dev, warmup=3, state=[po.flat, po.exp_avg, po.exp_avg_sq, po.step_dev])
 
@@ -517,6 +572,9 @@ class PoseFitStep:
 
     def __call__(self, batch):
         pose_batch_poses(batch)                  # refused before any device work
+        kp2d = kp2d_batch(self.args, batch)
+        if kp2d is None and any(k in batch for k in KP2D_KEYS):
+            batch = {k: v for k, v in batch.items() if k not in KP2D_KEYS}     # the term is off: nothing of it runs
         if self._graphed is None:
             return self._step(batch)
         # the poses come from the layer: the feed's tables would only be copied into static buffers
@@ -529,7 +587,7 @@ class PoseFitStep:
         # the graph reads the parameters through the raw pointers they had at capture: re-pointed storage recaptures
         ptrs = hash(tuple(p.data_ptr() for p in self.caster.network.parameters()))
         out = self._graphed(_param_ptrs=ptrs, **batch)
-        self.last_stats = {"MPJPC": out["MPJPC"]}
+        self.last_stats = {k: out[k] for k in ("MPJPC", "kp2d_px") if k in out}
         return out["loss"], out
 
     def _step(self, batch):
@@ -545,8 +603,12 @@ class PoseFitStep:
             tol=getattr(a, "opt_pose_tol", 0.), coef=getattr(a, "opt_pose_coef", 0.),
             ext_scale=getattr(a, "ext_scale", 0.001), grads_in_place=True)
         ex = lambda t: t[:, None].expand(G, skip, *t.shape[1:]).reshape(n, *t.shape[1:])
-        batch = dict(batch, kp_batch=ex(kps), skts=ex(skts), bones=ex(bones))
         self.last_stats = {"MPJPC": mpjpc}
+        kp2d = kp2d_batch(a, batch)
+        if kp2d is not None:
+            l2d, self.last_stats["kp2d_px"] = _kp2d_term(a, kps, kp2d, kernels=True)
+            reg = reg + l2d
+        batch = dict(batch, kp_batch=ex(kps), skts=ex(skts), bones=ex(bones))
         net.pose_kernels = True                  # the graph net's kernels return d pose
         try:
             with self._frozen():

@@ -295,6 +295,16 @@ int danbo_pose_bwd(const float* pelvis, const float* bones, const float* root_bo
                    const float* anchor_bones, const float* d_reg, float tol, float coef, float* g_pelvis,
                    float* g_bones, float* g_root_bones, void* stream);
 
+/* 2D keypoint reprojection term of the pose layer's joints.  kps (n_poses,24,3) as danbo_pose_fwd wrote them (world
+ * frame), kp2d (n_poses,24,3) = detections (pixel u, pixel v, confidence c >= 0) in SMPL joint order, proj
+ * (n_poses,3,4) one projection matrix per pose.  Per joint (u, v) = (P0 X, P1 X) / w with X = [kps, 1], w = P2 X, and
+ * the Geman-McClure penalty rho(r) = sigma^2 r^2 / (sigma^2 + r^2) on each coordinate of r = (u - u^, v - v^):
+ * stats[0] = coef / (n_poses * 24) * sum c (rho(r_u) + rho(r_v)), stats[1] = the mean |r| over the joints with c > 0
+ * in front of the camera (0 when there is none).  Writes d_kps (n_poses,24,3) = d stats[0] / d kps.  A joint with
+ * w <= 1e-6 (at or behind the camera) contributes 0 to both stats and to d_kps.  sigma > 0.  One launch. */
+int danbo_pose_kp2d(const float* kps, const float* kp2d, const float* proj, int n_poses, float sigma, float coef,
+                    float* d_kps, float* stats, void* stream);
+
 /* L*: the trainer's losses on the outputs of the path, value and gradients in one launch (core/trainer.py:396-422
  * _compute_nerf_loss with loss_fn L1 (loss_kind 0) or MSE (1) on rgb + (1 - acc) bg for the fine and, if rgb0 != NULL,
  * the coarse maps; :507-536 _compute_soft_softmax_loss when confd != NULL; :538-553 _compute_volume_scale_loss when
