@@ -63,6 +63,8 @@ _SIGNATURES = {
     "danbo_mlp_wgrad": [c_p, c_p, c_p, c_i, c_p, c_i, c_p, c_i, c_p, c_p, c_p, c_p, c_p],
     "danbo_composite_resample": [c_p, c_i, c_i, c_i, c_i, c_p, c_p, c_p, c_p, c_f, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_i, c_p],
     "danbo_merge_composite": [c_p, c_i, c_i, c_i, c_i, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_f, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p],
+    "danbo_merge_composite_parts": [c_p, c_i, c_i, c_i, c_i, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_f, c_p, c_p, c_p, c_p, c_p,
+                                    c_p, c_p, c_p, c_i, c_p, c_p],
 }
 
 EXPORTS = tuple(_SIGNATURES)

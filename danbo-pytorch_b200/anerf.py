@@ -71,6 +71,7 @@ class AnerfCaster(RayCaster):
     fine network is evaluated on all S_c + S_f merged samples (raycasters.py:345-371)."""
     _supports_fine_network = True
     _supports_normals = False             # its density also depends on the point through the cut-off encodings
+    _supports_parts = False               # no per-bone aggregation: every bone's encoding goes into one MLP
 
     def __init__(self, network, network_fine=None, single_net=True, rest_poses=None, align_bones="align", skel_type=None,
                  **kwargs):

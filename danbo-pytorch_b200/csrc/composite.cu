@@ -6,6 +6,7 @@
 // accumulate in fp64 like ATen's CPU kernels (acc_type<float>) and round each output to fp32.  16 B raw + 4 B z in,
 // 8 B (weight, alpha) out per sample: too few bytes to bind the forward kernels to HBM, they are bound by instruction issue.
 #include "common.cuh"
+#include "field_common.cuh"
 #include <math.h>
 
 namespace danbo {
@@ -366,6 +367,88 @@ merge_composite_kernel(const float* __restrict__ rays, int ray_stride, int n_ray
     }
 }
 
+// Fine pass of an eval render with its body-part map: merge_composite_kernel's composite, unchanged, then
+//   part_map[n, j] = sum_m w_m p_mj,  p_m = get_agg(logits_m, 1 - visible_m)  (danbo.py:388-415)
+// over the merged samples.  Each lane sums w p over the samples whose weights it wrote, in its sample order, into 24
+// registers; the group's xor butterfly then adds the lanes' sums in a fixed order (no atomics).  A sample no bone sees
+// (mask 0) has p = 0 and is skipped.  Sigmoid passes hold logits only at visible bones, so only those are read; a
+// softmax pass holds all 24 of an active row, and its max runs over all of them (field_common.cuh softmax_terms).
+template <int kL, int kEo>
+__global__ void __launch_bounds__(32 * kWarpsPerBlock)
+merge_composite_parts_kernel(const float* __restrict__ rays, int ray_stride, int n_rays, int S_c, int S_f,
+                             const float* __restrict__ raw0, const uint32_t* __restrict__ mask0,
+                             const float* __restrict__ raw1, const uint32_t* __restrict__ mask1,
+                             const float* __restrict__ z_all, const int* __restrict__ order, const float* __restrict__ noise,
+                             float inv_B, float* __restrict__ weights, float* __restrict__ alpha, float* __restrict__ rgb,
+                             float* __restrict__ disp, float* __restrict__ acc, float* __restrict__ raw_merged,
+                             const float* __restrict__ logits0, const float* __restrict__ logits1, int agg_mode,
+                             float* __restrict__ part_map /* (n,24) */) {
+    const int lane = threadIdx.x & 31, g = lane & (kL - 1), slot = threadIdx.x / kL;
+    const unsigned gmask = group_mask<kL>(lane);
+    const int n_slot = blockIdx.x * (blockDim.x / kL) + slot;
+    const bool valid = n_slot < n_rays;
+    const int n = valid ? n_slot : n_rays - 1;
+    const int St = S_c + S_f;
+    const float* r = rays + (size_t)n * ray_stride;
+    const float norm_d = __fsqrt_rn(__fadd_rn(__fadd_rn(__fmul_rn(r[3], r[3]), __fmul_rn(r[4], r[4])), __fmul_rn(r[5], r[5])));
+    const int* ord = order + (size_t)n * St;
+    const float4* r0 = reinterpret_cast<const float4*>(raw0);
+    const float4* r1 = reinterpret_cast<const float4*>(raw1);
+    const float4 empty = r0[(size_t)n_rays * S_c + n];
+    auto fetch = [&](int i) {
+        const int src = ord[i];
+        const bool coarse = src < S_c;
+        const size_t sidx = coarse ? (size_t)n * S_c + src : (size_t)n * S_f + src - S_c;
+        const uint32_t m = (coarse ? mask0 : mask1)[sidx];
+        const float4 raw = (coarse ? r0 : r1)[sidx];
+        const float4 v = m ? raw : empty;
+        if (raw_merged && valid) reinterpret_cast<float4*>(raw_merged)[(size_t)n * St + i] = v;
+        return v;
+    };
+    float* w_row = weights + (size_t)n * St;
+    composite_group<kL, kEo>(z_all + (size_t)n * St, St, g, gmask, valid, norm_d, inv_B,
+                             noise ? noise + (size_t)n * St : nullptr, fetch, nullptr, w_row,
+                             alpha + (size_t)n * St, rgb + (size_t)n * 3, disp + n, acc + n);
+    constexpr int R = 32 / kL;
+    float pm[DANBO_J];
+#pragma unroll
+    for (int j = 0; j < DANBO_J; ++j) pm[j] = 0.f;
+    if (valid) {                                        // a group past the last ray wrote no weights: it adds zeros
+#pragma unroll
+        for (int v = 0; v < R; ++v)
+#pragma unroll
+            for (int e = 0; e < kEo; ++e) {
+                const int i = (v * kL + g) * kEo + e;   // the samples whose weights this lane wrote (composite_group)
+                if (i >= St) continue;
+                const int src = ord[i];
+                const bool coarse = src < S_c;
+                const size_t sidx = coarse ? (size_t)n * S_c + src : (size_t)n * S_f + src - S_c;
+                const uint32_t m = (coarse ? mask0 : mask1)[sidx];
+                if (!m) continue;
+                const float w = w_row[i];
+                const float* l = (coarse ? logits0 : logits1) + sidx * DANBO_J;
+                if (agg_mode == 1) {
+                    float amax, inv_den;
+                    softmax_terms(l, m, amax, inv_den);
+#pragma unroll
+                    for (int j = 0; j < DANBO_J; ++j)
+                        if ((m >> j) & 1u) pm[j] = fmaf(w, expf(l[j] - amax) * inv_den, pm[j]);
+                } else {
+#pragma unroll
+                    for (int j = 0; j < DANBO_J; ++j)
+                        if ((m >> j) & 1u) pm[j] = fmaf(w, (1.f / (1.f + expf(-l[j]))) * 1.002f - 0.001f, pm[j]);
+                }
+            }
+    }
+#pragma unroll
+    for (int j = 0; j < DANBO_J; ++j) pm[j] = group_sum<kL>(pm[j]);
+    if (valid) {
+#pragma unroll
+        for (int j = 0; j < DANBO_J; ++j)
+            if ((j & (kL - 1)) == g) part_map[(size_t)n * DANBO_J + j] = pm[j];
+    }
+}
+
 }  // namespace danbo
 
 using namespace danbo;
@@ -422,6 +505,31 @@ extern "C" int danbo_merge_composite(const float* rays, int ray_stride, int n_ra
         default: DANBO_MC_LAUNCH(5); break;
     }
 #undef DANBO_MC_LAUNCH
+    DANBO_CHECK_LAUNCH();
+    return 0;
+}
+
+extern "C" int danbo_merge_composite_parts(const float* rays, int ray_stride, int n_rays, int S_c, int S_f,
+                                           const float* raw0, const unsigned int* mask0, const float* raw1,
+                                           const unsigned int* mask1, const float* z_all, const int* order,
+                                           const float* noise, float inv_B, float* weights, float* alpha, float* rgb,
+                                           float* disp, float* acc, float* raw_merged, const float* confd0,
+                                           const float* confd1, int agg_mode, float* part_map, void* stream) {
+    if (n_rays <= 0) return 0;
+    if (S_c + S_f > kMaxS || !weights || !confd0 || !confd1 || !part_map || agg_mode < 0 || agg_mode > 1) return -1;
+#define DANBO_MCP_LAUNCH(E) merge_composite_parts_kernel<kMcLanes[E - 1], E>                                          \
+        <<<(n_rays + 32 * kWarpsPerBlock / kMcLanes[E - 1] - 1) / (32 * kWarpsPerBlock / kMcLanes[E - 1]),               \
+           32 * kWarpsPerBlock, 0, (cudaStream_t)stream>>>(                                                              \
+        rays, ray_stride, n_rays, S_c, S_f, raw0, mask0, raw1, mask1, z_all, order, noise, inv_B, weights, alpha, rgb,  \
+        disp, acc, raw_merged, confd0, confd1, agg_mode, part_map)
+    switch ((S_c + S_f + 31) / 32) {
+        case 1: DANBO_MCP_LAUNCH(1); break;
+        case 2: DANBO_MCP_LAUNCH(2); break;
+        case 3: DANBO_MCP_LAUNCH(3); break;
+        case 4: DANBO_MCP_LAUNCH(4); break;
+        default: DANBO_MCP_LAUNCH(5); break;
+    }
+#undef DANBO_MCP_LAUNCH
     DANBO_CHECK_LAUNCH();
     return 0;
 }

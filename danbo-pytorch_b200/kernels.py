@@ -391,6 +391,36 @@ def merge_composite(rays, S_c, S_f, raw0, mask0, raw1, mask1, z_all, order, nois
     return out
 
 
+def merge_composite_parts(rays, S_c, S_f, raw0, mask0, raw1, mask1, z_all, order, logits0, logits1, agg_mode,
+                          noise=None, inv_B=1.0, want_raw=False):
+    """merge_composite (eval mode) plus part_map (n,24) = sum_m w_m p_m, p_m the aggregation weights of merged sample m
+    from its pass's field_agg logits (`logits0` (n*S_c,24), `logits1` (n*S_f,24)) and visibility mask; the other
+    outputs are bit-identical to merge_composite's -> dict (rgb_map, disp_map, acc_map, alpha, weights, part_map [, raw])."""
+    _need_cuda(rays, raw0, mask0, raw1, mask1, z_all, order, logits0, logits1, noise)
+    n = rays.shape[0]
+    if tuple(logits0.shape) != (n * S_c, J) or tuple(logits1.shape) != (n * S_f, J):
+        raise ValueError(f"logits (n*S_c,24) and (n*S_f,24) expected, got {tuple(logits0.shape)}, {tuple(logits1.shape)}")
+    if agg_mode not in (0, 1):
+        raise ValueError(f"agg_mode {agg_mode!r}: 0 (sigmoid) or 1 (softmax)")
+    lib = _lib.load()
+    dev = rays.device
+    St = S_c + S_f
+    f = lambda *s: torch.empty(*s, device=dev, dtype=torch.float32)
+    out = {"weights": f(n, St), "alpha": f(n, St), "rgb_map": f(n, 3), "disp_map": f(n), "acc_map": f(n),
+           "part_map": f(n, J)}
+    if want_raw:
+        out["raw"] = f(n, St, 4)
+    with _Timed("merge_composite"):
+        _lib.check(lib.danbo_merge_composite_parts(_p(rays), rays.stride(0), n, S_c, S_f, _p(raw0), _p(mask0), _p(raw1),
+                                                   _p(mask1), _p(z_all), _p(order), _p(noise), float(inv_B),
+                                                   _p(out["weights"]), _p(out["alpha"]), _p(out["rgb_map"]),
+                                                   _p(out["disp_map"]), _p(out["acc_map"]), _p(out.get("raw")),
+                                                   _p(logits0), _p(logits1), int(agg_mode),
+                                                   _p(out["part_map"]), _stream()), "danbo_merge_composite_parts")
+    _count(1)
+    return out
+
+
 # ------------------------------------------------------------------------------------------------------ backward
 class ActSave:
     """bf16 activations of the fused MLP kept for the backward pass."""

@@ -150,11 +150,22 @@ def mesh_volume(vertices, triangles):
     return float((a * torch.cross(b, c, dim=-1)).sum() / 6.0)
 
 
+# RGB of the part of each of the 24 SMPL joints (skeleton.JOINT_NAMES order) in part-labelled meshes: 24 distinct
+# colours of a common categorical palette, fixed so that a part has the same colour in every file.
+PART_COLORS = np.array([
+    [128, 128, 128], [230, 25, 75], [0, 130, 200], [170, 255, 195],        # pelvis, l/r hip, spine1
+    [245, 130, 48], [70, 240, 240], [60, 180, 75], [255, 225, 25],         # l/r knee, spine2, l ankle
+    [0, 0, 128], [210, 245, 60], [128, 0, 0], [145, 30, 180],              # r ankle, spine3, l/r foot
+    [255, 255, 255], [250, 190, 212], [220, 190, 255], [64, 64, 64],       # neck, l/r collar, head
+    [240, 50, 230], [0, 128, 128], [170, 110, 40], [255, 215, 180],        # l/r shoulder, l/r elbow
+    [128, 128, 0], [0, 0, 255], [255, 250, 200], [0, 255, 0]], np.uint8)   # l/r wrist, l/r hand
+
+
 # ---- writers (trimesh.export / imageio.imwrite of run_render.py:1280,1343-1346) -----------------------------------
-def write_ply(path, vertices, triangles, normals=None):
+def write_ply(path, vertices, triangles, normals=None, colors=None):
     """Binary little-endian PLY with float32 vertices and int32 triangle indices; with `normals` (V,3) each vertex also
-    carries float32 nx ny nz (viewers then shade the mesh smoothly).  Without normals the bytes are those of a plain
-    vertex + face file."""
+    carries float32 nx ny nz (viewers then shade the mesh smoothly), with `colors` (V,3) uint8 red green blue.  Without
+    either the bytes are those of a plain vertex + face file."""
     v = np.ascontiguousarray(torch.as_tensor(vertices).detach().cpu().numpy(), dtype="<f4")
     f = np.ascontiguousarray(torch.as_tensor(triangles).detach().cpu().numpy(), dtype="<i4")
     props = "property float x\nproperty float y\nproperty float z\n"
@@ -164,6 +175,14 @@ def write_ply(path, vertices, triangles, normals=None):
             raise ValueError(f"write_ply: normals {nrm.shape} must match vertices {v.shape}")
         v = np.ascontiguousarray(np.concatenate([v.reshape(-1, 3), nrm.reshape(-1, 3)], 1))
         props += "property float nx\nproperty float ny\nproperty float nz\n"
+    if colors is not None:
+        col = torch.as_tensor(colors).detach().cpu().numpy()
+        if col.dtype != np.uint8 or col.shape != (len(v), 3):
+            raise ValueError(f"write_ply: colors must be uint8 ({len(v)}, 3), got {col.dtype} {col.shape}")
+        rec_v = np.empty(len(v), dtype=[("p", "<f4", (v.shape[1],)), ("c", "u1", (3,))])
+        rec_v["p"], rec_v["c"] = v, col
+        v = rec_v
+        props += "property uchar red\nproperty uchar green\nproperty uchar blue\n"
     head = ("ply\nformat binary_little_endian 1.0\n"
             f"element vertex {len(v)}\n{props}"
             f"element face {len(f)}\nproperty list uchar int vertex_indices\nend_header\n").encode("ascii")
@@ -175,9 +194,9 @@ def write_ply(path, vertices, triangles, normals=None):
         fh.write(rec.tobytes())
 
 
-def read_ply(path, with_normals=False):
-    """Inverse of write_ply (for tests and round trips) -> (vertices, triangles), or (vertices, triangles, normals) with
-    `with_normals` (a file without nx ny nz raises)."""
+def read_ply(path, with_normals=False, with_colors=False):
+    """Inverse of write_ply (for tests and round trips) -> (vertices, triangles), followed by the normals with
+    `with_normals` and the uint8 colours with `with_colors` (a file without nx ny nz / red green blue raises)."""
     with open(path, "rb") as fh:
         data = fh.read()
     end = data.index(b"end_header\n") + len(b"end_header\n")
@@ -185,14 +204,21 @@ def read_ply(path, with_normals=False):
     nv = int([l for l in head if l.startswith("element vertex")][0].split()[-1])
     nf = int([l for l in head if l.startswith("element face")][0].split()[-1])
     has_n = "property float nx" in head
+    has_c = "property uchar red" in head
     if with_normals and not has_n:
         raise ValueError(f"{path} has no vertex normals")
+    if with_colors and not has_c:
+        raise ValueError(f"{path} has no vertex colours")
     width = 6 if has_n else 3
-    vn = np.frombuffer(data, dtype="<f4", count=nv * width, offset=end).reshape(nv, width)
-    rec = np.frombuffer(data, dtype=[("n", "u1"), ("idx", "<i4", (3,))], count=nf, offset=end + nv * 4 * width)
+    vrec = np.frombuffer(data, dtype=[("p", "<f4", (width,)), ("c", "u1", (3 if has_c else 0,))], count=nv, offset=end)
+    vn = vrec["p"]
+    rec = np.frombuffer(data, dtype=[("n", "u1"), ("idx", "<i4", (3,))], count=nf, offset=end + vrec.nbytes)
+    out = (vn[:, :3].copy(), rec["idx"].copy())
     if with_normals:
-        return vn[:, :3].copy(), rec["idx"].copy(), vn[:, 3:].copy()
-    return vn[:, :3].copy(), rec["idx"].copy()
+        out += (vn[:, 3:].copy(),)
+    if with_colors:
+        out += (vrec["c"].copy(),)
+    return out
 
 
 def write_png(path, img):
@@ -247,7 +273,7 @@ def save_renders(basedir, rgbs, accs, fps=14):
 
 @torch.no_grad()
 def render_mesh(ray_caster, kps, skts, bones, radius=1.80, res=255, threshold=10., out_dir=None, preproc_kwargs=None,
-                normals=False):
+                normals=False, parts=False):
     """run_render.py:1266-1281: per pose, the (res+1)^3 raw-density lattice (`fwd_type='mesh'`), relu, marching cubes at
     `threshold`, vertices scaled to `v / res - 0.5`; written as `meshes/{i:03d}.ply` when out_dir is given.
     -> list of (vertices, triangles).
@@ -255,13 +281,21 @@ def render_mesh(ray_caster, kps, skts, bones, radius=1.80, res=255, threshold=10
     normals=True: -> list of (vertices, triangles, normals), the same vertices and triangles, with the unit outward
     normal -grad sigma / |grad sigma| of the field at every vertex (0 where the gradient is 0), from
     `render_pts_gradient` at the vertex's world position root + 2 radius v (the lattice is in xyz index order around
-    the root joint, `render_mesh_density`); the PLY files carry them as nx ny nz."""
+    the root joint, `render_mesh_density`); the PLY files carry them as nx ny nz.
+
+    parts=True: each entry also ends with the (V,24) aggregation weights of the bones at those vertex positions
+    (`render_pts_parts`), after the normals when both are asked for; the PLY files carry the PART_COLORS entry of each
+    vertex's arg-max bone as red green blue."""
     import os
     caster = getattr(ray_caster, "module", ray_caster)          # the training handle wraps the caster
     if normals:
         if not hasattr(caster, "render_pts_gradient"):
             raise NotImplementedError("render_mesh(normals=True) needs a caster with render_pts_gradient")
         caster._refuse_normals("render_mesh(normals=True)")
+    if parts:
+        if not hasattr(caster, "render_pts_parts"):
+            raise NotImplementedError("render_mesh(parts=True) needs a caster with render_pts_parts")
+        caster._refuse_parts("render_mesh(parts=True)")
     out = []
     if out_dir is not None:
         os.makedirs(os.path.join(out_dir, "meshes"), exist_ok=True)
@@ -270,12 +304,18 @@ def render_mesh(ray_caster, kps, skts, bones, radius=1.80, res=255, threshold=10
                          render_kwargs=preproc_kwargs, fwd_type="mesh")
         v, t = marching_cubes(torch.relu(raw.reshape(res + 1, res + 1, res + 1)), threshold)
         v = v / res - 0.5
-        n = None
-        if normals:
+        n = p = col = None
+        if normals or parts:
             root = torch.as_tensor(kps[i:i + 1]).reshape(1, -1, 3)[0, 0].to(v.device).float()
+        if normals:
             _, g = caster.render_pts_gradient(root + 2. * radius * v, kps[i:i + 1], skts[i:i + 1], bones[i:i + 1])
             n = caster._unit_normals(g).to(v.device)
+        if parts:
+            _, p = caster.render_pts_parts(root + 2. * radius * v, kps[i:i + 1], skts[i:i + 1], bones[i:i + 1])
+            p = p.to(v.device)
         if out_dir is not None:
-            write_ply(os.path.join(out_dir, "meshes", f"{i:03d}.ply"), v, t, normals=n)
-        out.append((v, t) if n is None else (v, t, n))
+            if parts:
+                col = PART_COLORS[p.argmax(-1).cpu().numpy()]
+            write_ply(os.path.join(out_dir, "meshes", f"{i:03d}.ply"), v, t, normals=n, colors=col)
+        out.append((v, t) + tuple(x for x in (n, p) if x is not None))
     return out

@@ -35,6 +35,7 @@ class RayCaster(nn.Module):
 
     _supports_fine_network = False        # a separate fine network (single_net=False): the A-NeRF caster only
     _supports_normals = True              # density gradients / normals (render_pts_gradient, want_normals): DANBO only
+    _supports_parts = True                # body-part maps (render_pts_parts, want_parts): a field with an aggregation net
 
     def __init__(self, network, network_fine=None, single_net=True, rest_poses=None, align_bones="align",
                  skel_type=None, use_volume_near_far=False, view_mode="world", **kwargs):
@@ -95,6 +96,9 @@ class RayCaster(nn.Module):
             raise RuntimeError("render_graphed is for eval mode")
         if ignored.get("want_normals"):
             raise NotImplementedError("want_normals is not implemented for render_graphed (normals are not captured): "
+                                      "use the plain call")
+        if ignored.get("want_parts"):
+            raise NotImplementedError("want_parts is not implemented for render_graphed (part maps are not captured): "
                                       "use the plain call")
         if ignored.get("ray_noise_std", 0.) > 0 or ignored.get("pytest"):
             raise NotImplementedError("ray_noise_std > 0 and pytest are not implemented")
@@ -235,19 +239,28 @@ class RayCaster(nn.Module):
                     subject_idxs=None, retraw=False, lindisp=False, perturb=0., N_importance=0, network_fine=None,
                     raw_noise_std=0., ray_noise_std=0., verbose=False, ext_scale=0.001, pytest=False, N_uniques=1,
                     render_confd=False, render_entropy=False, preproc_kwargs=None, netchunk=1024 * 64,
-                    nerf_type="danbo", use_viewdirs=True, nanmean_chunk=None, want_normals=False, _rand=None,
-                    _stages=None):
+                    nerf_type="danbo", use_viewdirs=True, nanmean_chunk=None, want_normals=False, want_parts=False,
+                    _rand=None, _stages=None):
         """Same arguments and returned dict as raycasters.py:245-377,516-546,710-716.
 
         Extra (optional) keywords: `nanmean_chunk` keeps the reference's per-chunk near/far fill (F8) when more than
         one reference chunk is passed in a single call; `want_normals` adds `normal_map` (n,3), the composite of the
-        samples' unit normals (`_render_normals`; eval mode without gradients only); `_rand`/`_stages` are test hooks
-        (inject the four random tensors / collect stage tensors)."""
+        samples' unit normals (`_render_normals`; eval mode without gradients only); `want_parts` adds `part_map` (n,24),
+        the composite of the samples' aggregation weights p_j (eval mode without gradients only; not together with
+        `want_normals`); `_rand`/`_stages` are test hooks (inject the four random tensors / collect stage tensors)."""
         if want_normals:
             self._refuse_normals("render_rays(want_normals=True)")
             if self.training or torch.is_grad_enabled():
                 raise NotImplementedError("want_normals is for eval mode without gradients (caster.eval(), torch.no_grad()): "
                                           "normals in training are not implemented")
+        if want_parts:
+            self._refuse_parts("render_rays(want_parts=True)")
+            if self.training or torch.is_grad_enabled():
+                raise NotImplementedError("want_parts is for eval mode without gradients (caster.eval(), torch.no_grad()): "
+                                          "part maps in training are not implemented")
+            if want_normals:
+                raise NotImplementedError("want_parts together with want_normals in one call is not implemented: make two "
+                                          "calls")
         # render_confd / render_entropy / verbose / retraw are accepted and ignored, as in the reference's render_rays
         # (raycasters.py:245-377 never reads them)
         if ray_noise_std > 0 or pytest:
@@ -269,7 +282,8 @@ class RayCaster(nn.Module):
                                         nanmean_chunk, bool(lindisp), _stages)
         return self._render_prepared(rays, pose_skts, pose_bones, pose_cyls, cam_idx, skip=skip, N_samples=N_samples,
                                      N_importance=N_importance, B=B, raw_noise_std=raw_noise_std, perturb=perturb,
-                                     nanmean_chunk=nanmean_chunk, lindisp=bool(lindisp), _rand=_rand, _stages=_stages)
+                                     nanmean_chunk=nanmean_chunk, lindisp=bool(lindisp), _rand=_rand, _stages=_stages,
+                                     **({"want_parts": True} if want_parts else {}))
 
     def _prepare(self, ray_batch, skts, cyls, bones, cams, N_uniques):
         """Host-side reduction of the reference's per-ray stride-0 expands to per-pose tables (encoders.py:465-471)."""
@@ -287,7 +301,8 @@ class RayCaster(nn.Module):
         return rays, pose_skts, pose_bones, pose_cyls, cam_idx, skip
 
     def _render_prepared(self, rays, pose_skts, pose_bones, pose_cyls, cam_idx, skip=1, N_samples=64, N_importance=16,
-                         B=1.0, raw_noise_std=0., perturb=0., nanmean_chunk=None, lindisp=False, _rand=None, _stages=None):
+                         B=1.0, raw_noise_std=0., perturb=0., nanmean_chunk=None, lindisp=False, _rand=None, _stages=None,
+                         want_parts=False):
         dev = self._device()
         N = rays.shape[0]
         net = self.network
@@ -330,13 +345,13 @@ class RayCaster(nn.Module):
                     side.wait_stream(cur)                                   # inputs, packed weights, bone volumes
                     used.append(side)
                 with torch.cuda.stream(side):
-                    out = self._render_block(*args, lindisp=lindisp)
+                    out = self._render_block(*args, lindisp=lindisp, want_parts=want_parts)
                 if not torch.cuda.is_current_stream_capturing():           # a captured graph's memory is static anyway
                     for t in out.values():
                         t.record_stream(cur)                                # consumed (cat) on the caller's stream
                 outs.append(out)
             else:
-                outs.append(self._render_block(*args, lindisp=lindisp))
+                outs.append(self._render_block(*args, lindisp=lindisp, want_parts=want_parts))
         for side in used:
             cur.wait_stream(side)
         if len(outs) == 1:
@@ -360,10 +375,11 @@ class RayCaster(nn.Module):
 
     def _render_block(self, rays, ray0, skip, pose_skts, pose_cyls, vol, cam_idx, codes, consts, packed, S_c, S_f, B,
                       raw_noise_std, perturb, training, nanmean_chunk, rand, stages, keep=None, lindisp=False,
-                      nearfar=None):
+                      nearfar=None, want_parts=False):
         """One launch sequence over <= MAX_RAYS_PER_LAUNCH rays.  `keep` (dict) receives every intermediate the
         backward pass needs (train mode with gradients, and the normal map).  `nearfar`: the block's (near, far), when
-        the caller computed them over a larger range of rays (the normal map's blocks)."""
+        the caller computed them over a larger range of rays (the normal map's blocks).  `want_parts` (eval): the fine
+        composite also writes `part_map` (danbo_merge_composite_parts)."""
         n = rays.shape[0]
         # poses of this block: ray (ray0 + i) -> pose (ray0 + i) // skip
         if pose_skts.shape[0] == 1:
@@ -421,15 +437,21 @@ class RayCaster(nn.Module):
         else:
             K.mlp_forward(f1.xtiles, packed, rbias, act1, f1.row_ray, raw1)
         noise1 = (rand["noise1"] * (raw_noise_std * B)).contiguous() if ("noise1" in rand and raw_noise_std > 0) else None
-        c1 = K.merge_composite(rays, S_c, S_f, raw0, mask0, raw1, mask1, c0["z_all"], c0["order"], noise=noise1,
-                               inv_B=inv_B, want_raw=stages is not None, confd0=f0.logits if training else None,
-                               confd1=f1.logits if training else None, want_invalid=training)
+        if want_parts:
+            c1 = K.merge_composite_parts(rays, S_c, S_f, raw0, mask0, raw1, mask1, c0["z_all"], c0["order"], f0.logits,
+                                         f1.logits, agg_mode, noise=noise1, inv_B=inv_B, want_raw=stages is not None)
+        else:
+            c1 = K.merge_composite(rays, S_c, S_f, raw0, mask0, raw1, mask1, c0["z_all"], c0["order"], noise=noise1,
+                                   inv_B=inv_B, want_raw=stages is not None, confd0=f0.logits if training else None,
+                                   confd1=f1.logits if training else None, want_invalid=training)
         ret = {"rgb_map": c1["rgb_map"], "disp_map": c1["disp_map"], "acc_map": c1["acc_map"], "alpha": c1["alpha"],
                "T_i": c1["weights"], "rgb0": c0["rgb_map"], "disp0": c0["disp_map"], "acc0": c0["acc_map"],
                "alpha0": c0["alpha"]}
         if training:
             ret["confd"] = c1["confd"]
             ret["part_invalid"] = c1["part_invalid"]
+        if want_parts:
+            ret["part_map"] = c1["part_map"]
         if save:
             keep.update(dict(rays=rays, rays_v=rays_v, cam_idx=cam_idx, codes=codes, p_skts=p_skts, p_vol=p_vol, p0=p0, skip=skip,
                              consts=consts, S_c=S_c, S_f=S_f, inv_B=inv_B, z0=z0, mask0=mask0, act0=act0, f0=f0, raw0=raw0,
@@ -565,6 +587,11 @@ class RayCaster(nn.Module):
     def render_pts_density(self, pts, kps, skts, bones, netchunk=1024 * 64, network=None):
         """Raw sigma at points (P,1,3) or (P,3) for ONE pose (raycasters.py:439-453, nerf.py:136-154)."""
         assert kps.shape[0] == 1, f"Assuming only one poses are provided, got {kps.shape[0]} instead"
+        out, _, _ = self._pts_field(pts, skts, bones)
+        return out.reshape(pts.shape[0], 1, 1) if pts.dim() == 3 else out.reshape(pts.shape[0], 1)
+
+    def _pts_field(self, pts, skts, bones):
+        """render_pts_density's launches -> (raw sigma (P,), visibility masks (P,) int32, FieldOut of the points)."""
         dev = self._device()
         P = pts.shape[0]
         p = pts.reshape(P, 3).to(dev).float()
@@ -583,8 +610,31 @@ class RayCaster(nn.Module):
                              pairs_per_row=K.J)
         sigma = torch.empty(2 * P, device=dev)
         K.mlp_forward(fo.xtiles, packed, None, act, fo.row_ray, sigma, density_only=True)
-        out = torch.where(mask.reshape(-1) != 0, sigma[:P], sigma[2 * P - 1])
-        return out.reshape(P, 1, 1) if pts.dim() == 3 else out.reshape(P, 1)
+        return torch.where(mask.reshape(-1) != 0, sigma[:P], sigma[2 * P - 1]), mask.reshape(-1), fo
+
+    # ------------------------------------------------------------------------------------------------ part maps
+    def _refuse_parts(self, what):
+        if not self._supports_parts:
+            raise NotImplementedError(f"{what}: body-part weights are implemented for the DANBO field only (the A-NeRF "
+                                      "field has no per-bone aggregation)")
+
+    @torch.no_grad()
+    def render_pts_parts(self, pts, kps, skts, bones):
+        """Raw sigma and the aggregation weights p_j of every bone at points (P,1,3) or (P,3) for ONE pose
+        -> (sigma (P,1) or (P,1,1), p (P,24)).  sigma is render_pts_density's; p = network.get_agg(logits, invalid) with
+        the field's logits and visibility masks of the same launches, 0 for a point no bone sees."""
+        self._refuse_parts("render_pts_parts")
+        if kps.shape[0] != 1 or skts.shape[0] != 1 or bones.shape[0] != 1:
+            raise NotImplementedError("render_pts_parts takes one pose (kps, skts, bones with a leading 1)")
+        P = pts.shape[0]
+        sigma, mask, fo = self._pts_field(pts, skts, bones)
+        vis = ((mask.long()[:, None] >> torch.arange(K.J, device=mask.device)) & 1).bool()
+        # entries danbo_field_agg did not write are uninitialised (and x 0 may still be NaN): a sigmoid pass writes the
+        # visible bones only, a softmax pass all 24 of a row some bone sees (its max runs over all of them)
+        written = vis if self.network.agg_type == "sigmoid" else vis.any(-1, keepdim=True)
+        logits = torch.where(written, fo.logits[:P], torch.zeros((), device=mask.device))
+        p = self.network.get_agg(logits, (~vis).float())
+        return (sigma.reshape(P, 1, 1) if pts.dim() == 3 else sigma.reshape(P, 1)), p
 
     @torch.no_grad()
     def render_mesh_density(self, kps, skts, bones, subject_idxs=None, radius=1.0, res=64, render_kwargs=None,

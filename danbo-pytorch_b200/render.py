@@ -81,12 +81,27 @@ def projection_matrix(c2w, H, W, focal):
 
 @torch.no_grad()
 def render_images(caster, args, c2ws, poses, H, W, focal=None, cam_idx=0, white_bkgd=True, near=syn.NEAR, far=syn.FAR,
-                  graphed=False, distributed=False, normals=False):
+                  graphed=False, distributed=False, normals=False, parts=False):
     """Render one image per (camera, pose) pair.  poses: list of dicts from synthetic.make_pose (kps, skts, bones, cyl);
     image k uses c2ws[k] and poses[k % len(poses)], like render_path.  With distributed=True images are dealt round
     robin to the ranks and the finished images all-gathered: every rank returns all images (n, H, W, 3) float32.
     normals=True (single process, not graphed): -> (images, normal_images), the second (n, H, W, 3) float32 world-frame
-    normal maps (`render_rays(want_normals=True)`), 0 on the background."""
+    normal maps (`render_rays(want_normals=True)`), 0 on the background.
+    parts=True (single process, not graphed, not with normals): -> (images, part_maps), the second (n, H, W, 24) float32
+    body-part maps (`render_rays(want_parts=True)`: the composited aggregation weight of every bone), 0 on the
+    background; `part_labels` turns them into a segmentation."""
+    if parts:
+        if graphed:
+            raise NotImplementedError("render_images(parts=True) with graphed=True: part maps are not captured")
+        if distributed:
+            raise NotImplementedError("render_images(parts=True) with distributed=True is not implemented")
+        if normals:
+            raise NotImplementedError("render_images(parts=True) together with normals=True is not implemented: make "
+                                      "two calls")
+        if hasattr(caster, "_refuse_parts"):
+            caster._refuse_parts("render_images(parts=True)")
+        if caster.training:
+            raise NotImplementedError("render_images(parts=True) is for eval mode (caster.eval())")
     if normals:
         if graphed:
             raise NotImplementedError("render_images(normals=True) with graphed=True: normals are not captured")
@@ -102,6 +117,7 @@ def render_images(caster, args, c2ws, poses, H, W, focal=None, cam_idx=0, white_
     mine = list(range(rank, len(c2ws), world))
     out = torch.ones(len(mine), H * W, 3, device=dev) if white_bkgd else torch.zeros(len(mine), H * W, 3, device=dev)
     nmaps = torch.zeros(len(mine), H * W, 3, device=dev) if normals else None
+    pmaps = torch.zeros(len(mine), H * W, 24, device=dev) if parts else None
     call = caster.render_graphed if graphed else caster
     # every pose table and camera of this rank's images goes to the device ONCE (5 copies), not per image: a pageable
     # host-to-device copy is synchronous, and one per tensor per image kept the GPU idle for half of each image
@@ -122,14 +138,18 @@ def render_images(caster, args, c2ws, poses, H, W, focal=None, cam_idx=0, white_
                    bones=tab["bones"][ps:ps + 1].expand(n, -1, -1),
                    cams=torch.full((n, 1), cam_idx, dtype=torch.long, device=dev), N_uniques=1, perturb=False,
                    N_importance=args.N_importance, raw_noise_std=0., nanmean_chunk=args.chunk,
-                   **({"want_normals": True} if normals else {}))
+                   **({"want_normals": True} if normals else {}), **({"want_parts": True} if parts else {}))
         bg = 1.0 if white_bkgd else 0.0
         out[slot, idx] = ret["rgb_map"] + (1. - ret["acc_map"])[:, None] * bg         # run_nerf.py:103-133
         if normals:
             nmaps[slot, idx] = ret["normal_map"]
+        if parts:
+            pmaps[slot, idx] = ret["part_map"]
     out = out.reshape(len(mine), H, W, 3)
     if normals:
         return out, nmaps.reshape(len(mine), H, W, 3)
+    if parts:
+        return out, pmaps.reshape(len(mine), H, W, 24)
     if world == 1:
         return out
     counts = [len(range(r, len(c2ws), world)) for r in range(world)]
@@ -139,6 +159,13 @@ def render_images(caster, args, c2ws, poses, H, W, focal=None, cam_idx=0, white_
     inv = torch.empty(len(order), dtype=torch.long, device=dev)
     inv[torch.as_tensor(order, device=dev)] = torch.arange(len(order), device=dev)
     return gathered[inv]
+
+
+def part_labels(part_maps, min_weight=0.5):
+    """Body-part segmentation of part maps (..., 24) -> int64 (...): the bone of the largest weight, -1 where that
+    weight is below `min_weight` (background, and pixels no part explains clearly)."""
+    w, j = part_maps.max(-1)
+    return torch.where(w >= min_weight, j, torch.full_like(j, -1))
 
 
 @torch.no_grad()

@@ -152,6 +152,17 @@ int danbo_merge_composite(const float* rays, int ray_stride, int n_rays, int S_c
                           float* disp, float* acc, float* raw_merged, const float* confd0, const float* confd1,
                           float* confd_merged, float* invalid_merged, void* stream);
 
+/* Eval-mode R2 + C1 with the body-part map: the composite of danbo_merge_composite (rgb, disp, acc, weights, alpha and
+ * raw_merged bit-identical to it) plus part_map (n,24) = sum_m w_m p_m over the merged samples, with p_m the
+ * aggregation weights get_agg(confd_m, 1 - visible_m) of the sample (agg_mode 0 sigmoid, 1 masked softmax, as in
+ * danbo_field_agg) and 0 for a sample no bone sees.  confd0 / confd1: danbo_field_agg's logits of the two passes;
+ * weights, confd0, confd1 and part_map are required. */
+int danbo_merge_composite_parts(const float* rays, int ray_stride, int n_rays, int S_c, int S_f, const float* raw0,
+                                const unsigned int* mask0, const float* raw1, const unsigned int* mask1,
+                                const float* z_all, const int* order, const float* noise, float inv_B, float* weights,
+                                float* alpha, float* rgb, float* disp, float* acc, float* raw_merged,
+                                const float* confd0, const float* confd1, int agg_mode, float* part_map, void* stream);
+
 /* ---- backward (train mode; autograd of the same rows as reached from core/trainer.py:563-576) -------------------- */
 
 /* Train-mode M1 forward: danbo_mlp_forward plus the bf16 activations the backward needs: act_save [9][save_cap][256]
