@@ -65,6 +65,7 @@ _SIGNATURES = {
     "danbo_merge_composite": [c_p, c_i, c_i, c_i, c_i, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_f, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p],
     "danbo_merge_composite_parts": [c_p, c_i, c_i, c_i, c_i, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_f, c_p, c_p, c_p, c_p, c_p,
                                     c_p, c_p, c_p, c_i, c_p, c_p],
+    "danbo_scene_composite": [c_p, c_i, c_i, c_i, c_i, c_i, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p],
 }
 
 EXPORTS = tuple(_SIGNATURES)

@@ -72,6 +72,7 @@ class AnerfCaster(RayCaster):
     _supports_fine_network = True
     _supports_normals = False             # its density also depends on the point through the cut-off encodings
     _supports_parts = False               # no per-bone aggregation: every bone's encoding goes into one MLP
+    _supports_scene = False               # render_scene_rays composites the DANBO render block's merge inputs
 
     def __init__(self, network, network_fine=None, single_net=True, rest_poses=None, align_bones="align", skel_type=None,
                  **kwargs):

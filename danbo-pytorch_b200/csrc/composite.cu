@@ -77,12 +77,13 @@ __device__ __forceinline__ T group_sum(T v) {
     return v;
 }
 
-// Composites one ray of S samples (z[0..S), fetch(i) -> raw (rgb, sigma)) on the kL lanes of its group; kEo = ceil(S / 32).
-// Writes the weights / alpha rows and the maps when `store`; leaves the weights in w_sm when it is given.
-template <int kL, int kEo, class Fetch>
+// Composites one ray of S samples (z[0..S), fetch(i) -> raw (rgb, sigma)) on the kL lanes of its group; kEo >= ceil(S / 32).
+// dist(i): the z distance sample i's alpha is taken over (before the |d| scale).  Writes the weights / alpha rows and the
+// maps when `store`; leaves the weights in w_sm when it is given.
+template <int kL, int kEo, class Fetch, class Dist>
 __device__ __forceinline__ void composite_group(const float* z, int S, int g, unsigned gmask, bool store, float norm_d,
-                                                float inv_B, const float* __restrict__ noise_row, Fetch fetch, float* w_sm,
-                                                float* __restrict__ w_row, float* __restrict__ alpha_row,
+                                                float inv_B, const float* __restrict__ noise_row, Fetch fetch, Dist dist,
+                                                float* w_sm, float* __restrict__ w_row, float* __restrict__ alpha_row,
                                                 float* __restrict__ rgb_out, float* __restrict__ disp_out,
                                                 float* __restrict__ acc_out) {
     constexpr int R = 32 / kL;                          // virtual lanes per lane
@@ -97,7 +98,7 @@ __device__ __forceinline__ void composite_group(const float* z, int S, int g, un
             al[j][e] = 0.f; cr[j][e] = cg[j][e] = cb[j][e] = 0.f;
             if (i < S) {
                 const float4 raw = fetch(i);
-                float d = (i + 1 < S) ? __fsub_rn(z[i + 1], z[i]) : 1e10f;
+                float d = dist(i);
                 d = __fmul_rn(d, norm_d);
                 cr[j][e] = (1.f / (1.f + expf(-raw.x))) * 1.002f - 0.001f;
                 cg[j][e] = (1.f / (1.f + expf(-raw.y))) * 1.002f - 0.001f;
@@ -158,6 +159,18 @@ __device__ __forceinline__ void composite_group(const float* z, int S, int g, un
         *acc_out = fminf(sw, 1.f);
     }
     __syncwarp(gmask);
+}
+
+// One sorted list of its own (raw2outputs): a sample's distance runs to the next sample of the list, 1e10 after the last.
+template <int kL, int kEo, class Fetch>
+__device__ __forceinline__ void composite_group(const float* z, int S, int g, unsigned gmask, bool store, float norm_d,
+                                                float inv_B, const float* __restrict__ noise_row, Fetch fetch, float* w_sm,
+                                                float* __restrict__ w_row, float* __restrict__ alpha_row,
+                                                float* __restrict__ rgb_out, float* __restrict__ disp_out,
+                                                float* __restrict__ acc_out) {
+    composite_group<kL, kEo>(z, S, g, gmask, store, norm_d, inv_B, noise_row, fetch,
+                             [&](int i) { return (i + 1 < S) ? __fsub_rn(z[i + 1], z[i]) : 1e10f; }, w_sm, w_row,
+                             alpha_row, rgb_out, disp_out, acc_out);
 }
 
 // Coarse pass: composite + inverse-CDF importance sampling + merge order.  Dynamic shared memory: per ray, z[S], w[S],
@@ -449,6 +462,100 @@ merge_composite_parts_kernel(const float* __restrict__ rays, int ray_stride, int
     }
 }
 
+constexpr int kSceneMaxInst = 8;
+constexpr int kSceneMaxU = 8 * 144;                     // union bound: 8 instances of danbo_base (96 + 48 samples)
+
+// What danbo_merge_composite reads, per instance; passed by value, so that there is no device pointer table to upload.
+struct SceneInputs {
+    const float* raw0[kSceneMaxInst];
+    const uint32_t* mask0[kSceneMaxInst];
+    const float* raw1[kSceneMaxInst];
+    const uint32_t* mask1[kSceneMaxInst];
+    const float* z_all[kSceneMaxInst];
+    const int* order[kSceneMaxInst];
+};
+
+// Fine pass of a scene: the union U of n_inst instances' merged lists (each S_t = S_c + S_f samples sorted by z, as
+// merge_composite_kernel reads them) composited along each ray.  A sample keeps the alpha its own instance gives it:
+// its distance runs to the next sample of its own list (1e10 after the last), and a sample no bone sees reads its
+// instance's empty row.  The union is ordered by z, ties to the lower instance, then to the list position: the union
+// rank of sample i of list k is i + #{z_o <= z} over the lists o < k + #{z_o < z} over the lists o > k, one binary search
+// each.  composite_group then runs over U, and instance_map[n, k] sums the weights of instance k's samples.
+// Dynamic shared memory per ray (U entries each): the lists' z (the weights once the ranks are taken), the union's z, its
+// alpha, and the (instance, position) of each union entry as k * S_t + i.  Nothing of size U leaves the chip.
+template <int kL, int kEo>
+__global__ void __launch_bounds__(32 * kWarpsPerBlock)
+scene_composite_kernel(const float* __restrict__ rays, int ray_stride, int n_rays, int S_c, int S_f, int n_inst,
+                       const SceneInputs in, float* __restrict__ rgb, float* __restrict__ disp, float* __restrict__ acc,
+                       float* __restrict__ inst_map /* (n, n_inst) */) {
+    extern __shared__ float dsm[];
+    const int lane = threadIdx.x & 31, g = lane & (kL - 1), slot = threadIdx.x / kL, slots = blockDim.x / kL;
+    const unsigned gmask = group_mask<kL>(lane);
+    const int n_slot = blockIdx.x * slots + slot;
+    const bool valid = n_slot < n_rays;
+    const int n = valid ? n_slot : n_rays - 1;
+    const int St = S_c + S_f, U = n_inst * St;
+    float* zl = dsm + (size_t)slot * U;
+    float* zu = dsm + (size_t)(slots + slot) * U;
+    float* au = dsm + (size_t)(2 * slots + slot) * U;
+    unsigned short* su = reinterpret_cast<unsigned short*>(dsm + (size_t)3 * slots * U) + (size_t)slot * U;
+    const float* r = rays + (size_t)n * ray_stride;
+    const float norm_d = __fsqrt_rn(__fadd_rn(__fadd_rn(__fmul_rn(r[3], r[3]), __fmul_rn(r[4], r[4])), __fmul_rn(r[5], r[5])));
+    for (int e = g; e < U; e += kL) {
+        const int k = e / St;
+        zl[e] = in.z_all[k][(size_t)n * St + e - k * St];
+    }
+    __syncwarp(gmask);
+    for (int e = g; e < U; e += kL) {
+        const int k = e / St, i = e - k * St;
+        const float v = zl[e];
+        int rank = i;
+        for (int o = 0; o < n_inst; ++o) {
+            if (o == k) continue;
+            const float* l = zl + o * St;
+            int lo = 0, hi = St;
+            if (o < k) { while (lo < hi) { const int mid = (lo + hi) >> 1; if (l[mid] <= v) lo = mid + 1; else hi = mid; } }
+            else { while (lo < hi) { const int mid = (lo + hi) >> 1; if (l[mid] < v) lo = mid + 1; else hi = mid; } }
+            rank += lo;
+        }
+        zu[rank] = v;
+        su[rank] = (unsigned short)e;
+    }
+    __syncwarp(gmask);                                  // from here zl is dead: composite_group leaves the weights there
+    auto fetch = [&](int u) {
+        const int e = su[u], k = e / St, i = e - k * St;
+        const int src = in.order[k][(size_t)n * St + i];
+        const bool coarse = src < S_c;
+        const size_t sidx = coarse ? (size_t)n * S_c + src : (size_t)n * S_f + src - S_c;
+        const uint32_t m = (coarse ? in.mask0[k] : in.mask1[k])[sidx];
+        const float4* r0 = reinterpret_cast<const float4*>(in.raw0[k]);
+        return m ? (coarse ? r0 : reinterpret_cast<const float4*>(in.raw1[k]))[sidx] : r0[(size_t)n_rays * S_c + n];
+    };
+    auto dist = [&](int u) {
+        const int e = su[u], k = e / St, i = e - k * St;
+        const float* z = in.z_all[k] + (size_t)n * St;
+        return (i + 1 < St) ? __fsub_rn(z[i + 1], z[i]) : 1e10f;
+    };
+    composite_group<kL, kEo>(zu, U, g, gmask, valid, norm_d, 1.f, nullptr, fetch, dist, zl, nullptr, au,
+                             rgb + (size_t)n * 3, disp + n, acc + n);
+    float pk[kSceneMaxInst];
+#pragma unroll
+    for (int k = 0; k < kSceneMaxInst; ++k) pk[k] = 0.f;
+    for (int u = g; u < U; u += kL) {
+        const int k = su[u] / St;
+        const float w = zl[u];
+#pragma unroll
+        for (int o = 0; o < kSceneMaxInst; ++o) pk[o] += o == k ? w : 0.f;
+    }
+#pragma unroll
+    for (int k = 0; k < kSceneMaxInst; ++k) pk[k] = group_sum<kL>(pk[k]);
+    if (valid && g == 0) {
+#pragma unroll
+        for (int k = 0; k < kSceneMaxInst; ++k)
+            if (k < n_inst) inst_map[(size_t)n * n_inst + k] = pk[k];
+    }
+}
+
 }  // namespace danbo
 
 using namespace danbo;
@@ -530,6 +637,55 @@ extern "C" int danbo_merge_composite_parts(const float* rays, int ray_stride, in
         default: DANBO_MCP_LAUNCH(5); break;
     }
 #undef DANBO_MCP_LAUNCH
+    DANBO_CHECK_LAUNCH();
+    return 0;
+}
+
+extern "C" int danbo_scene_composite(const float* rays, int ray_stride, int n_rays, int S_c, int S_f, int n_inst,
+                                     const float* const* raw0, const unsigned int* const* mask0, const float* const* raw1,
+                                     const unsigned int* const* mask1, const float* const* z_all, const int* const* order,
+                                     float* rgb, float* disp, float* acc, float* inst_map, void* stream) {
+    if (n_rays <= 0) return 0;
+    if (n_inst < 1 || n_inst > kSceneMaxInst || S_c < 1 || S_f < 0 || S_c + S_f > kMaxS ||
+        n_inst * (S_c + S_f) > kSceneMaxU)
+        return -1;
+    if (!rays || !raw0 || !mask0 || !raw1 || !mask1 || !z_all || !order || !rgb || !disp || !acc || !inst_map) return -1;
+    SceneInputs in = {};
+    for (int k = 0; k < n_inst; ++k) {
+        if (!raw0[k] || !mask0[k] || (S_f > 0 && (!raw1[k] || !mask1[k])) || !z_all[k] || !order[k]) return -1;
+        in.raw0[k] = raw0[k]; in.mask0[k] = mask0[k]; in.raw1[k] = raw1[k]; in.mask1[k] = mask1[k];
+        in.z_all[k] = z_all[k]; in.order[k] = order[k];
+    }
+    const int U = n_inst * (S_c + S_f);
+    // per ray: three float rows (lists' z / weights, union z, alpha) and a 16-bit row of sources, U entries each
+    const size_t smem_per_ray = (size_t)U * (3 * sizeof(float) + sizeof(unsigned short));
+#define DANBO_SC_LAUNCH(L, E)                                                                                          \
+    do {                                                                                                               \
+        const int slots = 32 * kWarpsPerBlock / (L);                                                                   \
+        const size_t smem = slots * smem_per_ray;                                                                      \
+        if (smem > 48 * 1024) {                                                                                        \
+            const cudaError_t e = cudaFuncSetAttribute(scene_composite_kernel<L, E>,                                   \
+                                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);        \
+            if (e != cudaSuccess) return (int)e;                                                                       \
+        }                                                                                                              \
+        scene_composite_kernel<L, E><<<(n_rays + slots - 1) / slots, 32 * kWarpsPerBlock, smem, (cudaStream_t)stream>>>( \
+            rays, ray_stride, n_rays, S_c, S_f, n_inst, in, rgb, disp, acc, inst_map);                                 \
+    } while (0)
+    // up to 160 samples the plain merge's specialisation (a scene of one instance is then its composite bit for bit);
+    // beyond, one warp per ray and kEo in steps
+    const int E = (U + 31) / 32;
+    if (E == 1) DANBO_SC_LAUNCH(kMcLanes[0], 1);
+    else if (E == 2) DANBO_SC_LAUNCH(kMcLanes[1], 2);
+    else if (E == 3) DANBO_SC_LAUNCH(kMcLanes[2], 3);
+    else if (E == 4) DANBO_SC_LAUNCH(kMcLanes[3], 4);
+    else if (E == 5) DANBO_SC_LAUNCH(kMcLanes[4], 5);
+    else if (E <= 6) DANBO_SC_LAUNCH(32, 6);
+    else if (E <= 9) DANBO_SC_LAUNCH(32, 9);
+    else if (E <= 12) DANBO_SC_LAUNCH(32, 12);
+    else if (E <= 18) DANBO_SC_LAUNCH(32, 18);
+    else if (E <= 27) DANBO_SC_LAUNCH(32, 27);
+    else DANBO_SC_LAUNCH(32, 36);
+#undef DANBO_SC_LAUNCH
     DANBO_CHECK_LAUNCH();
     return 0;
 }

@@ -421,6 +421,42 @@ def merge_composite_parts(rays, S_c, S_f, raw0, mask0, raw1, mask1, z_all, order
     return out
 
 
+SCENE_MAX_INSTANCES = 8
+SCENE_MAX_UNION = 8 * 144                # samples of a ray's union: 8 instances of danbo_base (96 + 48)
+
+
+def scene_composite(rays, S_c, S_f, inputs):
+    """Eval-mode composite of a scene: `inputs` holds one dict per instance with what merge_composite reads for it
+    (raw0 (n*S_c+n,4), mask0 (n,S_c), raw1 (n*S_f,4), mask1 (n,S_f), z_all (n,S_t), order (n,S_t) int32).  The union of
+    the instances' merged lists is composited along each ray, every sample with the alpha of its own list
+    -> dict (rgb_map, disp_map, acc_map, instance_map (n,K)).  One instance gives merge_composite's maps bit for bit."""
+    n, K_, St = rays.shape[0], len(inputs), S_c + S_f
+    if not 1 <= K_ <= SCENE_MAX_INSTANCES or K_ * St > SCENE_MAX_UNION:
+        raise ValueError(f"{K_} instances of {St} samples: 1 to {SCENE_MAX_INSTANCES} instances and at most "
+                         f"{SCENE_MAX_UNION} samples per ray in all")
+    shapes = {"raw0": (n * S_c + n, 4), "mask0": (n, S_c), "raw1": (n * S_f, 4), "mask1": (n, S_f), "z_all": (n, St),
+              "order": (n, St)}
+    for k, inp in enumerate(inputs):
+        for name, shape in shapes.items():
+            t = inp[name]
+            _need_cuda(t)
+            if tuple(t.shape) != shape or not t.is_contiguous() or t.element_size() != 4 or t.device != rays.device:
+                raise ValueError(f"instance {k}: {name} must be a contiguous 4-byte tensor of shape {shape} on "
+                                 f"{rays.device}, got {tuple(t.shape)} {t.dtype} on {t.device}")
+    _need_cuda(rays)
+    lib = _lib.load()
+    f = lambda *s: torch.empty(*s, device=rays.device, dtype=torch.float32)
+    out = {"rgb_map": f(n, 3), "disp_map": f(n), "acc_map": f(n), "instance_map": f(n, K_)}
+    ptrs = {name: (ctypes.c_void_p * K_)(*[inp[name].data_ptr() for inp in inputs]) for name in shapes}
+    with _Timed("scene_composite"):
+        _lib.check(lib.danbo_scene_composite(_p(rays), rays.stride(0), n, S_c, S_f, K_, ptrs["raw0"], ptrs["mask0"],
+                                             ptrs["raw1"], ptrs["mask1"], ptrs["z_all"], ptrs["order"],
+                                             _p(out["rgb_map"]), _p(out["disp_map"]), _p(out["acc_map"]),
+                                             _p(out["instance_map"]), _stream()), "danbo_scene_composite")
+    _count(1)
+    return out
+
+
 # ------------------------------------------------------------------------------------------------------ backward
 class ActSave:
     """bf16 activations of the fused MLP kept for the backward pass."""

@@ -36,6 +36,7 @@ class RayCaster(nn.Module):
     _supports_fine_network = False        # a separate fine network (single_net=False): the A-NeRF caster only
     _supports_normals = True              # density gradients / normals (render_pts_gradient, want_normals): DANBO only
     _supports_parts = True                # body-part maps (render_pts_parts, want_parts): a field with an aggregation net
+    _supports_scene = True                # scenes of several bodies (render_scene_rays): DANBO only
 
     def __init__(self, network, network_fine=None, single_net=True, rest_poses=None, align_bones="align",
                  skel_type=None, use_volume_near_far=False, view_mode="world", **kwargs):
@@ -375,11 +376,12 @@ class RayCaster(nn.Module):
 
     def _render_block(self, rays, ray0, skip, pose_skts, pose_cyls, vol, cam_idx, codes, consts, packed, S_c, S_f, B,
                       raw_noise_std, perturb, training, nanmean_chunk, rand, stages, keep=None, lindisp=False,
-                      nearfar=None, want_parts=False):
+                      nearfar=None, want_parts=False, merge_inputs=False):
         """One launch sequence over <= MAX_RAYS_PER_LAUNCH rays.  `keep` (dict) receives every intermediate the
         backward pass needs (train mode with gradients, and the normal map).  `nearfar`: the block's (near, far), when
         the caller computed them over a larger range of rays (the normal map's blocks).  `want_parts` (eval): the fine
-        composite also writes `part_map` (danbo_merge_composite_parts)."""
+        composite also writes `part_map` (danbo_merge_composite_parts).  `merge_inputs` (eval): stop before the fine
+        composite and return what it would read (raw0, mask0, raw1, mask1, z_all, order), for render_scene_rays."""
         n = rays.shape[0]
         # poses of this block: ray (ray0 + i) -> pose (ray0 + i) // skip
         if pose_skts.shape[0] == 1:
@@ -436,6 +438,8 @@ class RayCaster(nn.Module):
             K.mlp_forward_save(f1.xtiles, packed, rbias, act1, f1.row_ray, raw1, sv1)
         else:
             K.mlp_forward(f1.xtiles, packed, rbias, act1, f1.row_ray, raw1)
+        if merge_inputs:
+            return {"raw0": raw0, "mask0": mask0, "raw1": raw1, "mask1": mask1, "z_all": c0["z_all"], "order": c0["order"]}
         noise1 = (rand["noise1"] * (raw_noise_std * B)).contiguous() if ("noise1" in rand and raw_noise_std > 0) else None
         if want_parts:
             c1 = K.merge_composite_parts(rays, S_c, S_f, raw0, mask0, raw1, mask1, c0["z_all"], c0["order"], f0.logits,
@@ -649,6 +653,74 @@ class RayCaster(nn.Module):
 
 
 GraphCaster = RayCaster
+
+
+# ------------------------------------------------------------------------------------------------------ scenes
+def check_scene(instances, N_samples, N_importance):
+    """The refusals of render_scene_rays and render.render_scene_images, raised before any device work."""
+    n_inst, S_t = len(instances), int(N_samples) + int(N_importance)
+    if not 1 <= n_inst <= K.SCENE_MAX_INSTANCES:
+        raise NotImplementedError(f"a scene of {n_inst} instances: 1 to {K.SCENE_MAX_INSTANCES} are implemented")
+    if int(N_importance) <= 0:
+        raise NotImplementedError("N_importance must be > 0 (the reference itself requires it, SURVEY F10)")
+    if S_t > 160 or n_inst * S_t > K.SCENE_MAX_UNION:
+        raise NotImplementedError(f"{n_inst} instances of {S_t} samples: a ray's union holds at most "
+                                  f"{K.SCENE_MAX_UNION} samples (8 instances of danbo_base), an instance at most 160")
+    dev = None
+    for k, inst in enumerate(instances):
+        caster = inst["caster"]
+        if not getattr(caster, "_supports_scene", False):
+            raise NotImplementedError(f"scene instance {k}: scenes are implemented for the DANBO field only (the A-NeRF "
+                                      "caster's render block has its own fine pass)")
+        if caster.training or torch.is_grad_enabled():
+            raise NotImplementedError("scenes are rendered in eval mode without gradients (caster.eval(), "
+                                      "torch.no_grad()): gradients through a scene are not implemented")
+        if any(inst[name].shape[0] != 1 for name in ("kps", "skts", "bones", "cyls")):
+            raise NotImplementedError(f"scene instance {k}: one pose per instance (kps, skts, bones, cyls with a leading "
+                                      "1): add one instance per pose")
+        if dev is None:
+            dev = caster._device()
+        elif caster._device() != dev:
+            raise ValueError(f"scene instance {k} is on {caster._device()}, instance 0 on {dev}")
+
+
+def render_scene_rays(rays, instances, N_samples, N_importance, nanmean_chunk=None, lindisp=False):
+    """Render a scene of several posed bodies along the same rays (n, 8+): one volume composite over the union of the
+    instances' samples, so that bodies occlude each other per sample, along the ray.
+
+    instances: 1 to 8 dicts with `caster` (a DANBO RayCaster in eval mode), `kps` (1,24,3), `skts` (1,24,4,4),
+    `bones` (1,24,3), `cyls` (1,5) and `cams` (frame-code index, < 0 for the mean code).  Instances may share a caster.
+    Each instance runs what render_rays runs for it alone in eval mode (density scale 1), its own coarse pass,
+    importance samples and near / far fill (F8, per `nanmean_chunk` rays) included, up to the fine composite; one
+    danbo_scene_composite per ray block then composites the union of their merged samples, each sample with the alpha
+    of its own list.  -> dict rgb_map (n,3), disp_map (n), acc_map (n) and instance_map (n,K): the summed weights of
+    each instance's samples.  A scene of one instance is render_rays' rgb, disp and acc bit for bit.  Call it under
+    torch.no_grad()."""
+    check_scene(instances, N_samples, N_importance)
+    S_c, S_f = int(N_samples), int(N_importance)
+    N = rays.shape[0]
+    per = []
+    for inst in instances:
+        c = inst["caster"]
+        dev = c._device()
+        cams = torch.full((N, 1), int(inst["cams"]), dtype=torch.long, device=dev)
+        rays_k, p_skts, p_bones, p_cyls, cam_idx, skip = c._prepare(rays, inst["skts"], inst["cyls"], inst["bones"], cams, 1)
+        per.append(dict(caster=c, rays=rays_k, p_skts=p_skts, p_cyls=p_cyls, cam_idx=cam_idx, skip=skip,
+                        consts=c._consts(), packed=c._packed_mlp(), codes=c._codes_with_mean(),
+                        vol=c.network.bone_volumes(p_bones).float().contiguous()))
+    rays = per[0]["rays"]
+    block, _ = RayCaster._plan_blocks(N, 1, per[0]["skip"], nanmean_chunk, 1)
+    outs = []
+    for s0 in range(0, N, block):
+        s1 = min(N, s0 + block)
+        inputs = [p["caster"]._render_block(p["rays"][s0:s1], s0, p["skip"], p["p_skts"], p["p_cyls"], p["vol"],
+                                            p["cam_idx"][s0:s1], p["codes"], p["consts"], p["packed"], S_c, S_f, 1.0,
+                                            0., 0., False, nanmean_chunk, {}, None, lindisp=bool(lindisp),
+                                            merge_inputs=True) for p in per]
+        outs.append(K.scene_composite(rays[s0:s1], S_c, S_f, inputs))
+    if len(outs) == 1:
+        return outs[0]
+    return {k: torch.cat([o[k] for o in outs], 0) for k in outs[0]}
 
 
 # ------------------------------------------------------------------------------------------------------ factory

@@ -52,10 +52,11 @@ def render(H, W, focal, chunk=1024 * 64, rays=None, near=0., far=1., use_viewdir
 def rays_in_box(H, W, focal, c2w, cyl, device, c2w_dev=None):
     """Pinhole rays of the pixels inside the image box of a bounding cylinder, generated on the device
     (ray_utils.py:7-29,84-138; skeleton_utils.py:633-720).  -> rays_o, rays_d (n,3), flat pixel index (n).
-    c2w / cyl: host arrays (the pixel box is a host-side computation over 100 projected points); c2w_dev: the same
-    camera already on the device (saves the per-image upload)."""
+    c2w / cyl: host arrays (the pixel box is a host-side computation over 100 projected points); cyl (5,) or (K,5),
+    whose boxes' union is taken; c2w_dev: the same camera already on the device (saves the per-image upload)."""
     c2w_np = np.asarray(c2w, dtype=np.float32)
-    tl, br = syn.cylinder_image_box(np.asarray(cyl, dtype=np.float32), H, W, float(focal), c2w_np)
+    boxes = [syn.cylinder_image_box(c, H, W, float(focal), c2w_np) for c in np.asarray(cyl, dtype=np.float32).reshape(-1, 5)]
+    tl, br = np.min([b[0] for b in boxes], 0), np.max([b[1] for b in boxes], 0)
     ys = torch.arange(int(tl[1]), int(br[1]), device=device, dtype=torch.float32)
     xs = torch.arange(int(tl[0]), int(br[0]), device=device, dtype=torch.float32)
     j, i = torch.meshgrid(ys, xs, indexing="ij")
@@ -161,9 +162,37 @@ def render_images(caster, args, c2ws, poses, H, W, focal=None, cam_idx=0, white_
     return gathered[inv]
 
 
+@torch.no_grad()
+def render_scene_images(instances, args, c2ws, H, W, focal=None, white_bkgd=True, near=syn.NEAR, far=syn.FAR):
+    """Render one image of a scene of several posed bodies per camera (`raycaster.render_scene_rays`; instances as
+    there, 1 to 8).  The rays are those of the union of the instances' cylinder boxes; every image is composited on
+    the background as render_images does.  -> (images (n,H,W,3), instance_maps (n,H,W,K)) float32, the second holding
+    each instance's summed weights per pixel, 0 on the background; `part_labels` turns it into an instance
+    segmentation.  A scene of one instance gives render_images' images bit for bit."""
+    from .raycaster import check_scene, render_scene_rays
+    check_scene(instances, args.N_samples, args.N_importance)
+    dev = instances[0]["caster"]._device()
+    focal = 1.2 * H if focal is None else focal
+    n_inst = len(instances)
+    cyls = np.stack([np.asarray(torch.as_tensor(inst["cyls"]).cpu(), dtype=np.float32).reshape(5) for inst in instances])
+    out = torch.ones(len(c2ws), H * W, 3, device=dev) if white_bkgd else torch.zeros(len(c2ws), H * W, 3, device=dev)
+    imaps = torch.zeros(len(c2ws), H * W, n_inst, device=dev)
+    c2w_dev = torch.as_tensor(np.stack([np.asarray(c, dtype=np.float32) for c in c2ws])).to(dev) if len(c2ws) else None
+    for k in range(len(c2ws)):
+        ro, rd, idx = rays_in_box(H, W, focal, c2ws[k], cyls, dev, c2w_dev=c2w_dev[k])
+        ones = torch.ones(ro.shape[0], 1, device=dev)
+        ray_batch = torch.cat([ro, rd, near * ones, far * ones, rd / torch.norm(rd, dim=-1, keepdim=True)], -1)
+        ret = render_scene_rays(ray_batch, instances, args.N_samples, args.N_importance, nanmean_chunk=args.chunk)
+        bg = 1.0 if white_bkgd else 0.0
+        out[k, idx] = ret["rgb_map"] + (1. - ret["acc_map"])[:, None] * bg         # run_nerf.py:103-133
+        imaps[k, idx] = ret["instance_map"]
+    return out.reshape(len(c2ws), H, W, 3), imaps.reshape(len(c2ws), H, W, n_inst)
+
+
 def part_labels(part_maps, min_weight=0.5):
     """Body-part segmentation of part maps (..., 24) -> int64 (...): the bone of the largest weight, -1 where that
-    weight is below `min_weight` (background, and pixels no part explains clearly)."""
+    weight is below `min_weight` (background, and pixels no part explains clearly).  Any last dimension works: on the
+    instance maps of render_scene_images (..., K) it gives an instance segmentation."""
     w, j = part_maps.max(-1)
     return torch.where(w >= min_weight, j, torch.full_like(j, -1))
 

@@ -163,6 +163,19 @@ int danbo_merge_composite_parts(const float* rays, int ray_stride, int n_rays, i
                                 float* alpha, float* rgb, float* disp, float* acc, float* raw_merged,
                                 const float* confd0, const float* confd1, int agg_mode, float* part_map, void* stream);
 
+/* Eval-mode composite of a scene of n_inst (1..8) instances along the same rays.  raw0 .. order are HOST arrays of
+ * n_inst device pointers, each entry what danbo_merge_composite takes for that instance (its merged list of
+ * S_t = S_c + S_f samples sorted by z, raw0 with its per-ray empty rows).  Each sample keeps the alpha of its own list
+ * (its distance runs to the next sample of its own list, density scale 1, no noise); the union of the n_inst lists,
+ * ordered by z (ties: lower instance, then list position), is composited with danbo_merge_composite's recurrence into
+ * rgb (n,3), disp (n), acc (n), and inst_map (n, n_inst), the sum of the weights of each instance's samples.  A scene
+ * of one instance gives danbo_merge_composite's rgb, disp and acc bit for bit.  Requires n_inst * S_t <= 8 * 144 and
+ * S_t <= 160; returns < 0 on a bad argument before any launch. */
+int danbo_scene_composite(const float* rays, int ray_stride, int n_rays, int S_c, int S_f, int n_inst,
+                          const float* const* raw0, const unsigned int* const* mask0, const float* const* raw1,
+                          const unsigned int* const* mask1, const float* const* z_all, const int* const* order,
+                          float* rgb, float* disp, float* acc, float* inst_map, void* stream);
+
 /* ---- backward (train mode; autograd of the same rows as reached from core/trainer.py:563-576) -------------------- */
 
 /* Train-mode M1 forward: danbo_mlp_forward plus the bf16 activations the backward needs: act_save [9][save_cap][256]
