@@ -54,6 +54,7 @@ _SIGNATURES = {
     "danbo_gemm_wgrad": [c_p, c_i, c_p, c_i, c_i, c_p, c_i, c_p, c_i, c_i, c_i, c_p],
     "danbo_colsum": [c_p, c_i, c_p, c_p, c_i, c_i, c_p],
     "danbo_ray_bias_bwd": [c_p, c_i, c_i, c_p, c_p, c_i, c_p, c_p, c_p, c_p, c_p, c_p],
+    "danbo_ray_bias_codes_bwd": [c_p, c_i, c_i, c_p, c_p, c_p, c_p],
     "danbo_view_root_bwd": [c_p, c_i, c_i, c_p, c_i, c_i, c_p, c_p, c_p, c_p],
     "danbo_field_agg_bwd": [c_p, c_i, c_i, c_i, c_p, c_p, c_p, c_p, c_i, c_p, c_p, c_i, c_i, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_i, c_p, c_i, c_i, c_p],
     "danbo_field_agg_bwd_pts": [c_p, c_i, c_i, c_i, c_p, c_p, c_p, c_p, c_i, c_p, c_p, c_i, c_i, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_i, c_p, c_p, c_p, c_i, c_i, c_p],

@@ -73,6 +73,7 @@ class AnerfCaster(RayCaster):
     _supports_normals = False             # its density also depends on the point through the cut-off encodings
     _supports_parts = False               # no per-bone aggregation: every bone's encoding goes into one MLP
     _supports_scene = False               # render_scene_rays composites the DANBO render block's merge inputs
+    _supports_frame_codes = False         # its code table feeds its own view branch (danbo_anerf_ray_encode)
 
     def __init__(self, network, network_fine=None, single_net=True, rest_poses=None, align_bones="align", skel_type=None,
                  **kwargs):

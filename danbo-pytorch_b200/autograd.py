@@ -14,7 +14,8 @@ When no network parameter needs a gradient and the poses do (training.PoseFitSte
 nodes take the pose-only path: the same data-gradient chain through compositing, MLP, field and graph net, with the
 kernel variants that form no weight gradient (no K = rows GEMMs, transposes, bias sums, aggregation-net or graph-net
 weight atomics, no ray-bias backward) and a transposed weight pack that is keyed on the weights instead of redone per
-call (RayCaster._packed_dgrad).
+call (RayCaster._packed_dgrad).  A fitted frame-code table (PoseFitStep's code fitting) is one more input of the render
+block; the pose-only backward then also forms its gradient (danbo_ray_bias_codes_bwd), never the network's.
 """
 import torch
 
@@ -51,7 +52,7 @@ def weight_grads(flags, core=None):
 class _RenderBlock(torch.autograd.Function):
 
     @staticmethod
-    def forward(ctx, caster, cfg, vol, pose_skts, *params):
+    def forward(ctx, caster, cfg, vol, pose_skts, frame_codes, *params):
         keep = {}
         with torch.no_grad():
             ret = caster._render_block(cfg["rays"], 0, cfg["skip"], pose_skts, cfg["pose_cyls"], vol, cfg["cam_idx"],
@@ -62,6 +63,7 @@ class _RenderBlock(torch.autograd.Function):
         ctx.caster = caster
         ctx.params = params
         ctx.vol_shape = vol.shape
+        ctx.codes_shape = None if frame_codes is None else frame_codes.shape
         outs = tuple(ret[k] for k in OUT_KEYS)
         ctx.mark_non_differentiable(*[ret[k] for k in OUT_KEYS if k not in DIFF_KEYS])
         return outs
@@ -78,7 +80,7 @@ class _RenderBlock(torch.autograd.Function):
         g_rgb0, g_acc0 = cg(g["rgb0"], n, 3), cg(g["acc0"], n)
         g_confd = None if g["confd"] is None else g["confd"].contiguous().float()
         P = dict(zip(PARAM_NAMES, ctx.params))
-        if not weight_grads(ctx.needs_input_grad[4:], N_TRAINED):
+        if not weight_grads(ctx.needs_input_grad[5:], N_TRAINED):
             return _RenderBlock._pose_only(ctx, P, g_rgb, g_acc, g_rgb0, g_acc0, g_confd)
         # Every backward kernel ACCUMULATES into its gradient buffers.  When the trainer keeps all gradients in one flat,
         # pre-zeroed bucket (parallel.GradBucket, opted in through caster.grads_in_place) the kernels add straight into
@@ -173,14 +175,15 @@ class _RenderBlock(torch.autograd.Function):
         ctx.keep = None
         del alive, wss
         if in_place:
-            return (None, None, d_vol, d_skts) + (None,) * len(PARAM_NAMES)
-        return (None, None, d_vol, d_skts) + tuple(G[name] for name in PARAM_NAMES)
+            return (None, None, d_vol, d_skts, None) + (None,) * len(PARAM_NAMES)
+        return (None, None, d_vol, d_skts, None) + tuple(G[name] for name in PARAM_NAMES)
 
     @staticmethod
     def _pose_only(ctx, P, g_rgb, g_acc, g_rgb0, g_acc0, g_confd):
-        """Backward to d vol and d skts only.  Compositing as in training; per pass the dX-only MLP chain (head backward
-        only where d ray_bias is read: root-local view directions) and the field backward without the aggregation-net
-        and axis-scale accumulators; no ray-bias backward; danbo_view_root_bwd on root-local view directions."""
+        """Backward to d vol, d skts and the fitted frame codes only.  Compositing as in training; per pass the dX-only
+        MLP chain (head backward only where d ray_bias is read: root-local view directions, fitted frame codes) and the
+        field backward without the aggregation-net and axis-scale accumulators; no ray-bias weight backward;
+        danbo_ray_bias_codes_bwd for fitted frame codes, danbo_view_root_bwd on root-local view directions."""
         if K.BACKWARD_IMPL != "tc":
             raise NotImplementedError("the pose-only backward runs on the tensor-core MLP kernels (BACKWARD_IMPL='tc')")
         k = ctx.keep
@@ -199,7 +202,8 @@ class _RenderBlock(torch.autograd.Function):
         grads = [None] * 7 + [d_vol[k["p0"]:], None]
         d_skts = zeros(*k["p_skts"].shape) if ctx.needs_input_grad[3] else None
         view_root = d_skts is not None and getattr(ctx.caster, "view_mode", "world") == "root_local"
-        d_ray_bias = zeros(n, 128) if view_root else None
+        want_codes = ctx.needs_input_grad[4]
+        d_ray_bias = zeros(n, 128) if (view_root or want_codes) else None
         packed_t = ctx.caster._packed_dgrad()
         cur = torch.cuda.current_stream(dev)
         side2 = None
@@ -222,17 +226,27 @@ class _RenderBlock(torch.autograd.Function):
             else:
                 K.field_agg_bwd(rays, S, z, mask, act, k["p_skts"], k["p_vol"], k["skip"], k["consts"], fo, dX, gl,
                                 grads, d_skts=d_skts)
+        d_codes = None
+        if want_codes:
+            # d_ray_bias is complete after the second pass's head backward (this stream): the code gradient overlaps
+            # the coarse pass's field backward on side2
+            d_codes = K.ray_bias_codes_bwd(k["cam_idx"], P["views_linears.0.weight"], d_ray_bias,
+                                           zeros(*ctx.codes_shape))
         if side2 is not None:
             cur.wait_stream(side2)
         if view_root:
             K.view_root_bwd(rays, k["p_skts"], k["skip"], P["views_linears.0.weight"], d_ray_bias, d_skts)
         ctx.keep = None
         del alive
-        return (None, None, d_vol if ctx.needs_input_grad[2] else None, d_skts) + (None,) * len(PARAM_NAMES)
+        return (None, None, d_vol if ctx.needs_input_grad[2] else None, d_skts, d_codes) + (None,) * len(PARAM_NAMES)
 
 
 def render_block_with_grad(caster, rays, skip, pose_skts, pose_cyls, vol, cam_idx, codes, consts, packed, S_c, S_f, B,
-                           raw_noise_std, perturb, nanmean_chunk, rand, stages, lindisp=False):
+                           raw_noise_std, perturb, nanmean_chunk, rand, stages, lindisp=False, frame_codes=None):
+    """`codes` is the code table the kernels read ((rows + 1,128), last row the mean code).  `frame_codes`: the fitted
+    table whose rows are codes[:-1] (training.PoseFitStep), an input of the node; when it requires a gradient the
+    pose-only backward forms d frame_codes (danbo_ray_bias_codes_bwd).  A backward that trains the network as well
+    is not implemented."""
     named = dict(caster.network.named_parameters())
     if not getattr(caster.network, "opt_framecode", True):
         # no frame codes (configs/surreal): the kernels keep the view layer's 411-input layout, so the node gets a
@@ -242,11 +256,14 @@ def render_block_with_grad(caster, rays, skip, pose_skts, pose_cyls, vol, cam_id
         named["views_linears.0.weight"] = torch.nn.functional.pad(named["views_linears.0.weight"], (0, 128))
         named["framecodes.codes.weight"] = torch.zeros(1, 128, device=rays.device)
     params = [named[n] for n in PARAM_NAMES]
-    weight_grads([p.requires_grad for p in params], N_TRAINED)          # a mixed set is refused before any launch
+    trains = weight_grads([p.requires_grad for p in params], N_TRAINED)  # a mixed set is refused before any launch
+    if trains and frame_codes is not None and frame_codes.requires_grad:
+        raise NotImplementedError("fitting frame codes while the network trains is not implemented: fit them with the "
+                                  "field frozen (training.PoseFitStep(code_kwargs=...))")
     cfg = dict(rays=rays, skip=skip, pose_cyls=pose_cyls, cam_idx=cam_idx, codes=codes, consts=consts,
                packed=packed, S_c=S_c, S_f=S_f, B=B, raw_noise_std=raw_noise_std, perturb=perturb,
                nanmean_chunk=nanmean_chunk, rand=rand, stages=stages, lindisp=lindisp)
-    outs = _RenderBlock.apply(caster, cfg, vol, pose_skts, *params)
+    outs = _RenderBlock.apply(caster, cfg, vol, pose_skts, frame_codes, *params)
     return dict(zip(OUT_KEYS, outs))
 
 

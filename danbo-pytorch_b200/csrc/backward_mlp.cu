@@ -7,6 +7,7 @@
 //   gemm_wgrad      : dW[M x N] += A[rows x M]^T . B[rows x N], split over rows, fp32 atomics
 //   colsum          : bias gradients
 //   ray_bias_bwd    : grads of views_linears.0[:, 256:], its bias and the frame codes
+//   ray_bias_codes_bwd : grads of the frame codes only (code fitting with a frozen field)
 //   view_root_bwd   : d skts of the root rotation through root-local view directions (perfcap configs, --opt_pose)
 // All row counts are device scalars (the active counters), so nothing synchronises with the host.
 // Training batches hold ~4e4 active rows, so these are launch/latency bound; the tensor-core (tcgen05) versions are the
@@ -314,6 +315,48 @@ ray_bias_bwd_kernel(const float* __restrict__ rays, int ray_stride, int n_rays, 
         if (i < nc) atomicAdd(d_w_view + (size_t)o * 411 + 256 + c0 + i, acc[i]);
 }
 
+// Frame codes only (code fitting with a frozen field, training.PoseFitStep): d code[cam][c'] += sum_o W_v[o][283 + c']
+// d_ray_bias[ray][o], with no weight or bias gradient.  A block owns CB_RAYS consecutive rays and thread o (= c') walks
+// them in order, summing its column of d_ray_bias while the (clamped) camera stays the same; at the end of each run
+// the sums go to shared memory and thread c' forms one 128-long dot product with column 283 + c' of W_v (coalesced
+// across the warp) and issues one atomic.  Rays arrive image-major, so a block normally holds one or two runs; mixed
+// runs take one product per run and stay exact.  cam < 0 (the mean code) takes no gradient, cam > n_codes - 1 clamps
+// to the last row: the index rule of danbo_ray_bias / ray_bias_bwd_kernel.
+constexpr int CB_RAYS = 64;
+
+__global__ void __launch_bounds__(128)
+ray_bias_codes_bwd_kernel(const int* __restrict__ cam_idx, int n_rays, int n_codes,
+                          const float* __restrict__ w_view /* (128,411) */, const float* __restrict__ d_ray_bias,
+                          float* __restrict__ d_codes /* (n_codes,128) */) {
+    __shared__ int s_cam[CB_RAYS];
+    __shared__ float dsum[128];
+    const int t = threadIdx.x;
+    const int base = blockIdx.x * CB_RAYS;
+    const int nr = min(CB_RAYS, n_rays - base);
+    if (t < nr) {
+        const int c = cam_idx[base + t];
+        s_cam[t] = c < 0 ? -1 : (c > n_codes - 1 ? n_codes - 1 : c);
+    }
+    __syncthreads();
+    const float* col = w_view + 283 + t;
+    float s = 0.f;
+    for (int r = 0; r < nr; ++r) {
+        const int cam = s_cam[r];                                     // block-uniform: every branch below is too
+        if (cam >= 0) s += __ldg(d_ray_bias + (size_t)(base + r) * 128 + t);
+        if (r + 1 < nr && s_cam[r + 1] == cam) continue;
+        if (cam >= 0) {                                               // end of a run with a trainable code
+            dsum[t] = s;
+            __syncthreads();
+            float s4[4] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll 8
+            for (int o = 0; o < 128; ++o) s4[o & 3] = fmaf(__ldg(col + (size_t)o * 411), dsum[o], s4[o & 3]);
+            atomicAdd(d_codes + (size_t)cam * 128 + t, (s4[0] + s4[1]) + (s4[2] + s4[3]));
+            __syncthreads();                                          // dsum is rewritten by the next run
+        }
+        s = 0.f;
+    }
+}
+
 // V1 backward to the root rotation (perfcap configs: ray_tr_type=root_local + view_type=relray, pose refinement).  There
 // the view branch encodes dn = normalize(m), m = R0 d_ray, R0 = skts[pose, 0, :3, :3] (RootLocalEncoder
 // encoders.py:570-578, VecNormEncoder :774-795), and PE(dn) = [dn, sin(2^f dn), cos(2^f dn)]_{f<4} meets columns 256..282
@@ -500,6 +543,16 @@ extern "C" int danbo_ray_bias_bwd(const float* rays, int ray_stride, int n_rays,
     if (rb_blocks > 1184) rb_blocks = 1184;
     bwd::ray_bias_bwd_kernel<<<rb_blocks, 256, 0, (cudaStream_t)stream>>>(
         rays, ray_stride, n_rays, cam_idx, codes, n_codes, w_view, d_ray_bias, d_w_view, d_b_view, d_codes);
+    DANBO_CHECK_LAUNCH();
+    return 0;
+}
+
+extern "C" int danbo_ray_bias_codes_bwd(const int* cam_idx, int n_rays, int n_codes, const float* w_view,
+                                        const float* d_ray_bias, float* d_codes, void* stream) {
+    if (n_rays <= 0) return 0;
+    if (!cam_idx || !w_view || !d_ray_bias || !d_codes || n_codes <= 0) return -1;
+    bwd::ray_bias_codes_bwd_kernel<<<(n_rays + bwd::CB_RAYS - 1) / bwd::CB_RAYS, 128, 0, (cudaStream_t)stream>>>(
+        cam_idx, n_rays, n_codes, w_view, d_ray_bias, d_codes);
     DANBO_CHECK_LAUNCH();
     return 0;
 }

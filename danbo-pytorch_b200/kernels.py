@@ -700,6 +700,36 @@ def ray_bias_bwd(rays, cam_idx, codes_with_mean, w_view, d_ray_bias, d_w_view, d
     _count(1)
 
 
+def ray_bias_codes_bwd(cam_idx, w_view, d_ray_bias, d_codes):
+    """d_codes (n_codes,128) += d loss / d code of every fitted frame code (danbo_ray_bias_codes_bwd): the frame-code
+    part of the view layer's backward alone, with no weight or bias gradient.  cam_idx (n,) int32 with danbo_ray_bias's
+    index rule (< 0: the mean code, no gradient; > n_codes - 1: the last row), w_view the (128,411) view weight,
+    d_ray_bias (n,128) the gradient of danbo_ray_bias's output."""
+    tensors = dict(cam_idx=cam_idx, w_view=w_view, d_ray_bias=d_ray_bias, d_codes=d_codes)
+    _need_cuda(*tensors.values())
+    for name, t in tensors.items():
+        if t.dtype != (torch.int32 if name == "cam_idx" else torch.float32):
+            raise ValueError(f"ray_bias_codes_bwd: {name} has dtype {t.dtype}")
+        if t.device != d_codes.device:
+            raise ValueError(f"ray_bias_codes_bwd: {name} is on {t.device}, d_codes on {d_codes.device}")
+        if not t.is_contiguous():
+            raise ValueError(f"ray_bias_codes_bwd: {name} must be contiguous")
+    n = cam_idx.shape[0]
+    if cam_idx.dim() != 1:
+        raise ValueError("ray_bias_codes_bwd: cam_idx must be a (n,) tensor")
+    if tuple(w_view.shape) != (128, 411):
+        raise ValueError(f"ray_bias_codes_bwd: w_view must be (128,411), got {tuple(w_view.shape)}")
+    if tuple(d_ray_bias.shape) != (n, 128):
+        raise ValueError(f"ray_bias_codes_bwd: d_ray_bias must be ({n},128), got {tuple(d_ray_bias.shape)}")
+    if d_codes.dim() != 2 or d_codes.shape[1] != 128 or d_codes.shape[0] < 1:
+        raise ValueError(f"ray_bias_codes_bwd: d_codes must be (n_codes >= 1,128), got {tuple(d_codes.shape)}")
+    with _Timed("ray_bias_codes_bwd"):
+        _lib.check(_lib.load().danbo_ray_bias_codes_bwd(_p(cam_idx), n, d_codes.shape[0], _p(w_view), _p(d_ray_bias),
+                                                        _p(d_codes), _stream()), "danbo_ray_bias_codes_bwd")
+    _count(1)
+    return d_codes
+
+
 def view_root_bwd(rays, pose_skts, rays_per_pose, w_view, d_ray_bias, d_skts):
     """d skts (n_poses,24,4,4) += d loss / d skts through root-local view directions (perfcap configs under --opt_pose,
     danbo_view_root_bwd): rows 0-2, columns 0-2 of joint 0 only.  rays (n,>=6) with unit column stride, w_view the

@@ -37,6 +37,7 @@ class RayCaster(nn.Module):
     _supports_normals = True              # density gradients / normals (render_pts_gradient, want_normals): DANBO only
     _supports_parts = True                # body-part maps (render_pts_parts, want_parts): a field with an aggregation net
     _supports_scene = True                # scenes of several bodies (render_scene_rays): DANBO only
+    _supports_frame_codes = True          # a fitted code table in place of the network's (frame_codes=): DANBO only
 
     def __init__(self, network, network_fine=None, single_net=True, rest_poses=None, align_bones="align",
                  skel_type=None, use_volume_near_far=False, view_mode="world", **kwargs):
@@ -103,6 +104,9 @@ class RayCaster(nn.Module):
                                       "use the plain call")
         if ignored.get("ray_noise_std", 0.) > 0 or ignored.get("pytest"):
             raise NotImplementedError("ray_noise_std > 0 and pytest are not implemented")
+        if ignored.get("frame_codes") is not None:
+            raise NotImplementedError("frame_codes is not implemented for render_graphed (the code table is not "
+                                      "captured): use the plain call")
         B = float((preproc_kwargs or {}).get("density_scale", 1.0))
         rays, pose_skts, pose_bones, pose_cyls, cam_idx, skip = self._prepare(ray_batch, skts, cyls, bones, cams, N_uniques)
         if self._graphed is None:
@@ -207,11 +211,31 @@ class RayCaster(nn.Module):
             self._packed_t_gen = self._pack_gen
         return self._packed_t
 
-    def _codes_with_mean(self):
+    def _codes_with_mean(self, frame_codes=None):
+        """The code table the kernels read: the frame codes and, as its last row, the network's mean code (cams < 0).
+        frame_codes (rows,128): a fitted table that replaces the network's rows (training.PoseFitStep, `render_rays`);
+        the mean row stays the network's."""
         if not getattr(self.network, "opt_framecode", True):
             return torch.zeros(2, 128, device=self._device())
         w = self.network.framecodes.codes.weight.detach()
-        return torch.cat([w, w.mean(0, keepdim=True)], 0).contiguous()
+        rows = w if frame_codes is None else frame_codes.detach()
+        return torch.cat([rows, w.mean(0, keepdim=True)], 0).contiguous()
+
+    def check_frame_codes(self, frame_codes, what="frame_codes"):
+        """A fitted frame-code table a render may use in place of the network's: raise, before any device work, for a
+        field without frame codes, a table that is not (rows >= 1, 128) fp32, or one off the caster's device."""
+        if not self._supports_frame_codes:
+            raise NotImplementedError(f"{what}: a fitted frame-code table is implemented for the DANBO field only")
+        if not getattr(self.network, "opt_framecode", True) or not hasattr(self.network, "framecodes"):
+            raise NotImplementedError(f"{what}: the field has no frame codes (opt_framecode=False)")
+        if not torch.is_tensor(frame_codes) or frame_codes.dim() != 2 or frame_codes.shape[0] < 1 or \
+                frame_codes.shape[1] != 128:
+            raise ValueError(f"{what} must be a (rows >= 1, 128) tensor, got "
+                             f"{tuple(frame_codes.shape) if torch.is_tensor(frame_codes) else type(frame_codes)}")
+        if frame_codes.dtype != torch.float32:
+            raise ValueError(f"{what} must be fp32, got {frame_codes.dtype}")
+        if frame_codes.device != self._device():
+            raise ValueError(f"{what} is on {frame_codes.device}, the caster on {self._device()}")
 
     @staticmethod
     def _unique(t, skip):
@@ -241,14 +265,17 @@ class RayCaster(nn.Module):
                     raw_noise_std=0., ray_noise_std=0., verbose=False, ext_scale=0.001, pytest=False, N_uniques=1,
                     render_confd=False, render_entropy=False, preproc_kwargs=None, netchunk=1024 * 64,
                     nerf_type="danbo", use_viewdirs=True, nanmean_chunk=None, want_normals=False, want_parts=False,
-                    _rand=None, _stages=None):
+                    frame_codes=None, _rand=None, _stages=None):
         """Same arguments and returned dict as raycasters.py:245-377,516-546,710-716.
 
         Extra (optional) keywords: `nanmean_chunk` keeps the reference's per-chunk near/far fill (F8) when more than
         one reference chunk is passed in a single call; `want_normals` adds `normal_map` (n,3), the composite of the
         samples' unit normals (`_render_normals`; eval mode without gradients only); `want_parts` adds `part_map` (n,24),
         the composite of the samples' aggregation weights p_j (eval mode without gradients only; not together with
-        `want_normals`); `_rand`/`_stages` are test hooks (inject the four random tensors / collect stage tensors)."""
+        `want_normals`); `frame_codes` (rows,128) fp32 on the caster's device, e.g. codes fitted to unseen frames by
+        training.PoseFitStep, replaces the network's code table for cams >= 0 (cams above rows - 1 take the last row;
+        cams < 0 keep the network's mean code); `_rand`/`_stages` are test hooks (inject the four random tensors /
+        collect stage tensors)."""
         if want_normals:
             self._refuse_normals("render_rays(want_normals=True)")
             if self.training or torch.is_grad_enabled():
@@ -273,6 +300,8 @@ class RayCaster(nn.Module):
             raise ValueError("skts, bones and cyls are required")
         if cams is None and getattr(self.network, "opt_framecode", True):
             raise ValueError("cams are required (the field has per-frame codes)")
+        if frame_codes is not None:
+            self.check_frame_codes(frame_codes)
         pk = preproc_kwargs or {}
         if pk.get("density_fn", F.relu) is not F.relu:
             raise NotImplementedError("density_type other than 'relu' is not implemented")
@@ -280,11 +309,12 @@ class RayCaster(nn.Module):
         rays, pose_skts, pose_bones, pose_cyls, cam_idx, skip = self._prepare(ray_batch, skts, cyls, bones, cams, N_uniques)
         if want_normals:
             return self._render_normals(rays, pose_skts, pose_bones, pose_cyls, cam_idx, skip, N_samples, N_importance, B,
-                                        nanmean_chunk, bool(lindisp), _stages)
+                                        nanmean_chunk, bool(lindisp), _stages, frame_codes=frame_codes)
         return self._render_prepared(rays, pose_skts, pose_bones, pose_cyls, cam_idx, skip=skip, N_samples=N_samples,
                                      N_importance=N_importance, B=B, raw_noise_std=raw_noise_std, perturb=perturb,
                                      nanmean_chunk=nanmean_chunk, lindisp=bool(lindisp), _rand=_rand, _stages=_stages,
-                                     **({"want_parts": True} if want_parts else {}))
+                                     **({"want_parts": True} if want_parts else {}),
+                                     **({"frame_codes": frame_codes} if frame_codes is not None else {}))
 
     def _prepare(self, ray_batch, skts, cyls, bones, cams, N_uniques):
         """Host-side reduction of the reference's per-ray stride-0 expands to per-pose tables (encoders.py:465-471)."""
@@ -303,14 +333,14 @@ class RayCaster(nn.Module):
 
     def _render_prepared(self, rays, pose_skts, pose_bones, pose_cyls, cam_idx, skip=1, N_samples=64, N_importance=16,
                          B=1.0, raw_noise_std=0., perturb=0., nanmean_chunk=None, lindisp=False, _rand=None, _stages=None,
-                         want_parts=False):
+                         want_parts=False, frame_codes=None):
         dev = self._device()
         N = rays.shape[0]
         net = self.network
         consts = self._consts()
         packed = self._packed_mlp()
         vol = net.bone_volumes(pose_bones).float().contiguous()            # GN1 + GN2 (PyTorch, <= 16 poses; autograd)
-        codes = self._codes_with_mean()
+        codes = self._codes_with_mean(frame_codes)
         training = self.training
         rand = _rand or {}
         if training and perturb > 0 and "t_rand" not in rand:
@@ -325,7 +355,8 @@ class RayCaster(nn.Module):
                 raise NotImplementedError(f"training batches above {MAX_RAYS_PER_LAUNCH} rays are not implemented")
             return render_block_with_grad(self, rays, skip, pose_skts, pose_cyls, vol, cam_idx, codes, consts, packed,
                                           N_samples, N_importance, B, raw_noise_std, perturb, nanmean_chunk,
-                                          {k: v.to(dev).contiguous() for k, v in rand.items()}, _stages, lindisp=lindisp)
+                                          {k: v.to(dev).contiguous() for k, v in rand.items()}, _stages,
+                                          lindisp=lindisp, frame_codes=frame_codes)
         outs = []
         # internal launches: any split works for a single pose; with several poses a block holds whole poses
         G = pose_skts.shape[0]
@@ -538,7 +569,7 @@ class RayCaster(nn.Module):
         return (sigma.reshape(P, 1, 1) if pts.dim() == 3 else sigma.reshape(P, 1)), grad
 
     def _render_normals(self, rays, pose_skts, pose_bones, pose_cyls, cam_idx, skip, S_c, S_f, B, nanmean_chunk,
-                        lindisp, stages):
+                        lindisp, stages, frame_codes=None):
         """render_rays(want_normals=True): the eval render (no perturbation, no noise) with its intermediates kept, the
         seeded backward of render_pts_gradient on both passes, and normal_map = sum_m w_m n_m over the merged samples
         with the fine composite's weights (world frame, not renormalised).  The plain call's blocks (and their near /
@@ -549,7 +580,7 @@ class RayCaster(nn.Module):
         net = self.network
         consts, packed, packed_t = self._consts(), self._packed_mlp(), self._packed_dgrad()
         vol = net.bone_volumes(pose_bones).float().contiguous()
-        codes = self._codes_with_mean()
+        codes = self._codes_with_mean(frame_codes)
         G = pose_skts.shape[0]
         block, _ = self._plan_blocks(N, G, skip, nanmean_chunk, 1)
         seg = 0 if not nanmean_chunk else int(nanmean_chunk)
@@ -675,6 +706,9 @@ def check_scene(instances, N_samples, N_importance):
         if caster.training or torch.is_grad_enabled():
             raise NotImplementedError("scenes are rendered in eval mode without gradients (caster.eval(), "
                                       "torch.no_grad()): gradients through a scene are not implemented")
+        if inst.get("frame_codes") is not None:
+            raise NotImplementedError(f"scene instance {k}: frame_codes (a fitted code table) is not implemented for "
+                                      "scenes")
         if any(inst[name].shape[0] != 1 for name in ("kps", "skts", "bones", "cyls")):
             raise NotImplementedError(f"scene instance {k}: one pose per instance (kps, skts, bones, cyls with a leading "
                                       "1): add one instance per pose")

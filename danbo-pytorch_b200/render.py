@@ -82,7 +82,7 @@ def projection_matrix(c2w, H, W, focal):
 
 @torch.no_grad()
 def render_images(caster, args, c2ws, poses, H, W, focal=None, cam_idx=0, white_bkgd=True, near=syn.NEAR, far=syn.FAR,
-                  graphed=False, distributed=False, normals=False, parts=False):
+                  graphed=False, distributed=False, normals=False, parts=False, frame_codes=None):
     """Render one image per (camera, pose) pair.  poses: list of dicts from synthetic.make_pose (kps, skts, bones, cyl);
     image k uses c2ws[k] and poses[k % len(poses)], like render_path.  With distributed=True images are dealt round
     robin to the ranks and the finished images all-gathered: every rank returns all images (n, H, W, 3) float32.
@@ -90,7 +90,17 @@ def render_images(caster, args, c2ws, poses, H, W, focal=None, cam_idx=0, white_
     normal maps (`render_rays(want_normals=True)`), 0 on the background.
     parts=True (single process, not graphed, not with normals): -> (images, part_maps), the second (n, H, W, 24) float32
     body-part maps (`render_rays(want_parts=True)`: the composited aggregation weight of every bone), 0 on the
-    background; `part_labels` turns them into a segmentation."""
+    background; `part_labels` turns them into a segmentation.
+    frame_codes (single process, not graphed): a (rows,128) fp32 code table on the caster's device, e.g. the codes
+    training.PoseFitStep fitted to unseen frames, that replaces the network's rows; cam_idx then indexes it (< 0: the
+    network's mean code)."""
+    if frame_codes is not None:
+        if graphed:
+            raise NotImplementedError("render_images(frame_codes=...) with graphed=True: the code table is not "
+                                      "captured")
+        if distributed:
+            raise NotImplementedError("render_images(frame_codes=...) with distributed=True is not implemented")
+        caster.check_frame_codes(frame_codes, "render_images(frame_codes=...)")
     if parts:
         if graphed:
             raise NotImplementedError("render_images(parts=True) with graphed=True: part maps are not captured")
@@ -139,7 +149,8 @@ def render_images(caster, args, c2ws, poses, H, W, focal=None, cam_idx=0, white_
                    bones=tab["bones"][ps:ps + 1].expand(n, -1, -1),
                    cams=torch.full((n, 1), cam_idx, dtype=torch.long, device=dev), N_uniques=1, perturb=False,
                    N_importance=args.N_importance, raw_noise_std=0., nanmean_chunk=args.chunk,
-                   **({"want_normals": True} if normals else {}), **({"want_parts": True} if parts else {}))
+                   **({"want_normals": True} if normals else {}), **({"want_parts": True} if parts else {}),
+                   **({"frame_codes": frame_codes} if frame_codes is not None else {}))
         bg = 1.0 if white_bkgd else 0.0
         out[slot, idx] = ret["rgb_map"] + (1. - ret["acc_map"])[:, None] * bg         # run_nerf.py:103-133
         if normals:

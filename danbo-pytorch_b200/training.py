@@ -116,9 +116,9 @@ def adam_state_from_dict(sd, params, exp_avg, exp_avg_sq):
     return step, float(sd["param_groups"][0]["lr"])
 
 
-def save_checkpoint(path, global_step, caster, optimizer, popt_kwargs=None, pose_optimizer=None):
+def save_checkpoint(path, global_step, caster, optimizer, popt_kwargs=None, pose_optimizer=None, extra=None):
     """Trainer.save_nerf (core/trainer.py:597-618): the same keys, so `create_raycaster` here or in the reference resumes
-    from the file."""
+    from the file.  `extra`: further top-level keys (PoseFitStep's fitted frame codes)."""
     popt_sd = poptim_sd = anchors = None
     if popt_kwargs is not None and popt_kwargs.get("popt_layer") is not None:
         popt_sd = popt_kwargs["popt_layer"].state_dict()
@@ -127,7 +127,7 @@ def save_checkpoint(path, global_step, caster, optimizer, popt_kwargs=None, pose
     torch.save({"global_step": global_step,
                 "optimizer_state_dict": optimizer.state_dict() if optimizer is not None else None,
                 "poseopt_layer_state_dict": popt_sd, "pose_optimizer_state_dict": poptim_sd, "poseopt_anchors": anchors,
-                **caster.state_dict()}, path)
+                **caster.state_dict(), **(extra or {})}, path)
 
 
 class FlatAdam(torch.optim.Optimizer):
@@ -502,6 +502,45 @@ class TrainStep:
         return loss.detach(), preds
 
 
+def create_code_fit(caster, n_frames, lr=5e-4, device=None):
+    """A table of frame codes to fit to frames the field was not trained on, with training.PoseFitStep(code_kwargs=...,
+    code_optimizer=...).  -> (code_optimizer, {"frame_codes": codes}): `codes` is an (n_frames,128) nn.Parameter whose
+    rows all start at the network's mean code (so a first step renders like cams < 0), separate from the network's
+    `framecodes.codes.weight`; `code_optimizer` is a FlatAdam over it (CUDA only).  A field without frame codes is
+    refused (NotImplementedError) before anything is allocated."""
+    caster.check_frame_codes(torch.zeros(1, 128, device=caster._device()), "code fitting")
+    if int(n_frames) < 1:
+        raise ValueError(f"code fitting needs n_frames >= 1, got {n_frames}")
+    with torch.no_grad():
+        # the reduction _codes_with_mean uses for the mean row, on the same device: the same bits
+        mean = caster.network.framecodes.codes.weight.detach().mean(0, keepdim=True)
+        codes = torch.nn.Parameter(mean.expand(int(n_frames), 128).to(device or mean.device).clone())
+    optimizer = FlatAdam([codes], parallel.GradBucket([codes]), lr=lr, betas=(0.9, 0.999))
+    return optimizer, {"frame_codes": codes}
+
+
+def _check_code_fit(caster, code_kwargs, code_optimizer):
+    """The refusals of PoseFitStep's code fitting, raised before any device work.  -> the fitted table or None."""
+    if code_kwargs is None and code_optimizer is None:
+        return None
+    if code_kwargs is None or code_optimizer is None or code_kwargs.get("frame_codes") is None:
+        raise ValueError("code fitting needs both code_kwargs ({'frame_codes': table}) and code_optimizer, as "
+                         "training.create_code_fit returns them")
+    codes = code_kwargs["frame_codes"]
+    caster.check_frame_codes(codes, "code fitting (PoseFitStep)")
+    if not isinstance(code_optimizer, FlatAdam):
+        raise NotImplementedError("code fitting (PoseFitStep) is not implemented for a code optimizer that is not a "
+                                  "training.FlatAdam (training.create_code_fit): a captured backward writes into fixed "
+                                  "gradient storage")
+    if not (codes.is_leaf and codes.requires_grad) or [id(p) for p in code_optimizer.bucket.params] != [id(codes)]:
+        raise ValueError("code fitting (PoseFitStep): the frame-code table must be a leaf that requires a gradient and "
+                         "the code optimizer's only parameter")
+    if codes is caster.network.framecodes.codes.weight:
+        raise ValueError("code fitting (PoseFitStep) fits a table of its own, not the network's "
+                         "framecodes.codes.weight (training.create_code_fit)")
+    return codes
+
+
 class PoseFitStep:
     """Fits the SMPL poses of frames to their images with the field frozen: forward -> losses -> pose-only backward ->
     pose backward -> the pose optimizer's Adam.  Call shape of TrainStep: `loss, preds = step(batch)`,
@@ -525,14 +564,26 @@ class PoseFitStep:
     before each replay, outside the graph, so a `caster.load_state_dict` between steps is seen.  graph=False runs the
     same kernels eagerly.  Refused (NotImplementedError, before any device work): the A-NeRF field, a separate fine
     network, world_size > 1, opt_rot6d, use_temp_loss, opt_pose_cache, a pose optimizer that is not a FlatAdam, and a
-    batch whose N_uniques does not divide it."""
+    batch whose N_uniques does not divide it.
 
-    def __init__(self, caster, args, popt_kwargs, pose_optimizer, graph=False, world_size=1):
+    Frame codes of the fitted frames: with `code_kwargs` / `code_optimizer` from `create_code_fit`, the batch's cams
+    index the rows of that table (a table of its own: the network's framecodes.codes.weight is not touched), and cams
+    < 0 still mean the network's mean code.  Each step renders with [fitted rows; network mean] as the code table,
+    backpropagates to the rows (danbo_ray_bias_codes_bwd after the pose-only MLP chain) and steps the code optimizer
+    after the pose optimizer; graph=True captures that too and restores the code arenas after capture.  `save` then
+    adds one key, `framecode_fit` = {codes, optimizer_state_dict}, which `resume` reads.  Refused before any device
+    work: a field without frame codes (NotImplementedError), a table that is not (rows,128) fp32 on the caster's device
+    (ValueError), a code optimizer that is not a FlatAdam (NotImplementedError)."""
+
+    def __init__(self, caster, args, popt_kwargs, pose_optimizer, graph=False, world_size=1, code_kwargs=None,
+                 code_optimizer=None):
         if not popt_kwargs or popt_kwargs.get("popt_layer") is None:
             raise ValueError("PoseFitStep needs the pose layer of pose_opt.create_popt (popt_kwargs['popt_layer'])")
         layer = popt_kwargs["popt_layer"]
+        self._codes = _check_code_fit(caster, code_kwargs, code_optimizer)
         _refuse_pose_graph(args, caster, world_size, pose_optimizer, layer, what="pose fitting (PoseFitStep)")
         self.caster, self.args, self.popt, self.pose_optimizer = caster, args, popt_kwargs, pose_optimizer
+        self.code_optimizer = code_optimizer if self._codes is not None else None
         self.last_stats = {}
         dev = next(caster.network.parameters()).device
         layer.to(dev)
@@ -550,8 +601,9 @@ class PoseFitStep:
             def run(_param_ptrs=None, **b):
                 loss, preds = self._step(b)
                 return dict(self.last_stats, loss=loss, rgb_map=preds["rgb_map"], acc_map=preds["acc_map"])
-            po = pose_optimizer
-            self._graphed = GraphedFn(run, dev, warmup=3, state=[po.flat, po.exp_avg, po.exp_avg_sq, po.step_dev])
+            state = [o for opt in (pose_optimizer, self.code_optimizer) if opt is not None
+                     for o in (opt.flat, opt.exp_avg, opt.exp_avg_sq, opt.step_dev)]
+            self._graphed = GraphedFn(run, dev, warmup=3, state=state)
 
     def _frozen(self):
         """Context: the network's parameters with requires_grad off (restored on exit)."""
@@ -598,6 +650,8 @@ class PoseFitStep:
         G, skip = pose_batch_poses(batch)
         n = G * skip
         self.pose_optimizer.zero_grad()
+        if self._codes is not None:
+            self.code_optimizer.zero_grad()
         kps, bones, skts, reg, mpjpc = pose_layer(
             self.popt["popt_layer"], batch["kp_idx"].long(), skip, G, self._pose_anchors, rest_idx=self._rest_idx,
             tol=getattr(a, "opt_pose_tol", 0.), coef=getattr(a, "opt_pose_coef", 0.),
@@ -615,7 +669,8 @@ class PoseFitStep:
                 preds = caster(batch["ray_batch"], N_samples=a.N_samples, kp_batch=batch["kp_batch"],
                                skts=batch["skts"], cyls=batch["cyls"], bones=batch["bones"], cams=batch["cams"],
                                N_uniques=batch["N_uniques"], perturb=a.perturb, N_importance=a.N_importance,
-                               raw_noise_std=a.raw_noise_std)
+                               raw_noise_std=a.raw_noise_std,
+                               **({"frame_codes": self._codes} if self._codes is not None else {}))
                 if fused_loss_supported(a, preds):
                     # axis_scale needs no gradient here, so the fused loss forms no volume-scale term
                     loss, _ = fused_loss_backward(a, preds, batch, net, extra_loss=reg)
@@ -628,12 +683,19 @@ class PoseFitStep:
         finally:
             net.pose_kernels = False
         self.pose_optimizer.step()
+        if self._codes is not None:
+            self.code_optimizer.step()
         return loss, preds
 
     def save(self, path, global_step):
         """Checkpoint in the reference's format with the (unchanged) network, the pose layer and the pose optimizer;
-        there is no network optimizer state (optimizer_state_dict is None)."""
-        save_checkpoint(path, global_step, self.caster, None, self.popt, self.pose_optimizer)
+        there is no network optimizer state (optimizer_state_dict is None).  With code fitting, one more key:
+        framecode_fit = {codes (rows,128) on the CPU, optimizer_state_dict}."""
+        extra = None
+        if self._codes is not None:
+            extra = {"framecode_fit": {"codes": self._codes.detach().cpu().clone(),
+                                       "optimizer_state_dict": self.code_optimizer.state_dict()}}
+        save_checkpoint(path, global_step, self.caster, None, self.popt, self.pose_optimizer, extra=extra)
 
     def resume(self, ckpt):
         """The pose layer and pose optimizer state of a loaded checkpoint dict (nothing of the network).
@@ -642,4 +704,12 @@ class PoseFitStep:
             self.popt["popt_layer"].load_state_dict(ckpt["poseopt_layer_state_dict"])
             if ckpt.get("pose_optimizer_state_dict") is not None:
                 self.pose_optimizer.load_state_dict(ckpt["pose_optimizer_state_dict"])
+        fit = ckpt.get("framecode_fit")
+        if self._codes is not None and fit is not None:
+            if tuple(fit["codes"].shape) != tuple(self._codes.shape):
+                raise ValueError(f"the checkpoint's fitted frame codes are {tuple(fit['codes'].shape)}, this step fits "
+                                 f"{tuple(self._codes.shape)}")
+            with torch.no_grad():
+                self._codes.copy_(fit["codes"])
+            self.code_optimizer.load_state_dict(fit["optimizer_state_dict"])
         return int(ckpt.get("global_step", 0))

@@ -237,6 +237,14 @@ int danbo_ray_bias_bwd(const float* rays, int ray_stride, int n_rays, const int*
                        const float* w_view, const float* d_ray_bias, float* d_w_view, float* d_b_view, float* d_codes,
                        void* stream);
 
+/* V1 backward to the frame codes only (code fitting with a frozen field): d_codes[c] += sum over the rays n with
+ * clamped cam_idx[n] == c of W_v[:, 283:411]^T d_ray_bias[n].  cam_idx (n_rays) int32 with danbo_ray_bias's index rule:
+ * cam < 0 is the mean code and takes no gradient, cam > n_codes - 1 clamps to row n_codes - 1.  w_view (128,411),
+ * d_ray_bias (n_rays,128) and d_codes (n_codes,128) fp32 row-major; d_codes is added to with atomics (zero it first).
+ * No weight or bias gradient is formed. */
+int danbo_ray_bias_codes_bwd(const int* cam_idx, int n_rays, int n_codes, const float* w_view, const float* d_ray_bias,
+                             float* d_codes, void* stream);
+
 /* V1 backward to the root rotation under root-local view directions (perfcap configs: ray_tr_type=root_local,
  * view_type=relray; pose refinement, --opt_pose): autograd of RootLocalEncoder (core/encoders.py:570-578) and
  * VecNormEncoder (:774-795), i.e. of dn = normalize(skts[pose, 0, :3, :3] . rays_d) and its 4-octave encoding, which
